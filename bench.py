@@ -2,7 +2,7 @@
 """bench.py — fwd+bwd samples/s of the review-encoder hot path on N B200s (one process per GPU).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--model all|deepconn|narre|dual_att] [--mode train|infer]
-                    [--impl ours|reference]
+                    [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = optimizer.zero_grad() + forward + nn.MSELoss + backward (+ the gradient all-reduce when N > 1), i.e.
 trainer/train_deepconn_pp.py:161-165 of the reference.  BASELINE.json's metric names DeepCoNN AND NARRE, so the default run
@@ -17,6 +17,11 @@ driven from pinned HOST buffers through the public API (H2D of every input and a
 region); roofline = the dominant kernel (tcgen05 conv) against the measured bf16 peak; cpu_baseline = the reference's own
 modules (oracle/_ref, unmodified) timed on this box's host cores; library_gpu_baseline = the reference's formulation on
 ATen/cuBLAS kernels on the same GPU.  `--impl reference` times the CPU path alone, as the reference arm.
+
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<workload>.<name>.npy (float32): the loss
+and every parameter gradient of a training step, the predictions of an inference step, the scores of `--pairs`.  Inputs,
+parameters and dropout masks depend on the arguments only, so two builds run with the same arguments can be compared
+array by array.
 """
 import argparse
 import json
@@ -30,7 +35,10 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
+
+DUMP_BYTES = 64 * 10 ** 6          # --dump-outputs writes at most this much in all
 
 CFG = {
     "deepconn": dict(B=4096, L=500, V=50000, E=300, H=100, K=32, U=20000, I=12000, ks=(3,)),
@@ -256,10 +264,12 @@ def make_batches(model_name, n, rank, b=None):
     return [synth_batch(model_name, b or CFG[model_name]["B"], synth.SEED_BASE + rank * 1000 + i) for i in range(n)]
 
 
-def eager_step(model, batch, ratings, loss_fn, post=None):
+def eager_step(model, batch, ratings, loss_fn, post=None, keep=None):
     if not model.training:                # inference scoring (configs[4]): eval forward under no_grad, no collective
         with torch.no_grad():
             pred = model(*batch)
+        if keep is not None:
+            keep["pred"] = pred
         return pred.sum()
     model.zero_grad(set_to_none=True)
     model.invalidate_operand_cache()      # as after an optimizer step: re-stage the bf16 table shadow + packed weights
@@ -295,9 +305,10 @@ def time_graph_loop(ctx, steps_objs, K):
 
 
 def measure(ctx, name, args):
-    """All measurements of one workload → dict (rank 0) / None."""
+    """All measurements of one workload → (dict, {name: output of the last timed step} with --dump-outputs) on rank 0,
+    (None, None) elsewhere."""
     import torch.distributed as dist
-    from rbr_b200 import ops, parallel
+    from rbr_b200 import ops, parallel, synth
     from rbr_b200._lib import lib
     from rbr_b200.graphs import GraphedTrainStep
     rank, world, dev, peaks, sampler = ctx.rank, ctx.world, ctx.dev, ctx.peaks, ctx.sampler
@@ -372,6 +383,7 @@ def measure(ctx, name, args):
 
     # ------------------------------ device-resident timing (value): CUDA-graph replays of the whole step ------------------------------
     graphs, graph_note, per_step, pool = None, "eager nn.Module calls", None, None
+    graph_grads = []                      # --dump-outputs: the .grad tensors each captured graph writes
     if args.graphs == "auto" and train:
         try:
             graphs = []
@@ -381,6 +393,8 @@ def measure(ctx, name, args):
                 per_step = (lib.rbr_launch_count() - c0) // 2          # one warm-up + one captured execution
                 pool = gs.pool
                 graphs.append(gs)
+                if args.dump_outputs:
+                    graph_grads.append({n: p.grad for n, p in model.named_parameters()})
             for gs in graphs:
                 gs.replay()
             torch.cuda.synchronize()
@@ -392,15 +406,29 @@ def measure(ctx, name, args):
             graphs, graph_note = None, f"eager (graph capture failed: {type(e).__name__}: {str(e)[:100]})"
             torch.cuda.synchronize()
     l0 = lib.rbr_launch_count()
+    keep = {}
     if graphs is not None:
         objs = [g.replay for g in graphs]
     else:
-        objs = [(lambda j=j: eager_step(model, *dev_batches[j], loss_fn, post)) for j in range(NB)]
+        objs = [(lambda j=j: eager_step(model, *dev_batches[j], loss_fn, post, keep)) for j in range(NB)]
+    # the warm-up above ran a timing-dependent number of steps: reseed so that the dropout masks of the timed steps (and what
+    # --dump-outputs writes) depend on the arguments only
+    torch.manual_seed(synth.SEED_BASE + rank)
     total_ms, loss = time_graph_loop(ctx, objs, K)
     value_clocks = sampler.take()
     launches = (per_step * K) if graphs is not None else (lib.rbr_launch_count() - l0)
     value = world * c["B"] * K / (total_ms * 1e-3)
     final_loss = float(loss.item())
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        outputs = {"loss": loss}
+        if train:
+            grads = graph_grads[(K - 1) % NB] if graphs is not None else {n: p.grad for n, p in model.named_parameters()}
+            outputs.update({"grad." + n: g for n, g in grads.items() if g is not None})
+        else:
+            outputs["pred"] = keep["pred"]
+        outputs = {f"{name}.{k}": v.detach().float().cpu() for k, v in outputs.items()}
+    graph_grads = keep = None
 
     # exposed collective time per step (N > 1): the same graphed step WITHOUT the gradient exchange
     exposed = None
@@ -761,7 +789,7 @@ def measure(ctx, name, args):
             out["full_trainer_step"] = full_step
     del model, dev_batches, pinned
     torch.cuda.empty_cache()
-    return out
+    return out, outputs
 
 
 def measure_infer_pairs(ctx, args):
@@ -819,6 +847,7 @@ def measure_infer_pairs(ctx, args):
     clocks = ctx.sampler.take()
     launches = lib.rbr_launch_count() - l0
     score_ms = sum(a.elapsed_time(b) for a, b in ev_score)
+    outputs = {f"{name}.scores": scores.cpu()} if args.dump_outputs and rank == 0 else None   # rank 0's slice
     t = torch.tensor([wall, score_ms], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -849,7 +878,7 @@ def measure_infer_pairs(ctx, args):
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     if rank != 0:
-        return None
+        return None, None
     return {
         "metric": METRIC[name], "value": args.pairs / (score_ms * 1e-3), "unit": "pairs/s", "n_gpus": world,
         "steps": len(ev_score), "warmup": args.warmup, "ms_per_step": score_ms / max(len(ev_score), 1), "higher_is_better": True,
@@ -867,7 +896,23 @@ def measure_infer_pairs(ctx, args):
                                   "(bit-identical scores, tests/test_gpu_benchcfg.py)"},
         "gpu_launches": int(launches), "gpu_launches_per_step": launches / max(len(ev_score), 1),
         "clocks": ctx.sampler.summarise(*clocks),
-    }
+    }, outputs
+
+
+def dump_outputs(outputs, out_dir):
+    """Write each CPU tensor of `outputs` as out_dir/<name>.npy in float32, DUMP_BYTES in all.  Smaller arrays are written
+    whole; an array over its share of what is left is cut to that many of its elements, flattened, at indices drawn by a
+    fixed seed (the same for the same arguments, so two builds write the same sample)."""
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(outputs.items(), key=lambda kv: (kv[1].numel(), kv[0]))
+    left = (DUMP_BYTES - 256 * len(items)) // 4          # float32 elements, after a 256-byte allowance per .npy header
+    for j, (name, t) in enumerate(items):
+        share = left // (len(items) - j)
+        if t.numel() > share:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:share].sort().values
+            t = t.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), t.to(torch.float32).numpy())
+        left -= t.numel()
 
 
 def main():
@@ -899,8 +944,15 @@ def main():
     ap.add_argument("--pairs", type=int, default=0,
                     help="--mode infer: score this many synthetic (user, item) pairs in total (BASELINE.json configs[4]: 10000000), "
                          "sharded over the ranks with no collective, ids generated on the device chunk by chunk")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<workload>.<name>.npy (float32, at most "
+                         "64 MB in all: larger arrays are cut to a fixed, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of --impl ours")
         return run_reference_arm(args)
 
     import torch.distributed as dist
@@ -927,9 +979,11 @@ def main():
     ctx.sync_all = sync_all
 
     if args.mode == "infer" and args.pairs > 0:
-        line = measure_infer_pairs(ctx, args)
+        line, outputs = measure_infer_pairs(ctx, args)
         ctx.sampler.stop()
         if ctx.rank == 0:
+            if args.dump_outputs:
+                dump_outputs(outputs, args.dump_outputs)
             print(json.dumps(line), flush=True)
         if ctx.world > 1:
             dist.barrier()
@@ -941,16 +995,19 @@ def main():
         models = ["deepconn", "narre"]
     else:
         models = [args.model]
-    line = None
+    line, outputs = None, {}
     for mi, m in enumerate(models):
-        d = measure(ctx, m, args)
+        d, o = measure(ctx, m, args)
         if ctx.rank == 0:
             if mi == 0:
                 line = d
             else:
                 line[m] = d
+            outputs.update(o or {})
     ctx.sampler.stop()
     if ctx.rank == 0:
+        if args.dump_outputs:
+            dump_outputs(outputs, args.dump_outputs)
         print(json.dumps(line), flush=True)
     if ctx.world > 1:
         dist.barrier()

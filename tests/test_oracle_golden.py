@@ -90,6 +90,21 @@ def test_vendored_reference_is_byte_identical_and_agrees_with_the_oracle():
         assert rel_err(p.grad, rg[k]) < 1e-5, k
 
 
+@pytest.mark.parametrize("kind", ["deepconn", "narre", "dual_att"])
+def test_restated_trainer_loop_reproduces_reference_trainer_goldens(kind):
+    """trainer_harness.run_loop (the loop body of the reference's train_one_epoch restated: zero_grad → forward → MSELoss →
+    backward → clip_grad_norm_(5.0) → Adam(lr 0.002).step) driving the oracle gives the losses and final parameters the
+    unmodified trainer wrote to tests/golden/trainer_*_3steps.npz, so the GPU test may use it where oracle/_ref is absent."""
+    import trainer_harness as th
+    params = {k: v.clone().requires_grad_(True) for k, v in th.initial_params(kind).items()}
+    for k in orc._PADDED_TABLES:               # nn.Embedding(padding_idx=0): row 0 gets no gradient
+        if k in params:
+            params[k].register_hook(lambda g: g.index_fill(0, torch.zeros(1, dtype=torch.long), 0.0))
+    forward = {"deepconn": orc.deepconn_forward, "narre": orc.narre_forward, "dual_att": orc.dual_att_forward}[kind]
+    losses, final = th.run_loop(kind, params, lambda *batch: forward(params, *batch))
+    th.assert_matches_golden(kind, losses, final, tol=1e-5)
+
+
 @pytest.mark.parametrize("case", ["deepconn_hier", "deepconn_hier_noproj"])
 def test_oracle_hier_pooling_matches_reference_golden(case):
     """arch="HierPooling" (models/deepconn/layers.py:62-98, 110-114): the oracle's avg-pool → max-pool → [Linear] → ReLU

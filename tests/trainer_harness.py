@@ -7,6 +7,9 @@ Nothing of the trainer is edited or re-implemented: the Experiment class is cons
 the reference's default_*.json with the sizes shrunk, dropout 0, logging off), parameters are loaded from a seeded set,
 `loss_func` is wrapped by a recorder, and `train_one_epoch(0)` runs zero_grad → forward → MSELoss → backward →
 clip_grad_norm_ → Adam.step over the stub loader's batches.
+
+The trainer needs the reference's sources (oracle/_ref).  Without them, `run_loop` runs the same loop body restated here;
+tests/test_oracle_golden.py pins that restatement, driving the CPU oracle, to the goldens the unmodified trainer wrote.
 """
 from __future__ import annotations
 
@@ -37,6 +40,8 @@ SHAPES = {
     "dual_att": dict(B=4, L=30, V=120, E=20, lw=5, lo=24, go=12, h1=30, h2=7),
 }
 N_STEPS = 3
+LR, MAX_GRAD_NORM = 0.002, 5.0          # lr and max_grad_norm of the reference's default_*.json
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 class _StubDataset:
@@ -140,3 +145,69 @@ def run_trainer_epoch(kind: str, model_module=None):
             sys.modules[model_mod_name] = saved
         else:
             sys.modules.pop(model_mod_name, None)
+
+
+def build_model(kind: str):
+    """This package's drop-in model at SHAPES[kind] (dropout 0), constructed with the arguments the trainer's build_model passes,
+    initial_params(kind) loaded."""
+    import rbr_b200
+    c = SHAPES[kind]
+    if kind == "deepconn":
+        model = rbr_b200.DeepCoNNpp(c["U"], c["I"], c["V"], list(c["ks"]), c["E"], c["H"], c["K"], c["L"], None, 0.0)
+    elif kind == "narre":
+        model = rbr_b200.NARRE(c["U"], c["I"], c["V"], list(c["ks"]), c["H"], c["E"], c["A"], c["K"], c["R"], c["T"], 0.0,
+                               0, 0, 0, None, "CNN")
+    else:
+        model = rbr_b200.DualAtt(c["V"], c["L"], c["lw"], c["lo"], c["go"], c["E"], c["h1"], c["h2"], 0.0, None)
+    model.load_state_dict(initial_params(kind))
+    return model
+
+
+def run_loop(kind: str, params: dict, forward):
+    """The body of `train_one_epoch` restated over batches(kind): optimizer.zero_grad() → forward → nn.MSELoss → backward →
+    clip_grad_norm_(5.0) → Adam(lr 0.002).step → loss.item(), with Adam and the clip over `params` in the order given.
+    params: {state_dict name: leaf tensor}; forward(*batch) returns pred, or a tuple led by pred, on the params' device.
+    Returns (losses per step, final params on the CPU)."""
+    dev = next(iter(params.values())).device
+    opt = torch.optim.Adam(list(params.values()), lr=LR)
+    loss_fn = torch.nn.MSELoss()
+    losses = []
+    for *batch, ratings in batches(kind):
+        opt.zero_grad()
+        out = forward(*[t.to(dev) for t in batch])
+        pred = out[0] if isinstance(out, tuple) else out
+        loss = loss_fn(pred, ratings.to(dev))
+        loss.backward()
+        torch.nn.utils.clip_grad_norm_(list(params.values()), MAX_GRAD_NORM)
+        opt.step()
+        losses.append(loss.item())
+    return losses, {k: v.detach().cpu().clone() for k, v in params.items()}
+
+
+def assert_matches_golden(kind: str, losses, final, tol: float, check_params: bool = True) -> None:
+    """Per-step losses within `tol` (relative) of tests/golden/trainer_<kind>_3steps.npz and, with check_params, the final
+    parameters: Adam's first updates are lr·sign(g), so an entry whose gradient is rounding noise can differ by a fraction of
+    one lr step between any two summation orders — bounded as a fraction of outliers (|diff| > 1e-5 on at most 0.2 % of the
+    entries) and the worst entry (< half an lr step); rows no batch touched must not have moved at all."""
+    import numpy as np
+    z = np.load(os.path.join(GOLDEN, f"trainer_{kind}_{N_STEPS}steps.npz"))
+    ref_losses = z["losses"]
+    assert len(losses) == N_STEPS
+    for a, b in zip(losses, ref_losses):
+        assert abs(a - b) <= tol * abs(b), (losses, ref_losses.tolist())
+    if not check_params:
+        return
+    init = initial_params(kind)
+    n_bad = n_all = 0
+    worst = 0.0
+    for k, v in final.items():
+        ref = torch.from_numpy(z["final/" + k])
+        d = (v - ref).abs()
+        n_bad += int((d > 1e-5).sum())
+        n_all += d.numel()
+        worst = max(worst, float(d.max()))
+        # rows no batch touched did not move at all (dense gradients with exact zeros, Adam leaves them in place)
+        untouched = (ref == init[k])
+        assert torch.equal(v[untouched], init[k][untouched]), k
+    assert n_bad <= 2e-3 * n_all, (n_bad, n_all)
+    assert worst < 1e-3, worst
