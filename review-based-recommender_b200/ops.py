@@ -618,6 +618,9 @@ class NarreAttnFn(torch.autograd.Function):
                                          _p(scores), _stream()), "rbr_narre_attn_fwd")
         ctx.save_for_backward(feat, other_id, scores, *args)
         ctx.padding_idx, ctx.arena, ctx.params = padding_idx, arena, params
+        # an output the loss does not use (usually the scores) reaches backward as None rather than a zero-filled tensor:
+        # the kernels then skip the score-gradient term
+        ctx.set_materialize_grads(False)
         return out, scores.view(B, R, 1)
 
     @staticmethod

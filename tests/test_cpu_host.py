@@ -315,3 +315,18 @@ def test_staged_inputs_wire_format_on_cpu():
     # masks that are NOT ids != 0 can still be sent
     st = StagedInputs(batch, ratings, "cpu", vocab=600, derive_masks=False)
     assert st.batch[2] is not None and st.batch[2].dtype == torch.uint8
+
+
+def test_narre_attn_pair_plan_boundary():
+    """Which NARRE attention shapes the two-sided tensor-core kernel takes (host code, no GPU).  NARRE falls back to the per-side
+    kernels outside this set, and test_attention_pair_tensor_core_kernels_vs_oracle runs the edge shapes pinned here."""
+    from rbr_b200._lib import lib
+    sup = lambda R, H, A: bool(lib.rbr_narre_attn_pair_supported(R, H, A))
+    assert sup(10, 150, 32)                                   # the benchmarked NARRE shape
+    for R, h_max in ((1, 128), (10, 160), (64, 192)):        # largest hidden per review count, whatever att_dim <= 32
+        for A in (1, 16, 32):
+            assert sup(R, h_max, A) and not sup(R, h_max + 1, A), (R, A)
+    assert sup(10, 101, 16) and sup(10, 1, 1)
+    assert not sup(65, 64, 32) and not sup(0, 64, 32)        # reviews in [1, 64]
+    assert not sup(10, 150, 33) and not sup(10, 150, 0)      # att_dim in [1, 32]
+    assert not sup(10, 0, 32)

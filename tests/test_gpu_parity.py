@@ -234,7 +234,10 @@ def test_two_pass_backward_with_table_hook_matches_single_pass():
 
 
 @pytest.mark.parametrize("shape", [(33, 10, 150, 32), (7, 4, 8, 5), (5, 5, 15, 6), (100, 6, 100, 16), (3, 2, 40, 8), (70, 17, 64, 32),
-                                   (4096, 10, 150, 32)])
+                                   (4096, 10, 150, 32),
+                                   # plan edges: one review; 64 reviews (one sample per tile); att_dim 1; the largest hidden
+                                   # accepted at 10 and at 64 reviews (pinned in test_cpu_host); hidden not a multiple of 8
+                                   (50, 1, 128, 32), (40, 64, 192, 32), (33, 10, 150, 1), (100, 10, 160, 32), (150, 10, 101, 16)])
 def test_attention_pair_tensor_core_kernels_vs_oracle(shape):
     """K3 on tensor cores (csrc/attn_tc.cu, 3xTF32 mma.sync, both sides in one launch): outputs, scores and every gradient
     against the oracle's LinearAttention at the fp32 tolerance; padded reviews (id 0) keep softmax mass and give the padding
@@ -277,7 +280,12 @@ def test_attention_pair_tensor_core_kernels_vs_oracle(shape):
         for j, name in enumerate(("W_rv", "W_id", "h", "b_1", "b_2", "ebd_vals")):
             # d loss / d b_2 is ~0 by the softmax's shift invariance: what any implementation stores there is the rounding
             # noise of a sum of B*R terms of size |d logit| — compare it on that scale
-            floor = float(B * R) ** 0.5 * 0.1 if name == "b_2" else 1e-6      # (R = 1: softmax of one review, gradients ~1e-8)
+            floor = float(B * R) ** 0.5 * 0.1 if name == "b_2" else 1e-6
+            if R == 1:
+                # one review: the score is 1 / (1 + 1e-8) and every logit gradient is ~1e-8 of the upstream gradient, below fp32's
+                # resolution of the score.  The parameters only see those logit gradients (~1e-7 here): compare them on an
+                # absolute scale (3e-6)
+                floor = max(floor, 0.1)
             assert rel_err(cu[s][2][j].grad.cpu(), ref[s][3][j], floor) < FP32_GRAD_TOL, (s, name)
         assert float(cu[s][2][5].grad[0].abs().max()) == 0.0
 
