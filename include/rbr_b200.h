@@ -332,6 +332,24 @@ int rbr_multimem_allreduce_f32(void* multicast_ptr, int64_t n_floats, int rank, 
 int rbr_p2p_allreduce_f32(const void* peer_ptrs, int64_t offset_floats, int64_t n_floats, int rank, int world, float scale,
                           int max_ctas, void* stream);
 
+/* ---- K10: per-row top-k of a factorised score matrix (full-catalogue recommendation) --------------------------------
+ * score[r, i] = sum_c A[r, c] * B[i, c] + row_bias[r] + col_bias[i]  (A [n_rows, dim], B [n_items, dim] fp32 row-major;
+ * row_bias [n_rows] / col_bias [n_items], either may be NULL = 0).  For each row, the k eligible items with the largest
+ * score, ordered by score descending then item id ascending, go to out_scores / out_items [n_rows, k]; the n_rows x n_items
+ * scores are never materialised.  Eligible: every i < n_items not listed in excl_idx[excl_ptr[r] : excl_ptr[r+1]]
+ * (CSR, each row's list sorted ascending without duplicates; both NULL = nothing excluded).  With fewer than k eligible
+ * items the remaining slots hold item -1, score -inf.  A NaN score is never returned (scores enter by strict '>').
+ * fp32-grade: each returned score is within ~1e-6 of |score|-scale of the exact dot product (3-piece bf16 split of both
+ * operands, six tcgen05 products).  The FM head is such a product: relu(u*i) = relu(u)*relu(i) + relu(-u)*relu(-i).
+ * Limits: 1 <= k <= 256, 1 <= dim <= 512, 1 <= n_items < 2^31; else RBR_EUNSUPPORTED.  The two queries are host-only and
+ * launch nothing; rbr_factor_topk_slices gives the number of item slices the call splits each row's scan into (one CTA
+ * per 128 rows and slice; a second kernel merges the slices' sorted lists, a copy when there is one slice).            */
+int64_t rbr_factor_topk_workspace_bytes(int64_t n_rows, int64_t n_items, int64_t dim, int64_t k);
+int64_t rbr_factor_topk_slices(int64_t n_rows, int64_t n_items, int64_t dim, int64_t k);
+int rbr_factor_topk(const float* A, const float* row_bias, int64_t n_rows, const float* B, const float* col_bias,
+                    int64_t n_items, int64_t dim, const int64_t* excl_ptr, const int64_t* excl_idx, int64_t k,
+                    float* out_scores, int64_t* out_items, void* ws, int64_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1,42 +1,111 @@
-"""Inference scoring (BASELINE.json configs[4]) and the per-entity feature cache (SURVEY §8f-2).
+"""Inference scoring (BASELINE.json configs[4]), the per-entity feature cache (SURVEY §8f-2) and full-catalogue top-k.
 
 The reference has no predict entry point: scoring is `valid_one_epoch` (trainer/train_deepconn_pp.py:191-212) — `model.eval()`,
 `torch.no_grad()`, the same forward — and every example carries its own two padded documents (:274), so the encoder runs
 twice per (user, item) pair although a user's document is the same in every pair the user appears in.
 
-`PairScorer.score_pairs` is that data flow on the fused kernels.  `PairScorer.build_cache` encodes each entity's document ONCE
-(K2 forward over [U, L] and [I, L]) and `score_cached` then scores pairs with a row gather (K1) + the head kernel (K4) only:
-10 M pairs over U + I = 32 k documents is ≈ 600x less encoder work, bit-identical scores.
+`PairScorer.score_pairs` is that data flow on the fused kernels.  `PairScorer.build_cache` encodes each entity's side ONCE
+and `score_cached` then scores pairs from the cached features only: 10 M pairs over U + I = 32 k documents is ≈ 600x less
+encoder work.  In eval mode every model puts an entity's side through that entity's inputs alone, so all three cache:
+  DeepCoNN  the entity's document (K2) → [U, H] / [I, H]; pairs score through K1 gather + K4 head, bit-identical;
+  NARRE     the entity's reviews (K2) + LinearAttention over the ids of the counterparts they review → [U, H] / [I, H];
+            pairs score through K1 + K4 as for DeepCoNN;
+  D-ATT     fc(encode(document)) per side → [U, 50] / [I, 50]; a pair's score is the dot product of its two rows.
+
+`PairScorer.recommend` answers "the k best items for these users out of the whole catalogue" with K10 (ops.factor_topk),
+which never materialises the users x items score matrix.  The FM head factorises exactly:
+  relu(u*i) = relu(u)*relu(i) + relu(-u)*relu(-i)   ⇒   score(u,i) = A[u] . B[i] + row_bias[u] + col_bias[i]
+with A = [h*relu(u_lat), h*relu(-u_lat)], B = [relu(i_lat), relu(-i_lat)], row_bias = ub + g, col_bias = ib (fm_factors);
+D-ATT's score is already a dot product of the two FC outputs.
 """
 from __future__ import annotations
 
-from typing import Optional
+from typing import Optional, Tuple
 
 import torch
 
 from . import ops
+from .deepconn import DeepCoNNpp
+from .dual_att import DualAtt
 from .layers import fused_head
+from .narre import NARRE
+
+
+def fm_factors(u_lat: torch.Tensor, i_lat: torch.Tensor, h: torch.Tensor, user_bias: torch.Tensor, item_bias: torch.Tensor,
+               g_bias: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """FM head (models/deepconn/layers.py:200-207) as a factor product: score(u, i) = A[u] . B[i] + row_bias[u] + col_bias[i]
+    for latents u_lat [U, K], i_lat [I, K] (LastFeat outputs of entity rows u / i), h [K, 1], user_bias [U, 1],
+    item_bias [I, 1], g_bias [1].  Returns (A [U, 2K], row_bias [U], B [I, 2K], col_bias [I]) in the inputs' dtype."""
+    hv = h.reshape(1, -1)
+    A = torch.cat([hv * torch.relu(u_lat), hv * torch.relu(-u_lat)], dim=1)
+    B = torch.cat([torch.relu(i_lat), torch.relu(-i_lat)], dim=1)
+    return A, user_bias.reshape(-1) + g_bias.reshape(()), B, item_bias.reshape(-1)
+
+
+def _is_narre(model) -> bool:
+    return isinstance(model, NARRE)
+
+
+def _is_datt(model) -> bool:
+    return isinstance(model, DualAtt)
 
 
 class PairScorer:
     def __init__(self, model):
-        if not hasattr(model, "ngram") or hasattr(model, "user_att"):
-            raise TypeError("PairScorer serves DeepCoNNpp (one document per entity); NARRE / D-ATT score through model.eval() forward")
+        if not isinstance(model, (DeepCoNNpp, NARRE, DualAtt)):
+            raise TypeError("PairScorer serves DeepCoNNpp, NARRE and DualAtt")
         self.model = model.eval()
         self.user_feat: Optional[torch.Tensor] = None
         self.item_feat: Optional[torch.Tensor] = None
+        self._factors = None         # (key, (A, row_bias, B, col_bias)) derived from the current head parameters
 
     @torch.no_grad()
-    def score_pairs(self, u_docs, i_docs, u_masks, i_masks, u_ids, i_ids) -> torch.Tensor:
-        """The reference's per-pair data flow: both documents encoded for every pair."""
-        return self.model(u_docs, i_docs, u_masks, i_masks, u_ids, i_ids)
+    def score_pairs(self, *inputs) -> torch.Tensor:
+        """The reference's per-pair data flow: both sides encoded for every pair (the model's own eval forward)."""
+        out = self.model(*inputs)
+        return out[0] if isinstance(out, tuple) else out
 
     @torch.no_grad()
     def build_cache(self, user_docs: torch.Tensor, item_docs: torch.Tensor, user_masks: Optional[torch.Tensor] = None,
-                    item_masks: Optional[torch.Tensor] = None, chunk: int = 4096) -> None:
-        """user_docs [U, L], item_docs [I, L]: row e = the document of entity id e (row 0 = the padding entity).
-        Masks default to ids != 0 (utils.py:30-42)."""
+                    item_masks: Optional[torch.Tensor] = None, chunk: int = 4096, *, user_rev_ids: Optional[torch.Tensor] = None,
+                    item_rev_ids: Optional[torch.Tensor] = None) -> None:
+        """Row e of every argument belongs to entity id e (row 0 = the padding entity).
+        DeepCoNN: user_docs [U, L], item_docs [I, L]; masks default to ids != 0 (utils.py:30-42).
+        NARRE: user_docs [U, R, T], item_docs [I, R, T] (the entity's reviews), optional masks of the same shapes, and
+          user_rev_ids [U, R] / item_rev_ids [I, R]: the ids of the items a user reviewed / the users who reviewed an item —
+          what NARRE's dataset supplies as reuid / reiid for a pair with that entity.
+        D-ATT: user_docs [U, L], item_docs [I, L] (no masks)."""
         m = self.model
+        self.model.eval()
+        self._factors = None
+        if _is_datt(m):
+            if user_masks is not None or item_masks is not None:
+                raise ValueError("DualAtt takes no masks")
+
+            def side(docs, s):
+                return torch.cat([m.fc(m.encode([docs[lo:lo + chunk]], [s])[0]) for lo in range(0, docs.shape[0], chunk)], 0)
+            self.user_feat, self.item_feat = side(user_docs, "u"), side(item_docs, "i")
+            return
+        if _is_narre(m):
+            if user_rev_ids is None or item_rev_ids is None:
+                raise ValueError("NARRE's build_cache needs user_rev_ids [U, R] and item_rev_ids [I, R]")
+            R, T = m.doc_num, m.doc_len
+            ent_chunk = max(1, chunk // R)
+
+            def side(docs, masks, rev_ids, att):
+                if docs.shape[1:] != (R, T) or rev_ids.shape != docs.shape[:2]:
+                    raise ValueError(f"NARRE was built for [*, {R}, {T}] reviews with [*, {R}] review ids, got "
+                                     f"{tuple(docs.shape)} / {tuple(rev_ids.shape)}")
+                outs = []
+                for lo in range(0, docs.shape[0], ent_chunk):
+                    d = docs[lo:lo + ent_chunk]
+                    mk = None if masks is None else masks[lo:lo + ent_chunk].reshape(-1, T)
+                    (f,) = m.ngram.encode(m.word_embeddings, [d.reshape(-1, T)], [mk])
+                    outs.append(att(f.view(d.shape[0], R, -1), rev_ids[lo:lo + ent_chunk])[0])
+                return torch.cat(outs, 0)
+            self.user_feat = side(user_docs, user_masks, user_rev_ids, m.user_att)
+            self.item_feat = side(item_docs, item_masks, item_rev_ids, m.item_att)
+            return
 
         def encode(docs, masks):
             outs = []
@@ -50,10 +119,67 @@ class PairScorer:
 
     @torch.no_grad()
     def score_cached(self, u_ids: torch.Tensor, i_ids: torch.Tensor) -> torch.Tensor:
-        """preds for pairs (u_ids[b], i_ids[b]) from the cached features: K1 row gather + K4 head, no encoder."""
+        """preds for pairs (u_ids[b], i_ids[b]) from the cached features, no encoder: K1 row gather + K4 head (DeepCoNN,
+        NARRE) or K1 + dot product (D-ATT, dual_att.py:59-61)."""
         if self.user_feat is None:
             raise RuntimeError("PairScorer.build_cache(...) first")
         m = self.model
         u_text = ops.gather_rows(self.user_feat, u_ids)
         i_text = ops.gather_rows(self.item_feat, i_ids)
+        if _is_datt(m):
+            return torch.sum(torch.mul(u_text, i_text), 1).view(-1)
         return fused_head(m.user_feat, m.item_feat, m.fm, u_text, i_text, u_ids, i_ids, False, None).view(-1)
+
+    def _head_params(self):
+        m = self.model
+        if _is_datt(m):
+            return []
+        return [m.user_feat.W, m.user_feat.b, m.user_feat.ebd.weight, m.item_feat.W, m.item_feat.b, m.item_feat.ebd.weight,
+                m.fm.h, m.fm.user_bias.weight, m.fm.item_bias.weight, m.fm.g_bias]
+
+    def factors(self) -> Tuple[torch.Tensor, Optional[torch.Tensor], torch.Tensor, Optional[torch.Tensor]]:
+        """(A [U, D], row_bias [U] or None, B [I, D], col_bias [I] or None) with score(u, i) = A[u] . B[i] + biases for the
+        cached entities under the CURRENT head parameters.  Re-derived when a parameter changed (optimizer steps bump
+        its version counter) or the cache was rebuilt."""
+        if self.user_feat is None:
+            raise RuntimeError("PairScorer.build_cache(...) first")
+        params = self._head_params()
+        key = tuple((p._version, p.data_ptr()) for p in params) + ((self.user_feat.data_ptr(), self.item_feat.data_ptr()),)
+        if self._factors is None or self._factors[0] != key:
+            if _is_datt(self.model):
+                f = (self.user_feat, None, self.item_feat, None)
+            else:
+                with torch.no_grad():
+                    # LastFeat (models/deepconn/layers.py:163) in float64: exact fp32 latents whatever the TF32 setting
+                    d = [p.detach().double() for p in params]
+                    Wu, bu, eu, Wi, bi, ei, h, ub, ib, g = d
+                    n_u, n_i = self.user_feat.shape[0], self.item_feat.shape[0]
+                    u_lat = self.user_feat.double() @ Wu + bu + eu[:n_u]
+                    i_lat = self.item_feat.double() @ Wi + bi + ei[:n_i]
+                    f = tuple(t.float().contiguous() for t in fm_factors(u_lat, i_lat, h, ub[:n_u], ib[:n_i], g))
+            self._factors = (key, f)
+        return self._factors[1]
+
+    @torch.no_grad()
+    def recommend(self, u_ids: torch.Tensor, k: int, exclude: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
+                  exclude_padding: bool = True) -> Tuple[torch.Tensor, torch.Tensor]:
+        """The k best cached items for each user u_ids[r], by score descending then item id ascending (K10: one fused
+        score GEMM + per-row top-k, the [len(u_ids), I] score matrix is never materialised).
+        exclude = (indptr [len(u_ids) + 1], indices) int64 CUDA CSR: items to leave out per row (e.g. those already rated).
+        exclude_padding drops the item padding row (fm.item_padding_idx; 0 for D-ATT).
+        Returns (scores [len(u_ids), k] fp32, items [len(u_ids), k] int64); rows with fewer than k eligible items end in
+        (-inf, -1).  Scores agree with score_cached on the same pairs to fp32 rounding."""
+        self.model.eval()
+        A, rb, B, cb = self.factors()
+        u_ids = u_ids.to(device=A.device, dtype=torch.int64).reshape(-1)
+        if u_ids.numel() and (int(u_ids.min()) < 0 or int(u_ids.max()) >= A.shape[0]):
+            raise ValueError(f"user ids must lie in [0, {A.shape[0]})")
+        A_rows = A.index_select(0, u_ids)
+        rb_rows = None if rb is None else rb.index_select(0, u_ids)
+        if exclude_padding:
+            pad = 0 if _is_datt(self.model) else self.model.fm.item_padding_idx
+            if pad is not None and 0 <= pad < B.shape[0]:
+                # a -inf column bias: the padding item's score never beats a threshold, so it is never returned
+                cb = torch.zeros(B.shape[0], dtype=torch.float32, device=B.device) if cb is None else cb.clone()
+                cb[pad] = float("-inf")
+        return ops.factor_topk(A_rows, rb_rows, B, cb, k, exclude=exclude)

@@ -998,3 +998,94 @@ class DattEncodeFn(torch.autograd.Function):
                                             _p(gate_g), _p(d_gate_l), _p(d_gate_g), cfg["padding_idx"], _p(grads[0]), _p(grads[1]),
                                             _p(grads[4]), _p(grads[5]), _p(g_table), _p(ws), ws_bytes, idf, _stream()),
                       "rbr_datt_gate_bwd")
+
+
+# ---------------------------------------------------------------------------------------------------
+# K10: per-row top-k of a factorised score matrix (full-catalogue recommendation)
+# ---------------------------------------------------------------------------------------------------
+FACTOR_TOPK_MAX_K, FACTOR_TOPK_MAX_DIM = 256, 512
+
+
+def normalize_exclusions(indptr: torch.Tensor, indices: torch.Tensor, n_rows: int, n_items: int
+                         ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """CSR exclusion lists (row r excludes indices[indptr[r]:indptr[r+1]], in any order, duplicates allowed) → the same
+    lists sorted ascending without duplicates, as rbr_factor_topk reads them.  Ids outside [0, n_items) raise ValueError."""
+    if indptr.dtype != torch.int64 or indices.dtype != torch.int64:
+        raise ValueError("rbr_b200: exclusion indptr / indices must be int64")
+    if indptr.dim() != 1 or indptr.numel() != n_rows + 1 or indices.dim() != 1:
+        raise ValueError(f"rbr_b200: exclusion indptr must be [n_rows + 1] = [{n_rows + 1}] and indices 1-D")
+    counts = indptr[1:] - indptr[:-1]
+    lo_hi = torch.stack([indices.min(), indices.max()]) if indices.numel() else indptr.new_zeros(2)
+    # one device-to-host read for every check
+    first, last, neg, lo, hi = torch.cat([indptr[:1], indptr[-1:], (counts < 0).any().view(1).long(), lo_hi]).tolist()
+    if first != 0 or last != indices.numel() or neg:
+        raise ValueError("rbr_b200: exclusion indptr must start at 0, be non-decreasing and end at len(indices)")
+    if lo < 0 or hi >= n_items:
+        raise ValueError(f"rbr_b200: excluded item ids must lie in [0, {n_items})")
+    rows = torch.repeat_interleave(torch.arange(n_rows, device=indices.device), counts)
+    keys = torch.unique(rows * n_items + indices, sorted=True)
+    new_counts = torch.bincount(torch.div(keys, n_items, rounding_mode="floor"), minlength=n_rows)
+    ptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=indices.device)
+    torch.cumsum(new_counts, 0, out=ptr[1:])
+    return ptr, keys % n_items
+
+
+def factor_topk_workspace_bytes(n_rows: int, n_items: int, dim: int, k: int) -> int:
+    n = lib.rbr_factor_topk_workspace_bytes(n_rows, n_items, dim, k)
+    if n < 0:
+        raise ValueError(f"rbr_b200: factor_topk does not take n_items={n_items}, dim={dim}, k={k} "
+                         f"(1 <= k <= {FACTOR_TOPK_MAX_K}, 1 <= dim <= {FACTOR_TOPK_MAX_DIM}, 1 <= n_items < 2^31)")
+    return int(n)
+
+
+def factor_topk_slices(n_rows: int, n_items: int, dim: int, k: int) -> int:
+    """How many item slices rbr_factor_topk splits each row's scan into on the current device (host-only plan query)."""
+    factor_topk_workspace_bytes(n_rows, n_items, dim, k)
+    return int(lib.rbr_factor_topk_slices(n_rows, n_items, dim, k))
+
+
+def factor_topk(A: torch.Tensor, row_bias: Optional[torch.Tensor], B: torch.Tensor, col_bias: Optional[torch.Tensor], k: int,
+                exclude: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """K10: for each row r, the k items i (excluding exclude = (indptr [n_rows+1], indices) CSR lists) with the largest
+    score A[r] . B[i] + row_bias[r] + col_bias[i], by score descending then item id ascending; fp32-grade scores.
+    Returns (scores [n_rows, k] fp32, items [n_rows, k] int64); slots past the eligible items hold (-inf, -1)."""
+    for t, name in ((A, "A"), (B, "B"), (row_bias, "row_bias"), (col_bias, "col_bias")):
+        if t is None:
+            continue
+        if not isinstance(t, torch.Tensor) or not t.is_cuda:
+            raise RuntimeError(f"rbr_b200: `{name}` must be a CUDA tensor (the hot path has no CPU implementation)")
+        if t.dtype != torch.float32:
+            raise ValueError(f"rbr_b200: `{name}` must be float32, got {t.dtype}")
+        if t.device != A.device:
+            raise ValueError(f"rbr_b200: `{name}` is on {t.device}, A on {A.device}")
+    if A.dim() != 2 or B.dim() != 2 or A.shape[1] != B.shape[1]:
+        raise ValueError(f"rbr_b200: A [n_rows, dim] and B [n_items, dim] must share dim, got {tuple(A.shape)} / {tuple(B.shape)}")
+    n_rows, dim = A.shape
+    n_items = B.shape[0]
+    k = int(k)
+    if row_bias is not None and row_bias.numel() != n_rows:
+        raise ValueError("rbr_b200: row_bias must hold n_rows values")
+    if col_bias is not None and col_bias.numel() != n_items:
+        raise ValueError("rbr_b200: col_bias must hold n_items values")
+    ws_bytes = factor_topk_workspace_bytes(n_rows, n_items, dim, k)
+    ptr = idx = None
+    if exclude is not None:
+        indptr, indices = exclude
+        for t, name in ((indptr, "exclude indptr"), (indices, "exclude indices")):
+            if not isinstance(t, torch.Tensor) or not t.is_cuda:
+                raise RuntimeError(f"rbr_b200: `{name}` must be a CUDA tensor")
+        ptr, idx = normalize_exclusions(indptr.contiguous(), indices.contiguous(), n_rows, n_items)
+        if idx.numel() == 0:
+            ptr = idx = None
+    A, B = A.contiguous(), B.contiguous()
+    rb = None if row_bias is None else row_bias.contiguous().view(-1)
+    cb = None if col_bias is None else col_bias.contiguous().view(-1)
+    scores = torch.empty(n_rows, k, dtype=torch.float32, device=A.device)
+    items = torch.empty(n_rows, k, dtype=torch.int64, device=A.device)
+    if n_rows == 0:
+        return scores, items
+    with torch.cuda.device(A.device):
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=A.device)
+        lib.check(lib.rbr_factor_topk(_p(A), _p(rb), n_rows, _p(B), _p(cb), n_items, dim, _p(ptr), _p(idx), k, _p(scores),
+                                      _p(items), _p(ws), ws_bytes, _stream(True)), "rbr_factor_topk")
+    return scores, items
