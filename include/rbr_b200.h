@@ -350,6 +350,25 @@ int rbr_factor_topk(const float* A, const float* row_bias, int64_t n_rows, const
                     int64_t n_items, int64_t dim, const int64_t* excl_ptr, const int64_t* excl_idx, int64_t k,
                     float* out_scores, int64_t* out_items, void* ws, int64_t ws_bytes, void* stream);
 
+/* ---- K11: exact full-catalogue rank of target items under a factorised score matrix ----------------------------------
+ * The score is K10's, from the same split operands, tcgen05 shape, K-step order, bias order and key (score descending,
+ * then item id ascending), so the results are bit-consistent with rbr_factor_topk on the same inputs.  Row r's targets are
+ * tgt_idx[tgt_ptr[r] : tgt_ptr[r+1]] (CSR, each row sorted ascending without duplicates, ids in [0, n_items), disjoint from
+ * the row's exclusions; n_targets = tgt_ptr[n_rows]; at most max_targets per row — a caller with longer rows splits them
+ * into several rows with the same A row, row bias and exclusions).  Exclusions as in rbr_factor_topk.  For each target t:
+ *   out_ranks[p]  = #{ eligible i : key(r, i) >= key(r, t) }, i.e. the 1-based position of t in rbr_factor_topk's output
+ *                   for k = infinity (other targets of the row are ordinary competitors; NaN and -inf scores never count);
+ *                   -1 when t's own score is NaN or -inf;
+ *   out_scores[p] = t's score, bit-identical to the score rbr_factor_topk returns for (r, t).
+ * Item slices as in K10; per-slice counts are integers, so the result does not depend on the slice count.
+ * Limits: 1 <= dim <= 512, 1 <= n_items < 2^31, 1 <= max_targets <= 64; else RBR_EUNSUPPORTED.  The workspace query is
+ * host-only and launches nothing; the call never synchronises.                                                       */
+int64_t rbr_factor_rank_workspace_bytes(int64_t n_rows, int64_t n_items, int64_t dim, int64_t n_targets, int64_t max_targets);
+int rbr_factor_rank(const float* A, const float* row_bias, int64_t n_rows, const float* B, const float* col_bias,
+                    int64_t n_items, int64_t dim, const int64_t* excl_ptr, const int64_t* excl_idx, const int64_t* tgt_ptr,
+                    const int64_t* tgt_idx, int64_t n_targets, int64_t max_targets, int64_t* out_ranks, float* out_scores,
+                    void* ws, int64_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -27,45 +27,22 @@
 
 #include <algorithm>
 
-#include "rbr_common.cuh"
-#include "tc_ptx.cuh"
+#include "factor_gemm.cuh"
 
 namespace rbr {
 
-constexpr int FT_M = 128;                              // rows per tile (UMMA M, TMEM lanes)
-constexpr int FT_N = 256;                              // items per tile (UMMA N)
-constexpr int FT_KC = 64;                              // contraction elements per ring stage (4 UMMA K-steps)
-constexpr int FT_A_BYTES = FT_M * FT_KC * 2;           // 16 KB
-constexpr int FT_B_BYTES = FT_N * FT_KC * 2;           // 32 KB
-constexpr int FT_STAGE_BYTES = FT_A_BYTES + FT_B_BYTES;
-constexpr int FT_THREADS = 192;                        // warps 0-3 epilogue, 4 producer, 5 MMA issuer
-constexpr int FT_PROD_WARP = 4, FT_MMA_WARP = 5;
-constexpr int FT_SMEM_MAX = 232448;                    // 227 KB opt-in dynamic shared memory per CTA
-constexpr int FT_MAX_SLICES = 16;
 constexpr int FT_QUEUE_BYTES = FT_M * 16 * 8;          // per row: the candidate keys of one 16-column chunk
 constexpr int64_t FT_PART_CAP = 96ll << 20;            // cap on the per-slice partial lists when choosing several slices
-constexpr int FT_MAX_K = 256, FT_MAX_DIM = 512;
+constexpr int FT_MAX_K = 256;
 
 struct FtPlan {
-    int64_t dimp;       // dim rounded up to 32 (6 * dimp is a whole number of 64-element chunks)
-    int64_t nq;         // ring stages per item tile = 6 * dimp / 64
-    int64_t rt, it;     // row tiles, item tiles
+    FtGemm g;           // split operands: A' | B' at the start of the workspace
     int64_t S, tps;     // item slices, item tiles per slice
     int nst;            // ring stages
     int heap_smem;      // 1: per-row heaps in shared memory
     int smem;           // dynamic shared memory bytes
-    int64_t off_b, off_part, total;   // workspace: A' | B' | partial top-k keys [n_rows][S][k]
+    int64_t off_part, total;   // workspace: A' | B' | partial top-k keys [n_rows][S][k]
 };
-
-static int ft_sm_count() {
-    int dev = 0, n = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
-        n <= 0) {
-        cudaGetLastError();
-        return 148;                                     // B200
-    }
-    return n;
-}
 
 static bool ft_supported(int64_t n_rows, int64_t n_items, int64_t dim, int64_t k) {
     return n_rows >= 0 && n_items >= 1 && n_items < (1ll << 31) && dim >= 1 && dim <= FT_MAX_DIM && k >= 1 && k <= FT_MAX_K;
@@ -73,28 +50,11 @@ static bool ft_supported(int64_t n_rows, int64_t n_items, int64_t dim, int64_t k
 
 static FtPlan ft_plan(int64_t n_rows, int64_t n_items, int64_t dim, int64_t k, int sms) {
     FtPlan p;
-    p.dimp = round_up(dim, 32);
-    p.nq = 6 * p.dimp / FT_KC;
-    p.rt = (n_rows + FT_M - 1) / FT_M;
-    p.it = (n_items + FT_N - 1) / FT_N;
-    // Slices: the CTA's cost is roughly its item tiles plus a share per slice that grows with k (filling, sorting and
-    // writing its heaps, and the threshold starting over); the grid runs in waves of one CTA per SM.  Take the slice
-    // count with the fewest wave-weighted tiles.  The share, in tiles, was fitted to timings at 20 000 x 12 000 on a
-    // B200 (k = 10: 3 slices best, k = 100: 1-2).
-    const double fill = 3.0 + (double)k / 16.0;
-    int64_t best = 1;
-    double best_cost = 1e300;
-    const int64_t smax = p.it < FT_MAX_SLICES ? p.it : FT_MAX_SLICES;
-    for (int64_t s = 1; s <= smax; ++s) {
-        if (s > 1 && n_rows * s * k * 8 > FT_PART_CAP) break;
-        const int64_t tps = (p.it + s - 1) / s;
-        if ((p.it + tps - 1) / tps != s) continue;     // every slice must own at least one tile
-        const int64_t waves = (p.rt * s + sms - 1) / sms;
-        const double cost = (double)waves * ((double)tps + fill);
-        if (cost < best_cost * 0.97) { best_cost = cost; best = s; }
-    }
-    p.S = best;
-    p.tps = (p.it + p.S - 1) / p.S;
+    p.g = ft_gemm_plan(n_rows, n_items, dim);
+    // The per-slice share, in tiles (filling, sorting and writing the heaps, and the threshold starting over), was fitted
+    // to timings at 20 000 x 12 000 on a B200 (k = 10: 3 slices best, k = 100: 1-2).
+    p.S = ft_choose_slices(p.g, sms, 3.0 + (double)k / 16.0, n_rows * k * 8, FT_PART_CAP);
+    p.tps = (p.g.it + p.S - 1) / p.S;
     const int64_t heap_bytes = (int64_t)FT_M * k * 8;
     const int64_t fixed = FT_QUEUE_BYTES + 1024;        // candidate queues, barriers + TMEM slot
     p.heap_smem = 0;
@@ -106,10 +66,7 @@ static FtPlan ft_plan(int64_t n_rows, int64_t n_items, int64_t dim, int64_t k, i
     int64_t smem = p.nst * FT_STAGE_BYTES + (p.heap_smem ? heap_bytes : 0) + fixed;
     if (smem < 116 * 1024) smem = 116 * 1024;
     p.smem = (int)smem;
-    const int64_t a_bytes = p.rt * p.nq * FT_A_BYTES;
-    const int64_t b_bytes = p.it * p.nq * FT_B_BYTES;
-    p.off_b = round_up(a_bytes, 1024);
-    p.off_part = p.off_b + round_up(b_bytes, 1024);
+    p.off_part = p.g.end;
     p.total = p.off_part + round_up(n_rows * p.S * k * 8, 1024);
     return p;
 }
@@ -165,16 +122,6 @@ __device__ __forceinline__ void heap_sift_down(unsigned long long* h, int64_t hs
 __device__ __forceinline__ void heap_make(unsigned long long* h, int64_t hs, int n) {
     for (int i = n / 2 - 1; i >= 0; --i) heap_sift_down(h, hs, n, i, h[i * hs]);
 }
-__device__ __forceinline__ float key_score(unsigned long long key) { return __uint_as_float(ord2f((uint32_t)(key >> 32))); }
-
-// first position in idx[lo, hi) holding a value >= j
-__device__ __forceinline__ int64_t lower_bound(const int64_t* __restrict__ idx, int64_t lo, int64_t hi, int64_t j) {
-    while (lo < hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (__ldg(idx + mid) < j) lo = mid + 1; else hi = mid;
-    }
-    return lo;
-}
 
 struct FtArgs {
     const __nv_bfloat16* a_split;
@@ -201,73 +148,15 @@ __global__ void __launch_bounds__(FT_THREADS, 1) factor_topk_kernel(const FtArgs
     unsigned long long* queue_s = reinterpret_cast<unsigned long long*>(smem + a.nst * FT_STAGE_BYTES);
     unsigned long long* heap_s = queue_s + FT_M * 16;
     const int heap_bytes = FT_QUEUE_BYTES + (a.heap_smem ? FT_M * a.k * 8 : 0);
-    const uint32_t bars = sbase + a.nst * FT_STAGE_BYTES + heap_bytes;
     // barrier slots: full[nst], empty[nst], acc_full[2], acc_empty[2]; then the TMEM address slot
-    const uint32_t bar_full = bars, bar_empty = bars + 8 * a.nst, bar_accf = bars + 16 * a.nst, bar_acce = bar_accf + 16;
+    const FtBars bar = ft_bars(sbase + a.nst * FT_STAGE_BYTES + heap_bytes, a.nst);
     volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem + a.nst * FT_STAGE_BYTES + heap_bytes + 16 * a.nst + 32);
-
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < a.nst; ++i) { mbar_init(bar_full + 8 * i, 1); mbar_init(bar_empty + 8 * i, 1); }
-        mbar_init(bar_accf, 1); mbar_init(bar_accf + 8, 1);
-        mbar_init(bar_acce, FT_M); mbar_init(bar_acce + 8, FT_M);
-        fence_barrier_init();
-    }
-    if (warp == FT_MMA_WARP) tmem_alloc(smem_u32((const void*)tmem_slot), 512);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = ft_setup(bar, a.nst, tmem_slot);
 
     if (warp == FT_PROD_WARP) {
-        // =========================== ring producer: two TMA bulk copies per stage ===========================
-        if (elect_one()) {
-            const uint8_t* asrc = reinterpret_cast<const uint8_t*>(a.a_split) + rt * a.nq * FT_A_BYTES;
-            int stage = 0;
-            uint32_t ph = 0;
-            for (int g = 0; g < ntiles; ++g) {
-                const uint8_t* bsrc = reinterpret_cast<const uint8_t*>(a.b_split) + (t0 + g) * a.nq * FT_B_BYTES;
-                for (int q = 0; q < nq; ++q) {
-                    mbar_wait(bar_empty + 8 * stage, ph ^ 1);
-                    const uint32_t dst = ring + (uint32_t)(stage * FT_STAGE_BYTES);
-                    mbar_expect_tx(bar_full + 8 * stage, (uint32_t)FT_STAGE_BYTES);
-                    bulk_g2s(dst, asrc + (int64_t)q * FT_A_BYTES, FT_A_BYTES, bar_full + 8 * stage);
-                    bulk_g2s(dst + FT_A_BYTES, bsrc + (int64_t)q * FT_B_BYTES, FT_B_BYTES, bar_full + 8 * stage);
-                    if (++stage == a.nst) { stage = 0; ph ^= 1; }
-                }
-            }
-        }
-        __syncwarp();
+        ft_produce(a.a_split, a.b_split, rt, t0, ntiles, nq, a.nst, ring, bar);
     } else if (warp == FT_MMA_WARP) {
-        // =========================== MMA issuer ===========================
-        const bool leader = elect_one();
-        const uint32_t idesc = umma_idesc(FT_M, FT_N);
-        int stage = 0;
-        uint32_t ph = 0;
-        for (int g = 0; g < ntiles; ++g) {
-            const int buf = g & 1;
-            mbar_wait(bar_acce + 8 * buf, (uint32_t)(((g >> 1) & 1) ^ 1));     // epilogue drained this accumulator
-            tc_fence_after();
-            const uint32_t d_tmem = tmem_base + (uint32_t)(buf * FT_N);
-            for (int q = 0; q < nq; ++q) {
-                mbar_wait(bar_full + 8 * stage, ph);
-                tc_fence_after();
-                if (leader) {
-                    const uint32_t sa = ring + (uint32_t)(stage * FT_STAGE_BYTES);
-                    // A block [8 chunks][128 rows][16 B]: chunk stride 2048 B; B block [8][256][16 B]: chunk stride 4096 B;
-                    // 8-row groups 128 B apart in both.  One K-step (16 elements) = two chunks.
-                    const uint64_t ad = umma_desc(sa, FT_M * 16u, 128u);
-                    const uint64_t bd = umma_desc(sa + FT_A_BYTES, FT_N * 16u, 128u);
-#pragma unroll
-                    for (int ks = 0; ks < FT_KC / 16; ++ks)
-                        umma_bf16(d_tmem, ad + (uint64_t)(ks * 2 * FT_M), bd + (uint64_t)(ks * 2 * FT_N), idesc,
-                                  (uint32_t)((q | ks) != 0));
-                    umma_commit(bar_empty + 8 * stage);                          // frees the ring slot when the MMAs retire
-                    if (q == nq - 1) umma_commit(bar_accf + 8 * buf);            // accumulator complete → epilogue
-                }
-                __syncwarp();
-                if (++stage == a.nst) { stage = 0; ph ^= 1; }
-            }
-        }
+        ft_mma(ntiles, nq, a.nst, ring, bar, tmem_base);
     } else {
         // =========================== epilogue: thread t = row rt*128 + t = TMEM lane t ===========================
         const int t = threadIdx.x;
@@ -292,7 +181,7 @@ __global__ void __launch_bounds__(FT_THREADS, 1) factor_topk_kernel(const FtArgs
         const uint32_t lane_base = tmem_base + ((uint32_t)(warp * 32) << 16);
         for (int g = 0; g < ntiles; ++g) {
             const int buf = g & 1;
-            mbar_wait(bar_accf + 8 * buf, (uint32_t)((g >> 1) & 1));
+            mbar_wait(bar.accf + 8 * buf, (uint32_t)((g >> 1) & 1));
             tc_fence_after();
             const int64_t jt = (t0 + g) * FT_N;
             for (int ch = 0; ch < FT_N / 16; ++ch) {
@@ -301,7 +190,7 @@ __global__ void __launch_bounds__(FT_THREADS, 1) factor_topk_kernel(const FtArgs
                 tmem_ld_wait();
                 if (ch == FT_N / 16 - 1) {                 // the whole tile is read: release the accumulator
                     tc_fence_before();
-                    mbar_arrive(bar_acce + 8 * buf);
+                    mbar_arrive(bar.acce + 8 * buf);
                 }
                 const int64_t j0 = jt + ch * 16;
                 // Pass 1: queue the chunk's candidates (a predicated store, no branch).  Handling a candidate on the spot
@@ -312,19 +201,15 @@ __global__ void __launch_bounds__(FT_THREADS, 1) factor_topk_kernel(const FtArgs
                 for (int i = 0; i < 16; ++i) {
                     const int64_t j = j0 + i;
                     const bool in = j < a.n_items;
-                    float s = __uint_as_float(v[i]);
-                    if (a.col_bias) s += in ? __ldg(a.col_bias + j) : 0.f;
-                    s += rb;
-                    s = s == 0.f ? 0.f : s;                      // -0 and +0 tie: one key, so the item id decides
-                    const unsigned long long key =
-                        ((unsigned long long)f2ord(__float_as_uint(s)) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)j);
+                    const float s = ft_score(v[i], a.col_bias, j, in, rb);
+                    const unsigned long long key = ft_key(s, j);
                     if (s > thr && in) q[(nc++) * FT_M] = key;
                 }
                 // Pass 2: in id order, against the threshold as it rises (a key compare: a later id that ties loses)
                 for (int c = 0; c < nc; ++c) {
                     const unsigned long long key = q[c * FT_M];
                     if (cnt == k && key <= root) continue;
-                    const int64_t j = (int64_t)(0xFFFFFFFFu - (uint32_t)key);
+                    const int64_t j = key_item(key);
                     while (enext < j) enext = ++ep < ehi ? __ldg(a.excl_idx + ep) : INT64_MAX;
                     if (enext == j) continue;
                     if (cnt < k) {
@@ -353,12 +238,7 @@ __global__ void __launch_bounds__(FT_THREADS, 1) factor_topk_kernel(const FtArgs
             }
         }
     }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == FT_MMA_WARP) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 512);
-    }
+    ft_teardown(tmem_base);
 }
 
 // one thread per row: merge the S descending key lists of the row into the final k
@@ -380,8 +260,20 @@ __global__ void factor_topk_merge_kernel(const unsigned long long* __restrict__ 
         }
         if (bs >= 0) ++pos[bs];
         out_scores[row * k + o] = best ? key_score(best) : -INFINITY;
-        out_items[row * k + o] = best ? (int64_t)(0xFFFFFFFFu - (uint32_t)(best & 0xFFFFFFFFull)) : -1;
+        out_items[row * k + o] = best ? key_item(best) : -1;
     }
+}
+
+int ft_stage(const float* A, int64_t n_rows, const float* B, int64_t n_items, int64_t dim, const FtGemm& g, uint8_t* ws,
+             cudaStream_t s) {
+    const int64_t a_chunks = g.rt * FT_M * (6 * g.dimp / 8), b_chunks = g.it * FT_N * (6 * g.dimp / 8);
+    factor_split_kernel<<<(unsigned)std::min<int64_t>((a_chunks + 255) / 256, 65535), 256, 0, s>>>(
+        A, n_rows, dim, g.dimp, g.nq, FT_M, 0, g.rt * FT_M, reinterpret_cast<__nv_bfloat16*>(ws));
+    RBR_LAUNCH_CHECK("factor_split_kernel(A)");
+    factor_split_kernel<<<(unsigned)std::min<int64_t>((b_chunks + 255) / 256, 65535), 256, 0, s>>>(
+        B, n_items, dim, g.dimp, g.nq, FT_N, 1, g.it * FT_N, reinterpret_cast<__nv_bfloat16*>(ws + g.off_b));
+    RBR_LAUNCH_CHECK("factor_split_kernel(B)");
+    return RBR_OK;
 }
 
 }  // namespace rbr
@@ -421,24 +313,19 @@ extern "C" int rbr_factor_topk(const float* A, const float* row_bias, int64_t n_
     cudaStream_t s = as_stream(stream);
     uint8_t* w = reinterpret_cast<uint8_t*>(ws);
     __nv_bfloat16* asp = reinterpret_cast<__nv_bfloat16*>(w);
-    __nv_bfloat16* bsp = reinterpret_cast<__nv_bfloat16*>(w + p.off_b);
+    __nv_bfloat16* bsp = reinterpret_cast<__nv_bfloat16*>(w + p.g.off_b);
     unsigned long long* part = reinterpret_cast<unsigned long long*>(w + p.off_part);
 
-    const int64_t a_chunks = p.rt * FT_M * (6 * p.dimp / 8), b_chunks = p.it * FT_N * (6 * p.dimp / 8);
-    factor_split_kernel<<<(unsigned)std::min<int64_t>((a_chunks + 255) / 256, 65535), 256, 0, s>>>(
-        A, n_rows, dim, p.dimp, p.nq, FT_M, 0, p.rt * FT_M, asp);
-    RBR_LAUNCH_CHECK("factor_split_kernel(A)");
-    factor_split_kernel<<<(unsigned)std::min<int64_t>((b_chunks + 255) / 256, 65535), 256, 0, s>>>(
-        B, n_items, dim, p.dimp, p.nq, FT_N, 1, p.it * FT_N, bsp);
-    RBR_LAUNCH_CHECK("factor_split_kernel(B)");
+    const int rc = ft_stage(A, n_rows, B, n_items, dim, p.g, w, s);
+    if (rc != RBR_OK) return rc;
 
     RBR_CUDA(cudaFuncSetAttribute(factor_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, p.smem));
     FtArgs a;
     a.a_split = asp; a.b_split = bsp; a.row_bias = row_bias; a.col_bias = col_bias;
     a.excl_ptr = excl_ptr; a.excl_idx = excl_idx; a.part = part;
-    a.n_rows = n_rows; a.n_items = n_items; a.nq = p.nq; a.it = p.it; a.S = p.S; a.tps = p.tps;
+    a.n_rows = n_rows; a.n_items = n_items; a.nq = p.g.nq; a.it = p.g.it; a.S = p.S; a.tps = p.tps;
     a.k = (int)k; a.nst = p.nst; a.heap_smem = p.heap_smem;
-    factor_topk_kernel<<<dim3((unsigned)p.rt, (unsigned)p.S), FT_THREADS, p.smem, s>>>(a);
+    factor_topk_kernel<<<dim3((unsigned)p.g.rt, (unsigned)p.S), FT_THREADS, p.smem, s>>>(a);
     RBR_LAUNCH_CHECK("factor_topk_kernel");
     factor_topk_merge_kernel<<<(unsigned)((n_rows + 127) / 128), 128, 0, s>>>(part, n_rows, (int)p.S, (int)k, out_scores, out_items);
     RBR_LAUNCH_CHECK("factor_topk_merge_kernel");

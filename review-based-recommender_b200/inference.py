@@ -13,7 +13,8 @@ encoder work.  In eval mode every model puts an entity's side through that entit
   D-ATT     fc(encode(document)) per side → [U, 50] / [I, 50]; a pair's score is the dot product of its two rows.
 
 `PairScorer.recommend` answers "the k best items for these users out of the whole catalogue" with K10 (ops.factor_topk),
-which never materialises the users x items score matrix.  The FM head factorises exactly:
+which never materialises the users x items score matrix; `rank_items` / `evaluate` give the exact full-catalogue rank of
+held-out items and HR@k / Recall@k / NDCG@k / MRR / AUC from it with K11 (ops.factor_rank), on the same scores.  The FM head factorises exactly:
   relu(u*i) = relu(u)*relu(i) + relu(-u)*relu(-i)   ⇒   score(u,i) = A[u] . B[i] + row_bias[u] + col_bias[i]
 with A = [h*relu(u_lat), h*relu(-u_lat)], B = [relu(i_lat), relu(-i_lat)], row_bias = ub + g, col_bias = ib (fm_factors);
 D-ATT's score is already a dot product of the two FC outputs.
@@ -169,6 +170,12 @@ class PairScorer:
         exclude_padding drops the item padding row (fm.item_padding_idx; 0 for D-ATT).
         Returns (scores [len(u_ids), k] fp32, items [len(u_ids), k] int64); rows with fewer than k eligible items end in
         (-inf, -1).  Scores agree with score_cached on the same pairs to fp32 rounding."""
+        A_rows, rb_rows, B, cb, _ = self._user_rows(u_ids, exclude_padding)
+        return ops.factor_topk(A_rows, rb_rows, B, cb, k, exclude=exclude)
+
+    def _user_rows(self, u_ids: torch.Tensor, exclude_padding: bool):
+        """(A rows, row_bias rows, B, col_bias, padding item or None) for users u_ids under the current head parameters;
+        with exclude_padding the padding item's column bias is -inf, so it never enters a top-k nor counts in a rank."""
         self.model.eval()
         A, rb, B, cb = self.factors()
         u_ids = u_ids.to(device=A.device, dtype=torch.int64).reshape(-1)
@@ -176,10 +183,106 @@ class PairScorer:
             raise ValueError(f"user ids must lie in [0, {A.shape[0]})")
         A_rows = A.index_select(0, u_ids)
         rb_rows = None if rb is None else rb.index_select(0, u_ids)
+        pad = None
         if exclude_padding:
             pad = 0 if _is_datt(self.model) else self.model.fm.item_padding_idx
             if pad is not None and 0 <= pad < B.shape[0]:
                 # a -inf column bias: the padding item's score never beats a threshold, so it is never returned
                 cb = torch.zeros(B.shape[0], dtype=torch.float32, device=B.device) if cb is None else cb.clone()
                 cb[pad] = float("-inf")
-        return ops.factor_topk(A_rows, rb_rows, B, cb, k, exclude=exclude)
+            else:
+                pad = None
+        return A_rows, rb_rows, B, cb, pad
+
+    @torch.no_grad()
+    def rank_items(self, u_ids: torch.Tensor, targets: Tuple[torch.Tensor, torch.Tensor],
+                   exclude: Optional[Tuple[torch.Tensor, torch.Tensor]] = None, exclude_padding: bool = True
+                   ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """The exact full-catalogue rank of each target item for user u_ids[r] (K11, ops.factor_rank): 1 + the number of
+        eligible items ahead of it by (score desc, item id asc), i.e. its 1-based position in recommend(k = inf).
+        targets = (indptr [len(u_ids) + 1], indices) int64 CUDA CSR, e.g. each user's held-out items; exclude as for
+        recommend, e.g. the items the user rated in training.  exclude_padding leaves the item padding row out of every
+        count (a target that is the padding item then raises ValueError).
+        Returns (ranks int64 [nnz], scores fp32 [nnz], both in the order of `indices` — rank -1 for a NaN / -inf score —,
+        n_candidates int64 [len(u_ids)]: the eligible items per row, the padding item not counted).  A target with
+        rank <= k is in recommend(u_ids, k) at position rank - 1 with the identical score."""
+        A_rows, rb_rows, B, cb, pad = self._user_rows(u_ids, exclude_padding)
+        if pad is not None:
+            t_idx = targets[1]
+            if bool((t_idx == pad).any()):
+                raise ValueError(f"target item {pad} is the padding item, which exclude_padding=True leaves out")
+        ranks, scores, n_cand = ops.factor_rank(A_rows, rb_rows, B, cb, targets, exclude=exclude)
+        if pad is not None:
+            pad_listed = torch.zeros(A_rows.shape[0], dtype=torch.bool, device=A_rows.device)
+            if exclude is not None:
+                e_ptr, e_idx = exclude
+                rows = torch.repeat_interleave(torch.arange(A_rows.shape[0], device=e_ptr.device), e_ptr[1:] - e_ptr[:-1])
+                pad_listed[rows[e_idx == pad]] = True
+            n_cand = n_cand - (~pad_listed).long()
+        return ranks, scores, n_cand
+
+    @torch.no_grad()
+    def evaluate(self, u_ids: torch.Tensor, targets: Tuple[torch.Tensor, torch.Tensor], ks=(10,),
+                 exclude: Optional[Tuple[torch.Tensor, torch.Tensor]] = None, exclude_padding: bool = True) -> dict:
+        """Full-catalogue ranking metrics of the held-out `targets` (rank_items, then ranking_metrics): hr@k, recall@k and
+        ndcg@k for each k in ks, mrr, auc and n_rows, averaged over the rows that have at least one target."""
+        ranks, _, n_cand = self.rank_items(u_ids, targets, exclude=exclude, exclude_padding=exclude_padding)
+        return ranking_metrics(ranks, targets[0], n_cand, ks)
+
+
+def ranking_metrics(ranks: torch.Tensor, indptr: torch.Tensor, n_candidates: torch.Tensor, ks=(10,)) -> dict:
+    """Binary-relevance ranking metrics from full-catalogue ranks (any device, no GPU needed).
+
+    ranks [nnz]: the 1-based rank of each target among its row's n_candidates eligible items, -1 for a target that cannot
+    be ranked (NaN / -inf score); row r's targets are ranks[indptr[r] : indptr[r+1]], m = their number.  Per row:
+      hr@k      1 if the row's best rank <= k, else 0
+      recall@k  hits@k / m
+      ndcg@k    sum over hits of 1 / log2(rank + 1), divided by sum_{j=1..min(m, k)} 1 / log2(j + 1)
+      mrr       1 / best rank (0 when no target has a rank)
+      auc       mean over the row's targets of 1 - (negatives above t) / (n_candidates - m), where negatives above t =
+                rank(t) - 1 - (other targets above t); a rank -1 target is below every negative (its term is 0)
+    Each metric is the mean over rows with m >= 1 (n_rows of them); auc leaves out rows with n_candidates == m."""
+    ranks = ranks.reshape(-1).to(torch.int64)
+    dev = ranks.device
+    indptr = indptr.to(device=dev, dtype=torch.int64)
+    n_cand = n_candidates.to(device=dev, dtype=torch.int64).reshape(-1)
+    n = indptr.numel() - 1
+    m = indptr[1:] - indptr[:-1]
+    rows = torch.repeat_interleave(torch.arange(n, device=dev), m)
+    has = m > 0
+    n_rows = int(has.sum())
+    out = {}
+    valid = ranks > 0
+    r = ranks.double()
+
+    def row_sum(x):
+        return torch.zeros(n, dtype=torch.float64, device=dev).index_add_(0, rows, x.double())
+
+    def mean(x, sel):
+        return float(x[sel].mean()) if bool(sel.any()) else 0.0
+
+    inf = float("inf")
+    best = torch.full((n,), inf, dtype=torch.float64, device=dev).scatter_reduce(
+        0, rows, torch.where(valid, r, torch.full_like(r, inf)), "amin")
+    max_m = int(m.max()) if n else 0
+    for k in ks:
+        hit = valid & (ranks <= k)
+        disc = 1.0 / torch.log2(torch.arange(2, max(min(max_m, k), 1) + 2, dtype=torch.float64, device=dev))
+        idcg = torch.cumsum(disc, 0)[(torch.clamp(m, max=k) - 1).clamp_min(0)]
+        out[f"hr@{k}"] = mean((best <= k).double(), has)
+        out[f"recall@{k}"] = mean(row_sum(hit) / m.clamp_min(1), has)
+        out[f"ndcg@{k}"] = mean(row_sum(torch.where(hit, 1.0 / torch.log2(r + 1), torch.zeros_like(r))) / idcg, has)
+    out["mrr"] = mean(1.0 / best, has)                                  # 1 / inf = 0 for rows without a ranked target
+    # other targets of the row above t: its position among the row's ranked targets (ranks within a row are distinct)
+    vrow = rows[valid]
+    order = torch.argsort(vrow * (int(ranks.max()) + 1) + ranks[valid]) if vrow.numel() else vrow
+    vcount = torch.bincount(vrow, minlength=n)
+    vstart = torch.cumsum(vcount, 0) - vcount
+    above = torch.empty_like(vrow)
+    above[order] = torch.arange(vrow.numel(), device=dev) - vstart[vrow[order]]
+    neg = (n_cand - m).double()
+    term = torch.zeros_like(r)
+    term[valid] = 1.0 - (r[valid] - 1 - above.double()) / neg[vrow].clamp_min(1)
+    out["auc"] = mean(row_sum(term) / m.clamp_min(1), has & (n_cand > m))
+    out["n_rows"] = n_rows
+    return out

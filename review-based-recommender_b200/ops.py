@@ -1006,28 +1006,78 @@ class DattEncodeFn(torch.autograd.Function):
 FACTOR_TOPK_MAX_K, FACTOR_TOPK_MAX_DIM = 256, 512
 
 
+def _csr_keys(indptr: torch.Tensor, indices: torch.Tensor, n_rows: int, n_items: int, what: str
+              ) -> Tuple[torch.Tensor, torch.Tensor, int]:
+    """Validates a CSR of item lists (what: "exclusion" / "target") → (row of each entry, row * n_items + item per entry,
+    longest row).  Ids outside [0, n_items) and a malformed indptr raise ValueError."""
+    if indptr.dtype != torch.int64 or indices.dtype != torch.int64:
+        raise ValueError(f"rbr_b200: {what} indptr / indices must be int64")
+    if indptr.dim() != 1 or indptr.numel() != n_rows + 1 or indices.dim() != 1:
+        raise ValueError(f"rbr_b200: {what} indptr must be [n_rows + 1] = [{n_rows + 1}] and indices 1-D")
+    counts = indptr[1:] - indptr[:-1]
+    lo_hi = torch.stack([indices.min(), indices.max()]) if indices.numel() else indptr.new_zeros(2)
+    longest = counts.max().view(1) if n_rows else indptr.new_zeros(1)
+    # one device-to-host read for every check
+    first, last, neg, lo, hi, longest = torch.cat([indptr[:1], indptr[-1:], (counts < 0).any().view(1).long(), lo_hi,
+                                                   longest]).tolist()
+    if first != 0 or last != indices.numel() or neg:
+        raise ValueError(f"rbr_b200: {what} indptr must start at 0, be non-decreasing and end at len(indices)")
+    if lo < 0 or hi >= n_items:
+        raise ValueError(f"rbr_b200: {what} item ids must lie in [0, {n_items})")
+    rows = torch.repeat_interleave(torch.arange(n_rows, device=indices.device), counts)
+    return rows, rows * n_items + indices, int(longest)
+
+
 def normalize_exclusions(indptr: torch.Tensor, indices: torch.Tensor, n_rows: int, n_items: int
                          ) -> Tuple[torch.Tensor, torch.Tensor]:
     """CSR exclusion lists (row r excludes indices[indptr[r]:indptr[r+1]], in any order, duplicates allowed) → the same
     lists sorted ascending without duplicates, as rbr_factor_topk reads them.  Ids outside [0, n_items) raise ValueError."""
-    if indptr.dtype != torch.int64 or indices.dtype != torch.int64:
-        raise ValueError("rbr_b200: exclusion indptr / indices must be int64")
-    if indptr.dim() != 1 or indptr.numel() != n_rows + 1 or indices.dim() != 1:
-        raise ValueError(f"rbr_b200: exclusion indptr must be [n_rows + 1] = [{n_rows + 1}] and indices 1-D")
-    counts = indptr[1:] - indptr[:-1]
-    lo_hi = torch.stack([indices.min(), indices.max()]) if indices.numel() else indptr.new_zeros(2)
-    # one device-to-host read for every check
-    first, last, neg, lo, hi = torch.cat([indptr[:1], indptr[-1:], (counts < 0).any().view(1).long(), lo_hi]).tolist()
-    if first != 0 or last != indices.numel() or neg:
-        raise ValueError("rbr_b200: exclusion indptr must start at 0, be non-decreasing and end at len(indices)")
-    if lo < 0 or hi >= n_items:
-        raise ValueError(f"rbr_b200: excluded item ids must lie in [0, {n_items})")
-    rows = torch.repeat_interleave(torch.arange(n_rows, device=indices.device), counts)
-    keys = torch.unique(rows * n_items + indices, sorted=True)
+    _, keys, _ = _csr_keys(indptr, indices, n_rows, n_items, "exclusion")
+    keys = torch.unique(keys, sorted=True)
     new_counts = torch.bincount(torch.div(keys, n_items, rounding_mode="floor"), minlength=n_rows)
     ptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=indices.device)
     torch.cumsum(new_counts, 0, out=ptr[1:])
     return ptr, keys % n_items
+
+
+def _check_factors(A: torch.Tensor, row_bias: Optional[torch.Tensor], B: torch.Tensor, col_bias: Optional[torch.Tensor]
+                   ) -> Tuple[int, int, int]:
+    """Validates the factor operands of K10 / K11 → (n_rows, n_items, dim)."""
+    for t, name in ((A, "A"), (B, "B"), (row_bias, "row_bias"), (col_bias, "col_bias")):
+        if t is None:
+            continue
+        if not isinstance(t, torch.Tensor) or not t.is_cuda:
+            raise RuntimeError(f"rbr_b200: `{name}` must be a CUDA tensor (the hot path has no CPU implementation)")
+        if t.dtype != torch.float32:
+            raise ValueError(f"rbr_b200: `{name}` must be float32, got {t.dtype}")
+        if t.device != A.device:
+            raise ValueError(f"rbr_b200: `{name}` is on {t.device}, A on {A.device}")
+    if A.dim() != 2 or B.dim() != 2 or A.shape[1] != B.shape[1]:
+        raise ValueError(f"rbr_b200: A [n_rows, dim] and B [n_items, dim] must share dim, got {tuple(A.shape)} / {tuple(B.shape)}")
+    n_rows, dim = A.shape
+    n_items = B.shape[0]
+    if row_bias is not None and row_bias.numel() != n_rows:
+        raise ValueError("rbr_b200: row_bias must hold n_rows values")
+    if col_bias is not None and col_bias.numel() != n_items:
+        raise ValueError("rbr_b200: col_bias must hold n_items values")
+    return n_rows, n_items, dim
+
+
+def _cuda_csr(csr: Tuple[torch.Tensor, torch.Tensor], what: str) -> Tuple[torch.Tensor, torch.Tensor]:
+    indptr, indices = csr
+    for t, name in ((indptr, f"{what} indptr"), (indices, f"{what} indices")):
+        if not isinstance(t, torch.Tensor) or not t.is_cuda:
+            raise RuntimeError(f"rbr_b200: `{name}` must be a CUDA tensor")
+    return indptr.contiguous(), indices.contiguous()
+
+
+def _exclusions(exclude: Optional[Tuple[torch.Tensor, torch.Tensor]], n_rows: int, n_items: int
+                ) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """Normalised exclusion CSR, or (None, None) when nothing is excluded."""
+    if exclude is None:
+        return None, None
+    ptr, idx = normalize_exclusions(*_cuda_csr(exclude, "exclude"), n_rows, n_items)
+    return (None, None) if idx.numel() == 0 else (ptr, idx)
 
 
 def factor_topk_workspace_bytes(n_rows: int, n_items: int, dim: int, k: int) -> int:
@@ -1049,34 +1099,10 @@ def factor_topk(A: torch.Tensor, row_bias: Optional[torch.Tensor], B: torch.Tens
     """K10: for each row r, the k items i (excluding exclude = (indptr [n_rows+1], indices) CSR lists) with the largest
     score A[r] . B[i] + row_bias[r] + col_bias[i], by score descending then item id ascending; fp32-grade scores.
     Returns (scores [n_rows, k] fp32, items [n_rows, k] int64); slots past the eligible items hold (-inf, -1)."""
-    for t, name in ((A, "A"), (B, "B"), (row_bias, "row_bias"), (col_bias, "col_bias")):
-        if t is None:
-            continue
-        if not isinstance(t, torch.Tensor) or not t.is_cuda:
-            raise RuntimeError(f"rbr_b200: `{name}` must be a CUDA tensor (the hot path has no CPU implementation)")
-        if t.dtype != torch.float32:
-            raise ValueError(f"rbr_b200: `{name}` must be float32, got {t.dtype}")
-        if t.device != A.device:
-            raise ValueError(f"rbr_b200: `{name}` is on {t.device}, A on {A.device}")
-    if A.dim() != 2 or B.dim() != 2 or A.shape[1] != B.shape[1]:
-        raise ValueError(f"rbr_b200: A [n_rows, dim] and B [n_items, dim] must share dim, got {tuple(A.shape)} / {tuple(B.shape)}")
-    n_rows, dim = A.shape
-    n_items = B.shape[0]
+    n_rows, n_items, dim = _check_factors(A, row_bias, B, col_bias)
     k = int(k)
-    if row_bias is not None and row_bias.numel() != n_rows:
-        raise ValueError("rbr_b200: row_bias must hold n_rows values")
-    if col_bias is not None and col_bias.numel() != n_items:
-        raise ValueError("rbr_b200: col_bias must hold n_items values")
     ws_bytes = factor_topk_workspace_bytes(n_rows, n_items, dim, k)
-    ptr = idx = None
-    if exclude is not None:
-        indptr, indices = exclude
-        for t, name in ((indptr, "exclude indptr"), (indices, "exclude indices")):
-            if not isinstance(t, torch.Tensor) or not t.is_cuda:
-                raise RuntimeError(f"rbr_b200: `{name}` must be a CUDA tensor")
-        ptr, idx = normalize_exclusions(indptr.contiguous(), indices.contiguous(), n_rows, n_items)
-        if idx.numel() == 0:
-            ptr = idx = None
+    ptr, idx = _exclusions(exclude, n_rows, n_items)
     A, B = A.contiguous(), B.contiguous()
     rb = None if row_bias is None else row_bias.contiguous().view(-1)
     cb = None if col_bias is None else col_bias.contiguous().view(-1)
@@ -1089,3 +1115,123 @@ def factor_topk(A: torch.Tensor, row_bias: Optional[torch.Tensor], B: torch.Tens
         lib.check(lib.rbr_factor_topk(_p(A), _p(rb), n_rows, _p(B), _p(cb), n_items, dim, _p(ptr), _p(idx), k, _p(scores),
                                       _p(items), _p(ws), ws_bytes, _stream(True)), "rbr_factor_topk")
     return scores, items
+
+
+# ---------------------------------------------------------------------------------------------------
+# K11: exact full-catalogue rank of target items under a factorised score matrix (evaluation)
+# ---------------------------------------------------------------------------------------------------
+FACTOR_RANK_MAX_TARGETS = 64
+
+
+def factor_rank_workspace_bytes(n_rows: int, n_items: int, dim: int, n_targets: int, max_targets: int) -> int:
+    n = lib.rbr_factor_rank_workspace_bytes(n_rows, n_items, dim, n_targets, max_targets)
+    if n < 0:
+        raise ValueError(f"rbr_b200: factor_rank does not take n_items={n_items}, dim={dim}, max_targets={max_targets} "
+                         f"(1 <= dim <= {FACTOR_TOPK_MAX_DIM}, 1 <= n_items < 2^31, "
+                         f"1 <= max_targets <= {FACTOR_RANK_MAX_TARGETS})")
+    return int(n)
+
+
+def split_target_rows(counts: torch.Tensor, cap: int = FACTOR_RANK_MAX_TARGETS) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Cuts rows holding `counts` targets each into pieces of at most `cap` consecutive targets; rows without targets get no
+    piece.  Returns (row of each piece, piece indptr into the rows' concatenated target lists).  A piece is ranked as a row
+    of its own with its row's factors and exclusions: exact, since the row's targets in other pieces are ordinary items."""
+    counts = counts.to(torch.int64)
+    n_pieces = torch.div(counts + cap - 1, cap, rounding_mode="floor")
+    piece_row = torch.repeat_interleave(torch.arange(counts.numel(), device=counts.device), n_pieces)
+    first = torch.zeros(counts.numel() + 1, dtype=torch.int64, device=counts.device)
+    torch.cumsum(n_pieces, 0, out=first[1:])                   # first piece of each row
+    start = torch.zeros_like(first)
+    torch.cumsum(counts, 0, out=start[1:])                     # first target of each row
+    k = torch.arange(piece_row.numel(), device=counts.device) - first[piece_row]
+    # pieces tile the target lists in order, so each piece starts where the previous one ends
+    hi = torch.minimum(start[piece_row] + (k + 1) * cap, start[piece_row + 1])
+    return piece_row, torch.cat([hi.new_zeros(1), hi])
+
+
+def gather_csr_rows(indptr: torch.Tensor, indices: torch.Tensor, rows: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """CSR whose row p is row rows[p] of (indptr, indices)."""
+    counts = indptr[1:] - indptr[:-1]
+    c = counts[rows]
+    ptr = torch.zeros(rows.numel() + 1, dtype=torch.int64, device=indptr.device)
+    torch.cumsum(c, 0, out=ptr[1:])
+    within = torch.arange(int(ptr[-1]), device=indptr.device) - torch.repeat_interleave(ptr[:-1], c)
+    return ptr, indices[torch.repeat_interleave(indptr[:-1][rows], c) + within]
+
+
+def rank_inputs(t_ptr: torch.Tensor, t_idx: torch.Tensor, n_rows: int, n_items: int,
+                exclude: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> dict:
+    """Host side of factor_rank (any device): validates the target CSR against the exclusions and lays it out as
+    rbr_factor_rank reads it.  Raises ValueError for a target id outside [0, n_items), a target listed twice in its row
+    and a target in its row's exclusion list.  Returns a dict:
+      order         [nnz]: caller position of each target in the kernel's order (rows ascending, ids ascending)
+      targets       [nnz]: the target ids in the kernel's order
+      piece_row, piece_ptr, max_targets: rows of at most FACTOR_RANK_MAX_TARGETS targets (split_target_rows)
+      excl_ptr, excl_idx: the normalised exclusions of each piece's row (None when nothing is excluded)
+      n_candidates  [n_rows]: n_items minus the row's distinct excluded items"""
+    _, keys, longest = _csr_keys(t_ptr, t_idx, n_rows, n_items, "target")
+    dev = t_idx.device
+    ptr = idx = None
+    if exclude is not None:
+        ptr, idx = normalize_exclusions(exclude[0], exclude[1], n_rows, n_items)
+    n_excl = torch.zeros(n_rows, dtype=torch.int64, device=dev) if ptr is None else ptr[1:] - ptr[:-1]
+    sorted_keys, order = torch.sort(keys)
+    checks = [(sorted_keys[1:] == sorted_keys[:-1]).any()]
+    if idx is not None and idx.numel() and sorted_keys.numel():
+        excl_keys = torch.repeat_interleave(torch.arange(n_rows, device=dev), n_excl) * n_items + idx     # ascending
+        pos = torch.searchsorted(excl_keys, sorted_keys).clamp_max(excl_keys.numel() - 1)
+        checks.append((excl_keys[pos] == sorted_keys).any())
+    dup, *overlap = torch.stack(checks).tolist()
+    if dup:
+        raise ValueError("rbr_b200: a target is listed twice in its row")
+    if overlap and overlap[0]:
+        raise ValueError("rbr_b200: a target is also in its row's exclusion list")
+    # rows without targets are not scanned; longer rows become several pieces
+    piece_row, piece_ptr = split_target_rows(t_ptr[1:] - t_ptr[:-1])
+    e_ptr = e_idx = None
+    if idx is not None and idx.numel():
+        e_ptr, e_idx = gather_csr_rows(ptr, idx, piece_row)
+        if e_idx.numel() == 0:
+            e_ptr = e_idx = None
+    return {"order": order, "targets": sorted_keys % n_items, "piece_row": piece_row, "piece_ptr": piece_ptr,
+            "max_targets": max(1, min(longest, FACTOR_RANK_MAX_TARGETS)), "excl_ptr": e_ptr, "excl_idx": e_idx,
+            "n_candidates": n_items - n_excl}
+
+
+def factor_rank(A: torch.Tensor, row_bias: Optional[torch.Tensor], B: torch.Tensor, col_bias: Optional[torch.Tensor],
+                targets: Tuple[torch.Tensor, torch.Tensor], exclude: Optional[Tuple[torch.Tensor, torch.Tensor]] = None
+                ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """K11: the exact rank of each target item among all eligible items of its row, under factor_topk's score and order.
+
+    targets = (indptr [n_rows+1], indices) int64 CUDA CSR: row r's targets, in any order, without duplicates, none of them
+    in the row's exclusion list (exclude, as for factor_topk: any order, duplicates allowed).
+    rank = #{ eligible i : (score_i, -i) >= (score_t, -t) }, 1-based: the position + 1 that t takes in factor_topk(k = inf).
+    Other targets of the row count as ordinary competitors; NaN and -inf scores never count; a target whose own score is
+    NaN or -inf gets rank -1.  Returns (ranks int64 [nnz], scores fp32 [nnz], both in the order of `indices`,
+    n_candidates int64 [n_rows] = n_items minus the row's distinct excluded items)."""
+    n_rows, n_items, dim = _check_factors(A, row_bias, B, col_bias)
+    factor_rank_workspace_bytes(n_rows, n_items, dim, 0, 1)             # the shape limits, before any device work
+    t_ptr, t_idx = _cuda_csr(targets, "targets")
+    plan = rank_inputs(t_ptr, t_idx, n_rows, n_items, None if exclude is None else _cuda_csr(exclude, "exclude"))
+    dev = A.device
+    nnz = t_idx.numel()
+    ranks = torch.empty(nnz, dtype=torch.int64, device=dev)
+    scores = torch.empty(nnz, dtype=torch.float32, device=dev)
+    if nnz == 0:
+        return ranks, scores, plan["n_candidates"]
+    piece_row = plan["piece_row"]
+    n_pieces, mt = piece_row.numel(), plan["max_targets"]
+    A_p = A.contiguous().index_select(0, piece_row)
+    rb_p = None if row_bias is None else row_bias.contiguous().view(-1).index_select(0, piece_row)
+    cb = None if col_bias is None else col_bias.contiguous().view(-1)
+    ws_bytes = factor_rank_workspace_bytes(n_pieces, n_items, dim, nnz, mt)
+    r_sorted = torch.empty(nnz, dtype=torch.int64, device=dev)
+    s_sorted = torch.empty(nnz, dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        lib.check(lib.rbr_factor_rank(_p(A_p), _p(rb_p), n_pieces, _p(B.contiguous()), _p(cb), n_items, dim,
+                                      _p(plan["excl_ptr"]), _p(plan["excl_idx"]), _p(plan["piece_ptr"]), _p(plan["targets"]),
+                                      nnz, mt, _p(r_sorted), _p(s_sorted), _p(ws), ws_bytes, _stream(True)), "rbr_factor_rank")
+    ranks[plan["order"]] = r_sorted
+    scores[plan["order"]] = s_sorted
+    return ranks, scores, plan["n_candidates"]
