@@ -175,8 +175,9 @@ int rbr_conv_act_maxpool_bwd(int precision, int activation, const void* table, c
  * 2 = table gradient, 4 = weight gradient — data-parallel training runs 1|2, starts the table all-reduce, then 4; 8 (with 2) =
  * the table gradient is OVERWRITTEN (every row and column is written, the padding row with zeros) instead of accumulated
  * into: the caller then need not zero-fill table_grad, and the epilogue stores without reading (halves its HBM traffic).
- * Shapes: emb % 4 == 0, emb <= 512, vocab * round_up(filters*ksize, 64) * 4 bytes <= 3 GiB, no gate
- * (rbr_conv_bwd_cmat_supported; otherwise use K2b).                                                                     */
+ * Shapes: emb % 4 == 0, emb <= 448 (the weight GEMM's shared-memory ring outgrows 227 KB at rbr_emb_pad(emb) = 512),
+ * filters <= 1024, ksize <= 8, round_up(filters*ksize, 64) <= 4096, vocab * round_up(filters*ksize, 64) * 4 bytes <= 3 GiB,
+ * no gate (rbr_conv_bwd_cmat_supported; otherwise use K2b).                                                             */
 int rbr_conv_bwd_cmat_supported(int64_t vocab, int64_t emb, int64_t filters, int64_t ksize);
 int64_t rbr_conv_bwd_cmat_workspace_bytes(int64_t vocab, int64_t emb, int64_t filters, int64_t ksize);
 int rbr_conv_bwd_cmat_chunks(int64_t vocab, int64_t emb, int64_t filters, int64_t ksize);

@@ -20,7 +20,7 @@
 //
 // Pipeline (all on the caller's stream):
 //   cmat_scatter_kernel      per document side: C32[v][hj] += g (red.global.add.f32), bias_grad[h] += g
-//   cmat_split_kernel        C32 → Chl = [hi | lo] bf16, and C32 re-zeroed (the workspace stays clean for the next step)
+//   cmat_split_kernel        C32 → Chl = [hi | lo] bf16 (each C32 block is zero-filled by rbr_conv_bwd_cmat_begin before its scatter)
 //   cmat_table_gemm_kernel   D[128 tokens x 160] = Chl[128 x 2HJp] · Wt2ᵀ   — A, B K-major SWIZZLE_128B via TMA, cta_group::1,
 //                            2 CTAs/SM; epilogue adds the tile into table_grad (the padding row is skipped)
 //   cmat_weight_gemm_kernel  D[128 hj x emb_pad] = sum over a slice of the vocabulary of Chlᵀ · x   — both operands MN-MAJOR
@@ -493,9 +493,27 @@ __global__ void cmat_unpack_kernel(float* __restrict__ dw_hke, int H, int E, int
     }
 }
 
+// Dynamic shared memory of the two GEMMs of rbr_conv_bwd_cmat_finish (rings + barriers + TMEM slot + 1024-byte alignment slack),
+// and the most each may take.  cmat_shape_ok declines a shape that exceeds either, so "supported" means "finish will run": the
+// weight GEMM's ring grows with the embedding width (emb_pad 512 needs 240 KB) and such shapes go to the sparse backward instead.
+constexpr int CM_SMEM_T_MAX = 116 * 1024;  // two table-GEMM CTAs per SM
+constexpr int CM_SMEM_W_MAX = 227 * 1024;
+struct CmatSmem { int table, weight; };
+static CmatSmem cmat_smem(int64_t emb) {
+    int64_t NT, tiles;
+    cmat_ntile(emb, &NT, &tiles);
+    const int64_t nch = rbr_emb_pad(emb) / 64;
+    CmatSmem s;
+    s.table = CM_STAGES_T * (16384 + (int)NT * 128) + 8 * (2 * CM_STAGES_T + 1) + 16 + 1024;
+    s.weight = CM_STAGES_W * (2 + (int)nch) * 8192 + 8 * (2 * CM_STAGES_W + 1) + 16 + 1024;
+    return s;
+}
+
 static bool cmat_shape_ok(int64_t vocab, int64_t emb, int64_t filters, int64_t ksize) {
     if (vocab < 1 || vocab >= (1ll << 31) || emb < 4 || emb % 4 != 0 || emb > 512 || filters < 1 || ksize < 1 || ksize > 8) return false;
     if (filters > 1024) return false;
+    const CmatSmem sm = cmat_smem(emb);
+    if (sm.table > CM_SMEM_T_MAX || sm.weight > CM_SMEM_W_MAX) return false;
     const int64_t hjp = cmat_hjp(filters, ksize);
     if (hjp > 4096) return false;
     return vocab * hjp * 4 <= (3ll << 30);          // coefficient matrix up to 3 GiB (fp32) + the same again in bf16
@@ -660,13 +678,13 @@ extern "C" int rbr_conv_bwd_cmat_finish(int what, int chunk, int64_t row_lo, int
         RBR_REQUIRE(row_lo >= 0 && row_lo < row_hi && row_hi <= vocab && row_lo % 128 == 0 && (row_hi % 128 == 0 || row_hi == vocab), RBR_EINVAL,
                     "conv_bwd_cmat_finish: the table row range must be cut on multiples of 128 rows");
         a.tile0 = (int)(row_lo / 128);
-        const int smem = CM_STAGES_T * (16384 + (int)pl.NT * 128) + 8 * (2 * CM_STAGES_T + 1) + 16 + 1024;
+        const int smem = cmat_smem(emb).table;
         static bool attr = false;
         if (!attr) {
-            RBR_CUDA(cudaFuncSetAttribute(cmat_table_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 116 * 1024));
+            RBR_CUDA(cudaFuncSetAttribute(cmat_table_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_T_MAX));
             attr = true;
         }
-        RBR_REQUIRE(smem <= 116 * 1024, RBR_EUNSUPPORTED, "conv_bwd_cmat_finish: shared memory");
+        RBR_REQUIRE(smem <= CM_SMEM_T_MAX, RBR_EUNSUPPORTED, "conv_bwd_cmat_finish: shared memory");
         dim3 grid((unsigned)((row_hi - row_lo + 127) / 128), (unsigned)pl.n_tiles);
         cmat_table_gemm_kernel<<<grid, CM_THREADS, smem, s>>>(tmA, tmB, a);
         RBR_LAUNCH_CHECK("cmat_table_gemm_kernel");
@@ -690,13 +708,13 @@ extern "C" int rbr_conv_bwd_cmat_finish(int what, int chunk, int64_t row_lo, int
         a.ksplit = sms / m_tiles < 1 ? 1 : sms / m_tiles;
         if (a.ksplit > a.n_tb) a.ksplit = a.n_tb;
         a.dw_hke = dw;
-        const int smem = CM_STAGES_W * (2 + a.nch) * 8192 + 8 * (2 * CM_STAGES_W + 1) + 16 + 1024;
+        const int smem = cmat_smem(emb).weight;
         static bool attr = false;
         if (!attr) {
-            RBR_CUDA(cudaFuncSetAttribute(cmat_weight_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            RBR_CUDA(cudaFuncSetAttribute(cmat_weight_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_W_MAX));
             attr = true;
         }
-        RBR_REQUIRE(smem <= 227 * 1024, RBR_EUNSUPPORTED, "conv_bwd_cmat_finish: shared memory");
+        RBR_REQUIRE(smem <= CM_SMEM_W_MAX, RBR_EUNSUPPORTED, "conv_bwd_cmat_finish: shared memory");
         dim3 grid((unsigned)m_tiles, (unsigned)a.ksplit);
         cmat_weight_gemm_kernel<<<grid, CM_THREADS, smem, s>>>(tmA, tmX, a);
         RBR_LAUNCH_CHECK("cmat_weight_gemm_kernel");

@@ -321,6 +321,7 @@ class EncodeDocsFn(torch.autograd.Function):
         ctx.mask_present = [m is not None for m in mask_l]
         ctx.flags_l = flags_l
         ctx.mark_non_differentiable(*argmaxes)
+        ctx.set_materialize_grads(False)              # a side the loss does not use arrives as None and is skipped, not scattered as zeros
         return tuple(feats) + tuple(argmaxes)          # [n_docs, H] features per side, then the int32 arg-max positions
 
     @staticmethod
@@ -480,8 +481,9 @@ _CMAT_WS: Dict[tuple, torch.Tensor] = {}
 
 
 def _cmat_workspace(table: torch.Tensor, conv_index: int, vocab: int, emb: int, filters: int, ksize: int) -> torch.Tensor:
-    """Persistent, self-cleaning workspace of the dense tensor-core backward (K2c) for one (table, conv): zero-filled ONCE here;
-    rbr_conv_bwd_cmat_finish leaves it zeroed again, so steps — eager or CUDA-graph replays — never memset its 130-200 MB."""
+    """Persistent workspace of the dense tensor-core backward (K2c) for one (table, conv), allocated once per shape.  Only the
+    weight scratch is self-cleaning (the unpack kernel re-zeroes what it reads); each filter block of the coefficient matrix C32 is
+    zero-filled by rbr_conv_bwd_cmat_begin right before its scatter, while the block is about to be hot in L2."""
     key = (table.device.index, table.data_ptr(), conv_index, vocab, emb, filters, ksize)
     ws = _CMAT_WS.get(key)
     if ws is None:

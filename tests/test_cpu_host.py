@@ -317,6 +317,28 @@ def test_staged_inputs_wire_format_on_cpu():
     assert st.batch[2] is not None and st.batch[2].dtype == torch.uint8
 
 
+def test_conv_bwd_cmat_filter_blocks_and_declined_shapes():
+    """Filter blocks of the dense tensor-core backward's coefficient matrix (host code, no GPU): C32 = V x round_up(H k, 64) fp32 is
+    cut into ceil(bytes / 80 MiB) blocks (at most 16) of round_up(ceil(H / blocks), 4) filters.  tests/test_gpu_conv_bwd_variants.py
+    runs these shapes on the GPU.  Shapes the backward cannot finish get no workspace, and go to the sparse kernels."""
+    from rbr_b200._lib import lib
+    chunks, ws = lib.rbr_conv_bwd_cmat_chunks, lib.rbr_conv_bwd_cmat_workspace_bytes
+    assert chunks(327680, 64, 16, 4) == 1 and chunks(327681, 64, 16, 4) == 2          # C32 exactly 80 MiB, and one row more
+    for shape, n in {(3000, 300, 100, 3): 1, (60000, 300, 150, 3): 2, (100000, 100, 150, 3): 3, (350000, 64, 512, 4): 16,
+                     (200000, 64, 9, 8): 2, (400000, 64, 9, 4): 2, (2000, 32, 1024, 4): 1, (2000, 100, 820, 3): 1}.items():
+        assert chunks(*shape) == n, shape
+    rup = lambda x, m: (x + m - 1) // m * m
+    for V, E, H, k in ((350000, 64, 512, 4), (3000, 300, 100, 3), (1, 4, 1, 1), (1000, 448, 24, 3)):
+        hjp = rup(H * k, 64)                                           # C32 fp32 + [hi | lo] bf16 + the [H k][E] weight scratch
+        assert ws(V, E, H, k) == rup(V * hjp * 4, 1024) + rup(V * 2 * hjp * 2, 1024) + rup(H * k * rup(E, 4) * 4, 1024), (V, E, H, k)
+    # declined: E in (448, 512] (the weight GEMM's ring would need 240 KB of shared memory), E % 4, E > 512, k > 8, H > 1024,
+    # H k beyond 4096 columns, C32 over 3 GiB
+    for shape in ((5000, 452, 100, 3), (5000, 480, 100, 3), (5000, 512, 100, 3), (5000, 30, 100, 3), (5000, 516, 100, 3),
+                  (5000, 64, 100, 9), (5000, 64, 1025, 1), (5000, 64, 1024, 5), (2000, 100, 820, 5), (800000, 64, 1024, 1)):
+        assert ws(*shape) == 0 and chunks(*shape) == 0, shape
+    assert ws(5000, 448, 100, 3) > 0 and ws(5000, 444, 100, 3) > 0
+
+
 def test_narre_attn_pair_plan_boundary():
     """Which NARRE attention shapes the two-sided tensor-core kernel takes (host code, no GPU).  NARRE falls back to the per-side
     kernels outside this set, and test_attention_pair_tensor_core_kernels_vs_oracle runs the edge shapes pinned here."""
