@@ -370,6 +370,44 @@ int rbr_factor_rank(const float* A, const float* row_bias, int64_t n_rows, const
                     const int64_t* tgt_idx, int64_t n_targets, int64_t max_targets, int64_t* out_ranks, float* out_scores,
                     void* ws, int64_t ws_bytes, void* stream);
 
+/* ---- K12: token attributions of a predicted rating from the per-entity feature cache ---------------------------------
+ * After max-over-time (NgramFeat.forward, models/deepconn/layers.py:123-136; MyConv1d :54-58 with nn.Conv1d's [H, E, k]
+ * weights, :44) feature (n, h) depends on the one window starting at t*[n,h] - pad, t* = the forward's first arg-max.
+ *
+ * rbr_conv_window_contrib: the tap contributions of that window,
+ *   contrib[n * contrib_ld + h*ksize + j] = sum_e W[h,e,j] * x[n, argmax[n * argmax_ld + h] + j - pad, e]
+ * in fp32 from the fp32 `table` and the fp32 [H][k][E] copy of W inside `packed` (rbr_conv_pack), whatever precision the
+ * forward ran in.  x rows read as zeros exactly where the forward's do: outside the document, where the mask is false (mask
+ * NULL: all true, or ids != 0 with RBR_MASK_FROM_IDS) and for ids outside [0, vocab).  `ids` as in K2 (RBR_IDS_I32 /
+ * RBR_IDS_U16).  Several convs share one [n_docs, sum_c H_c * k_c] output through pointer offsets (argmax + first filter
+ * column, contrib + first tap column) and the leading dimensions.  One table-row read per (n, h, j).
+ *
+ * rbr_explain_attrib: for n_rows (pair, side) rows — row p covers the docs_per_entity consecutive cached documents starting at
+ * ent_row[p] (DeepCoNN 1, NARRE R reviews), each doc_len tokens — with g [n_rows, docs_per_entity, Htot] = d pred / d feat:
+ *   attr[r, t] = sum_{h : feat > 0} sum_{j : t*[r,h] + j - pad = t} g[r,h] * contrib[r,h,j]    (gradient x input on x)
+ * over the n_conv convs given by host_convs = {filters, ksize, pad} per conv (their filter columns are consecutive in
+ * feat / argmax / g, Htot = sum of filters; their taps consecutive in contrib).  Writes
+ *   text_total [n_rows]           sum_{h : feat > 0} g * sum_j contrib (= the sum of the map);
+ *   top_pos / top_attr [n_rows, m]    the m windows of `width` consecutive positions with the largest summed attribution,
+ *                                     greedily without overlap, ties to the lower start, never across a document boundary;
+ *   bottom_pos / bottom_attr          the same for the smallest sums; positions are flat (r * doc_len + t), slots without a
+ *                                     window left hold -1 / NaN;
+ *   map [n_rows, docs_per_entity * doc_len] (optional: NULL = not written), review_attr [n_rows, docs_per_entity] (optional).
+ * The map is built on chip with fixed-point integer atomics: results are bit-identical between calls and independent of the
+ * batch and the row order.  A row whose ent_row lies outside [0, n_docs - docs_per_entity] gets NaN / -1.
+ * Limits (rbr_explain_supported, host-only): 1 <= docs_per_entity * doc_len <= 16384, 1 <= m <= 32, 1 <= width <= 16,
+ * 1 <= n_conv <= 8; otherwise rbr_explain_attrib returns RBR_EUNSUPPORTED.                                              */
+int rbr_explain_supported(int64_t positions, int64_t m, int64_t width, int64_t n_conv);
+int rbr_conv_window_contrib(const float* table, int64_t vocab, int64_t emb, const void* ids, const uint8_t* mask,
+                            int64_t n_docs, int64_t doc_len, const void* packed, int64_t filters, int64_t ksize, int64_t pad,
+                            const int32_t* argmax, int64_t argmax_ld, float* contrib, int64_t contrib_ld, int flags,
+                            void* stream);
+int rbr_explain_attrib(const int64_t* ent_row, int64_t n_rows, int64_t docs_per_entity, int64_t doc_len, const float* g,
+                       const float* feat, const int32_t* argmax, int64_t feat_ld, const float* contrib, int64_t contrib_ld,
+                       int64_t n_docs, int64_t n_conv, const int64_t* host_convs, int64_t m, int64_t width, float* text_total,
+                       int64_t* top_pos, float* top_attr, int64_t* bottom_pos, float* bottom_attr, float* map,
+                       float* review_attr, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -21,6 +21,7 @@ D-ATT's score is already a dot product of the two FC outputs.
 """
 from __future__ import annotations
 
+from dataclasses import dataclass
 from typing import Optional, Tuple
 
 import torch
@@ -59,6 +60,7 @@ class PairScorer:
         self.user_feat: Optional[torch.Tensor] = None
         self.item_feat: Optional[torch.Tensor] = None
         self._factors = None         # (key, (A, row_bias, B, col_bias)) derived from the current head parameters
+        self._explain = None         # per-side tensors kept by build_cache(explain=True)
 
     @torch.no_grad()
     def score_pairs(self, *inputs) -> torch.Tensor:
@@ -69,16 +71,23 @@ class PairScorer:
     @torch.no_grad()
     def build_cache(self, user_docs: torch.Tensor, item_docs: torch.Tensor, user_masks: Optional[torch.Tensor] = None,
                     item_masks: Optional[torch.Tensor] = None, chunk: int = 4096, *, user_rev_ids: Optional[torch.Tensor] = None,
-                    item_rev_ids: Optional[torch.Tensor] = None) -> None:
+                    item_rev_ids: Optional[torch.Tensor] = None, explain: bool = False) -> None:
         """Row e of every argument belongs to entity id e (row 0 = the padding entity).
         DeepCoNN: user_docs [U, L], item_docs [I, L]; masks default to ids != 0 (utils.py:30-42).
         NARRE: user_docs [U, R, T], item_docs [I, R, T] (the entity's reviews), optional masks of the same shapes, and
           user_rev_ids [U, R] / item_rev_ids [I, R]: the ids of the items a user reviewed / the users who reviewed an item —
           what NARRE's dataset supplies as reuid / reiid for a pair with that entity.
-        D-ATT: user_docs [U, L], item_docs [I, L] (no masks)."""
+        D-ATT: user_docs [U, L], item_docs [I, L] (no masks).
+        explain=True also keeps what `explain` needs per entity (references to the documents and masks; for DeepCoNN and
+        NARRE the conv arg-max and the tap contributions of every pooled window (K12a), for NARRE the per-review features
+        and attention weights; for D-ATT the two K5 gates).  The cached features are the same either way."""
         m = self.model
         self.model.eval()
         self._factors = None
+        self._explain = None
+        if explain and not _is_datt(m) and m.ngram.arch != "CNN":
+            raise NotImplementedError("PairScorer.explain covers the CNN encoder; arch='HierPooling' pools averages, "
+                                      "which have no per-window tap contributions")
         if _is_datt(m):
             if user_masks is not None or item_masks is not None:
                 raise ValueError("DualAtt takes no masks")
@@ -86,6 +95,18 @@ class PairScorer:
             def side(docs, s):
                 return torch.cat([m.fc(m.encode([docs[lo:lo + chunk]], [s])[0]) for lo in range(0, docs.shape[0], chunk)], 0)
             self.user_feat, self.item_feat = side(user_docs, "u"), side(item_docs, "i")
+            if explain:
+                table = m.word_embeddings.embedding.weight.detach()
+
+                def gates(docs, s):
+                    la, ga = getattr(m, f"{s}_local_atten"), getattr(m, f"{s}_global_atten")
+                    parts = [ops.datt_gates(table, docs[lo:lo + chunk], la.attn[0].weight, la.attn[0].bias, ga.attn[0].weight,
+                                            ga.attn[0].bias) for lo in range(0, docs.shape[0], chunk)]
+                    return {"docs": docs, "gate_l": torch.cat([p[0] for p in parts]), "gate_g": torch.cat([p[1] for p in parts])}
+                self._explain = {"user": gates(user_docs, "u"), "item": gates(item_docs, "i")}
+            return
+        if explain:
+            self._build_explain_cache(user_docs, item_docs, user_masks, item_masks, chunk, user_rev_ids, item_rev_ids)
             return
         if _is_narre(m):
             if user_rev_ids is None or item_rev_ids is None:
@@ -118,6 +139,66 @@ class PairScorer:
         self.user_feat = encode(user_docs, user_masks)
         self.item_feat = encode(item_docs, item_masks)
 
+    def _conv_specs(self):
+        conv = self.model.ngram.conv
+        return [(c.weight.shape[0], k, (k - 1) // 2) for c, k in zip(conv.list_of_conv1d, conv.kernel_sizes)]
+
+    def _encode_explain(self, docs: torch.Tensor, masks: Optional[torch.Tensor], chunk: int):
+        """docs [N, L] (masks None: ids != 0) → (feat [N, H], argmax int32 [N, H], contrib [N, sum_c H_c * k_c]): the encoder's
+        own features and first arg-max (EncodeDocsFn), then the tap contributions of every pooled window (K12a)."""
+        m = self.model
+        conv = m.ngram.conv
+        table = m.word_embeddings.embedding.weight.detach()
+        specs = self._conv_specs()
+        taps = sum(h * k for h, k, _ in specs)
+        feats, amaxes = [], []
+        contrib = torch.empty(docs.shape[0], taps, dtype=torch.float32, device=table.device)
+        for lo in range(0, docs.shape[0], chunk):
+            d = docs[lo:lo + chunk]
+            mk = None if masks is None else masks[lo:lo + chunk]
+            f, a = m.ngram.encode(m.word_embeddings, [d], [mk], return_argmax=True)
+            col = tcol = 0
+            for i, (h, k, pad) in enumerate(specs):
+                ops.conv_window_contrib(table, d, mk, conv.list_of_conv1d[i].weight.detach(), pad, a[:, col:col + h],
+                                        packed=conv.packed(i), mask_from_ids=True, out=contrib[lo:lo + chunk, tcol:tcol + h * k])
+                col += h
+                tcol += h * k
+            feats.append(f)
+            amaxes.append(a)
+        return torch.cat(feats), torch.cat(amaxes), contrib
+
+    def _build_explain_cache(self, user_docs, item_docs, user_masks, item_masks, chunk, user_rev_ids, item_rev_ids):
+        m = self.model
+        if not _is_narre(m):
+            sides = {}
+            for name, docs, masks in (("user", user_docs, user_masks), ("item", item_docs, item_masks)):
+                feat, amax, contrib = self._encode_explain(docs, masks, chunk)
+                sides[name] = {"docs": docs, "masks": masks, "feat": feat, "argmax": amax, "contrib": contrib}
+            self.user_feat, self.item_feat = sides["user"]["feat"], sides["item"]["feat"]
+            self._explain = sides
+            return
+        if user_rev_ids is None or item_rev_ids is None:
+            raise ValueError("NARRE's build_cache needs user_rev_ids [U, R] and item_rev_ids [I, R]")
+        R, T = m.doc_num, m.doc_len
+        ent_chunk = max(1, chunk // R)
+        sides = {}
+        for name, docs, masks, rev_ids, att in (("user", user_docs, user_masks, user_rev_ids, m.user_att),
+                                                ("item", item_docs, item_masks, item_rev_ids, m.item_att)):
+            if docs.shape[1:] != (R, T) or rev_ids.shape != docs.shape[:2]:
+                raise ValueError(f"NARRE was built for [*, {R}, {T}] reviews with [*, {R}] review ids, got "
+                                 f"{tuple(docs.shape)} / {tuple(rev_ids.shape)}")
+            n = docs.shape[0]
+            feat, amax, contrib = self._encode_explain(docs.reshape(n * R, T), None if masks is None else masks.reshape(n * R, T),
+                                                       ent_chunk * R)
+            outs, scores = [], []
+            for lo in range(0, n, ent_chunk):
+                o, s = att(feat[lo * R:(lo + ent_chunk) * R].view(-1, R, feat.shape[1]), rev_ids[lo:lo + ent_chunk])
+                outs.append(o)
+                scores.append(s.view(-1, R))
+            sides[name] = {"docs": docs, "masks": masks, "rev_ids": rev_ids, "feat": feat, "argmax": amax, "contrib": contrib,
+                           "att": torch.cat(scores), "out": torch.cat(outs)}
+        self.user_feat, self.item_feat = sides["user"].pop("out"), sides["item"].pop("out")
+        self._explain = sides
     @torch.no_grad()
     def score_cached(self, u_ids: torch.Tensor, i_ids: torch.Tensor) -> torch.Tensor:
         """preds for pairs (u_ids[b], i_ids[b]) from the cached features, no encoder: K1 row gather + K4 head (DeepCoNN,
@@ -228,6 +309,129 @@ class PairScorer:
         ndcg@k for each k in ks, mrr, auc and n_rows, averaged over the rows that have at least one target."""
         ranks, _, n_cand = self.rank_items(u_ids, targets, exclude=exclude, exclude_padding=exclude_padding)
         return ranking_metrics(ranks, targets[0], n_cand, ks)
+
+    @torch.no_grad()
+    def explain(self, u_ids: torch.Tensor, i_ids: torch.Tensor, m: int = 5, width: Optional[int] = None,
+                return_maps: bool = False, chunk: int = 16384) -> "Explanation":
+        """Why the model predicts what score_cached(u_ids, i_ids) returns, from the cache of build_cache(explain=True).
+
+        DeepCoNN / NARRE: gradient x input on the embedded tokens of each side's document(s), at the model's own arg-max and
+        ReLU decisions (K12, DESIGN.md): attr[t] = sum over pooled features h whose window covers t (feat > 0) of
+        g[h] * c[h, j], g = d pred / d feat from K4's backward (NARRE: further through K3's backward to each review's
+        feature), c = the cached tap contribution.  Per side: text_total (= the map's sum), the top-m / bottom-m windows of
+        `width` positions (default: the largest kernel size; greedy without overlap, ties to the lower start, never across a
+        review) and, with return_maps, the map itself ([B, L], NARRE [B, R, T]; 4 bytes per position and pair, so it is
+        only written when asked for).  NARRE also gives review_weight (the entity's attention weights) and review_attr
+        (per-review sums of the map).  D-ATT: the local gate per token, the global gate per document (K5) and the m
+        positions with the largest local gate.  Positions are flat (NARRE: r * T + t); `tokens_at` turns them into ids.
+        Pairs run in chunks of `chunk`, so scratch memory does not grow with B."""
+        if self._explain is None or self.user_feat is None:
+            raise RuntimeError("PairScorer.build_cache(..., explain=True) first")
+        mdl = self.model
+        mdl.eval()
+        dev = self.user_feat.device
+        u_ids = u_ids.to(device=dev, dtype=torch.int64).reshape(-1)
+        i_ids = i_ids.to(device=dev, dtype=torch.int64).reshape(-1)
+        if u_ids.numel() != i_ids.numel():
+            raise ValueError("u_ids and i_ids must hold one id per pair")
+        n_u, n_i = self.user_feat.shape[0], self.item_feat.shape[0]
+        if u_ids.numel():
+            lo_u, hi_u, lo_i, hi_i = torch.stack([u_ids.min(), u_ids.max(), i_ids.min(), i_ids.max()]).tolist()
+            if lo_u < 0 or hi_u >= n_u or lo_i < 0 or hi_i >= n_i:
+                raise ValueError(f"user ids must lie in [0, {n_u}) and item ids in [0, {n_i})")
+        m = int(m)
+        pred = self.score_cached(u_ids, i_ids)
+        if _is_datt(mdl):
+            L = self._explain["user"]["gate_l"].shape[1]
+            if not 1 <= m <= L:
+                raise ValueError(f"m must lie in [1, {L}]")
+            sides = []
+            for name, ids in (("user", u_ids), ("item", i_ids)):
+                c = self._explain[name]
+                gl = c["gate_l"].index_select(0, ids)
+                # stable sort: equal gates keep the lower position first
+                order = torch.sort(gl, dim=1, descending=True, stable=True).indices[:, :m]
+                sides.append(SideExplanation(local_att=gl, global_att=c["gate_g"].index_select(0, ids), top_pos=order,
+                                             top_attr=gl.gather(1, order)))
+            return Explanation(pred, *sides)
+        specs = self._conv_specs()
+        R, T = (mdl.doc_num, mdl.doc_len) if _is_narre(mdl) else (1, self._explain["user"]["docs"].shape[1])
+        width = max(k for _, k, _ in specs) if width is None else int(width)
+        if not ops.explain_supported(R * T, m, width, len(specs)):
+            raise ValueError(f"explain takes 1 <= m <= {ops.EXPLAIN_MAX_M}, 1 <= width <= {ops.EXPLAIN_MAX_WIDTH} and at most "
+                             f"{ops.EXPLAIN_MAX_POSITIONS} positions per entity (got m={m}, width={width}, {R} x {T})")
+        head = self._head_params()
+        pads = (mdl.user_feat.padding_idx, mdl.item_feat.padding_idx, mdl.fm.padding_idx, mdl.fm.item_padding_idx)
+        head_scratch = [torch.empty_like(p) for p in head]
+        if _is_narre(mdl):
+            att_prm = [[a.W_rv, a.W_id, a.h, a.b_1, a.b_2, a.ebd_vals.weight] for a in (mdl.user_att, mdl.item_att)]
+            att_scratch = [[torch.empty_like(p) for p in sp] for sp in att_prm]
+            att_pads = (mdl.user_att.padding_idx, mdl.item_att.padding_idx)
+        parts = {"user": [], "item": []}
+        for lo in range(0, u_ids.numel(), chunk):
+            u, i = u_ids[lo:lo + chunk], i_ids[lo:lo + chunk]
+            g_u, g_i = ops.head_text_grads(ops.gather_rows(self.user_feat, u), ops.gather_rows(self.item_feat, i), u, i, head,
+                                           pads, head_scratch)
+            if _is_narre(mdl):
+                cu, ci = self._explain["user"], self._explain["item"]
+                H = cu["feat"].shape[1]
+                g_u, g_i = ops.narre_feat_grads(
+                    [cu["feat"].view(-1, R, H).index_select(0, u), ci["feat"].view(-1, R, H).index_select(0, i)],
+                    [cu["rev_ids"].index_select(0, u), ci["rev_ids"].index_select(0, i)],
+                    [cu["att"].index_select(0, u), ci["att"].index_select(0, i)], [g_u, g_i], att_prm, att_pads, att_scratch)
+            for name, ids, g in (("user", u, g_u), ("item", i, g_i)):
+                c = self._explain[name]
+                parts[name].append(ops.explain_attrib(ids * R, g.view(ids.numel(), R, -1), c["feat"], c["argmax"], c["contrib"],
+                                                      specs, R, T, m, width, return_map=return_maps,
+                                                      return_review_attr=_is_narre(mdl)))
+        sides = []
+        for name, ids in (("user", u_ids), ("item", i_ids)):
+            p = parts[name]
+            cat = {k: torch.cat([x[k] for x in p]) if p else None for k in (p[0] if p else {})}
+            if not p:                                   # no pairs: empty results of the right shapes
+                cat = ops.explain_attrib(ids, torch.empty(0, R, sum(h for h, _, _ in specs), device=dev),
+                                         self._explain[name]["feat"], self._explain[name]["argmax"],
+                                         self._explain[name]["contrib"], specs, R, T, m, width, return_maps, _is_narre(mdl))
+            mp = cat.get("map")
+            sides.append(SideExplanation(
+                text_total=cat["text_total"], top_pos=cat["top_pos"], top_attr=cat["top_attr"], bottom_pos=cat["bottom_pos"],
+                bottom_attr=cat["bottom_attr"], map=None if mp is None else (mp.view(-1, R, T) if _is_narre(mdl) else mp),
+                review_weight=self._explain[name]["att"].index_select(0, ids) if _is_narre(mdl) else None,
+                review_attr=cat.get("review_attr")))
+        return Explanation(pred, *sides)
+
+    def tokens_at(self, side: str, ent_ids: torch.Tensor, pos: torch.Tensor) -> torch.Tensor:
+        """Token ids at flat positions pos [B, m] (explain's top_pos / bottom_pos) of the kept documents of entities
+        ent_ids [B] on `side` ("user" / "item"); -1 where pos is -1."""
+        if self._explain is None:
+            raise RuntimeError("PairScorer.build_cache(..., explain=True) first")
+        docs = self._explain[side]["docs"]
+        flat = docs.reshape(docs.shape[0], -1).index_select(0, ent_ids.to(device=docs.device, dtype=torch.int64).reshape(-1))
+        pos = pos.to(device=docs.device, dtype=torch.int64)
+        tok = flat.to(torch.int64).gather(1, pos.clamp_min(0))
+        return torch.where(pos >= 0, tok, torch.full_like(tok, -1))
+
+
+@dataclass
+class SideExplanation:
+    """One side (user or item) of PairScorer.explain, one row per pair; fields a model does not have are None."""
+    text_total: Optional[torch.Tensor] = None       # [B] sum of the attribution map
+    top_pos: Optional[torch.Tensor] = None          # [B, m] int64 window starts (D-ATT: positions by local gate), -1 = none
+    top_attr: Optional[torch.Tensor] = None         # [B, m] window sums (D-ATT: the local gate), NaN where top_pos is -1
+    bottom_pos: Optional[torch.Tensor] = None       # [B, m] most negative windows
+    bottom_attr: Optional[torch.Tensor] = None
+    map: Optional[torch.Tensor] = None              # [B, L] (NARRE [B, R, T]) with return_maps
+    review_weight: Optional[torch.Tensor] = None    # NARRE [B, R]: the entity's review attention weights
+    review_attr: Optional[torch.Tensor] = None      # NARRE [B, R]: per-review sums of the map
+    local_att: Optional[torch.Tensor] = None        # D-ATT [B, L]: local attention gate per token
+    global_att: Optional[torch.Tensor] = None       # D-ATT [B]: global attention gate of the document
+
+
+@dataclass
+class Explanation:
+    pred: torch.Tensor                              # [B], bit-identical to score_cached
+    user: SideExplanation
+    item: SideExplanation
 
 
 def ranking_metrics(ranks: torch.Tensor, indptr: torch.Tensor, n_candidates: torch.Tensor, ks=(10,)) -> dict:

@@ -1237,3 +1237,251 @@ def factor_rank(A: torch.Tensor, row_bias: Optional[torch.Tensor], B: torch.Tens
     ranks[plan["order"]] = r_sorted
     scores[plan["order"]] = s_sorted
     return ranks, scores, plan["n_candidates"]
+
+
+# ---------------------------------------------------------------------------------------------------
+# K12: token attributions of a predicted rating from the per-entity feature cache
+# ---------------------------------------------------------------------------------------------------
+EXPLAIN_MAX_POSITIONS, EXPLAIN_MAX_M, EXPLAIN_MAX_WIDTH, EXPLAIN_MAX_CONVS = 16384, 32, 16, 8
+
+
+def explain_supported(positions: int, m: int, width: int, n_conv: int = 1) -> bool:
+    """Whether rbr_explain_attrib takes rows of `positions` = docs_per_entity * doc_len tokens with m windows of `width`
+    positions over n_conv convs (host-only query)."""
+    return bool(lib.rbr_explain_supported(int(positions), int(m), int(width), int(n_conv)))
+
+
+def _check_argmax(argmax: torch.Tensor, n_docs: int, filters: int, n_pos: int, what: str) -> torch.Tensor:
+    if not isinstance(argmax, torch.Tensor) or not argmax.is_cuda:
+        raise RuntimeError(f"rbr_b200: `{what}` must be a CUDA tensor")
+    if argmax.dtype != torch.int32 or argmax.dim() != 2 or argmax.shape[0] != n_docs or argmax.shape[1] < filters:
+        raise ValueError(f"rbr_b200: `{what}` must be int32 [{n_docs}, >= {filters}], got {argmax.dtype} {tuple(argmax.shape)}")
+    if argmax.stride(1) != 1:
+        raise ValueError(f"rbr_b200: `{what}` must have unit column stride")
+    if argmax.numel():
+        lo, hi = torch.stack([argmax[:, :filters].min(), argmax[:, :filters].max()]).tolist()
+        if lo < 0 or hi >= n_pos:
+            raise ValueError(f"rbr_b200: `{what}` positions must lie in [0, {n_pos}) (the pooled conv outputs)")
+    return argmax
+
+
+def conv_window_contrib(table: torch.Tensor, ids: torch.Tensor, mask: Optional[torch.Tensor], weight: torch.Tensor, pad: int,
+                        argmax: torch.Tensor, packed: Optional[torch.Tensor] = None, mask_from_ids: bool = False,
+                        out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """K12a: the tap contributions c[n, h, j] = sum_e weight[h, e, j] * x[n, argmax[n, h] + j - pad, e] of every pooled
+    window, in fp32 from the fp32 table (x reads as zeros outside the document, where the mask is false — mask None with
+    mask_from_ids: ids != 0 — and for ids outside the table, as in the forward).  ids [n_docs, doc_len] int64 / int32 /
+    uint16; weight [H, E, k] (nn.Conv1d); argmax int32 [n_docs, H] (or a column slice of a wider array, e.g. one conv's
+    filters of EncodeDocsFn's arg-max).  Returns contrib [n_docs, H * k] (column h * k + j), or writes into `out`, which may
+    be a column slice of a wider [n_docs, sum_c H_c * k_c] array shared by several convs."""
+    table = _req(table, torch.float32, "table")
+    ids = _ids(ids, "ids")
+    weight = _req(weight, torch.float32, "conv weight")
+    if ids.dim() < 1 or table.dim() != 2 or weight.dim() != 3 or weight.shape[1] != table.shape[1]:
+        raise ValueError(f"rbr_b200: table [V, E], weight [H, E, k] and ids [..., L] do not fit: {tuple(table.shape)} / "
+                         f"{tuple(weight.shape)} / {tuple(ids.shape)}")
+    h, emb, k = weight.shape
+    pad = int(pad)
+    doc_len = ids.shape[-1]
+    n_docs = ids.numel() // max(doc_len, 1)
+    if pad < 0 or doc_len < 1:
+        raise ValueError("rbr_b200: pad must be >= 0 and documents non-empty")
+    if mask is not None and tuple(mask.shape) != tuple(ids.shape):
+        raise ValueError(f"rbr_b200: mask {tuple(mask.shape)} does not match ids {tuple(ids.shape)}")
+    flags = _id_flags(ids, mask, mask_from_ids)
+    mask = _mask_u8(mask, "mask")
+    argmax = _check_argmax(argmax, n_docs, h, doc_len + 2 * pad - k + 1, "argmax")
+    if packed is None:
+        packed = conv_pack(weight)
+    if out is None:
+        out = torch.empty(n_docs, h * k, dtype=torch.float32, device=table.device)
+    elif (out.dtype != torch.float32 or out.dim() != 2 or out.shape[0] != n_docs or out.shape[1] < h * k or out.stride(1) != 1
+          or out.device != table.device):
+        raise ValueError(f"rbr_b200: `out` must be fp32 [{n_docs}, >= {h * k}] with unit column stride")
+    if n_docs == 0:
+        return out
+    lib.check(lib.rbr_conv_window_contrib(_p(table), table.shape[0], emb, _p(ids), _p(mask), n_docs, doc_len, _p(packed), h, k,
+                                          pad, _p(argmax), argmax.stride(0), _p(out), out.stride(0), flags, _stream(True)),
+              "rbr_conv_window_contrib")
+    return out
+
+
+def explain_attrib(ent_row: torch.Tensor, g: torch.Tensor, feat: torch.Tensor, argmax: torch.Tensor, contrib: torch.Tensor,
+                   convs: Sequence[Tuple[int, int, int]], docs_per_entity: int, doc_len: int, m: int, width: int,
+                   return_map: bool = False, return_review_attr: bool = False) -> dict:
+    """K12b: per (pair, side) row p, the token attribution map of the docs_per_entity cached documents starting at row
+    ent_row[p] of feat / argmax / contrib, under g [P, docs_per_entity, Htot] = d pred / d feat, and its top-m / bottom-m
+    windows of `width` positions (greedy, no overlap, ties to the lower start, never across a document boundary).
+    convs = [(filters, ksize, pad)] per conv, in the column order of feat / argmax (Htot = sum of filters) and contrib
+    (sum of filters * ksize, conv_window_contrib's layout).
+    Returns a dict of text_total [P], top_pos / bottom_pos int64 [P, m] (flat positions r * doc_len + t, -1 = no window
+    left), top_attr / bottom_attr [P, m] (NaN where -1), and with return_map `map` [P, docs_per_entity * doc_len], with
+    return_review_attr `review_attr` [P, docs_per_entity]."""
+    R, T, m, width = int(docs_per_entity), int(doc_len), int(m), int(width)
+    convs = [tuple(int(x) for x in c) for c in convs]
+    if R < 1 or T < 1 or not explain_supported(R * T, m, width, len(convs)):
+        raise ValueError(f"rbr_b200: explain_attrib takes 1 <= docs_per_entity * doc_len <= {EXPLAIN_MAX_POSITIONS}, "
+                         f"1 <= m <= {EXPLAIN_MAX_M}, 1 <= width <= {EXPLAIN_MAX_WIDTH} and 1 to {EXPLAIN_MAX_CONVS} convs "
+                         f"(got {R} x {T}, m={m}, width={width}, {len(convs)} convs)")
+    if any(h < 1 or k < 1 or pad < 0 for h, k, pad in convs):
+        raise ValueError(f"rbr_b200: bad conv description {convs}")
+    h_tot = sum(h for h, _, _ in convs)
+    taps = sum(h * k for h, k, _ in convs)
+    feat = _req(feat, torch.float32, "feat")
+    contrib = _req(contrib, torch.float32, "contrib")
+    ent_row = _req(ent_row, torch.int64, "ent_row").view(-1)
+    g = _req(g, torch.float32, "g")
+    n_docs = feat.shape[0] if feat.dim() == 2 else -1
+    if feat.dim() != 2 or feat.shape[1] < h_tot or contrib.dim() != 2 or contrib.shape[0] != n_docs or contrib.shape[1] < taps:
+        raise ValueError(f"rbr_b200: feat [n_docs, >= {h_tot}] and contrib [n_docs, >= {taps}] expected, got "
+                         f"{tuple(feat.shape)} / {tuple(contrib.shape)}")
+    P = ent_row.numel()
+    if tuple(g.shape) != (P, R, h_tot):
+        raise ValueError(f"rbr_b200: g must be [{P}, {R}, {h_tot}], got {tuple(g.shape)}")
+    if tuple(argmax.shape) != tuple(feat.shape):
+        raise ValueError(f"rbr_b200: argmax {tuple(argmax.shape)} must match feat {tuple(feat.shape)}")
+    argmax = _req(argmax, torch.int32, "argmax")
+    for t, name in ((g, "g"), (contrib, "contrib"), (argmax, "argmax"), (ent_row, "ent_row")):
+        if t.device != feat.device:
+            raise ValueError(f"rbr_b200: `{name}` is on {t.device}, feat on {feat.device}")
+    if P and n_docs % R:
+        raise ValueError(f"rbr_b200: {n_docs} cached documents are not whole entities of {R}")
+    if P:
+        lo, hi, odd = torch.stack([ent_row.min(), ent_row.max(), (ent_row % R != 0).any().long()]).tolist()
+        if lo < 0 or hi > n_docs - R or odd:
+            raise ValueError(f"rbr_b200: ent_row must be multiples of {R} in [0, {n_docs - R}]")
+    dev = feat.device
+    out = {"text_total": torch.empty(P, dtype=torch.float32, device=dev)}
+    for side in ("top", "bottom"):
+        out[f"{side}_pos"] = torch.empty(P, m, dtype=torch.int64, device=dev)
+        out[f"{side}_attr"] = torch.empty(P, m, dtype=torch.float32, device=dev)
+    if return_map:
+        out["map"] = torch.empty(P, R * T, dtype=torch.float32, device=dev)
+    if return_review_attr:
+        out["review_attr"] = torch.empty(P, R, dtype=torch.float32, device=dev)
+    if P == 0:
+        return out
+    lib.check(lib.rbr_explain_attrib(
+        _p(ent_row), P, R, T, _p(g), _p(feat), _p(argmax), feat.shape[1], _p(contrib), contrib.shape[1], n_docs, len(convs),
+        _i64_array([x for c in convs for x in c]), m, width, _p(out["text_total"]), _p(out["top_pos"]), _p(out["top_attr"]),
+        _p(out["bottom_pos"]), _p(out["bottom_attr"]), _p(out.get("map")), _p(out.get("review_attr")), _stream(True)),
+        "rbr_explain_attrib")
+    return out
+
+
+def window_select(attr: torch.Tensor, doc_len: int, m: int, width: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor,
+                                                                                  torch.Tensor]:
+    """The window rule of explain_attrib in plain torch (any device; a statement of the rule, not a hot path): for each row
+    of attr [P, S] (S = docs * doc_len flat positions), the m windows of `width` consecutive positions with the largest
+    float64 sum, chosen greedily without overlap, ties to the lower start, no window across a multiple of doc_len; then
+    the same for the smallest sums.  Returns (top_pos, top_attr, bottom_pos, bottom_attr), -1 / NaN where no window is left."""
+    P, S = attr.shape
+    a = attr.double()
+    starts = torch.arange(S, device=attr.device)
+    valid = (starts % doc_len) + width <= doc_len
+    ws = torch.zeros(P, S, dtype=torch.float64, device=attr.device)
+    for j in range(min(width, S)):  # window sums as in-order additions (what the kernel does), not a cumsum difference
+        ws[:, :S - j] += a[:, j:]
+    out = []
+    for top in (True, False):
+        pos = torch.full((P, m), -1, dtype=torch.int64, device=attr.device)
+        val = torch.full((P, m), float("nan"), dtype=torch.float32, device=attr.device)
+        avail = valid.unsqueeze(0).expand(P, S).clone()
+        for it in range(m):
+            key = torch.where(avail, ws if top else -ws, torch.full_like(ws, float("-inf")))
+            best = key.max(1).values
+            hit = avail & (key == best.unsqueeze(1))
+            s = torch.where(hit, starts, torch.full_like(starts, S)).min(1).values      # lowest start among the ties
+            has = avail.any(1)
+            pos[:, it] = torch.where(has, s, torch.full_like(s, -1))
+            val[:, it] = torch.where(has, ws.gather(1, s.clamp_max(S - 1).view(-1, 1)).view(-1).float(),
+                                     torch.full((P,), float("nan"), device=attr.device))
+            block = (starts.view(1, -1) > (s.view(-1, 1) - width)) & (starts.view(1, -1) < (s.view(-1, 1) + width))
+            avail &= ~(block & has.view(-1, 1))
+        out += [pos, val]
+    return tuple(out)
+
+
+def datt_gates(table: torch.Tensor, ids: torch.Tensor, w_local: torch.Tensor, b_local: torch.Tensor, w_global: torch.Tensor,
+               b_global: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """K5's two D-ATT gates for documents ids [n_docs, doc_len]: (local [n_docs, doc_len], global [n_docs]), the values the
+    gated convs of DattEncodeFn multiply the token rows by."""
+    table = _req(table, torch.float32, "table")
+    ids = _ids(ids, "ids")
+    n_docs, doc_len = ids.shape
+    vocab, emb = table.shape
+    prm = [_req(t, torch.float32, n) for t, n in ((w_local, "w_local"), (b_local, "b_local"), (w_global, "w_global"),
+                                                  (b_global, "b_global"))]
+    win = prm[0].shape[2]
+    gate_l = torch.empty(n_docs, doc_len, dtype=torch.float32, device=table.device)
+    gate_g = torch.empty(n_docs, dtype=torch.float32, device=table.device)
+    ws_bytes = lib.rbr_datt_gate_workspace_bytes(n_docs, doc_len, emb, win, vocab)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=table.device)
+    lib.check(lib.rbr_datt_gate_fwd(_p(table), vocab, emb, _p(ids), n_docs, doc_len, _p(prm[0]), _p(prm[1]), win, _p(prm[2]),
+                                    _p(prm[3]), _p(gate_l), _p(gate_g), _p(ws), ws_bytes, _id_width_flag(ids), _stream(True)),
+              "rbr_datt_gate_fwd")
+    return gate_l, gate_g
+
+
+def head_text_grads(u_text: torch.Tensor, i_text: torch.Tensor, u_id: torch.Tensor, i_id: torch.Tensor,
+                    params: Sequence[torch.Tensor], padding_idx: Sequence[int], scratch: Optional[List[torch.Tensor]] = None
+                    ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """d pred / d u_text and d pred / d i_text [B, H] of K4 in eval mode (rbr_head_fwd, then rbr_head_bwd at pred_grad = 1).
+    params: (Wu, bu, ebd_u, Wi, bi, ebd_i, fm_h, user_bias, item_bias, g_bias); the parameter gradients the backward
+    accumulates go to `scratch` (one buffer per parameter, reused across calls and never read), not to `.grad`."""
+    u_text = _req(u_text, torch.float32, "u_text")
+    i_text = _req(i_text, torch.float32, "i_text")
+    u_id = _req(u_id, torch.int64, "u_id")
+    i_id = _req(i_id, torch.int64, "i_id")
+    fl = [_req(t.detach(), torch.float32, "head parameter") for t in params]
+    B, H = u_text.shape
+    K = fl[0].shape[1]
+    dev = u_text.device
+    if scratch is None:
+        scratch = [torch.empty_like(t) for t in fl]
+    pred = torch.empty(B, dtype=torch.float32, device=dev)
+    u_lat = torch.empty(B, K, dtype=torch.float32, device=dev)
+    i_lat = torch.empty(B, K, dtype=torch.float32, device=dev)
+    s = _stream(True)
+    lib.check(lib.rbr_head_fwd(_p(u_text), _p(i_text), _p(u_id), _p(i_id), B, H, K, *[_p(t) for t in fl], fl[2].shape[0],
+                               fl[5].shape[0], 0.0, 0, None, _p(pred), _p(u_lat), _p(i_lat), None, 0.0, None, None, s),
+              "rbr_head_fwd")
+    ones = torch.ones(B, dtype=torch.float32, device=dev)
+    g_ut, g_it = torch.empty_like(u_text), torch.empty_like(i_text)
+    pads = [-1 if x is None else int(x) for x in padding_idx]
+    lib.check(lib.rbr_head_bwd(_p(u_text), _p(i_text), _p(u_id), _p(i_id), B, H, K, _p(fl[0]), _p(fl[3]), _p(fl[6]), _p(u_lat),
+                               _p(i_lat), 0.0, 0, None, *pads, fl[2].shape[0], fl[5].shape[0], _p(ones), _p(g_ut), _p(g_it),
+                               *[_p(t) for t in scratch], s), "rbr_head_bwd")
+    return g_ut, g_it
+
+
+def narre_feat_grads(feats: Sequence[torch.Tensor], other_ids: Sequence[torch.Tensor], scores: Sequence[torch.Tensor],
+                     out_grads: Sequence[torch.Tensor], side_params: Sequence[Sequence[torch.Tensor]],
+                     padding_idx: Sequence[int], scratch: Optional[List[List[torch.Tensor]]] = None) -> List[torch.Tensor]:
+    """d pred / d feat [B, R, H] of each NARRE side from d pred / d out [B, H], through K3's backward (the tensor-core pair
+    kernel when the shape allows, else one K3 launch per side) with the forward's attention scores [B, R].  side_params: per
+    side (W_rv, W_id, h, b_1, b_2, ebd_vals); the parameter gradients go to `scratch`, never to `.grad`."""
+    feats = [_req(f, torch.float32, "feat") for f in feats]
+    ids = [_req(i, torch.int64, "other_id") for i in other_ids]
+    scores = [_req(s, torch.float32, "scores") for s in scores]
+    g_outs = [_req(g, torch.float32, "out_grad") for g in out_grads]
+    prm = [[_req(t.detach(), torch.float32, "attention parameter") for t in sp] for sp in side_params]
+    if scratch is None:
+        scratch = [[torch.empty_like(t) for t in sp] for sp in prm]
+    B, R, H = feats[0].shape
+    A = prm[0][0].shape[1]
+    pads = [-1 if x is None else int(x) for x in padding_idx]
+    g_feats = [torch.empty_like(f) for f in feats]
+    s = _stream(True)
+    if narre_attn_pair_supported(R, H, A) and len(feats) == 2:
+        lib.check(lib.rbr_narre_attn_pair_bwd(
+            2, _ptr_array([_p(f) for f in feats]), _ptr_array([_p(i) for i in ids]), B, R, H, A,
+            *[_ptr_array([_p(prm[0][j]), _p(prm[1][j])]) for j in range(6)],
+            _i64_array([prm[0][5].shape[0], prm[1][5].shape[0]]), _i64_array(pads), _ptr_array([_p(x) for x in scores]),
+            _ptr_array([_p(g) for g in g_outs]), None, _ptr_array([_p(g) for g in g_feats]),
+            *[_ptr_array([_p(scratch[0][j]), _p(scratch[1][j])]) for j in range(6)], s), "rbr_narre_attn_pair_bwd")
+        return g_feats
+    for f, i, sc, go, p, pad, gf, scr in zip(feats, ids, scores, g_outs, prm, pads, g_feats, scratch):
+        lib.check(lib.rbr_narre_attn_bwd(_p(f), _p(i), B, R, H, A, *[_p(t) for t in p], p[5].shape[0], pad, _p(sc), _p(go), None,
+                                         _p(gf), *[_p(t) for t in scr], s), "rbr_narre_attn_bwd")
+    return g_feats

@@ -1,0 +1,185 @@
+"""Explanations of served recommendations: PairScorer.explain (K12) for every user's top-10 from recommend, against gradient x
+input by autograd on the oracle formulation (fp32 on the GPU, TF32 off, in chunks, with the embedded tokens materialised).
+
+Set-up: U = 20 000 users x I = 12 000 items, vocabulary 50 000, E = 300, seeded parameters and documents:
+  DeepCoNN  documents of L = 500 tokens (lengths 200..500), H = 100 filters of width 3;
+  NARRE     10 reviews of 60 tokens per entity (lengths 20..60, trailing all-padding reviews), H = 150, attention 32.
+Pairs: each user's top-10 from recommend = 200 000 pairs.
+
+Reported per model: build_cache() and build_cache(explain=True) times and the bytes the explain cache adds; explain time
+(CUDA events over --reps calls after warm-up) and peak memory on the 200 000 pairs with and without maps, and on the first
+--baseline-pairs pairs; the baseline's time and peak memory on those same pairs, and the largest map difference between the
+two relative to each pair's largest |attribution| (the baseline routes through the cache's arg-max, so both compute the same
+quantity).
+
+    python tools/bench_explain.py --out DIR [--precision bf16|fp32] [--reps 3] [--baseline-pairs 4096]
+        → DIR/bench_explain_<precision>.json
+"""
+import argparse
+import json
+import os
+import sys
+
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+
+import rbr_b200  # noqa: E402
+from bench_recommend import I, U, gpu_info, timed  # noqa: E402
+from oracle import rbr_oracle as orc  # noqa: E402
+from rbr_b200 import synth  # noqa: E402
+from rbr_b200.inference import PairScorer  # noqa: E402
+
+VOCAB, EMB = 50000, 300
+
+
+def docs(n, L, seed, min_len):
+    g = torch.Generator(device="cuda").manual_seed(seed)
+    d = torch.randint(1, VOCAB, (n, L), device="cuda", generator=g)
+    lens = torch.randint(min_len, L + 1, (n, 1), device="cuda", generator=g)
+    return torch.where(torch.arange(L, device="cuda").view(1, -1) < lens, d, torch.zeros_like(d))
+
+
+def build(model, precision):
+    if model == "narre":
+        R, T = 10, 60
+        m = rbr_b200.NARRE(U, I, VOCAB, [3], 150, EMB, 32, 32, R, T, 0.0, 0, 0, 0, None, "CNN", precision=precision)
+        m.load_state_dict(synth.narre_params(U, I, VOCAB, EMB, 150, 32, 32, (3,), seed=0))
+        ud, idd = docs(U * R, T, 1, 20).view(U, R, T), docs(I * R, T, 2, 20).view(I, R, T)
+        nrev_u = torch.randint(1, R + 1, (U, 1), device="cuda")              # trailing reviews are all padding
+        nrev_i = torch.randint(1, R + 1, (I, 1), device="cuda")
+        ud = torch.where((torch.arange(R, device="cuda").view(1, -1) < nrev_u).unsqueeze(-1), ud, torch.zeros_like(ud))
+        idd = torch.where((torch.arange(R, device="cuda").view(1, -1) < nrev_i).unsqueeze(-1), idd, torch.zeros_like(idd))
+        kw = {"user_rev_ids": torch.randint(1, I, (U, R), device="cuda"), "item_rev_ids": torch.randint(1, U, (I, R), device="cuda")}
+    else:
+        m = rbr_b200.DeepCoNNpp(U, I, VOCAB, [3], EMB, 100, 32, 500, None, 0.0, precision=precision)
+        m.load_state_dict(synth.deepconn_params(U, I, VOCAB, EMB, 100, 32, (3,), seed=0))
+        ud, idd = docs(U, 500, 1, 200), docs(I, 500, 2, 200)
+        kw = {}
+    return PairScorer(m.cuda()), (ud, idd), kw
+
+
+def once_ms(fn):
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    out = fn()
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1), out
+
+
+def peak_mb(fn):
+    torch.cuda.synchronize()
+    base = torch.cuda.memory_allocated()
+    torch.cuda.reset_peak_memory_stats()
+    fn()
+    torch.cuda.synchronize()
+    return round((torch.cuda.max_memory_allocated() - base) / 2 ** 20, 1)
+
+
+def baseline(sc, inputs, kw, u_all, i_all, chunk):
+    """fp32 autograd gradient x input on the oracle formulation, chunk pairs at a time → (user maps, item maps)"""
+    p = {k: v.detach().float() for k, v in sc.model.state_dict().items()}
+    table = p["word_embeddings.embedding.weight"]
+    ws, bs = orc._conv_params(p, "ngram.feature_layer.0.list_of_conv1d")
+    c = sc._explain
+    ud, idd = inputs
+    narre = isinstance(sc.model, rbr_b200.NARRE)
+    maps_u, maps_i = [], []
+    for lo in range(0, u_all.numel(), chunk):
+        u, i = u_all[lo:lo + chunk], i_all[lo:lo + chunk]
+        ux = orc.embedding_gather(table, ud[u]).requires_grad_()
+        ix = orc.embedding_gather(table, idd[i]).requires_grad_()
+        if narre:
+            b, R, T = ud[u].shape
+            H = c["user"]["feat"].shape[1]
+            feats = []
+            for x, d, ids, side, rev in ((ux, ud[u], u, "user", kw["user_rev_ids"]), (ix, idd[i], i, "item", kw["item_rev_ids"])):
+                rf = orc.ngram_feat(x.view(b * R, T, -1), (d != 0).view(b * R, T), ws, bs,
+                                    argmax_override=c[side]["argmax"].view(-1, R, H)[ids].reshape(-1, H)).view(b, R, H)
+                att = {k: p[f"{side}_att.{k}"] for k in ("W_rv", "W_id", "h", "b_1", "b_2")}
+                feats.append(orc.linear_attention(rf, rev[ids], ebd_vals=p[f"{side}_att.ebd_vals.weight"], **att)[0])
+            uf, itf = feats
+        else:
+            uf = orc.ngram_feat(ux, ud[u] != 0, ws, bs, argmax_override=c["user"]["argmax"][u])
+            itf = orc.ngram_feat(ix, idd[i] != 0, ws, bs, argmax_override=c["item"]["argmax"][i])
+        u_f = orc.last_feat(uf, u, p["user_feat.W"], p["user_feat.b"], p["user_feat.ebd.weight"])
+        i_f = orc.last_feat(itf, i, p["item_feat.W"], p["item_feat.b"], p["item_feat.ebd.weight"])
+        pred = orc.fm_head(u_f, i_f, u, i, p["fm.h"], p["fm.g_bias"], p["fm.user_bias.weight"], p["fm.item_bias.weight"])
+        pred.sum().backward()
+        maps_u.append((ux * ux.grad).sum(-1).detach())
+        maps_i.append((ix * ix.grad).sum(-1).detach())
+    return torch.cat(maps_u), torch.cat(maps_i)
+
+
+def rel_per_pair(a, b):
+    """per pair: the largest |difference| over its positions relative to the pair's largest |attribution|"""
+    a, b = a.flatten(1).double(), b.flatten(1).double()
+    return (a - b).abs().amax(1) / b.abs().amax(1).clamp_min(1e-30)
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", required=True)
+    ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--baseline-pairs", type=int, default=4096)
+    ap.add_argument("--baseline-chunk", type=int, default=256)
+    ap.add_argument("--precision", choices=("bf16", "fp32"), default="bf16", help="the conv forward's precision")
+    args = ap.parse_args()
+    if not torch.cuda.is_available():
+        raise SystemExit("bench_explain needs a CUDA device")
+    torch.backends.cuda.matmul.allow_tf32 = False
+    torch.backends.cudnn.allow_tf32 = False
+    os.makedirs(args.out, exist_ok=True)
+    info = gpu_info()
+    runs = []
+    for model in ("deepconn", "narre"):
+        sc, inputs, kw = build(model, args.precision)
+        sc.build_cache(*inputs, **kw)                                         # warm-up (module loads, operand staging)
+        t_plain, _ = once_ms(lambda: sc.build_cache(*inputs, **kw))
+        sc.build_cache(*inputs, **kw, explain=True)
+        t_expl, _ = once_ms(lambda: sc.build_cache(*inputs, **kw, explain=True))
+        cache_mb = {k: round(sum(v[k].numel() * v[k].element_size() for v in sc._explain.values()) / 2 ** 20, 1)
+                    for k in ("feat", "argmax", "contrib")}
+        u_ids = torch.arange(U, device="cuda")
+        _, items = sc.recommend(u_ids, 10)
+        uu = u_ids.view(-1, 1).expand(-1, 10).reshape(-1)
+        ii = items.reshape(-1)
+        t_nomap, e = timed(lambda: sc.explain(uu, ii), args.reps)
+        t_map, _ = timed(lambda: sc.explain(uu, ii, return_maps=True), args.reps)
+        mem_nomap = peak_mb(lambda: sc.explain(uu, ii))
+        mem_map = peak_mb(lambda: sc.explain(uu, ii, return_maps=True))
+        nb = args.baseline_pairs
+        ub, ib = uu[:nb], ii[:nb]
+        t_sub, es = timed(lambda: sc.explain(ub, ib, return_maps=True), args.reps)
+        t_base, (bu, bi) = timed(lambda: baseline(sc, inputs, kw, ub, ib, args.baseline_chunk), 1)
+        mem_base = peak_mb(lambda: baseline(sc, inputs, kw, ub, ib, args.baseline_chunk))
+        diff = torch.cat([rel_per_pair(es.user.map, bu), rel_per_pair(es.item.map, bi)])
+        runs.append({
+            "model": model, "precision": sc.model.ngram.precision, "pairs": uu.numel(),
+            "build_cache_ms": round(t_plain, 2), "build_cache_explain_ms": round(t_expl, 2), "explain_cache_mb": cache_mb,
+            "explain_ms": round(t_nomap, 3), "explain_maps_ms": round(t_map, 3),
+            "explain_peak_mb": mem_nomap, "explain_maps_peak_mb": mem_map,
+            "baseline_pairs": nb, "explain_baseline_pairs_ms": round(t_sub, 3),
+            "autograd_baseline_ms": round(t_base, 2), "autograd_baseline_peak_mb": mem_base,
+            "speedup_on_baseline_pairs": round(t_base / t_sub, 1),
+            "map_diff_rel_to_pair_max": {"max": float(diff.max()), "p99": float(diff.quantile(0.99)),
+                                         "median": float(diff.median()),
+                                         "fraction_below_1e-2": float((diff <= 1e-2).double().mean()),
+                                         "fraction_below_1e-5": float((diff <= 1e-5).double().mean())},
+            "nan_windows": int(e.user.top_pos.lt(0).sum() + e.item.top_pos.lt(0).sum()),
+        })
+        print(json.dumps(runs[-1]), flush=True)
+        del sc, e, es
+        torch.cuda.empty_cache()
+    res = {**info, "U": U, "I": I, "vocab": VOCAB, "emb": EMB, "precision": args.precision, "reps": args.reps, "runs": runs}
+    with open(os.path.join(args.out, f"bench_explain_{args.precision}.json"), "w") as f:
+        json.dump(res, f, indent=1)
+    print(json.dumps({k: v for k, v in res.items() if k != "runs"}))
+
+
+if __name__ == "__main__":
+    main()
