@@ -407,6 +407,64 @@ int rbr_explain_attrib(const int64_t* ent_row, int64_t n_rows, int64_t docs_per_
                        int64_t n_docs, int64_t n_conv, const int64_t* host_convs, int64_t m, int64_t width, float* text_total,
                        int64_t* top_pos, float* top_attr, int64_t* bottom_pos, float* bottom_attr, float* map,
                        float* review_attr, void* stream);
+/* rbr_explain_attrib_ex: rbr_explain_attrib (which is this call with dense_coef = dense_vec = NULL) with
+ *   feat NULL (in either call): every filter counts (no liveness predicate: D-ATT's tanh features);
+ *   a dense term (dense_coef non-NULL): for document r of the row (cached document ent_row[p] + r),
+ *     attr[r, t] += (sum_h g[r, h] * dense_coef[doc * dense_coef_ld + h]) * dense_vec[doc * dense_vec_ld + t]
+ *   where the scalar is reduced in float64 in a fixed order; each product enters the map (and the total) as one more
+ *   fixed-point term, and the scale bound counts it, so results stay bit-identical across calls, batches and row orders.
+ * Limits as above; with a dense term also docs_per_entity * 8 bytes more shared memory (RBR_EUNSUPPORTED past 227 KB).     */
+int rbr_explain_attrib_ex(const int64_t* ent_row, int64_t n_rows, int64_t docs_per_entity, int64_t doc_len, const float* g,
+                          const float* feat, const int32_t* argmax, int64_t feat_ld, const float* contrib, int64_t contrib_ld,
+                          int64_t n_docs, int64_t n_conv, const int64_t* host_convs, const float* dense_coef,
+                          int64_t dense_coef_ld, const float* dense_vec, int64_t dense_vec_ld, int64_t m, int64_t width,
+                          float* text_total, int64_t* top_pos, float* top_attr, int64_t* bottom_pos, float* bottom_attr,
+                          float* map, float* review_attr, void* stream);
+
+/* ---- K12 for D-ATT: gradient x input through both attention gates and the FC stack ----------------------------------------
+ * D-ATT (models/dual_att/layers.py:25-89, dual_att.py:31-61): per side, gl = sigmoid(local gate conv, k = window, pad
+ * (window-1)/2) per token, gg = sigmoid(global gate conv, k = doc_len) per document; features f = max_t tanh(conv(gate * x))
+ * of a k = 1 conv on gl * x (l_out filters) and k = 2, 3, 4 convs on gg * x (g_out filters each, no padding), at the
+ * forward's first arg-max t*.  x = the table row of each token (zero for ids outside the table; no masks).  With
+ * d = 1 - f^2 and g = d pred / d f, gradient x input on x is the sum of
+ *   local filter h:  g d gl[t*] (W_h . x[t*]) at t*, and g d (W_h . x[t*]) gl(1-gl)[t*] (w_l[:, j] . x[t* + j - pad]) at
+ *                    t* + j - pad (the gate's taps);
+ *   global filter h: g d gg (W_h[:, j] . x[t* + j]) at t* + j, and g d (sum_j W_h[:, j] . x[t* + j]) gg(1-gg) (w_g[:, s] . x[s])
+ *                    at every position s.
+ * Everything but g depends on the entity alone.
+ *
+ * rbr_datt_explain_contrib: those per-entity terms of n_docs documents, in fp32 from the fp32 table and the fp32 weight
+ * copies inside `packed_*` (rbr_conv_pack of the four conv weights: local [l_out, E, 1], global [g_out, E, 2 / 3 / 4]),
+ * whatever precision the forward ran in:
+ *   contrib [n_docs, contrib_ld >= l_out * window + g_out * 9]: the local filters as one width-`window` conv with pad
+ *     (window-1)/2 (column h * window + j; the direct term is folded into the centre tap), then the three global convs as
+ *     pad-0 convs (columns h * k + j) — rbr_explain_attrib's layout for convs {l_out, window, (window-1)/2}, {g_out, 2, 0},
+ *     {g_out, 3, 0}, {g_out, 4, 0};
+ *   gate_coef [n_docs, coef_ld >= l_out + 3 g_out]: d * sum_j c_j on the global filters, 0 on the local ones;
+ *   gate_vec [n_docs, vec_ld >= doc_len]: gg(1-gg) (w_g[:, s] . x[s]).
+ * w_local_t [window][emb] and w_global_t [doc_len][emb] are the gate weights transposed (nn.Conv1d's [1, E, k] → [k, E]).
+ * gate_local [n_docs, doc_len], gate_global [n_docs], feat / argmax [n_docs, feat_ld] (filter columns local, conv k=2, 3, 4)
+ * are the forward's (rbr_datt_gate_fwd, rbr_conv_act_maxpool_fwd).  `flags`: RBR_IDS_I32 for int32 ids.
+ * Limits: window odd and <= 16, doc_len >= 4; else RBR_EUNSUPPORTED before any launch.
+ * The per-pair map is then rbr_explain_attrib_ex with feat NULL, g, this contrib and the dense term (gate_coef, gate_vec).
+ *
+ * rbr_datt_fc_grads: g for n_pairs pairs (u_ids[p], i_ids[p]) and both sides:
+ *   g_user[p] = W0^T (user_mask[u] * W3^T item_out[i]),  g_item[p] = W0^T (item_mask[i] * W3^T user_out[u])
+ * with user_out / item_out [n_users / n_items, out_dim] the cached FC outputs, user_mask / item_mask [*, hidden] (uint8 / bool)
+ * the cached hidden ReLU masks 1[z > 0], w0 = fc.0.weight [hidden, in_dim], w3 = fc.3.weight [out_dim, hidden]; outputs
+ * [n_pairs, in_dim].  Tensor cores at fp32 grade (3xTF32 mma.sync); every element is reduced in a fixed order, so results are
+ * bit-identical whatever the batch, the chunking or the pair order.  Ids outside the tables give zero rows.
+ * Limits: 1 <= hidden <= 768; else RBR_EUNSUPPORTED before any launch.                                                      */
+int rbr_datt_explain_contrib(const float* table, int64_t vocab, int64_t emb, const void* ids, int64_t n_docs, int64_t doc_len,
+                             const float* w_local_t, int64_t window, const float* w_global_t, const void* packed_local,
+                             int64_t l_out, const void* packed_g2, const void* packed_g3, const void* packed_g4, int64_t g_out,
+                             const float* gate_local, const float* gate_global, const float* feat, const int32_t* argmax,
+                             int64_t feat_ld, float* contrib, int64_t contrib_ld, float* gate_coef, int64_t coef_ld,
+                             float* gate_vec, int64_t vec_ld, int flags, void* stream);
+int rbr_datt_fc_grads(const int64_t* u_ids, const int64_t* i_ids, int64_t n_pairs, const float* user_out, int64_t n_users,
+                      const float* item_out, int64_t n_items, int64_t out_dim, const uint8_t* user_mask,
+                      const uint8_t* item_mask, int64_t hidden, const float* w0, int64_t in_dim, const float* w3,
+                      float* g_user, float* g_item, void* stream);
 
 #ifdef __cplusplus
 }

@@ -80,7 +80,8 @@ class PairScorer:
         D-ATT: user_docs [U, L], item_docs [I, L] (no masks).
         explain=True also keeps what `explain` needs per entity (references to the documents and masks; for DeepCoNN and
         NARRE the conv arg-max and the tap contributions of every pooled window (K12a), for NARRE the per-review features
-        and attention weights; for D-ATT the two K5 gates).  The cached features are the same either way."""
+        and attention weights; for D-ATT the two K5 gates, the conv arg-max, the FC hidden ReLU mask and the per-entity
+        terms of gradient x input, rbr_datt_explain_contrib).  The cached features are the same either way."""
         m = self.model
         self.model.eval()
         self._factors = None
@@ -92,18 +93,13 @@ class PairScorer:
             if user_masks is not None or item_masks is not None:
                 raise ValueError("DualAtt takes no masks")
 
+            if explain:
+                self._build_datt_explain_cache(user_docs, item_docs, chunk)
+                return
+
             def side(docs, s):
                 return torch.cat([m.fc(m.encode([docs[lo:lo + chunk]], [s])[0]) for lo in range(0, docs.shape[0], chunk)], 0)
             self.user_feat, self.item_feat = side(user_docs, "u"), side(item_docs, "i")
-            if explain:
-                table = m.word_embeddings.embedding.weight.detach()
-
-                def gates(docs, s):
-                    la, ga = getattr(m, f"{s}_local_atten"), getattr(m, f"{s}_global_atten")
-                    parts = [ops.datt_gates(table, docs[lo:lo + chunk], la.attn[0].weight, la.attn[0].bias, ga.attn[0].weight,
-                                            ga.attn[0].bias) for lo in range(0, docs.shape[0], chunk)]
-                    return {"docs": docs, "gate_l": torch.cat([p[0] for p in parts]), "gate_g": torch.cat([p[1] for p in parts])}
-                self._explain = {"user": gates(user_docs, "u"), "item": gates(item_docs, "i")}
             return
         if explain:
             self._build_explain_cache(user_docs, item_docs, user_masks, item_masks, chunk, user_rev_ids, item_rev_ids)
@@ -138,6 +134,40 @@ class PairScorer:
             return torch.cat(outs, dim=0)
         self.user_feat = encode(user_docs, user_masks)
         self.item_feat = encode(item_docs, item_masks)
+
+    def _datt_side_prm(self, s: str):
+        m = self.model
+        return [p.detach() for p in m._side_params(getattr(m, f"{s}_local_atten"), getattr(m, f"{s}_global_atten"))]
+
+    def _build_datt_explain_cache(self, user_docs, item_docs, chunk):
+        """D-ATT with explain=True: the encoder once per chunk (ops.datt_encode_side, the kernels DualAtt.encode runs), the FC
+        stack layer by layer (the same modules in the same order as m.fc, so the cached features are bit-identical to
+        build_cache(explain=False)) to keep its hidden ReLU mask, then K12's per-entity terms (ops.datt_explain_contrib)."""
+        m = self.model
+        table = m.word_embeddings.embedding.weight.detach()
+        shadow = m.word_embeddings.bf16_shadow() if m.precision == "bf16" else None
+        lin0, relu, drop, lin1 = m.fc
+        sides, outs = {}, {}
+        for name, s, docs in (("user", "u", user_docs), ("item", "i", item_docs)):
+            if docs.shape[-1] != m.doc_len:
+                raise ValueError(f"DualAtt was built for doc_len={m.doc_len}, got {docs.shape[-1]}")
+            prm = self._datt_side_prm(s)
+            packed = ops.datt_side_packs(prm)
+            keep = {k: [] for k in ("gate_l", "gate_g", "argmax", "contrib", "gate_coef", "gate_vec", "hid_mask")}
+            out = []
+            for lo in range(0, docs.shape[0], chunk):
+                d = docs[lo:lo + chunk]
+                feat, amax, _, gl, gg = ops.datt_encode_side(table, d, prm, m.precision, shadow, packed)
+                z = lin0(feat)
+                out.append(lin1(drop(relu(z))))
+                contrib, coef, vec = ops.datt_explain_contrib(table, d, prm, gl, gg, feat, amax, packed)
+                for k, v in (("gate_l", gl), ("gate_g", gg), ("argmax", amax), ("contrib", contrib), ("gate_coef", coef),
+                             ("gate_vec", vec), ("hid_mask", z > 0)):
+                    keep[k].append(v)
+            sides[name] = {"docs": docs, **{k: torch.cat(v) for k, v in keep.items()}}
+            outs[name] = torch.cat(out, 0)
+        self.user_feat, self.item_feat = outs["user"], outs["item"]
+        self._explain = sides
 
     def _conv_specs(self):
         conv = self.model.ngram.conv
@@ -312,7 +342,7 @@ class PairScorer:
 
     @torch.no_grad()
     def explain(self, u_ids: torch.Tensor, i_ids: torch.Tensor, m: int = 5, width: Optional[int] = None,
-                return_maps: bool = False, chunk: int = 16384) -> "Explanation":
+                return_maps: bool = False, chunk: int = 16384, *, attribution: bool = False) -> "Explanation":
         """Why the model predicts what score_cached(u_ids, i_ids) returns, from the cache of build_cache(explain=True).
 
         DeepCoNN / NARRE: gradient x input on the embedded tokens of each side's document(s), at the model's own arg-max and
@@ -322,9 +352,13 @@ class PairScorer:
         `width` positions (default: the largest kernel size; greedy without overlap, ties to the lower start, never across a
         review) and, with return_maps, the map itself ([B, L], NARRE [B, R, T]; 4 bytes per position and pair, so it is
         only written when asked for).  NARRE also gives review_weight (the entity's attention weights) and review_attr
-        (per-review sums of the map).  D-ATT: the local gate per token, the global gate per document (K5) and the m
-        positions with the largest local gate.  Positions are flat (NARRE: r * T + t); `tokens_at` turns them into ids.
-        Pairs run in chunks of `chunk`, so scratch memory does not grow with B."""
+        (per-review sums of the map).  D-ATT: the local gate per token and the global gate per document (K5); by default
+        also the m positions with the largest local gate.  With attribution=True (D-ATT only; DeepCoNN and NARRE always
+        attribute) D-ATT's top / bottom windows, text_total and map are gradient x input as for DeepCoNN, through both
+        gates and the FC stack at the model's own arg-max and ReLU decisions: g = d pred / d feat from the cached FC outputs
+        and hidden ReLU masks (ops.datt_fc_grads), then K12b over the cached per-entity terms with the global gate as a
+        dense term; the default width is the local window size.  Positions are flat (NARRE: r * T + t); `tokens_at` turns
+        them into ids.  Pairs run in chunks of `chunk`, so scratch memory does not grow with B."""
         if self._explain is None or self.user_feat is None:
             raise RuntimeError("PairScorer.build_cache(..., explain=True) first")
         mdl = self.model
@@ -341,6 +375,8 @@ class PairScorer:
                 raise ValueError(f"user ids must lie in [0, {n_u}) and item ids in [0, {n_i})")
         m = int(m)
         pred = self.score_cached(u_ids, i_ids)
+        if _is_datt(mdl) and attribution:
+            return self._explain_datt(u_ids, i_ids, pred, m, width, return_maps, chunk)
         if _is_datt(mdl):
             L = self._explain["user"]["gate_l"].shape[1]
             if not 1 <= m <= L:
@@ -400,6 +436,41 @@ class PairScorer:
                 review_attr=cat.get("review_attr")))
         return Explanation(pred, *sides)
 
+    def _explain_datt(self, u_ids, i_ids, pred, m, width, return_maps, chunk) -> "Explanation":
+        mdl = self.model
+        L = mdl.doc_len
+        specs = ops.datt_explain_convs(self._datt_side_prm("u"))
+        width = specs[0][1] if width is None else int(width)
+        if not ops.explain_supported(L, m, width, len(specs)):
+            raise ValueError(f"explain takes 1 <= m <= {ops.EXPLAIN_MAX_M}, 1 <= width <= {ops.EXPLAIN_MAX_WIDTH} and at most "
+                             f"{ops.EXPLAIN_MAX_POSITIONS} positions per entity (got m={m}, width={width}, L={L})")
+        cu, ci = self._explain["user"], self._explain["item"]
+        w0, w3 = mdl.fc[0].weight.detach(), mdl.fc[3].weight.detach()
+        parts = {"user": [], "item": []}
+        for lo in range(0, u_ids.numel(), chunk):
+            u, i = u_ids[lo:lo + chunk], i_ids[lo:lo + chunk]
+            g_u, g_i = ops.datt_fc_grads(u, i, self.user_feat, self.item_feat, cu["hid_mask"], ci["hid_mask"], w0, w3)
+            for name, ids, g in (("user", u, g_u), ("item", i, g_i)):
+                c = self._explain[name]
+                parts[name].append(ops.explain_attrib(ids, g.view(ids.numel(), 1, -1), None, c["argmax"], c["contrib"], specs, 1,
+                                                      L, m, width, return_map=return_maps, dense_coef=c["gate_coef"],
+                                                      dense_vec=c["gate_vec"]))
+        sides = []
+        for name, ids in (("user", u_ids), ("item", i_ids)):
+            c = self._explain[name]
+            p = parts[name]
+            if p:
+                cat = {k: torch.cat([x[k] for x in p]) for k in p[0]}
+            else:                                       # no pairs: empty results of the right shapes
+                cat = ops.explain_attrib(ids, torch.empty(0, 1, c["argmax"].shape[1], device=ids.device), None, c["argmax"],
+                                         c["contrib"], specs, 1, L, m, width, return_maps, dense_coef=c["gate_coef"],
+                                         dense_vec=c["gate_vec"])
+            sides.append(SideExplanation(
+                text_total=cat["text_total"], top_pos=cat["top_pos"], top_attr=cat["top_attr"], bottom_pos=cat["bottom_pos"],
+                bottom_attr=cat["bottom_attr"], map=cat.get("map"), local_att=c["gate_l"].index_select(0, ids),
+                global_att=c["gate_g"].index_select(0, ids)))
+        return Explanation(pred, *sides)
+
     def tokens_at(self, side: str, ent_ids: torch.Tensor, pos: torch.Tensor) -> torch.Tensor:
         """Token ids at flat positions pos [B, m] (explain's top_pos / bottom_pos) of the kept documents of entities
         ent_ids [B] on `side` ("user" / "item"); -1 where pos is -1."""
@@ -416,8 +487,10 @@ class PairScorer:
 class SideExplanation:
     """One side (user or item) of PairScorer.explain, one row per pair; fields a model does not have are None."""
     text_total: Optional[torch.Tensor] = None       # [B] sum of the attribution map
-    top_pos: Optional[torch.Tensor] = None          # [B, m] int64 window starts (D-ATT: positions by local gate), -1 = none
-    top_attr: Optional[torch.Tensor] = None         # [B, m] window sums (D-ATT: the local gate), NaN where top_pos is -1
+    top_pos: Optional[torch.Tensor] = None          # [B, m] int64 window starts (D-ATT without attribution: positions by
+                                                    # local gate), -1 = none
+    top_attr: Optional[torch.Tensor] = None         # [B, m] window sums (D-ATT without attribution: the local gate), NaN
+                                                    # where top_pos is -1
     bottom_pos: Optional[torch.Tensor] = None       # [B, m] most negative windows
     bottom_attr: Optional[torch.Tensor] = None
     map: Optional[torch.Tensor] = None              # [B, L] (NARRE [B, R, T]) with return_maps

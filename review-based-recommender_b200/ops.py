@@ -869,6 +869,65 @@ def conv_act_maxpool(table: torch.Tensor, ids: torch.Tensor, mask: Optional[torc
 # ---------------------------------------------------------------------------------------------------
 # K5 + gated K2: one side of the D-ATT encoder (local attention + global attention), ids → [N, l_out + 3*g_out]
 # ---------------------------------------------------------------------------------------------------
+def datt_side_packs(prm: Sequence[torch.Tensor]) -> List[torch.Tensor]:
+    """conv_pack of one D-ATT side's four conv weights (local k = 1, then global k = 2, 3, 4) from its 12 parameters
+    (DattEncodeFn's order)."""
+    return [conv_pack(prm[i]) for i in (2, 6, 8, 10)]
+
+
+def datt_encode_side(table: torch.Tensor, ids: torch.Tensor, prm: Sequence[torch.Tensor], precision: str = "bf16",
+                     shadow: Optional[torch.Tensor] = None, packed: Optional[Sequence[torch.Tensor]] = None,
+                     stream: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """One side of the D-ATT encoder forward (models/dual_att/layers.py:43-53, 81-89): K5's two gates, then the four gated
+    tanh convs with max-over-time.  ids [n_docs, doc_len] int64 / int32; prm = the side's 12 parameters in DattEncodeFn's
+    order; shadow = the bf16 table (bf16 only; made here when None); packed = datt_side_packs(prm) (made here when None);
+    stream = a raw stream handle (None: torch's current stream).
+    Returns (feat [n_docs, l_out + 3 g_out], argmax int32, pre-activation at the arg-max, gate_local [n_docs, doc_len],
+    gate_global [n_docs]); filter columns: local conv, then the k = 2, 3, 4 global convs."""
+    table = _req(table, torch.float32, "embedding table")
+    ids = _ids(ids, "token ids")
+    prm = [_req(t, torch.float32, "D-ATT parameter") for t in prm]
+    prec = _PREC[precision]
+    if prec == PREC_BF16 and shadow is None:
+        shadow = table_to_bf16(table)
+    if packed is None:
+        packed = datt_side_packs(prm)
+    vocab, emb = table.shape
+    dev = table.device
+    idf = _id_width_flag(ids)
+    la_w, la_b, lc_w, lc_b, ga_w, ga_b = prm[:6]
+    g_convs = [(prm[6 + 2 * i], prm[7 + 2 * i]) for i in range(3)]
+    n_docs, doc_len = ids.shape
+    win = la_w.shape[2]
+    s = _stream(True) if stream is None else stream
+    ws_bytes = lib.rbr_datt_gate_workspace_bytes(n_docs, doc_len, emb, win, vocab)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    gate_l = torch.empty(n_docs, doc_len, dtype=torch.float32, device=dev)
+    gate_g = torch.empty(n_docs, dtype=torch.float32, device=dev)
+    lib.check(lib.rbr_datt_gate_fwd(_p(table), vocab, emb, _p(ids), n_docs, doc_len, _p(la_w), _p(la_b), win, _p(ga_w),
+                                    _p(ga_b), _p(gate_l), _p(gate_g), _p(ws), ws_bytes, idf, s), "rbr_datt_gate_fwd")
+    convs = [(lc_w, lc_b, gate_l, 1)] + [(w, b, gate_g, 2) for w, b in g_convs]
+    h_total = sum(w.shape[0] for w, _, _, _ in convs)
+    feat = torch.empty(n_docs, h_total, dtype=torch.float32, device=dev)
+    amax = torch.empty(n_docs, h_total, dtype=torch.int32, device=dev)
+    pre = torch.empty(n_docs, h_total, dtype=torch.float32, device=dev)
+    col = 0
+    ws_bytes = (max(lib.rbr_conv_fwd_workspace_bytes2(n_docs, doc_len, w.shape[2], 0) for w, _, _, _ in convs)
+                if prec == PREC_BF16 else 0)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev) if ws_bytes else None
+    for (w, b, gate, mode), pk in zip(convs, packed):
+        h, _, k = w.shape
+        lib.check(lib.rbr_conv_act_maxpool_fwd(prec, ACT_TANH, _p(table), _p(shadow), vocab, emb, _p(ids), None, _p(gate),
+                                               mode, n_docs, doc_len, _p(pk), _p(b), h, k, 0, feat.data_ptr() + 4 * col,
+                                               amax.data_ptr() + 4 * col, pre.data_ptr() + 4 * col, h_total, _p(ws), ws_bytes,
+                                               idf, s), "rbr_conv_act_maxpool_fwd")
+        col += h
+    return feat, amax, pre, gate_l, gate_g
+
+
+# ---------------------------------------------------------------------------------------------------
+# K5 + gated K2: one side of the D-ATT encoder (local attention + global attention), ids → [N, l_out + 3*g_out]
+# ---------------------------------------------------------------------------------------------------
 class DattEncodeFn(torch.autograd.Function):
     """feats[s] = cat(LocalAttention_s(x_s), *GlobalAttention_s(x_s)) for x_s = table[ids_s], s in (user, item)
     (reference models/dual_att/layers.py:43-53, 81-89 and dual_att.py:45-50, 53-56), without materialising x, its
@@ -887,41 +946,13 @@ class DattEncodeFn(torch.autograd.Function):
         stride = 1 + DattEncodeFn.N_PRM
         n_sides = len(rest) // stride
         prec = _PREC[cfg["precision"]]
-        vocab, emb = table.shape
-        dev = table.device
         shadow = cfg["shadow_fn"]() if prec == PREC_BF16 else None
         saved, feats, side_ctx = [], [], []
         for s in range(n_sides):
             ids = _ids(rest[s * stride], "token ids")
-            idf = _id_width_flag(ids)
             prm = [_req(t, torch.float32, "D-ATT parameter") for t in rest[s * stride + 1:(s + 1) * stride]]
-            la_w, la_b, lc_w, lc_b, ga_w, ga_b = prm[:6]
-            g_convs = [(prm[6 + 2 * i], prm[7 + 2 * i]) for i in range(3)]
-            n_docs, doc_len = ids.shape
-            win = la_w.shape[2]
-            ws_bytes = lib.rbr_datt_gate_workspace_bytes(n_docs, doc_len, emb, win, vocab)
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-            gate_l = torch.empty(n_docs, doc_len, dtype=torch.float32, device=dev)
-            gate_g = torch.empty(n_docs, dtype=torch.float32, device=dev)
-            lib.check(lib.rbr_datt_gate_fwd(_p(table), vocab, emb, _p(ids), n_docs, doc_len, _p(la_w), _p(la_b), win, _p(ga_w),
-                                            _p(ga_b), _p(gate_l), _p(gate_g), _p(ws), ws_bytes, idf, _stream()), "rbr_datt_gate_fwd")
-            convs = [(lc_w, lc_b, gate_l, 1)] + [(w, b, gate_g, 2) for w, b in g_convs]
-            packed = [conv_pack(w) for w, _, _, _ in convs]
-            h_total = sum(w.shape[0] for w, _, _, _ in convs)
-            feat = torch.empty(n_docs, h_total, dtype=torch.float32, device=dev)
-            amax = torch.empty(n_docs, h_total, dtype=torch.int32, device=dev)
-            pre = torch.empty(n_docs, h_total, dtype=torch.float32, device=dev)
-            col = 0
-            ws_bytes = (max(lib.rbr_conv_fwd_workspace_bytes2(n_docs, doc_len, w.shape[2], 0) for w, _, _, _ in convs)
-                        if prec == PREC_BF16 else 0)
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev) if ws_bytes else None
-            for (w, b, gate, mode), pk in zip(convs, packed):
-                h, _, k = w.shape
-                lib.check(lib.rbr_conv_act_maxpool_fwd(prec, ACT_TANH, _p(table), _p(shadow), vocab, emb, _p(ids), None, _p(gate),
-                                                       mode, n_docs, doc_len, _p(pk), _p(b), h, k, 0, feat.data_ptr() + 4 * col,
-                                                       amax.data_ptr() + 4 * col, pre.data_ptr() + 4 * col, h_total, _p(ws), ws_bytes,
-                                                       idf, _stream()), "rbr_conv_act_maxpool_fwd")
-                col += h
+            packed = datt_side_packs(prm)
+            feat, amax, pre, gate_l, gate_g = datt_encode_side(table, ids, prm, cfg["precision"], shadow, packed, _stream())
             saved += [ids, gate_l, gate_g, feat, amax, pre]
             feats.append(feat)
             side_ctx.append((prm, packed))
@@ -1306,9 +1337,10 @@ def conv_window_contrib(table: torch.Tensor, ids: torch.Tensor, mask: Optional[t
     return out
 
 
-def explain_attrib(ent_row: torch.Tensor, g: torch.Tensor, feat: torch.Tensor, argmax: torch.Tensor, contrib: torch.Tensor,
-                   convs: Sequence[Tuple[int, int, int]], docs_per_entity: int, doc_len: int, m: int, width: int,
-                   return_map: bool = False, return_review_attr: bool = False) -> dict:
+def explain_attrib(ent_row: torch.Tensor, g: torch.Tensor, feat: Optional[torch.Tensor], argmax: torch.Tensor,
+                   contrib: torch.Tensor, convs: Sequence[Tuple[int, int, int]], docs_per_entity: int, doc_len: int, m: int,
+                   width: int, return_map: bool = False, return_review_attr: bool = False,
+                   dense_coef: Optional[torch.Tensor] = None, dense_vec: Optional[torch.Tensor] = None) -> dict:
     """K12b: per (pair, side) row p, the token attribution map of the docs_per_entity cached documents starting at row
     ent_row[p] of feat / argmax / contrib, under g [P, docs_per_entity, Htot] = d pred / d feat, and its top-m / bottom-m
     windows of `width` positions (greedy, no overlap, ties to the lower start, never across a document boundary).
@@ -1316,7 +1348,10 @@ def explain_attrib(ent_row: torch.Tensor, g: torch.Tensor, feat: torch.Tensor, a
     (sum of filters * ksize, conv_window_contrib's layout).
     Returns a dict of text_total [P], top_pos / bottom_pos int64 [P, m] (flat positions r * doc_len + t, -1 = no window
     left), top_attr / bottom_attr [P, m] (NaN where -1), and with return_map `map` [P, docs_per_entity * doc_len], with
-    return_review_attr `review_attr` [P, docs_per_entity]."""
+    return_review_attr `review_attr` [P, docs_per_entity].
+    feat None: every filter counts (D-ATT's tanh features have no liveness predicate).  dense_coef [n_docs, >= Htot] with
+    dense_vec [n_docs, doc_len] add a dense term per cached document: (sum_h g * dense_coef) * dense_vec (D-ATT's global
+    gate, datt_explain_contrib), reduced in a fixed order (rbr_explain_attrib_ex)."""
     R, T, m, width = int(docs_per_entity), int(doc_len), int(m), int(width)
     convs = [tuple(int(x) for x in c) for c in convs]
     if R < 1 or T < 1 or not explain_supported(R * T, m, width, len(convs)):
@@ -1327,22 +1362,32 @@ def explain_attrib(ent_row: torch.Tensor, g: torch.Tensor, feat: torch.Tensor, a
         raise ValueError(f"rbr_b200: bad conv description {convs}")
     h_tot = sum(h for h, _, _ in convs)
     taps = sum(h * k for h, k, _ in convs)
-    feat = _req(feat, torch.float32, "feat")
     contrib = _req(contrib, torch.float32, "contrib")
     ent_row = _req(ent_row, torch.int64, "ent_row").view(-1)
     g = _req(g, torch.float32, "g")
+    argmax = _req(argmax, torch.int32, "argmax")
+    feat = argmax if feat is None else _req(feat, torch.float32, "feat")       # only shapes and the device are read from it
     n_docs = feat.shape[0] if feat.dim() == 2 else -1
     if feat.dim() != 2 or feat.shape[1] < h_tot or contrib.dim() != 2 or contrib.shape[0] != n_docs or contrib.shape[1] < taps:
-        raise ValueError(f"rbr_b200: feat [n_docs, >= {h_tot}] and contrib [n_docs, >= {taps}] expected, got "
+        raise ValueError(f"rbr_b200: feat / argmax [n_docs, >= {h_tot}] and contrib [n_docs, >= {taps}] expected, got "
                          f"{tuple(feat.shape)} / {tuple(contrib.shape)}")
     P = ent_row.numel()
     if tuple(g.shape) != (P, R, h_tot):
         raise ValueError(f"rbr_b200: g must be [{P}, {R}, {h_tot}], got {tuple(g.shape)}")
     if tuple(argmax.shape) != tuple(feat.shape):
         raise ValueError(f"rbr_b200: argmax {tuple(argmax.shape)} must match feat {tuple(feat.shape)}")
-    argmax = _req(argmax, torch.int32, "argmax")
-    for t, name in ((g, "g"), (contrib, "contrib"), (argmax, "argmax"), (ent_row, "ent_row")):
-        if t.device != feat.device:
+    if (dense_coef is None) != (dense_vec is None):
+        raise ValueError("rbr_b200: dense_coef and dense_vec go together")
+    if dense_coef is not None:
+        dense_coef = _req(dense_coef, torch.float32, "dense_coef")
+        dense_vec = _req(dense_vec, torch.float32, "dense_vec")
+        if (dense_coef.dim() != 2 or dense_coef.shape[0] != n_docs or dense_coef.shape[1] < h_tot
+                or tuple(dense_vec.shape) != (n_docs, T)):
+            raise ValueError(f"rbr_b200: dense_coef [{n_docs}, >= {h_tot}] and dense_vec [{n_docs}, {T}] expected, got "
+                             f"{tuple(dense_coef.shape)} / {tuple(dense_vec.shape)}")
+    for t, name in ((g, "g"), (contrib, "contrib"), (argmax, "argmax"), (ent_row, "ent_row"), (dense_coef, "dense_coef"),
+                    (dense_vec, "dense_vec")):
+        if t is not None and t.device != feat.device:
             raise ValueError(f"rbr_b200: `{name}` is on {t.device}, feat on {feat.device}")
     if P and n_docs % R:
         raise ValueError(f"rbr_b200: {n_docs} cached documents are not whole entities of {R}")
@@ -1361,11 +1406,19 @@ def explain_attrib(ent_row: torch.Tensor, g: torch.Tensor, feat: torch.Tensor, a
         out["review_attr"] = torch.empty(P, R, dtype=torch.float32, device=dev)
     if P == 0:
         return out
-    lib.check(lib.rbr_explain_attrib(
-        _p(ent_row), P, R, T, _p(g), _p(feat), _p(argmax), feat.shape[1], _p(contrib), contrib.shape[1], n_docs, len(convs),
-        _i64_array([x for c in convs for x in c]), m, width, _p(out["text_total"]), _p(out["top_pos"]), _p(out["top_attr"]),
-        _p(out["bottom_pos"]), _p(out["bottom_attr"]), _p(out.get("map")), _p(out.get("review_attr")), _stream(True)),
-        "rbr_explain_attrib")
+    if dense_coef is None and feat is not argmax:
+        lib.check(lib.rbr_explain_attrib(
+            _p(ent_row), P, R, T, _p(g), _p(feat), _p(argmax), feat.shape[1], _p(contrib), contrib.shape[1], n_docs, len(convs),
+            _i64_array([x for c in convs for x in c]), m, width, _p(out["text_total"]), _p(out["top_pos"]), _p(out["top_attr"]),
+            _p(out["bottom_pos"]), _p(out["bottom_attr"]), _p(out.get("map")), _p(out.get("review_attr")), _stream(True)),
+            "rbr_explain_attrib")
+        return out
+    lib.check(lib.rbr_explain_attrib_ex(
+        _p(ent_row), P, R, T, _p(g), None if feat is argmax else _p(feat), _p(argmax), feat.shape[1], _p(contrib),
+        contrib.shape[1], n_docs, len(convs), _i64_array([x for c in convs for x in c]), _p(dense_coef),
+        0 if dense_coef is None else dense_coef.shape[1], _p(dense_vec), T, m, width, _p(out["text_total"]),
+        _p(out["top_pos"]), _p(out["top_attr"]), _p(out["bottom_pos"]), _p(out["bottom_attr"]), _p(out.get("map")),
+        _p(out.get("review_attr")), _stream(True)), "rbr_explain_attrib_ex")
     return out
 
 
@@ -1421,6 +1474,133 @@ def datt_gates(table: torch.Tensor, ids: torch.Tensor, w_local: torch.Tensor, b_
                                     _p(prm[3]), _p(gate_l), _p(gate_g), _p(ws), ws_bytes, _id_width_flag(ids), _stream(True)),
               "rbr_datt_gate_fwd")
     return gate_l, gate_g
+
+
+def _datt_side_prm(prm: Sequence[torch.Tensor]) -> List[torch.Tensor]:
+    prm = [_req(t.detach(), torch.float32, "D-ATT parameter") for t in prm]
+    if len(prm) != DattEncodeFn.N_PRM:
+        raise ValueError(f"rbr_b200: a D-ATT side has {DattEncodeFn.N_PRM} parameters, got {len(prm)}")
+    return prm
+
+
+def datt_explain_contrib(table: torch.Tensor, ids: torch.Tensor, prm: Sequence[torch.Tensor], gate_l: torch.Tensor,
+                         gate_g: torch.Tensor, feat: torch.Tensor, argmax: torch.Tensor,
+                         packed: Optional[Sequence[torch.Tensor]] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """The per-entity terms of D-ATT's gradient x input (rbr_datt_explain_contrib) for documents ids [n_docs, L] (int64 /
+    int32) of one side: prm = the side's 12 parameters (DattEncodeFn's order), gate_l [n_docs, L] / gate_g [n_docs] / feat /
+    argmax [n_docs, l_out + 3 g_out] from datt_encode_side.  In fp32 from the fp32 table whatever the forward's precision.
+    Returns (contrib [n_docs, l_out * window + 9 g_out], gate_coef [n_docs, l_out + 3 g_out], gate_vec [n_docs, L]): the
+    contributions for explain_attrib with convs datt_explain_convs(prm) and feat None, and its dense term."""
+    table = _req(table, torch.float32, "table")
+    ids = _ids(ids, "ids")
+    if ids.dtype == torch.uint16:
+        raise TypeError("rbr_b200: D-ATT takes int64 or int32 ids")
+    prm = _datt_side_prm(prm)
+    if table.dim() != 2 or ids.dim() != 2:
+        raise ValueError(f"rbr_b200: table [V, E] and ids [n_docs, L] expected, got {tuple(table.shape)} / {tuple(ids.shape)}")
+    vocab, emb = table.shape
+    n_docs, L = ids.shape
+    la_w, ga_w = prm[0], prm[4]
+    win = la_w.shape[-1]
+    l_out, g_out = prm[2].shape[0], prm[6].shape[0]
+    if (tuple(la_w.shape) != (1, emb, win) or tuple(ga_w.shape) != (1, emb, L) or tuple(prm[2].shape) != (l_out, emb, 1)
+            or any(tuple(prm[6 + 2 * c].shape) != (g_out, emb, c + 2) for c in range(3))):
+        raise ValueError(f"rbr_b200: D-ATT parameters do not fit emb={emb}, doc_len={L}: "
+                         f"{[tuple(p.shape) for p in prm[::2]]}")
+    if L < 4 or win % 2 == 0 or not 1 <= win <= EXPLAIN_MAX_WIDTH:
+        raise ValueError(f"rbr_b200: datt_explain_contrib takes doc_len >= 4 and an odd window <= {EXPLAIN_MAX_WIDTH} "
+                         f"(got {L}, {win})")
+    htot = l_out + 3 * g_out
+    gate_l = _req(gate_l, torch.float32, "gate_l")
+    gate_g = _req(gate_g, torch.float32, "gate_g")
+    feat = _req(feat, torch.float32, "feat")
+    if tuple(gate_l.shape) != (n_docs, L) or tuple(gate_g.reshape(-1).shape) != (n_docs,) or tuple(feat.shape) != (n_docs, htot):
+        raise ValueError(f"rbr_b200: gate_l [{n_docs}, {L}], gate_g [{n_docs}] and feat [{n_docs}, {htot}] expected, got "
+                         f"{tuple(gate_l.shape)} / {tuple(gate_g.shape)} / {tuple(feat.shape)}")
+    argmax = _req(argmax, torch.int32, "argmax")
+    if tuple(argmax.shape) != (n_docs, htot):
+        raise ValueError(f"rbr_b200: argmax must be int32 [{n_docs}, {htot}], got {tuple(argmax.shape)}")
+    if n_docs:
+        for c, (lo, hi) in enumerate(((0, l_out), (l_out, l_out + g_out), (l_out + g_out, l_out + 2 * g_out),
+                                      (l_out + 2 * g_out, htot))):
+            _check_argmax(argmax[:, lo:hi], n_docs, hi - lo, L - (c + 1) + 1 if c else L, "argmax")
+    for t, name in ((ids, "ids"), (gate_l, "gate_l"), (gate_g, "gate_g"), (feat, "feat"), (argmax, "argmax")):
+        if t.device != table.device:
+            raise ValueError(f"rbr_b200: `{name}` is on {t.device}, the table on {table.device}")
+    if packed is None:
+        packed = datt_side_packs(prm)
+    wlT = la_w.reshape(emb, win).t().contiguous()
+    wgT = ga_w.reshape(emb, L).t().contiguous()
+    dev = table.device
+    contrib = torch.empty(n_docs, l_out * win + 9 * g_out, dtype=torch.float32, device=dev)
+    gate_coef = torch.empty(n_docs, htot, dtype=torch.float32, device=dev)
+    gate_vec = torch.empty(n_docs, L, dtype=torch.float32, device=dev)
+    if n_docs == 0:
+        return contrib, gate_coef, gate_vec
+    lib.check(lib.rbr_datt_explain_contrib(
+        _p(table), vocab, emb, _p(ids), n_docs, L, _p(wlT), win, _p(wgT), _p(packed[0]), l_out, _p(packed[1]), _p(packed[2]),
+        _p(packed[3]), g_out, _p(gate_l), _p(gate_g), _p(feat), _p(argmax), htot, _p(contrib), contrib.shape[1], _p(gate_coef),
+        htot, _p(gate_vec), L, _id_width_flag(ids), _stream(True)), "rbr_datt_explain_contrib")
+    return contrib, gate_coef, gate_vec
+
+
+def datt_explain_convs(prm: Sequence[torch.Tensor]) -> List[Tuple[int, int, int]]:
+    """explain_attrib's conv description of datt_explain_contrib's layout: the local filters as one width-`window` conv with
+    pad (window - 1) / 2, then the k = 2, 3, 4 global convs without padding."""
+    win = prm[0].shape[-1]
+    return [(prm[2].shape[0], win, (win - 1) // 2)] + [(prm[6 + 2 * c].shape[0], c + 2, 0) for c in range(3)]
+
+
+DATT_FC_MAX_HIDDEN = 768
+
+
+def datt_fc_grads(u_ids: torch.Tensor, i_ids: torch.Tensor, user_out: torch.Tensor, item_out: torch.Tensor,
+                  user_mask: torch.Tensor, item_mask: torch.Tensor, w0: torch.Tensor, w3: torch.Tensor
+                  ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """g = d pred / d cat [P, in_dim] of both D-ATT sides for pairs (u_ids[p], i_ids[p]) (rbr_datt_fc_grads): pred =
+    fc(cat_u) . fc(cat_i) with the shared FC stack, so g_u = W0^T (user_mask[u] * W3^T item_out[i]) and symmetrically.
+    user_out [U, out_dim] / item_out [I, out_dim]: the cached FC outputs; user_mask / item_mask [*, hidden] bool: the cached
+    hidden ReLU masks; w0 = fc.0.weight [hidden, in_dim], w3 = fc.3.weight [out_dim, hidden].  3xTF32 tensor cores, one
+    fixed summation order per element: bit-identical whatever the batch or the pair order."""
+    u_ids = _req(u_ids, torch.int64, "u_ids").view(-1)
+    i_ids = _req(i_ids, torch.int64, "i_ids").view(-1)
+    user_out = _req(user_out, torch.float32, "user_out")
+    item_out = _req(item_out, torch.float32, "item_out")
+    user_mask = _mask_u8(user_mask, "user_mask")
+    item_mask = _mask_u8(item_mask, "item_mask")
+    w0 = _req(w0.detach(), torch.float32, "w0")
+    w3 = _req(w3.detach(), torch.float32, "w3")
+    if w0.dim() != 2 or w3.dim() != 2:
+        raise ValueError("rbr_b200: w0 [hidden, in_dim] and w3 [out_dim, hidden] expected")
+    hidden, in_dim = w0.shape
+    out_dim = w3.shape[0]
+    if not 1 <= hidden <= DATT_FC_MAX_HIDDEN:
+        raise ValueError(f"rbr_b200: datt_fc_grads takes 1 <= hidden <= {DATT_FC_MAX_HIDDEN}, got {hidden}")
+    if tuple(w3.shape) != (out_dim, hidden):
+        raise ValueError(f"rbr_b200: w3 must be [out_dim, {hidden}], got {tuple(w3.shape)}")
+    for out, mask, name in ((user_out, user_mask, "user"), (item_out, item_mask, "item")):
+        if out.dim() != 2 or out.shape[1] != out_dim or mask.dim() != 2 or tuple(mask.shape) != (out.shape[0], hidden):
+            raise ValueError(f"rbr_b200: {name}_out [n, {out_dim}] and {name}_mask [n, {hidden}] expected, got "
+                             f"{tuple(out.shape)} / {tuple(mask.shape)}")
+    P = u_ids.numel()
+    if i_ids.numel() != P:
+        raise ValueError("rbr_b200: u_ids and i_ids must hold one id per pair")
+    for t, name in ((i_ids, "i_ids"), (user_out, "user_out"), (item_out, "item_out"), (user_mask, "user_mask"),
+                    (item_mask, "item_mask"), (w0, "w0"), (w3, "w3")):
+        if t.device != u_ids.device:
+            raise ValueError(f"rbr_b200: `{name}` is on {t.device}, u_ids on {u_ids.device}")
+    if P:
+        lo_u, hi_u, lo_i, hi_i = torch.stack([u_ids.min(), u_ids.max(), i_ids.min(), i_ids.max()]).tolist()
+        if lo_u < 0 or hi_u >= user_out.shape[0] or lo_i < 0 or hi_i >= item_out.shape[0]:
+            raise ValueError(f"rbr_b200: user ids must lie in [0, {user_out.shape[0]}) and item ids in [0, {item_out.shape[0]})")
+    g_u = torch.empty(P, in_dim, dtype=torch.float32, device=u_ids.device)
+    g_i = torch.empty(P, in_dim, dtype=torch.float32, device=u_ids.device)
+    if P == 0:
+        return g_u, g_i
+    lib.check(lib.rbr_datt_fc_grads(_p(u_ids), _p(i_ids), P, _p(user_out), user_out.shape[0], _p(item_out), item_out.shape[0],
+                                    out_dim, _p(user_mask), _p(item_mask), hidden, _p(w0), in_dim, _p(w3), _p(g_u), _p(g_i),
+                                    _stream(True)), "rbr_datt_fc_grads")
+    return g_u, g_i
 
 
 def head_text_grads(u_text: torch.Tensor, i_text: torch.Tensor, u_id: torch.Tensor, i_id: torch.Tensor,
