@@ -338,12 +338,13 @@ extern "C" int rbr_datt_gate_fwd(const float* table, int64_t vocab, int64_t emb,
     cudaStream_t s = as_stream(stream);
     DattWs w = datt_ws(ws, n_docs, doc_len, emb, window, vocab);
     const int E = (int)emb, L = (int)doc_len, win = (int)window, Ep = (E + 3) & ~3;
+    // declined before anything is enqueued: the caller's workspace and outputs stay untouched
+    const size_t smem = ((size_t)((win * L + 3) & ~3) + (size_t)win * Ep + DA_WARPS) * 4;
+    RBR_REQUIRE(smem <= 200 * 1024, RBR_EUNSUPPORTED, "rbr_datt_gate_fwd: doc_len too large for shared memory");
     datt_transpose_kernel<<<4, 256, 0, s>>>(w_local, E, Ep, win, w.waT);
     RBR_LAUNCH_CHECK("datt_transpose(local)");
     datt_transpose_kernel<<<(Ep * L + 255) / 256, 256, 0, s>>>(w_global, E, Ep, L, w.wgT);
     RBR_LAUNCH_CHECK("datt_transpose(global)");
-    const size_t smem = ((size_t)((win * L + 3) & ~3) + (size_t)win * Ep + DA_WARPS) * 4;
-    RBR_REQUIRE(smem <= 200 * 1024, RBR_EUNSUPPORTED, "rbr_datt_gate_fwd: doc_len too large for shared memory");
     void (*kern)(const float*, int64_t, int, IdView, int, const float*, const float*, int, const float*, const float*, float*,
                  float*) = nullptr;
 #define RBR_GF(W_) case W_: kern = (E % 4 == 0) ? datt_gate_fwd_kernel<true, W_> : datt_gate_fwd_kernel<false, W_>; break;

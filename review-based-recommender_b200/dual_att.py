@@ -59,6 +59,7 @@ class DualAtt(HotPathModule):
                                 nn.Linear(hidden_size_1, hidden_size_2))
         self.precision = precision or default_precision()
         self.last_arena = None
+        self.conv_flags = 0             # ops.CONV_TC_* kernel-selection flags passed with every gated conv (tests, A/B timing)
 
     def invalidate_operand_cache(self):
         self.word_embeddings.invalidate_operand_cache()
@@ -84,7 +85,7 @@ class DualAtt(HotPathModule):
         table = self.word_embeddings.embedding.weight
         pidx = self.word_embeddings.padding_idx
         cfg = {"precision": self.precision, "shadow_fn": self.word_embeddings.bf16_shadow, "arena": arena,
-               "table_param": table, "params": params, "padding_idx": -1 if pidx is None else pidx}
+               "table_param": table, "params": params, "padding_idx": -1 if pidx is None else pidx, "flags": self.conv_flags}
         return list(ops.DattEncodeFn.apply(table, cfg, *args))
 
     def forward(self, u_docs, i_docs):

@@ -836,10 +836,16 @@ def head_dropout_mask(batch: int, latent: int, drop_p: float, drop_seed: int, se
 def conv_act_maxpool(table: torch.Tensor, ids: torch.Tensor, mask: Optional[torch.Tensor], weight: torch.Tensor,
                      bias: torch.Tensor, pad: int, act: int = ACT_RELU, precision: str = "bf16",
                      shadow: Optional[torch.Tensor] = None, packed: Optional[torch.Tensor] = None, flags: int = 0,
-                     mask_from_ids: bool = False, select_docs: bool = True, row_index_table: bool = True):
+                     mask_from_ids: bool = False, select_docs: bool = True, row_index_table: bool = True,
+                     gate: Optional[torch.Tensor] = None, gate_mode: int = 0, return_pool_raw: bool = False,
+                     feat_ld: Optional[int] = None):
     """One K2 launch: returns (feat [n_docs, H] fp32, argmax [n_docs, H] int32).  `flags`: CONV_TC_* kernel selection.
     `select_docs=False`: no scratch at all; `row_index_table=False`: scratch for the document selection only, so the kernel's
-    index warp resolves ids and masks itself (rbr_conv_fwd_workspace_bytes vs ..._bytes2)."""
+    index warp resolves ids and masks itself (rbr_conv_fwd_workspace_bytes vs ..._bytes2).
+    `gate` / `gate_mode`: D-ATT's gate, passed straight to the C-ABI (1: per token [n_docs, doc_len], k = 1; 2: per document
+    [n_docs]).  `return_pool_raw`: also return pool_raw [n_docs, H], the pooled value before bias and activation.
+    `feat_ld` (>= H): row stride of the outputs, which are then [n_docs, feat_ld]; columns H.. are NaN (feat, pool_raw) and
+    -1 (argmax) unless the kernel wrote past its filters."""
     table = _req(table, torch.float32, "table")
     ids = _ids(ids, "ids")
     flags |= _id_flags(ids, mask, mask_from_ids)
@@ -849,21 +855,30 @@ def conv_act_maxpool(table: torch.Tensor, ids: torch.Tensor, mask: Optional[torc
         shadow = table_to_bf16(table)
     if packed is None:
         packed = conv_pack(weight)
+    if gate is not None:
+        gate = _req(gate, torch.float32, "gate")
     h, emb, k = weight.shape
     doc_len = ids.shape[-1]
     n_docs = ids.numel() // doc_len
-    feat = torch.empty(n_docs, h, dtype=torch.float32, device=table.device)
-    amax = torch.empty(n_docs, h, dtype=torch.int32, device=table.device)
+    ld = h if feat_ld is None else feat_ld
+    dev = table.device
+    if ld > h:
+        feat = torch.full((n_docs, ld), float("nan"), device=dev)
+        amax = torch.full((n_docs, ld), -1, dtype=torch.int32, device=dev)
+    else:
+        feat = torch.empty(n_docs, h, dtype=torch.float32, device=dev)
+        amax = torch.empty(n_docs, h, dtype=torch.int32, device=dev)
+    pool_raw = torch.full((n_docs, ld), float("nan"), device=dev) if return_pool_raw else None
     ws_bytes = 0
     if prec == PREC_BF16 and select_docs:
         ws_bytes = (lib.rbr_conv_fwd_workspace_bytes2(n_docs, doc_len, k, pad) if row_index_table
                     else lib.rbr_conv_fwd_workspace_bytes(n_docs))
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=table.device) if ws_bytes else None
-    lib.check(lib.rbr_conv_act_maxpool_fwd(prec, act, _p(table), _p(shadow), table.shape[0], emb, _p(ids), _p(mask), None, 0,
-                                           n_docs, doc_len, _p(packed), _p(_req(bias, torch.float32, "bias")), h, k, pad,
-                                           _p(feat), _p(amax), None, h, _p(ws), ws_bytes, flags, _stream(True)),
+    lib.check(lib.rbr_conv_act_maxpool_fwd(prec, act, _p(table), _p(shadow), table.shape[0], emb, _p(ids), _p(mask), _p(gate),
+                                           gate_mode, n_docs, doc_len, _p(packed), _p(_req(bias, torch.float32, "bias")), h, k, pad,
+                                           _p(feat), _p(amax), _p(pool_raw), ld, _p(ws), ws_bytes, flags, _stream(True)),
               "rbr_conv_act_maxpool_fwd")
-    return feat, amax
+    return (feat, amax, pool_raw) if return_pool_raw else (feat, amax)
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -877,11 +892,12 @@ def datt_side_packs(prm: Sequence[torch.Tensor]) -> List[torch.Tensor]:
 
 def datt_encode_side(table: torch.Tensor, ids: torch.Tensor, prm: Sequence[torch.Tensor], precision: str = "bf16",
                      shadow: Optional[torch.Tensor] = None, packed: Optional[Sequence[torch.Tensor]] = None,
-                     stream: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+                     stream: Optional[int] = None, conv_flags: int = 0
+                     ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
     """One side of the D-ATT encoder forward (models/dual_att/layers.py:43-53, 81-89): K5's two gates, then the four gated
     tanh convs with max-over-time.  ids [n_docs, doc_len] int64 / int32; prm = the side's 12 parameters in DattEncodeFn's
     order; shadow = the bf16 table (bf16 only; made here when None); packed = datt_side_packs(prm) (made here when None);
-    stream = a raw stream handle (None: torch's current stream).
+    stream = a raw stream handle (None: torch's current stream); conv_flags = CONV_TC_* kernel selection for the four convs.
     Returns (feat [n_docs, l_out + 3 g_out], argmax int32, pre-activation at the arg-max, gate_local [n_docs, doc_len],
     gate_global [n_docs]); filter columns: local conv, then the k = 2, 3, 4 global convs."""
     table = _req(table, torch.float32, "embedding table")
@@ -920,7 +936,7 @@ def datt_encode_side(table: torch.Tensor, ids: torch.Tensor, prm: Sequence[torch
         lib.check(lib.rbr_conv_act_maxpool_fwd(prec, ACT_TANH, _p(table), _p(shadow), vocab, emb, _p(ids), None, _p(gate),
                                                mode, n_docs, doc_len, _p(pk), _p(b), h, k, 0, feat.data_ptr() + 4 * col,
                                                amax.data_ptr() + 4 * col, pre.data_ptr() + 4 * col, h_total, _p(ws), ws_bytes,
-                                               idf, s), "rbr_conv_act_maxpool_fwd")
+                                               idf | conv_flags, s), "rbr_conv_act_maxpool_fwd")
         col += h
     return feat, amax, pre, gate_l, gate_g
 
@@ -952,7 +968,8 @@ class DattEncodeFn(torch.autograd.Function):
             ids = _ids(rest[s * stride], "token ids")
             prm = [_req(t, torch.float32, "D-ATT parameter") for t in rest[s * stride + 1:(s + 1) * stride]]
             packed = datt_side_packs(prm)
-            feat, amax, pre, gate_l, gate_g = datt_encode_side(table, ids, prm, cfg["precision"], shadow, packed, _stream())
+            feat, amax, pre, gate_l, gate_g = datt_encode_side(table, ids, prm, cfg["precision"], shadow, packed, _stream(),
+                                                               cfg.get("flags", 0))
             saved += [ids, gate_l, gate_g, feat, amax, pre]
             feats.append(feat)
             side_ctx.append((prm, packed))

@@ -352,3 +352,15 @@ def test_narre_attn_pair_plan_boundary():
     assert not sup(65, 64, 32) and not sup(0, 64, 32)        # reviews in [1, 64]
     assert not sup(10, 150, 33) and not sup(10, 150, 0)      # att_dim in [1, 32]
     assert not sup(10, 0, 32)
+
+
+def test_datt_gate_entry_points_decline_unsupported_shapes_without_a_device():
+    """K5 takes E <= 128 and odd windows up to 7: the gate forward and backward return RBR_EUNSUPPORTED for E = 129, window 2
+    and window 9 before they look at any pointer (all NULL here) or touch a device."""
+    from rbr_b200._lib import lib
+    for emb, win in ((129, 5), (100, 2), (100, 9)):
+        assert lib.rbr_datt_gate_fwd(None, 10, emb, None, 1, 8, None, None, win, None, None, None, None, None, 0, 0, None) == -4
+        assert b"rbr_datt_gate_fwd" in lib.rbr_last_error()
+        assert lib.rbr_datt_gate_bwd(None, 10, emb, None, 1, 8, None, win, None, None, None, None, None, 0, None, None, None,
+                                     None, None, None, 0, 0, None) == -4
+        assert b"rbr_datt_gate_bwd" in lib.rbr_last_error()
