@@ -466,6 +466,40 @@ int rbr_datt_fc_grads(const int64_t* u_ids, const int64_t* i_ids, int64_t n_pair
                       const uint8_t* item_mask, int64_t hidden, const float* w0, int64_t in_dim, const float* w3,
                       float* g_user, float* g_item, void* stream);
 
+/* ---- K13: token attributions for SimpleSiamese (masked average pooling + additive review attention) -----------------------
+ * One side of an entity in eval mode (models/simple_siamese/simple_siamese.py:55-88): reviews r < R of T tokens, pooled
+ * p_r = sum_t m[r,t] x[r,t] / (n_r + 1e-8) (K9; n_r = the review's masked-in tokens), v_r = tanh(Lt p_r + bt) with the latent
+ * transform (else v_r = p_r), s = softmax(l) with l_r = w . tanh(P v_r + c) (-1e8 where the review mask is false), and the side
+ * feature f = sum_r s_r v_r.  With g = d pred / d f, gradient x input on the embedded tokens is
+ *   a_r  = P^T (w * (1 - tanh^2(P v_r + c)))          (0 for a masked review: its logit is a constant)
+ *   dv_r = s_r (g + (g . (v_r - f)) a_r),   G_r = Lt^T ((1 - v_r^2) * dv_r)   (G_r = dv_r without the latent transform)
+ *   attr[r,t] = m[r,t] (x[r,t] . G_r) / (n_r + 1e-8)
+ * where a_r, v_r, s_r and f depend on the entity alone (kept per entity at cache build time).
+ *
+ * rbr_explain_avgpool_attrib: n_rows (pair, side) rows; row p is entity ent[p] of this side, whose reviews are
+ * ids [n_ent, reviews, doc_len] (`flags`: RBR_IDS_I32 / RBR_IDS_U16, RBR_MASK_FROM_IDS) with word mask [same shape] (NULL: as
+ * `flags` say); x rows read as zeros where the mask is false and for ids outside [0, vocab).  Per entity: v, att_a [n_ent,
+ * reviews, feat] (v_r, a_r), att_s [n_ent, reviews] (s_r), f [n_ent, feat].  lt_w = Lt [feat, emb] (latent_transform_layer's
+ * weight) or NULL (then feat == emb).  g: [n_rows, feat], or NULL to form it from the FM head at its ReLU decision,
+ *   g = w_side (fm_h * 1[lat[ent] * lat_other[other] > 0] * lat_other[other])        (summed over k = 0 .. latent-1 in order)
+ * with lat [n_ent, latent] / lat_other [n_other, latent] the two sides' LastFeat outputs, other [n_rows] the pair's other
+ * entity, w_side [feat, latent] this side's LastFeat.W and fm_h [latent].  Writes rbr_explain_attrib's outputs for one
+ * document of reviews * doc_len flat positions: text_total, top / bottom windows of `width` positions (never across a review),
+ * optional map [n_rows, reviews * doc_len] and review_attr [n_rows, reviews].  Each position's term is one fp32 dot rounded once
+ * onto the fixed-point grid, so text_total is the map's exact sum and every output is bit-identical across calls, batches and
+ * row orders.  A row whose ent (or other) lies outside its table gets NaN / -1.
+ * Limits (rbr_explain_avgpool_supported, host-only): positions = reviews * doc_len with 1 <= positions <= 16384, 1 <= m <= 32,
+ * 1 <= width <= 16, and the row's shared memory — 13 * positions + 4 * (feat + 2 reviews + reviews * (feat + emb)) bytes,
+ * roughly — at most 227 KB; otherwise rbr_explain_avgpool_attrib returns RBR_EUNSUPPORTED before any launch.                */
+int rbr_explain_avgpool_supported(int64_t positions, int64_t reviews, int64_t emb, int64_t feat, int64_t m, int64_t width);
+int rbr_explain_avgpool_attrib(const float* table, int64_t vocab, int64_t emb, const void* ids, const uint8_t* mask,
+                               int64_t n_ent, int64_t reviews, int64_t doc_len, const int64_t* ent, int64_t n_rows,
+                               const float* g, const int64_t* other, const float* lat, const float* lat_other, int64_t n_other,
+                               const float* w_side, const float* fm_h, int64_t latent, const float* v, const float* att_a,
+                               const float* att_s, const float* f, int64_t feat, const float* lt_w, int64_t m, int64_t width,
+                               float* text_total, int64_t* top_pos, float* top_attr, int64_t* bottom_pos, float* bottom_attr,
+                               float* map, float* review_attr, int flags, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

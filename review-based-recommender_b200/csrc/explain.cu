@@ -155,6 +155,14 @@ struct ExConvs {
 __host__ __device__ inline int64_t ex_dscal_off(int64_t S) { return (S * 13 + 7) & ~(int64_t)7; }
 __host__ inline size_t ex_smem_bytes(int64_t S, int64_t R, bool dense) { return (size_t)(ex_dscal_off(S) + (dense ? R * 8 : 0)); }
 
+// where a row's outputs go: text_total [P], top / bottom windows [P, m], map [P, R*T] and review_attr [P, R] (both optional)
+struct ExOut {
+    float* text_total;
+    int64_t* top_pos; float* top_attr; int64_t* bot_pos; float* bot_attr;
+    float* map;
+    float* review_attr;
+};
+
 struct ExArgs {
     const int64_t* ent_row;
     const float* g;          // [P, R, Htot]
@@ -166,10 +174,7 @@ struct ExArgs {
     int64_t n_docs, feat_ld, contrib_ld, coef_ld, vec_ld, htot;
     int R, T, m, width;
     ExConvs cv;
-    float* text_total;       // [P]
-    int64_t* top_pos; float* top_attr; int64_t* bot_pos; float* bot_attr;   // [P, m]
-    float* map;              // [P, R*T] or NULL
-    float* review_attr;      // [P, R] or NULL
+    ExOut out;
 };
 
 __device__ __forceinline__ int ex_conv_of(const ExConvs& cv, int hh) {
@@ -179,7 +184,7 @@ __device__ __forceinline__ int ex_conv_of(const ExConvs& cv, int hh) {
 }
 
 // block-wide reductions (EX_THREADS threads); `red` holds EX_THREADS / 32 entries of the widest type
-__device__ float ex_block_max(float v, double* red) {
+__device__ __forceinline__ float ex_block_max(float v, double* red) {
     v = warp_max(v);
     __syncthreads();
     if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
@@ -189,13 +194,13 @@ __device__ float ex_block_max(float v, double* red) {
     return r;
 }
 
-__device__ long long ex_warp_sum_ll(long long v) {
+__device__ __forceinline__ long long ex_warp_sum_ll(long long v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
 
-__device__ long long ex_block_sum_ll(long long v, double* red) {
+__device__ __forceinline__ long long ex_block_sum_ll(long long v, double* red) {
     v = ex_warp_sum_ll(v);
     long long* r = reinterpret_cast<long long*>(red);
     __syncthreads();
@@ -214,7 +219,7 @@ __device__ __forceinline__ bool ex_better(double v, int s, double bv, int bs, bo
     return s < bs;
 }
 
-__device__ void ex_block_pick(double& v, int& s, bool top, double* red_v, int* red_s) {
+__device__ __forceinline__ void ex_block_pick(double& v, int& s, bool top, double* red_v, int* red_s) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         const double ov = __shfl_xor_sync(0xffffffffu, v, o);
@@ -227,6 +232,77 @@ __device__ void ex_block_pick(double& v, int& s, bool top, double* red_v, int* r
     v = 0.0; s = -1;
     for (int w = 0; w < EX_THREADS / 32; ++w)
         if (ex_better(red_v[w], red_s[w], v, s, top)) { v = red_v[w]; s = red_s[w]; }
+}
+
+// The fixed-point grid of a row whose |total| is at most n_terms * mx: with mx * n_terms < 2^e, terms on a grid of 2^(e-61)
+// keep every partial sum below 2^61 in magnitude.  0 when there is nothing to add.
+__device__ __forceinline__ double ex_fixed_scale(float mx, double n_terms) {
+    double scale = 0.0;
+    if (mx > 0.f && isfinite(mx)) {
+        int e;
+        frexp((double)mx * n_terms, &e);
+        scale = ldexp(1.0, 61 - e);
+    }
+    return scale;
+}
+
+// Everything of row p after its fixed-point map acc [S] (S = R * T) and total are known: text_total, the fp32 map (mapf and,
+// if asked, out.map), the per-review sums and the top / bottom windows of `width` positions (greedy without overlap, ties to
+// the lower start, never across a review).  A row that is not `ok` gets NaN / -1.  Block-wide; acc becomes the window sums.
+__device__ __forceinline__ void ex_emit_row(long long* acc, float* mapf, uint8_t* avail, double* red_v, int* red_s, long long tot,
+                            double scale, bool ok, int64_t p, int R, int T, int m, int w, const ExOut& out) {
+    const int S = R * T;
+    const float nanf_ = __int_as_float(0x7fc00000);
+    const double inv = scale > 0.0 ? 1.0 / scale : 0.0;
+    if (threadIdx.x == 0) out.text_total[p] = ok ? (float)((double)tot * inv) : nanf_;
+    __syncthreads();                                                   // the map has landed
+    for (int i = threadIdx.x; i < S; i += EX_THREADS) {
+        const float v = ok ? (float)((double)acc[i] * inv) : nanf_;
+        mapf[i] = v;
+        if (out.map) out.map[p * S + i] = v;
+    }
+    if (out.review_attr) {
+        for (int r = threadIdx.x >> 5; r < R; r += EX_THREADS / 32) {
+            long long s = 0;
+            for (int t = threadIdx.x & 31; t < T; t += 32) s += acc[r * T + t];
+            s = ex_warp_sum_ll(s);
+            if ((threadIdx.x & 31) == 0) out.review_attr[p * R + r] = ok ? (float)((double)s * inv) : nanf_;
+        }
+    }
+    __syncthreads();                                                   // acc is read for the last time above
+    double* wsum = reinterpret_cast<double*>(acc);
+    for (int s = threadIdx.x; s < S; s += EX_THREADS) {
+        double v = 0.0;
+        if ((s % T) + w <= T)
+            for (int j = 0; j < w; ++j) v += (double)mapf[s + j];
+        wsum[s] = v;
+    }
+    for (int pass = 0; pass < 2; ++pass) {
+        const bool top = pass == 0;
+        int64_t* out_pos = (top ? out.top_pos : out.bot_pos) + p * m;
+        float* out_attr = (top ? out.top_attr : out.bot_attr) + p * m;
+        for (int s = threadIdx.x; s < S; s += EX_THREADS) avail[s] = ok && (s % T) + w <= T;
+        __syncthreads();
+        for (int it = 0; it < m; ++it) {
+            double bv = 0.0;
+            int bs = -1;
+            for (int s = threadIdx.x; s < S; s += EX_THREADS)
+                if (avail[s] && ex_better(wsum[s], s, bv, bs, top)) { bv = wsum[s]; bs = s; }
+            ex_block_pick(bv, bs, top, red_v, red_s);
+            if (threadIdx.x == 0) {
+                out_pos[it] = bs;
+                out_attr[it] = bs >= 0 ? (float)bv : nanf_;
+            }
+            if (bs < 0) {
+                for (int j = it + 1 + (int)threadIdx.x; j < m; j += EX_THREADS) { out_pos[j] = -1; out_attr[j] = nanf_; }
+                break;
+            }
+            // windows never cross a review boundary, so every start whose window overlaps [bs, bs + w) lies in (bs - w, bs + w)
+            for (int s = max(0, bs - w + 1) + (int)threadIdx.x; s < min(S, bs + w); s += EX_THREADS) avail[s] = 0;
+            __syncthreads();
+        }
+        __syncthreads();
+    }
 }
 
 __global__ void __launch_bounds__(EX_THREADS) explain_attrib_kernel(const ExArgs a) {
@@ -281,14 +357,8 @@ __global__ void __launch_bounds__(EX_THREADS) explain_attrib_kernel(const ExArgs
         }
     }
     mx = ex_block_max(mx, red_v);
-    // |total| <= (n_items * max_k + dense positions) * mx < 2^e  →  terms on a grid of 2^(e-61): every partial sum stays
-    // below 2^61 in magnitude
-    double scale = 0.0;
-    if (mx > 0.f && isfinite(mx)) {
-        int e;
-        frexp((double)mx * ((double)n_items * (double)max_k + (dense ? (double)S : 0.0)), &e);
-        scale = ldexp(1.0, 61 - e);
-    }
+    // |total| <= (n_items * max_k + dense positions) * mx
+    const double scale = ex_fixed_scale(mx, (double)n_items * (double)max_k + (dense ? (double)S : 0.0));
     __syncthreads();
     // pass 2: scatter the rounded terms; every term enters the total, the ones at a position inside the document also the map
     long long tot = 0;
@@ -321,58 +391,160 @@ __global__ void __launch_bounds__(EX_THREADS) explain_attrib_kernel(const ExArgs
         }
     }
     tot = ex_block_sum_ll(tot, red_v);
-    const float nanf_ = __int_as_float(0x7fc00000);
-    const double inv = scale > 0.0 ? 1.0 / scale : 0.0;
-    if (threadIdx.x == 0) a.text_total[p] = ok ? (float)((double)tot * inv) : nanf_;
-    __syncthreads();                                                   // the atomics have landed
+    ex_emit_row(acc, mapf, avail, red_v, red_s, tot, scale, ok, p, a.R, a.T, a.m, a.width, a.out);
+}
+
+// ---- K13: SimpleSiamese — gradient x input through masked average pooling and the review attention ------------------------
+// One side of an entity (models/simple_siamese/simple_siamese.py:55-88, eval mode): pooled p_r = sum_t m x / (n_r + 1e-8),
+// v_r = tanh(Lt p_r + bt) (or p_r), s = softmax(l), l_r = w . tanh(P v_r + c) (-1e8 where the review is masked), f = sum_r s_r v_r.
+// With g = d pred / d f and the per-entity a_r = P^T (w * (1 - tanh^2(P v_r + c))) (0 for a masked review):
+//   dv_r = s_r (g + (g . (v_r - f)) a_r),   G_r = Lt^T ((1 - v_r^2) * dv_r) (or dv_r),   attr[r,t] = m x[r,t] . G_r / (n_r + 1e-8)
+// Every token has exactly one term, so the map is one fp32 dot per position, rounded once onto K12b's fixed-point grid.
+constexpr int XA_RB = 4;      // reviews per pass of the G_r product (each Lt element read once per XA_RB reviews)
+
+struct XaArgs {
+    const float* table;
+    int64_t vocab, emb;
+    IdView iv;
+    const uint8_t* mask;     // [n_ent, R, T] or NULL (iv.mask_ids: ids != 0)
+    int64_t n_ent;
+    int R, T, F, K;
+    const int64_t* ent;      // [P] entity of each row
+    const float* g;          // [P, F] d pred / d f, or NULL: from the latents below
+    const int64_t* other;    // [P] the pair's other entity
+    const float* lat;        // [n_ent, K] this side's LastFeat outputs
+    const float* lat_other;  // [n_other, K]
+    int64_t n_other;
+    const float* w_side;     // [F, K] this side's LastFeat.W
+    const float* fm_h;       // [K]
+    const float* v;          // [n_ent, R, F]
+    const float* att_a;      // [n_ent, R, F]
+    const float* att_s;      // [n_ent, R]
+    const float* f;          // [n_ent, F]
+    const float* lt_w;       // [F, emb] or NULL (F == emb)
+    int m, width;
+    ExOut out;
+};
+
+// dynamic shared memory: K12b's map region, then g [F], dots [R], 1 / (n_r + 1e-8) [R], dv [R, F], G [R, emb]
+__host__ __device__ inline int64_t xa_smem_bytes(int64_t R, int64_t T, int64_t emb, int64_t F) {
+    return ex_dscal_off(R * T) + 4 * (F + 2 * R + R * F + R * emb);
+}
+
+__global__ void __launch_bounds__(EX_THREADS) explain_avgpool_attrib_kernel(const XaArgs a) {
+    extern __shared__ __align__(16) unsigned char ex_smem[];
+    __shared__ double red_v[EX_THREADS / 32];
+    __shared__ int red_s[EX_THREADS / 32];
+    const int R = a.R, T = a.T, S = R * T, F = a.F, E = (int)a.emb;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    long long* acc = reinterpret_cast<long long*>(ex_smem);
+    float* mapf = reinterpret_cast<float*>(acc + S);
+    uint8_t* avail = reinterpret_cast<uint8_t*>(mapf + S);
+    float* gv = reinterpret_cast<float*>(ex_smem + ex_dscal_off(S));
+    float* dots = gv + F;
+    float* inv_n = dots + R;
+    float* dv = inv_n + R;
+    float* G = dv + R * F;
+    const int64_t p = blockIdx.x;
+    const int64_t e = __ldg(a.ent + p);
+    const int64_t o = a.g ? 0 : __ldg(a.other + p);
+    const bool ok = e >= 0 && e < a.n_ent && (a.g || (o >= 0 && o < a.n_other));   // the host validates; else NaN / -1
+    if (ok) {
+        // g: given, or W_side (h * 1[lat * lat_other > 0] * lat_other), k in order
+        for (int i = threadIdx.x; i < F; i += EX_THREADS) {
+            float x = 0.f;
+            if (a.g) {
+                x = __ldg(a.g + p * F + i);
+            } else {
+                const float* ls = a.lat + e * a.K;
+                const float* lo = a.lat_other + o * a.K;
+                for (int k = 0; k < a.K; ++k) {
+                    const float us = __ldg(ls + k), ot = __ldg(lo + k);
+                    if ((us > 0.f && ot > 0.f) || (us < 0.f && ot < 0.f))
+                        x = fmaf(__ldg(a.w_side + (int64_t)i * a.K + k), __ldg(a.fm_h + k) * ot, x);
+                }
+            }
+            gv[i] = x;
+        }
+        // the forward's token count per review (masked-in ids outside the table count, as in K9)
+        for (int r = warp; r < R; r += EX_THREADS / 32) {
+            int c = 0;
+            for (int t = lane; t < T; t += 32) {
+                const int64_t idx = (e * R + r) * T + t;
+                c += ld_mask(a.iv, a.mask, idx, ld_id(a.iv, idx)) ? 1 : 0;
+            }
+#pragma unroll
+            for (int s = 16; s > 0; s >>= 1) c += __shfl_xor_sync(0xffffffffu, c, s);
+            if (lane == 0) inv_n[r] = 1.f / ((float)c + 1e-8f);
+        }
+        __syncthreads();
+        const float* vr = a.v + e * R * F;
+        const float* fe = a.f + e * F;
+        for (int r = warp; r < R; r += EX_THREADS / 32) {
+            float d = 0.f;
+            for (int i = lane; i < F; i += 32) d = fmaf(gv[i], __ldg(vr + r * F + i) - __ldg(fe + i), d);
+            d = warp_sum(d);
+            if (lane == 0) dots[r] = d;
+        }
+        __syncthreads();
+        const float* ar = a.att_a + e * R * F;
+        for (int i = threadIdx.x; i < R * F; i += EX_THREADS) {
+            const int r = i / F;
+            float d = __ldg(a.att_s + e * R + r) * fmaf(dots[r], __ldg(ar + i), gv[i % F]);
+            if (a.lt_w) {
+                const float vv = __ldg(vr + i);
+                d *= 1.f - vv * vv;
+            }
+            dv[i] = d;
+        }
+        __syncthreads();
+        // G[r, c] = (sum_k Lt[k, c] dv[r, k]) / (n_r + 1e-8), k in order
+        if (a.lt_w) {
+            for (int i = threadIdx.x; i < ((R + XA_RB - 1) / XA_RB) * E; i += EX_THREADS) {
+                const int r0 = (i / E) * XA_RB, c = i % E;
+                float x[XA_RB] = {};
+                for (int k = 0; k < F; ++k) {
+                    const float wk = __ldg(a.lt_w + (int64_t)k * E + c);
+#pragma unroll
+                    for (int j = 0; j < XA_RB; ++j)
+                        if (r0 + j < R) x[j] = fmaf(wk, dv[(r0 + j) * F + k], x[j]);
+                }
+#pragma unroll
+                for (int j = 0; j < XA_RB; ++j)
+                    if (r0 + j < R) G[(r0 + j) * E + c] = x[j] * inv_n[r0 + j];
+            }
+        } else {
+            for (int i = threadIdx.x; i < R * E; i += EX_THREADS) G[i] = dv[i] * inv_n[i / E];
+        }
+        __syncthreads();
+        // one warp per position: attr = x . G_r (0 where masked and for ids outside the table)
+        const int64_t base = e * S;
+        for (int i = warp; i < S; i += EX_THREADS / 32) {
+            const int64_t id = ld_id(a.iv, base + i);
+            float s = 0.f;
+            if (ld_mask(a.iv, a.mask, base + i, id) && id >= 0 && id < a.vocab) {
+                const float* x = a.table + id * E;
+                const float* gr = G + (i / T) * E;
+                for (int c = lane; c < E; c += 32) s = fmaf(__ldg(x + c), gr[c], s);
+                s = warp_sum(s);
+            }
+            if (lane == 0) mapf[i] = s;
+        }
+    }
+    __syncthreads();
+    float mx = 0.f;
+    if (ok)
+        for (int i = threadIdx.x; i < S; i += EX_THREADS) mx = fmaxf(mx, fabsf(mapf[i]));
+    mx = ex_block_max(mx, red_v);
+    const double scale = ex_fixed_scale(mx, (double)S);                // one term per position: |total| <= S * mx
+    long long tot = 0;
     for (int i = threadIdx.x; i < S; i += EX_THREADS) {
-        const float v = ok ? (float)((double)acc[i] * inv) : nanf_;
-        mapf[i] = v;
-        if (a.map) a.map[p * S + i] = v;
+        const long long q = (ok && scale > 0.0) ? llrint((double)mapf[i] * scale) : 0;
+        acc[i] = q;
+        tot += q;
     }
-    if (a.review_attr) {
-        for (int r = threadIdx.x >> 5; r < a.R; r += EX_THREADS / 32) {
-            long long s = 0;
-            for (int t = threadIdx.x & 31; t < a.T; t += 32) s += acc[r * a.T + t];
-            s = ex_warp_sum_ll(s);
-            if ((threadIdx.x & 31) == 0) a.review_attr[p * a.R + r] = ok ? (float)((double)s * inv) : nanf_;
-        }
-    }
-    __syncthreads();                                                   // acc is read for the last time above
-    double* wsum = reinterpret_cast<double*>(acc);
-    const int w = a.width;
-    for (int s = threadIdx.x; s < S; s += EX_THREADS) {
-        double v = 0.0;
-        if ((s % a.T) + w <= a.T)
-            for (int j = 0; j < w; ++j) v += (double)mapf[s + j];
-        wsum[s] = v;
-    }
-    for (int pass = 0; pass < 2; ++pass) {
-        const bool top = pass == 0;
-        int64_t* out_pos = (top ? a.top_pos : a.bot_pos) + p * a.m;
-        float* out_attr = (top ? a.top_attr : a.bot_attr) + p * a.m;
-        for (int s = threadIdx.x; s < S; s += EX_THREADS) avail[s] = ok && (s % a.T) + w <= a.T;
-        __syncthreads();
-        for (int it = 0; it < a.m; ++it) {
-            double bv = 0.0;
-            int bs = -1;
-            for (int s = threadIdx.x; s < S; s += EX_THREADS)
-                if (avail[s] && ex_better(wsum[s], s, bv, bs, top)) { bv = wsum[s]; bs = s; }
-            ex_block_pick(bv, bs, top, red_v, red_s);
-            if (threadIdx.x == 0) {
-                out_pos[it] = bs;
-                out_attr[it] = bs >= 0 ? (float)bv : nanf_;
-            }
-            if (bs < 0) {
-                for (int j = it + 1 + (int)threadIdx.x; j < a.m; j += EX_THREADS) { out_pos[j] = -1; out_attr[j] = nanf_; }
-                break;
-            }
-            // windows never cross a review boundary, so every start whose window overlaps [bs, bs + w) lies in (bs - w, bs + w)
-            for (int s = max(0, bs - w + 1) + (int)threadIdx.x; s < min(S, bs + w); s += EX_THREADS) avail[s] = 0;
-            __syncthreads();
-        }
-        __syncthreads();
-    }
+    tot = ex_block_sum_ll(tot, red_v);
+    ex_emit_row(acc, mapf, avail, red_v, red_s, tot, scale, ok, p, R, T, a.m, a.width, a.out);
 }
 
 // ---- D-ATT: g = d pred / d cat per pair and side, through the shared FC stack (dual_att.py:31-35, 51, 57-61) ----------------
@@ -563,8 +735,7 @@ extern "C" int rbr_explain_attrib_ex(const int64_t* ent_row, int64_t n_rows, int
     a.dense_coef = dense_coef; a.dense_vec = dense_vec; a.coef_ld = dense_coef_ld; a.vec_ld = dense_vec_ld;
     a.n_docs = n_docs; a.feat_ld = feat_ld; a.contrib_ld = contrib_ld; a.htot = hcol;
     a.R = (int)docs_per_entity; a.T = (int)doc_len; a.m = (int)m; a.width = (int)width;
-    a.text_total = text_total; a.top_pos = top_pos; a.top_attr = top_attr; a.bot_pos = bottom_pos; a.bot_attr = bottom_attr;
-    a.map = map; a.review_attr = review_attr;
+    a.out = {text_total, top_pos, top_attr, bottom_pos, bottom_attr, map, review_attr};
     RBR_CUDA(cudaFuncSetAttribute(explain_attrib_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     explain_attrib_kernel<<<(unsigned)n_rows, EX_THREADS, smem, as_stream(stream)>>>(a);
     RBR_LAUNCH_CHECK("explain_attrib_kernel");
@@ -579,6 +750,53 @@ extern "C" int rbr_explain_attrib(const int64_t* ent_row, int64_t n_rows, int64_
     return rbr_explain_attrib_ex(ent_row, n_rows, docs_per_entity, doc_len, g, feat, argmax, feat_ld, contrib, contrib_ld, n_docs,
                                  n_conv, host_convs, nullptr, 0, nullptr, 0, m, width, text_total, top_pos, top_attr, bottom_pos,
                                  bottom_attr, map, review_attr, stream);
+}
+
+static bool xa_supported(int64_t positions, int64_t reviews, int64_t emb, int64_t feat, int64_t m, int64_t width) {
+    return reviews >= 1 && positions >= reviews && positions % reviews == 0 && emb >= 1 && feat >= 1 &&
+           ex_supported(positions, m, width, 1) && xa_smem_bytes(reviews, positions / reviews, emb, feat) <= EX_MAX_SMEM;
+}
+
+extern "C" int rbr_explain_avgpool_supported(int64_t positions, int64_t reviews, int64_t emb, int64_t feat, int64_t m,
+                                             int64_t width) {
+    return xa_supported(positions, reviews, emb, feat, m, width) ? 1 : 0;
+}
+
+extern "C" int rbr_explain_avgpool_attrib(const float* table, int64_t vocab, int64_t emb, const void* ids, const uint8_t* mask,
+                                          int64_t n_ent, int64_t reviews, int64_t doc_len, const int64_t* ent, int64_t n_rows,
+                                          const float* g, const int64_t* other, const float* lat, const float* lat_other,
+                                          int64_t n_other, const float* w_side, const float* fm_h, int64_t latent,
+                                          const float* v, const float* att_a, const float* att_s, const float* f, int64_t feat,
+                                          const float* lt_w, int64_t m, int64_t width, float* text_total, int64_t* top_pos,
+                                          float* top_attr, int64_t* bottom_pos, float* bottom_attr, float* map,
+                                          float* review_attr, int flags, void* stream) {
+    RBR_REQUIRE(reviews >= 1 && doc_len >= 1 && xa_supported(reviews * doc_len, reviews, emb, feat, m, width), RBR_EUNSUPPORTED,
+                "rbr_explain_avgpool_attrib: need 1 <= reviews * doc_len <= %d, 1 <= m <= %d, 1 <= width <= %d and %lld bytes "
+                "of shared memory at most %d (got %lld x %lld, emb=%lld, feat=%lld, m=%lld, width=%lld)", EX_MAX_POSITIONS,
+                EX_MAX_M, EX_MAX_WIDTH, (long long)(reviews >= 1 && doc_len >= 1 ? xa_smem_bytes(reviews, doc_len, emb, feat) : 0),
+                EX_MAX_SMEM, (long long)reviews, (long long)doc_len, (long long)emb, (long long)feat, (long long)m,
+                (long long)width);
+    RBR_REQUIRE(n_ent >= 0 && n_rows >= 0 && vocab >= 1 && (lt_w || feat == emb) && (g || (latent >= 1 && n_other >= 0)),
+                RBR_EINVAL, "rbr_explain_avgpool_attrib: bad shape (n_ent=%lld n_rows=%lld vocab=%lld emb=%lld feat=%lld "
+                "latent=%lld; without the latent transform feat must equal emb)", (long long)n_ent, (long long)n_rows,
+                (long long)vocab, (long long)emb, (long long)feat, (long long)latent);
+    if (n_rows == 0) return RBR_OK;
+    RBR_REQUIRE(table && ids && ent && v && att_a && att_s && f && text_total && top_pos && top_attr && bottom_pos &&
+                    bottom_attr && (g || (other && lat && lat_other && w_side && fm_h)),
+                RBR_EINVAL, "rbr_explain_avgpool_attrib: null pointer");
+    XaArgs a;
+    a.table = table; a.vocab = vocab; a.emb = emb; a.iv = id_view(ids, flags); a.mask = mask; a.n_ent = n_ent;
+    a.R = (int)reviews; a.T = (int)doc_len; a.F = (int)feat; a.K = g ? 0 : (int)latent;
+    a.ent = ent; a.g = g; a.other = other; a.lat = lat; a.lat_other = lat_other; a.n_other = n_other;
+    a.w_side = w_side; a.fm_h = fm_h;
+    a.v = v; a.att_a = att_a; a.att_s = att_s; a.f = f; a.lt_w = lt_w;
+    a.m = (int)m; a.width = (int)width;
+    a.out = {text_total, top_pos, top_attr, bottom_pos, bottom_attr, map, review_attr};
+    const size_t smem = (size_t)xa_smem_bytes(reviews, doc_len, emb, feat);
+    RBR_CUDA(cudaFuncSetAttribute(explain_avgpool_attrib_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    explain_avgpool_attrib_kernel<<<(unsigned)n_rows, EX_THREADS, smem, as_stream(stream)>>>(a);
+    RBR_LAUNCH_CHECK("explain_avgpool_attrib_kernel");
+    return RBR_OK;
 }
 
 extern "C" int rbr_datt_explain_contrib(const float* table, int64_t vocab, int64_t emb, const void* ids, int64_t n_docs,

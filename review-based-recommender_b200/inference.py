@@ -11,6 +11,8 @@ encoder work.  In eval mode every model puts an entity's side through that entit
   NARRE     the entity's reviews (K2) + LinearAttention over the ids of the counterparts they review → [U, H] / [I, H];
             pairs score through K1 + K4 as for DeepCoNN;
   D-ATT     fc(encode(document)) per side → [U, 50] / [I, 50]; a pair's score is the dot product of its two rows.
+  SimpleSiamese  the entity's reviews, masked average pooling (K9), the optional latent transform and the review attention
+            (SimpleSiamese.encode_side) → [U, F] / [I, F]; pairs score through the model's own head (K4 where it is fused).
 
 `PairScorer.recommend` answers "the k best items for these users out of the whole catalogue" with K10 (ops.factor_topk),
 which never materialises the users x items score matrix; `rank_items` / `evaluate` give the exact full-catalogue rank of
@@ -29,8 +31,9 @@ import torch
 from . import ops
 from .deepconn import DeepCoNNpp
 from .dual_att import DualAtt
-from .layers import fused_head
+from .layers import FM, fused_head
 from .narre import NARRE
+from .simple_siamese import SimpleSiamese
 
 
 def fm_factors(u_lat: torch.Tensor, i_lat: torch.Tensor, h: torch.Tensor, user_bias: torch.Tensor, item_bias: torch.Tensor,
@@ -52,10 +55,14 @@ def _is_datt(model) -> bool:
     return isinstance(model, DualAtt)
 
 
+def _is_siamese(model) -> bool:
+    return isinstance(model, SimpleSiamese)
+
+
 class PairScorer:
     def __init__(self, model):
-        if not isinstance(model, (DeepCoNNpp, NARRE, DualAtt)):
-            raise TypeError("PairScorer serves DeepCoNNpp, NARRE and DualAtt")
+        if not isinstance(model, (DeepCoNNpp, NARRE, DualAtt, SimpleSiamese)):
+            raise TypeError("PairScorer serves DeepCoNNpp, NARRE, DualAtt and SimpleSiamese")
         self.model = model.eval()
         self.user_feat: Optional[torch.Tensor] = None
         self.item_feat: Optional[torch.Tensor] = None
@@ -71,21 +78,31 @@ class PairScorer:
     @torch.no_grad()
     def build_cache(self, user_docs: torch.Tensor, item_docs: torch.Tensor, user_masks: Optional[torch.Tensor] = None,
                     item_masks: Optional[torch.Tensor] = None, chunk: int = 4096, *, user_rev_ids: Optional[torch.Tensor] = None,
-                    item_rev_ids: Optional[torch.Tensor] = None, explain: bool = False) -> None:
+                    item_rev_ids: Optional[torch.Tensor] = None, user_rev_masks: Optional[torch.Tensor] = None,
+                    item_rev_masks: Optional[torch.Tensor] = None, explain: bool = False) -> None:
         """Row e of every argument belongs to entity id e (row 0 = the padding entity).
         DeepCoNN: user_docs [U, L], item_docs [I, L]; masks default to ids != 0 (utils.py:30-42).
         NARRE: user_docs [U, R, T], item_docs [I, R, T] (the entity's reviews), optional masks of the same shapes, and
           user_rev_ids [U, R] / item_rev_ids [I, R]: the ids of the items a user reviewed / the users who reviewed an item —
           what NARRE's dataset supplies as reuid / reiid for a pair with that entity.
         D-ATT: user_docs [U, L], item_docs [I, L] (no masks).
+        SimpleSiamese: user_docs [U, R_u, T], item_docs [I, R_i, T] (the entity's reviews; R_u and R_i may differ), optional
+          word masks of the same shapes (default ids != 0) and user_rev_masks [U, R_u] / item_rev_masks [I, R_i] (default:
+          the review has a masked-in word, models/simple_siamese/utils.py get_rev_mask).
         explain=True also keeps what `explain` needs per entity (references to the documents and masks; for DeepCoNN and
         NARRE the conv arg-max and the tap contributions of every pooled window (K12a), for NARRE the per-review features
         and attention weights; for D-ATT the two K5 gates, the conv arg-max, the FC hidden ReLU mask and the per-entity
-        terms of gradient x input, rbr_datt_explain_contrib).  The cached features are the same either way."""
+        terms of gradient x input, rbr_datt_explain_contrib; for SimpleSiamese the attention's inputs v, weights s and
+        logit gradients a (K13), and the LastFeat outputs where the head is not fused).  The cached features are the same
+        either way."""
         m = self.model
         self.model.eval()
         self._factors = None
         self._explain = None
+        if _is_siamese(m):
+            self._build_siamese_cache(user_docs, item_docs, user_masks, item_masks, user_rev_masks, item_rev_masks, chunk,
+                                      explain)
+            return
         if explain and not _is_datt(m) and m.ngram.arch != "CNN":
             raise NotImplementedError("PairScorer.explain covers the CNN encoder; arch='HierPooling' pools averages, "
                                       "which have no per-window tap contributions")
@@ -229,6 +246,49 @@ class PairScorer:
                            "att": torch.cat(scores), "out": torch.cat(outs)}
         self.user_feat, self.item_feat = sides["user"].pop("out"), sides["item"].pop("out")
         self._explain = sides
+
+    def _build_siamese_cache(self, user_docs, item_docs, user_masks, item_masks, user_rev_masks, item_rev_masks, chunk, explain):
+        """SimpleSiamese: SimpleSiamese.encode_side over chunks of chunk // R entities.  explain=True also keeps per entity the
+        attention's inputs v [R, F] and weights s [R], a = P^T (w * (1 - tanh^2(P v + c))) [R, F] (zero for a masked review;
+        in float64, then fp32) and, where the head is not fused (K13 then forms g itself), the LastFeat outputs [K]."""
+        m = self.model
+        proj = m.review_att_layer.proj_layer[0]
+        P, c = proj.weight.detach().double(), proj.bias.detach().double()
+        w = m.review_att_layer.inner_product.weight.detach().double().view(-1)
+        feats, sides = {}, {}
+        for name, docs, wm, rm in (("user", user_docs, user_masks, user_rev_masks), ("item", item_docs, item_masks, item_rev_masks)):
+            if (docs.dim() != 3 or (wm is not None and tuple(wm.shape) != tuple(docs.shape))
+                    or (rm is not None and tuple(rm.shape) != tuple(docs.shape[:2]))):
+                raise ValueError(f"SimpleSiamese takes {name}_docs [n, R, T] with word masks [n, R, T] and review masks [n, R], "
+                                 f"got {tuple(docs.shape)} / {None if wm is None else tuple(wm.shape)} / "
+                                 f"{None if rm is None else tuple(rm.shape)}")
+            R = docs.shape[1]
+            step = max(1, chunk // R)
+            keep = {k: [] for k in ("feat", "v", "att", "a")}
+            for lo in range(0, docs.shape[0], step):
+                d = docs[lo:lo + step]
+                wmk = None if wm is None else wm[lo:lo + step]
+                rmk = ((d != 0) if wmk is None else wmk).any(-1) if rm is None else rm[lo:lo + step]
+                f, s, v = m.encode_side(d, wmk, rmk)
+                keep["feat"].append(f)
+                if explain:
+                    th = torch.tanh(v.double() @ P.t() + c)
+                    keep["a"].append((((w * (1 - th * th)) @ P) * rmk.unsqueeze(-1)).float())
+                    keep["v"].append(v.contiguous())
+                    keep["att"].append(s.reshape(-1, R))
+            feats[name] = torch.cat(keep.pop("feat"))
+            if explain:
+                sides[name] = {"docs": docs, "masks": wm, **{k: torch.cat(t) for k, t in keep.items()}}
+        self.user_feat, self.item_feat = feats["user"], feats["item"]
+        if explain:
+            if not self._siamese_fused_g():
+                sides["user"]["lat"], sides["item"]["lat"] = (t.float() for t in self._latents64())
+            self._explain = sides
+
+    def _siamese_fused_g(self) -> bool:
+        """Whether g = d pred / d feat comes from K4's backward (ops.head_text_grads) rather than from K13 itself."""
+        return ops.head_supported(self.user_feat.shape[1], self.model.fm.h.shape[0])
+
     @torch.no_grad()
     def score_cached(self, u_ids: torch.Tensor, i_ids: torch.Tensor) -> torch.Tensor:
         """preds for pairs (u_ids[b], i_ids[b]) from the cached features, no encoder: K1 row gather + K4 head (DeepCoNN,
@@ -240,14 +300,28 @@ class PairScorer:
         i_text = ops.gather_rows(self.item_feat, i_ids)
         if _is_datt(m):
             return torch.sum(torch.mul(u_text, i_text), 1).view(-1)
+        if _is_siamese(m):
+            return m.head(u_text, i_text, u_ids, i_ids).view(-1)
         return fused_head(m.user_feat, m.item_feat, m.fm, u_text, i_text, u_ids, i_ids, False, None).view(-1)
+
+    def _last_feats(self):
+        m = self.model
+        return (m.user_last_feat_layer, m.item_last_feat_layer) if _is_siamese(m) else (m.user_feat, m.item_feat)
 
     def _head_params(self):
         m = self.model
         if _is_datt(m):
             return []
-        return [m.user_feat.W, m.user_feat.b, m.user_feat.ebd.weight, m.item_feat.W, m.item_feat.b, m.item_feat.ebd.weight,
-                m.fm.h, m.fm.user_bias.weight, m.fm.item_bias.weight, m.fm.g_bias]
+        uf, itf = self._last_feats()
+        bias = [m.fm.user_bias.weight, m.fm.item_bias.weight] if isinstance(m.fm, FM) else []     # not FMWithoutUIBias
+        return [uf.W, uf.b, uf.ebd.weight, itf.W, itf.b, itf.ebd.weight, m.fm.h, *bias, m.fm.g_bias]
+
+    def _latents64(self) -> Tuple[torch.Tensor, torch.Tensor]:
+        """LastFeat (models/deepconn/layers.py:163) of every cached entity in float64, [U, K] / [I, K]: exact fp32 latents
+        whatever the TF32 setting."""
+        (Wu, bu, eu, Wi, bi, ei) = [p.detach().double() for p in self._head_params()[:6]]
+        return (self.user_feat.double() @ Wu + bu + eu[:self.user_feat.shape[0]],
+                self.item_feat.double() @ Wi + bi + ei[:self.item_feat.shape[0]])
 
     def factors(self) -> Tuple[torch.Tensor, Optional[torch.Tensor], torch.Tensor, Optional[torch.Tensor]]:
         """(A [U, D], row_bias [U] or None, B [I, D], col_bias [I] or None) with score(u, i) = A[u] . B[i] + biases for the
@@ -262,13 +336,16 @@ class PairScorer:
                 f = (self.user_feat, None, self.item_feat, None)
             else:
                 with torch.no_grad():
-                    # LastFeat (models/deepconn/layers.py:163) in float64: exact fp32 latents whatever the TF32 setting
-                    d = [p.detach().double() for p in params]
-                    Wu, bu, eu, Wi, bi, ei, h, ub, ib, g = d
-                    n_u, n_i = self.user_feat.shape[0], self.item_feat.shape[0]
-                    u_lat = self.user_feat.double() @ Wu + bu + eu[:n_u]
-                    i_lat = self.item_feat.double() @ Wi + bi + ei[:n_i]
-                    f = tuple(t.float().contiguous() for t in fm_factors(u_lat, i_lat, h, ub[:n_u], ib[:n_i], g))
+                    u_lat, i_lat = self._latents64()
+                    n_u, n_i = u_lat.shape[0], i_lat.shape[0]
+                    h, g = params[6].detach().double(), params[-1].detach().double()
+                    if len(params) == 10:
+                        ub, ib = params[7].detach().double()[:n_u], params[8].detach().double()[:n_i]
+                    else:                                # FMWithoutUIBias: row_bias = g_bias, no column bias
+                        ub, ib = u_lat.new_zeros(n_u, 1), i_lat.new_zeros(n_i, 1)
+                    f = tuple(t.float().contiguous() for t in fm_factors(u_lat, i_lat, h, ub, ib, g))
+                    if len(params) != 10:
+                        f = f[:3] + (None,)
             self._factors = (key, f)
         return self._factors[1]
 
@@ -296,7 +373,7 @@ class PairScorer:
         rb_rows = None if rb is None else rb.index_select(0, u_ids)
         pad = None
         if exclude_padding:
-            pad = 0 if _is_datt(self.model) else self.model.fm.item_padding_idx
+            pad = 0 if _is_datt(self.model) or _is_siamese(self.model) else self.model.fm.item_padding_idx
             if pad is not None and 0 <= pad < B.shape[0]:
                 # a -inf column bias: the padding item's score never beats a threshold, so it is never returned
                 cb = torch.zeros(B.shape[0], dtype=torch.float32, device=B.device) if cb is None else cb.clone()
@@ -357,8 +434,12 @@ class PairScorer:
         attribute) D-ATT's top / bottom windows, text_total and map are gradient x input as for DeepCoNN, through both
         gates and the FC stack at the model's own arg-max and ReLU decisions: g = d pred / d feat from the cached FC outputs
         and hidden ReLU masks (ops.datt_fc_grads), then K12b over the cached per-entity terms with the global gate as a
-        dense term; the default width is the local window size.  Positions are flat (NARRE: r * T + t); `tokens_at` turns
-        them into ids.  Pairs run in chunks of `chunk`, so scratch memory does not grow with B."""
+        dense term; the default width is the local window size.  SimpleSiamese: gradient x input through the masked average
+        pooling, the latent transform and the review attention (K13, DESIGN.md), g from K4's backward where the head is
+        fused, else from the cached LastFeat outputs at the FM's ReLU decision; the outputs are NARRE's (map [B, R, T],
+        review_weight, review_attr) and the default width is 1, the token (the model is a bag of words per review).
+        Positions are flat (NARRE, SimpleSiamese: r * T + t); `tokens_at` turns them into ids.  Pairs run in chunks of
+        `chunk`, so scratch memory does not grow with B."""
         if self._explain is None or self.user_feat is None:
             raise RuntimeError("PairScorer.build_cache(..., explain=True) first")
         mdl = self.model
@@ -375,6 +456,8 @@ class PairScorer:
                 raise ValueError(f"user ids must lie in [0, {n_u}) and item ids in [0, {n_i})")
         m = int(m)
         pred = self.score_cached(u_ids, i_ids)
+        if _is_siamese(mdl):
+            return self._explain_siamese(u_ids, i_ids, pred, m, width, return_maps, chunk)
         if _is_datt(mdl) and attribution:
             return self._explain_datt(u_ids, i_ids, pred, m, width, return_maps, chunk)
         if _is_datt(mdl):
@@ -471,6 +554,60 @@ class PairScorer:
                 global_att=c["gate_g"].index_select(0, ids)))
         return Explanation(pred, *sides)
 
+    def _explain_siamese(self, u_ids, i_ids, pred, m, width, return_maps, chunk) -> "Explanation":
+        """SimpleSiamese: K13 per side, with g from K4's backward where the head is fused (zero bias tables for
+        FMWithoutUIBias: the biases do not enter g), else formed in K13 from the cached LastFeat outputs."""
+        mdl = self.model
+        table = mdl.word_embedding.embedding.weight.detach()
+        feat_w, emb = self.user_feat.shape[1], table.shape[1]
+        width = 1 if width is None else int(width)
+        for name in ("user", "item"):
+            _, R, T = self._explain[name]["docs"].shape
+            if not ops.explain_avgpool_supported(R * T, R, emb, feat_w, m, width):
+                raise ValueError(f"explain takes 1 <= m <= {ops.EXPLAIN_MAX_M}, 1 <= width <= {ops.EXPLAIN_MAX_WIDTH} and at most "
+                                 f"{ops.EXPLAIN_MAX_POSITIONS} positions per entity within 227 KB of shared memory (got m={m}, "
+                                 f"width={width}, {R} x {T}, emb={emb}, feat={feat_w})")
+        uf, itf = self._last_feats()
+        fm = mdl.fm
+        lt_w = mdl.latent_transform_layer[0].weight.detach() if mdl.latent_transform else None
+        fused = self._siamese_fused_g()
+        if fused:
+            head = self._head_params()
+            if not isinstance(fm, FM):
+                head = head[:7] + [torch.zeros(e.shape[0], 1, device=e.device) for e in (head[2], head[5])] + head[7:]
+            pads = (uf.padding_idx, itf.padding_idx, getattr(fm, "padding_idx", 0), getattr(fm, "item_padding_idx", 0))
+            head_scratch = [torch.empty_like(p) for p in head]
+        sides = {"user": (uf, "item"), "item": (itf, "user")}
+
+        def attrib(name, ids, other, g):
+            c, (lf, oname) = self._explain[name], sides[name]
+            return ops.explain_avgpool_attrib(table, c["docs"], c["masks"], ids, c["v"], c["a"], c["att"],
+                                              self.user_feat if name == "user" else self.item_feat, m, width, g=g, other=other,
+                                              lat=c.get("lat"), lat_other=self._explain[oname].get("lat"), w_side=lf.W,
+                                              fm_h=fm.h, lt_w=lt_w, return_map=return_maps)
+        parts = {"user": [], "item": []}
+        for lo in range(0, u_ids.numel(), chunk):
+            u, i = u_ids[lo:lo + chunk], i_ids[lo:lo + chunk]
+            g_u = g_i = None
+            if fused:
+                g_u, g_i = ops.head_text_grads(ops.gather_rows(self.user_feat, u), ops.gather_rows(self.item_feat, i), u, i, head,
+                                               pads, head_scratch)
+            parts["user"].append(attrib("user", u, i, g_u))
+            parts["item"].append(attrib("item", i, u, g_i))
+        out = []
+        for name, ids in (("user", u_ids), ("item", i_ids)):
+            c, p = self._explain[name], parts[name]
+            if p:
+                cat = {k: torch.cat([x[k] for x in p]) for k in p[0]}
+            else:                                       # no pairs: empty results of the right shapes
+                cat = attrib(name, ids, ids, torch.empty(0, feat_w, device=ids.device) if fused else None)
+            mp = cat.get("map")
+            out.append(SideExplanation(
+                text_total=cat["text_total"], top_pos=cat["top_pos"], top_attr=cat["top_attr"], bottom_pos=cat["bottom_pos"],
+                bottom_attr=cat["bottom_attr"], map=None if mp is None else mp.view(-1, *c["docs"].shape[1:]),
+                review_weight=c["att"].index_select(0, ids), review_attr=cat["review_attr"]))
+        return Explanation(pred, *out)
+
     def tokens_at(self, side: str, ent_ids: torch.Tensor, pos: torch.Tensor) -> torch.Tensor:
         """Token ids at flat positions pos [B, m] (explain's top_pos / bottom_pos) of the kept documents of entities
         ent_ids [B] on `side` ("user" / "item"); -1 where pos is -1."""
@@ -493,9 +630,9 @@ class SideExplanation:
                                                     # where top_pos is -1
     bottom_pos: Optional[torch.Tensor] = None       # [B, m] most negative windows
     bottom_attr: Optional[torch.Tensor] = None
-    map: Optional[torch.Tensor] = None              # [B, L] (NARRE [B, R, T]) with return_maps
-    review_weight: Optional[torch.Tensor] = None    # NARRE [B, R]: the entity's review attention weights
-    review_attr: Optional[torch.Tensor] = None      # NARRE [B, R]: per-review sums of the map
+    map: Optional[torch.Tensor] = None              # [B, L] (NARRE, SimpleSiamese [B, R, T]) with return_maps
+    review_weight: Optional[torch.Tensor] = None    # NARRE, SimpleSiamese [B, R]: the entity's review attention weights
+    review_attr: Optional[torch.Tensor] = None      # NARRE, SimpleSiamese [B, R]: per-review sums of the map
     local_att: Optional[torch.Tensor] = None        # D-ATT [B, L]: local attention gate per token
     global_att: Optional[torch.Tensor] = None       # D-ATT [B]: global attention gate of the document
 

@@ -1682,3 +1682,109 @@ def narre_feat_grads(feats: Sequence[torch.Tensor], other_ids: Sequence[torch.Te
         lib.check(lib.rbr_narre_attn_bwd(_p(f), _p(i), B, R, H, A, *[_p(t) for t in p], p[5].shape[0], pad, _p(sc), _p(go), None,
                                          _p(gf), *[_p(t) for t in scr], s), "rbr_narre_attn_bwd")
     return g_feats
+
+
+# ---------------------------------------------------------------------------------------------------
+# K13: token attributions for SimpleSiamese (masked average pooling + additive review attention)
+# ---------------------------------------------------------------------------------------------------
+def explain_avgpool_supported(positions: int, reviews: int, emb: int, feat: int, m: int, width: int) -> bool:
+    """Whether rbr_explain_avgpool_attrib takes entities of `reviews` reviews with `positions` = reviews * doc_len tokens,
+    embedding width emb, side feature width feat, m windows of `width` positions (host-only query)."""
+    return bool(lib.rbr_explain_avgpool_supported(int(positions), int(reviews), int(emb), int(feat), int(m), int(width)))
+
+
+def explain_avgpool_attrib(table: torch.Tensor, ids: torch.Tensor, mask: Optional[torch.Tensor], ent: torch.Tensor,
+                           v: torch.Tensor, att_a: torch.Tensor, att_s: torch.Tensor, feat: torch.Tensor, m: int, width: int, *,
+                           g: Optional[torch.Tensor] = None, other: Optional[torch.Tensor] = None,
+                           lat: Optional[torch.Tensor] = None, lat_other: Optional[torch.Tensor] = None,
+                           w_side: Optional[torch.Tensor] = None, fm_h: Optional[torch.Tensor] = None,
+                           lt_w: Optional[torch.Tensor] = None, return_map: bool = False) -> dict:
+    """K13: gradient x input on the embedded tokens of one SimpleSiamese side (rbr_explain_avgpool_attrib), per (pair, side)
+    row p for entity ent[p]: ids [n_ent, R, T] (int64 / int32 / uint16) are the entities' reviews, mask [n_ent, R, T] bool
+    their word masks (None: ids != 0); v / att_a [n_ent, R, F] and att_s [n_ent, R] the review attention's inputs, logit
+    gradients and weights; feat [n_ent, F] the side features; lt_w [F, E] the latent transform's weight (None: F == E).
+    g [P, F] = d pred / d feat, or None to form it in the kernel from the FM head: other [P] (the pair's other entity),
+    lat [n_ent, K] / lat_other [n_other, K] (the two sides' LastFeat outputs), w_side [F, K] (this side's LastFeat.W) and
+    fm_h [K].  Returns explain_attrib's dict for one document of R * T flat positions: text_total [P], top_pos /
+    bottom_pos int64 [P, m] (-1 = none), top_attr / bottom_attr [P, m], review_attr [P, R] and with return_map `map`
+    [P, R * T]."""
+    table = _req(table, torch.float32, "table")
+    ids = _ids(ids, "ids")
+    if table.dim() != 2 or ids.dim() != 3:
+        raise ValueError(f"rbr_b200: table [V, E] and ids [n_ent, R, T] expected, got {tuple(table.shape)} / {tuple(ids.shape)}")
+    emb = table.shape[1]
+    n_ent, R, T = ids.shape
+    m, width = int(m), int(width)
+    feat = _req(feat, torch.float32, "feat")
+    F = feat.shape[1] if feat.dim() == 2 else 0
+    if R < 1 or T < 1 or F < 1 or not explain_avgpool_supported(R * T, R, emb, F, m, width):
+        raise ValueError(f"rbr_b200: explain_avgpool_attrib takes 1 <= R * T <= {EXPLAIN_MAX_POSITIONS}, 1 <= m <= "
+                         f"{EXPLAIN_MAX_M}, 1 <= width <= {EXPLAIN_MAX_WIDTH} within 227 KB of shared memory (got {R} x {T}, "
+                         f"emb={emb}, feat={F}, m={m}, width={width})")
+    v, att_a = _req(v, torch.float32, "v"), _req(att_a, torch.float32, "att_a")
+    att_s = _req(att_s, torch.float32, "att_s")
+    if (feat.shape[0] != n_ent or tuple(v.shape) != (n_ent, R, F) or tuple(att_a.shape) != (n_ent, R, F)
+            or tuple(att_s.shape) != (n_ent, R)):
+        raise ValueError(f"rbr_b200: feat [{n_ent}, F], v / att_a [{n_ent}, {R}, F] and att_s [{n_ent}, {R}] expected, got "
+                         f"{tuple(feat.shape)} / {tuple(v.shape)} / {tuple(att_a.shape)} / {tuple(att_s.shape)}")
+    if mask is not None and tuple(mask.shape) != tuple(ids.shape):
+        raise ValueError(f"rbr_b200: mask {tuple(mask.shape)} does not match ids {tuple(ids.shape)}")
+    flags = _id_flags(ids, mask, True)
+    mask = _mask_u8(mask, "mask")
+    if lt_w is not None:
+        lt_w = _req(lt_w.detach(), torch.float32, "lt_w")
+        if tuple(lt_w.shape) != (F, emb):
+            raise ValueError(f"rbr_b200: lt_w must be [{F}, {emb}], got {tuple(lt_w.shape)}")
+    elif F != emb:
+        raise ValueError(f"rbr_b200: without the latent transform the side feature width ({F}) must be emb ({emb})")
+    ent = _req(ent, torch.int64, "ent").view(-1)
+    P = ent.numel()
+    n_other, K = 0, 0
+    if g is not None:
+        g = _req(g, torch.float32, "g")
+        if tuple(g.shape) != (P, F):
+            raise ValueError(f"rbr_b200: g must be [{P}, {F}], got {tuple(g.shape)}")
+        checked = (g,)
+    else:
+        if any(t is None for t in (other, lat, lat_other, w_side, fm_h)):
+            raise ValueError("rbr_b200: without g, other, lat, lat_other, w_side and fm_h are needed")
+        other = _req(other, torch.int64, "other").view(-1)
+        lat, lat_other = _req(lat, torch.float32, "lat"), _req(lat_other, torch.float32, "lat_other")
+        w_side = _req(w_side.detach(), torch.float32, "w_side")
+        fm_h = _req(fm_h.detach(), torch.float32, "fm_h").view(-1)
+        K = fm_h.numel()
+        n_other = lat_other.shape[0] if lat_other.dim() == 2 else -1
+        if (other.numel() != P or tuple(lat.shape) != (n_ent, K) or lat_other.dim() != 2 or lat_other.shape[1] != K
+                or tuple(w_side.shape) != (F, K) or K < 1):
+            raise ValueError(f"rbr_b200: other [{P}], lat [{n_ent}, K], lat_other [n, K], w_side [{F}, K] and fm_h [K] expected, "
+                             f"got {tuple(other.shape)} / {tuple(lat.shape)} / {tuple(lat_other.shape)} / "
+                             f"{tuple(w_side.shape)} / {tuple(fm_h.shape)}")
+        if P:
+            lo, hi = torch.stack([other.min(), other.max()]).tolist()
+            if lo < 0 or hi >= n_other:
+                raise ValueError(f"rbr_b200: other ids must lie in [0, {n_other})")
+        checked = (other, lat, lat_other, w_side, fm_h)
+    for t, name in ((ids, "ids"), (mask, "mask"), (ent, "ent"), (v, "v"), (att_a, "att_a"), (att_s, "att_s"), (feat, "feat"),
+                    (lt_w, "lt_w")) + tuple((t, "head input") for t in checked):
+        if t is not None and t.device != table.device:
+            raise ValueError(f"rbr_b200: `{name}` is on {t.device}, the table on {table.device}")
+    if P:
+        lo, hi = torch.stack([ent.min(), ent.max()]).tolist()
+        if lo < 0 or hi >= n_ent:
+            raise ValueError(f"rbr_b200: ent must lie in [0, {n_ent})")
+    dev = table.device
+    out = {"text_total": torch.empty(P, dtype=torch.float32, device=dev)}
+    for side in ("top", "bottom"):
+        out[f"{side}_pos"] = torch.empty(P, m, dtype=torch.int64, device=dev)
+        out[f"{side}_attr"] = torch.empty(P, m, dtype=torch.float32, device=dev)
+    if return_map:
+        out["map"] = torch.empty(P, R * T, dtype=torch.float32, device=dev)
+    out["review_attr"] = torch.empty(P, R, dtype=torch.float32, device=dev)
+    if P == 0:
+        return out
+    lib.check(lib.rbr_explain_avgpool_attrib(
+        _p(table), table.shape[0], emb, _p(ids), _p(mask), n_ent, R, T, _p(ent), P, _p(g), _p(other), _p(lat), _p(lat_other),
+        n_other, _p(w_side), _p(fm_h), K, _p(v), _p(att_a), _p(att_s), _p(feat), F, _p(lt_w), m, width, _p(out["text_total"]),
+        _p(out["top_pos"]), _p(out["top_attr"]), _p(out["bottom_pos"]), _p(out["bottom_attr"]), _p(out.get("map")),
+        _p(out["review_attr"]), flags, _stream(True)), "rbr_explain_avgpool_attrib")
+    return out

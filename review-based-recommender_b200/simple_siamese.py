@@ -95,25 +95,44 @@ class SimpleSiamese(HotPathModule):
         self.last_arena = arena
         bz, ur, T = u_revs.shape
         ir = i_revs.shape[1]
-        table = self.word_embedding.embedding.weight
-        cfg = {"padding_idx": 0 if self.word_embedding.padding_idx is None else self.word_embedding.padding_idx, "arena": arena,
-               "table_param": table, "mask_from_ids": True}
         um = None if u_rev_word_masks is None else u_rev_word_masks.reshape(-1, T)
         im = None if i_rev_word_masks is None else i_rev_word_masks.reshape(-1, T)
-        u_pool, i_pool = ops.MaskedAvgPoolFn.apply(table, cfg, u_revs.reshape(-1, T), um, i_revs.reshape(-1, T), im)
-        u = self.var_dropout(u_pool).view(bz, ur, self.embedding_dim)                    # simple_siamese.py:59-64
-        i = self.var_dropout(i_pool).view(bz, ir, self.embedding_dim)
-        if self.latent_transform:
-            u, i = self.latent_transform_layer(u), self.latent_transform_layer(i)
-        u, i = self.review_dropout(u), self.review_dropout(i)
-        u_feat, _ = self.review_att_layer(u, u_rev_masks)
-        i_feat, _ = self.review_att_layer(i, i_rev_masks)
-        if self.use_ui_bias and ops.head_supported(u_feat.shape[1], self.fm.h.shape[0]):
-            out = fused_head(self.user_last_feat_layer, self.item_last_feat_layer, self.fm, u_feat.contiguous(), i_feat.contiguous(),
-                             u_ids, i_ids, self.training, arena)
-        elif self.use_ui_bias:                   # feature width beyond the fused head's shared-memory budget: the layers' own forwards
-            out = self.fm(self.user_last_feat_layer(u_feat, u_ids), self.item_last_feat_layer(i_feat, i_ids), u_ids, i_ids)
-        else:
-            out = self.fm(self.user_last_feat_layer(u_feat, u_ids), self.item_last_feat_layer(i_feat, i_ids))
+        u_pool, i_pool = ops.MaskedAvgPoolFn.apply(self.word_embedding.embedding.weight, self._pool_cfg(arena), u_revs.reshape(-1, T),
+                                                   um, i_revs.reshape(-1, T), im)
+        (u_feat, _, _), (i_feat, _, _) = self._attend([u_pool.view(bz, ur, -1), i_pool.view(bz, ir, -1)],
+                                                      [u_rev_masks, i_rev_masks])
+        out = self.head(u_feat, i_feat, u_ids, i_ids, arena)
         self._after_forward()
         return out.view(bz), None, None
+
+    def _pool_cfg(self, arena):
+        pad = self.word_embedding.padding_idx
+        return {"padding_idx": 0 if pad is None else pad, "arena": arena, "table_param": self.word_embedding.embedding.weight,
+                "mask_from_ids": True}
+
+    def _attend(self, pooled, rev_masks):
+        """Pooled reviews [bz, R, E] of each side → per side (feat [bz, feat], the attention's inputs v [bz, R, feat], its
+        weights [bz, R, 1]); stage by stage across the sides, so training draws its dropout masks in the reference's order."""
+        xs = [self.var_dropout(p) for p in pooled]                                         # simple_siamese.py:59-64
+        if self.latent_transform:
+            xs = [self.latent_transform_layer(x) for x in xs]
+        xs = [self.review_dropout(x) for x in xs]
+        return [(*self.review_att_layer(x, m), x) for x, m in zip(xs, rev_masks)]
+
+    def encode_side(self, revs, word_masks, rev_masks):
+        """One side's text feature as forward computes it — revs [bz, R, T], word_masks [bz, R, T] bool or None (ids != 0),
+        rev_masks [bz, R] bool → (feat [bz, feat], the review attention's weights [bz, R, 1] and inputs v [bz, R, feat])."""
+        bz, R, T = revs.shape
+        wm = None if word_masks is None else word_masks.reshape(-1, T)
+        (pool,) = ops.MaskedAvgPoolFn.apply(self.word_embedding.embedding.weight, self._pool_cfg(None), revs.reshape(-1, T), wm)
+        ((feat, scores, v),) = self._attend([pool.view(bz, R, -1)], [rev_masks])
+        return feat, scores, v
+
+    def head(self, u_feat, i_feat, u_ids, i_ids, arena=None):
+        """LastFeat x2 + FM(WithoutUIBias) on the two text features → [bz, 1]."""
+        if self.use_ui_bias and ops.head_supported(u_feat.shape[1], self.fm.h.shape[0]):
+            return fused_head(self.user_last_feat_layer, self.item_last_feat_layer, self.fm, u_feat.contiguous(),
+                              i_feat.contiguous(), u_ids, i_ids, self.training, arena)
+        if self.use_ui_bias:                     # feature width beyond the fused head's shared-memory budget: the layers' own forwards
+            return self.fm(self.user_last_feat_layer(u_feat, u_ids), self.item_last_feat_layer(i_feat, i_ids), u_ids, i_ids)
+        return self.fm(self.user_last_feat_layer(u_feat, u_ids), self.item_last_feat_layer(i_feat, i_ids))

@@ -6,6 +6,9 @@ Set-up: U = 20 000 users x I = 12 000 items, vocabulary 50 000, seeded parameter
   NARRE     E = 300, 10 reviews of 60 tokens per entity (lengths 20..60, trailing all-padding reviews), H = 150, attention 32;
   D-ATT     E = 100, documents of L = 500 tokens (lengths 200..500), local window 5, 200 local and 3 x 100 global filters,
             FC 500 → 500 → 50; explain(attribution=True).
+  SimpleSiamese  E = 300, K = 32, 10 reviews of 60 tokens per entity (as NARRE's), with the FM's user / item biases, without
+            (siamese: F = 300, K13 forms g itself) and with the latent transform (siamese_lt: F = 32, g from K4's backward);
+            explain at width 1.
 Pairs: each user's top-10 from recommend = 200 000 pairs.
 
 Reported per model: build_cache() and build_cache(explain=True) times and the bytes the explain cache adds; explain time
@@ -14,7 +17,7 @@ Reported per model: build_cache() and build_cache(explain=True) times and the by
 two relative to each pair's largest |attribution| (the baseline routes through the cache's arg-max, so both compute the same
 quantity).
 
-    python tools/bench_explain.py --out DIR [--model deepconn|narre|datt|all] [--precision bf16|fp32] [--reps 3]
+    python tools/bench_explain.py --out DIR [--model deepconn|narre|datt|siamese|all] [--precision bf16|fp32] [--reps 3]
         [--baseline-pairs 4096]   → DIR/bench_explain_<precision>.json (--model all, the default: DeepCoNN and NARRE),
                                     DIR/bench_explain_<model>_<precision>.json otherwise
 """
@@ -47,6 +50,11 @@ def docs(n, L, seed, min_len):
 
 
 def build(model, precision):
+    if model.startswith("siamese"):
+        R, T, lt = 10, 60, model == "siamese_lt"
+        m = rbr_b200.SimpleSiamese(EMB, 32, VOCAB, U, I, None, False, 0.0, 0.0, 0.0, True, lt)
+        m.load_state_dict(synth.simple_siamese_params(U, I, VOCAB, EMB, 32, True, lt, seed=0))
+        return PairScorer(m.cuda()), reviews(R, T), {}
     if model == "datt":
         m = rbr_b200.DualAtt(VOCAB, DATT_L, 5, 200, 100, DATT_EMB, 500, 50, 0.0, None, precision=precision)
         m.load_state_dict(synth.dual_att_params(VOCAB, DATT_L, 5, 200, 100, DATT_EMB, 500, 50, seed=0))
@@ -55,11 +63,7 @@ def build(model, precision):
         R, T = 10, 60
         m = rbr_b200.NARRE(U, I, VOCAB, [3], 150, EMB, 32, 32, R, T, 0.0, 0, 0, 0, None, "CNN", precision=precision)
         m.load_state_dict(synth.narre_params(U, I, VOCAB, EMB, 150, 32, 32, (3,), seed=0))
-        ud, idd = docs(U * R, T, 1, 20).view(U, R, T), docs(I * R, T, 2, 20).view(I, R, T)
-        nrev_u = torch.randint(1, R + 1, (U, 1), device="cuda")              # trailing reviews are all padding
-        nrev_i = torch.randint(1, R + 1, (I, 1), device="cuda")
-        ud = torch.where((torch.arange(R, device="cuda").view(1, -1) < nrev_u).unsqueeze(-1), ud, torch.zeros_like(ud))
-        idd = torch.where((torch.arange(R, device="cuda").view(1, -1) < nrev_i).unsqueeze(-1), idd, torch.zeros_like(idd))
+        ud, idd = reviews(R, T)
         kw = {"user_rev_ids": torch.randint(1, I, (U, R), device="cuda"), "item_rev_ids": torch.randint(1, U, (I, R), device="cuda")}
     else:
         m = rbr_b200.DeepCoNNpp(U, I, VOCAB, [3], EMB, 100, 32, 500, None, 0.0, precision=precision)
@@ -67,6 +71,28 @@ def build(model, precision):
         ud, idd = docs(U, 500, 1, 200), docs(I, 500, 2, 200)
         kw = {}
     return PairScorer(m.cuda()), (ud, idd), kw
+
+
+def reviews(R, T):
+    """R reviews of T tokens per entity (lengths 20..T, trailing reviews all padding)"""
+    ud, idd = docs(U * R, T, 1, 20).view(U, R, T), docs(I * R, T, 2, 20).view(I, R, T)
+    nrev_u = torch.randint(1, R + 1, (U, 1), device="cuda")
+    nrev_i = torch.randint(1, R + 1, (I, 1), device="cuda")
+    ud = torch.where((torch.arange(R, device="cuda").view(1, -1) < nrev_u).unsqueeze(-1), ud, torch.zeros_like(ud))
+    idd = torch.where((torch.arange(R, device="cuda").view(1, -1) < nrev_i).unsqueeze(-1), idd, torch.zeros_like(idd))
+    return ud, idd
+
+
+def siamese_side(p, x, wm):
+    """oracle.simple_siamese_forward's side on embedded tokens x [B, R, T, E]"""
+    B, R, T, E = x.shape
+    pooled = orc.masked_avg_pool(x.reshape(-1, T, E), wm.reshape(-1, T)).view(B, R, E)
+    if "latent_transform_layer.0.weight" in p:
+        pooled = torch.tanh(pooled @ p["latent_transform_layer.0.weight"].t() + p["latent_transform_layer.0.bias"])
+    hid = torch.tanh(pooled @ p["review_att_layer.proj_layer.0.weight"].t() + p["review_att_layer.proj_layer.0.bias"])
+    logits = hid @ p["review_att_layer.inner_product.weight"].t()
+    logits = torch.where(wm.any(-1).unsqueeze(2), logits, torch.full((), -1e8, dtype=logits.dtype, device=logits.device))
+    return (torch.softmax(logits, dim=1) * pooled).sum(dim=1)
 
 
 def once_ms(fn):
@@ -109,6 +135,22 @@ def datt_side(p, x, s, amax):
 def baseline(sc, inputs, kw, u_all, i_all, chunk):
     """fp32 autograd gradient x input on the oracle formulation, chunk pairs at a time → (user maps, item maps)"""
     p = {k: v.detach().float() for k, v in sc.model.state_dict().items()}
+    if isinstance(sc.model, rbr_b200.SimpleSiamese):
+        table = p["word_embedding.embedding.weight"]
+        ud, idd = inputs
+        maps_u, maps_i = [], []
+        for lo in range(0, u_all.numel(), chunk):
+            u, i = u_all[lo:lo + chunk], i_all[lo:lo + chunk]
+            ux = orc.embedding_gather(table, ud[u]).requires_grad_()
+            ix = orc.embedding_gather(table, idd[i]).requires_grad_()
+            u_f = orc.last_feat(siamese_side(p, ux, ud[u] != 0), u, p["user_last_feat_layer.W"], p["user_last_feat_layer.b"],
+                                p["user_last_feat_layer.ebd.weight"])
+            i_f = orc.last_feat(siamese_side(p, ix, idd[i] != 0), i, p["item_last_feat_layer.W"], p["item_last_feat_layer.b"],
+                                p["item_last_feat_layer.ebd.weight"])
+            orc.fm_head(u_f, i_f, u, i, p["fm.h"], p["fm.g_bias"], p["fm.user_bias.weight"], p["fm.item_bias.weight"]).sum().backward()
+            maps_u.append((ux * ux.grad).sum(-1).detach())
+            maps_i.append((ix * ix.grad).sum(-1).detach())
+        return torch.cat(maps_u), torch.cat(maps_i)
     table = p["word_embeddings.embedding.weight"]
     if isinstance(sc.model, rbr_b200.DualAtt):
         c = sc._explain
@@ -157,6 +199,24 @@ def baseline(sc, inputs, kw, u_all, i_all, chunk):
     return torch.cat(maps_u), torch.cat(maps_i)
 
 
+def k13_alone(sc, uu, ii, reps):
+    """K13 (ops.explain_avgpool_attrib) alone on the user side of the pairs, and the table-row bytes it reads over that time
+    (one E-float row per masked-in token; the host wrapper's id-range check is inside the timed window)"""
+    from rbr_b200 import ops
+    m, c = sc.model, sc._explain["user"]
+    table = m.word_embedding.embedding.weight.detach()
+    lt_w = m.latent_transform_layer[0].weight.detach() if m.latent_transform else None
+    if "lat" in c:
+        kw = dict(other=ii, lat=c["lat"], lat_other=sc._explain["item"]["lat"], w_side=m.user_last_feat_layer.W, fm_h=m.fm.h)
+    else:
+        kw = dict(g=torch.randn(uu.numel(), sc.user_feat.shape[1], device="cuda"))
+    t, _ = timed(lambda: ops.explain_avgpool_attrib(table, c["docs"], c["masks"], uu, c["v"], c["a"], c["att"], sc.user_feat, 5,
+                                                    1, lt_w=lt_w, **kw), reps)
+    rows = int((c["docs"] != 0).sum((1, 2))[uu].sum())
+    return {"k13_user_side_ms": round(t, 3), "k13_rows_read": rows, "k13_row_gb": round(rows * EMB * 4 / 1e9, 2),
+            "k13_row_read_gb_per_s": round(rows * EMB * 4 / (t * 1e-3) / 1e9, 1), "k13_g_in_kernel": "lat" in c}
+
+
 def rel_per_pair(a, b):
     """per pair: the largest |difference| over its positions relative to the pair's largest |attribution|"""
     a, b = a.flatten(1).double(), b.flatten(1).double()
@@ -170,8 +230,9 @@ def main():
     ap.add_argument("--baseline-pairs", type=int, default=4096)
     ap.add_argument("--baseline-chunk", type=int, default=256)
     ap.add_argument("--precision", choices=("bf16", "fp32"), default="bf16", help="the conv forward's precision")
-    ap.add_argument("--model", choices=("all", "deepconn", "narre", "datt"), default="all",
-                    help="all: DeepCoNN and NARRE; datt: D-ATT's gradient x input (explain(attribution=True))")
+    ap.add_argument("--model", choices=("all", "deepconn", "narre", "datt", "siamese"), default="all",
+                    help="all: DeepCoNN and NARRE; datt: D-ATT's gradient x input (explain(attribution=True)); siamese: "
+                         "SimpleSiamese without and with the latent transform")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_explain needs a CUDA device")
@@ -180,7 +241,7 @@ def main():
     os.makedirs(args.out, exist_ok=True)
     info = gpu_info()
     runs = []
-    models = ("deepconn", "narre") if args.model == "all" else (args.model,)
+    models = {"all": ("deepconn", "narre"), "siamese": ("siamese", "siamese_lt")}.get(args.model, (args.model,))
     for model in models:
         sc, inputs, kw = build(model, args.precision)
         datt = model == "datt"
@@ -189,7 +250,9 @@ def main():
         t_plain, _ = once_ms(lambda: sc.build_cache(*inputs, **kw))
         sc.build_cache(*inputs, **kw, explain=True)
         t_expl, _ = once_ms(lambda: sc.build_cache(*inputs, **kw, explain=True))
-        keys = ("argmax", "contrib", "gate_coef", "gate_vec", "hid_mask") if datt else ("feat", "argmax", "contrib")
+        keys = (("argmax", "contrib", "gate_coef", "gate_vec", "hid_mask") if datt else
+                ("v", "a", "att", "lat") if model.startswith("siamese") else ("feat", "argmax", "contrib"))
+        keys = tuple(k for k in keys if k in sc._explain["user"])
         cache_mb = {k: round(sum(v[k].numel() * v[k].element_size() for v in sc._explain.values()) / 2 ** 20, 1)
                     for k in keys}
         cache_bytes_per_entity = round(sum(v[k].numel() * v[k].element_size() for v in sc._explain.values() for k in keys)
@@ -209,7 +272,8 @@ def main():
         mem_base = peak_mb(lambda: baseline(sc, inputs, kw, ub, ib, args.baseline_chunk))
         diff = torch.cat([rel_per_pair(es.user.map, bu), rel_per_pair(es.item.map, bi)])
         runs.append({
-            "model": model, "precision": sc.model.precision if datt else sc.model.ngram.precision, "pairs": uu.numel(),
+            "model": model, "pairs": uu.numel(),
+            "precision": sc.model.precision if datt else "fp32" if model.startswith("siamese") else sc.model.ngram.precision,
             "build_cache_ms": round(t_plain, 2), "build_cache_explain_ms": round(t_expl, 2), "explain_cache_mb": cache_mb,
             "explain_cache_bytes_per_entity": cache_bytes_per_entity,
             "explain_ms": round(t_nomap, 3), "explain_maps_ms": round(t_map, 3),
@@ -222,6 +286,7 @@ def main():
                                          "fraction_below_1e-2": float((diff <= 1e-2).double().mean()),
                                          "fraction_below_1e-5": float((diff <= 1e-5).double().mean())},
             "nan_windows": int(e.user.top_pos.lt(0).sum() + e.item.top_pos.lt(0).sum()),
+            **(k13_alone(sc, uu, ii, args.reps) if model.startswith("siamese") else {}),
         })
         print(json.dumps(runs[-1]), flush=True)
         del sc, e, es

@@ -2,7 +2,8 @@
 torch.topk), on the synthetic sizes of SURVEY §8d: U = 20 000 users (all of them as rows), I = 12 000 items, k = 10 / 100.
 
 The entity caches are filled with seeded random features of the shape build_cache produces ([U, H] / [I, H]; D-ATT: the FC
-outputs [U, 50] / [I, 50]); recommend's cost does not depend on how they were computed.  The factors (a few MB) sit in
+outputs [U, 50] / [I, 50]; SimpleSiamese: the review attention's output, [U, 300] / [I, 300] with the FM's biases and no
+latent transform, [U, 32] / [I, 32] with the latent transform and FMWithoutUIBias); recommend's cost does not depend on how they were computed.  The factors (a few MB) sit in
 L2, so K10 is compute / issue bound, not HBM bound.  Both results are compared in the same run: per row, the k returned
 scores must agree within 1e-5 of the row's largest |score| (items may differ only where scores tie to that tolerance).
 
@@ -40,6 +41,11 @@ def scorer(model: str):
         m = rbr_b200.DualAtt(1000, 64, 5, 200, 100, 100, 500, 50, 0.0, None)
         m.load_state_dict(synth.dual_att_params(1000, 64, 5, 200, 100, 100, 500, 50, seed=0))
         H = 50
+    elif model.startswith("siamese"):
+        lt = model == "siamese_lt_nobias"
+        m = rbr_b200.SimpleSiamese(300, 32, 1000, U, I, None, False, 0.0, 0.0, 0.0, not lt, lt)
+        m.load_state_dict(synth.simple_siamese_params(U, I, 1000, 300, 32, not lt, lt, seed=0))
+        H = 32 if lt else 300
     elif model == "narre":
         m = rbr_b200.NARRE(U, I, 1000, [3], 150, 64, 32, 32, 10, 60, 0.0, 0, 0, 0, None, "CNN")
         m.load_state_dict(synth.narre_params(U, I, 1000, 64, 150, 32, 32, (3,), seed=0))
@@ -51,7 +57,7 @@ def scorer(model: str):
     sc = PairScorer(m.cuda())
     # pooled ReLU / attention outputs are >= 0 (ReLU) or in (-1, 1) (D-ATT FC: any sign)
     feats = [torch.rand(n, H, generator=g) * 0.5 for n in (U, I)]
-    if model == "dual_att":
+    if model == "dual_att" or model.startswith("siamese"):
         feats = [f * 4 - 1 for f in feats]
     sc.user_feat, sc.item_feat = feats[0].cuda(), feats[1].cuda()
     return sc
@@ -105,7 +111,8 @@ def main():
     excl_idx = torch.randint(1, I, (U * 50,), device="cuda", generator=g)
     excl = (torch.arange(0, U * 50 + 1, 50, device="cuda"), excl_idx)
     runs = []
-    for model, ex in (("deepconn", None), ("narre", None), ("dual_att", None), ("deepconn", excl)):
+    for model, ex in (("deepconn", None), ("narre", None), ("dual_att", None), ("siamese", None), ("siamese_lt_nobias", None),
+                      ("deepconn", excl)):
         sc = scorer(model)
         A, _, B, _ = sc.factors()
         for k in (10, 100):
