@@ -64,6 +64,11 @@ class DualAtt(HotPathModule):
     def invalidate_operand_cache(self):
         self.word_embeddings.invalidate_operand_cache()
 
+    def side_params(self, s: str):
+        """The 12 parameters of side s ("u" / "i") in DattEncodeFn's order: local attn w, b; local conv w, b; global attn
+        w, b; conv1 w, b; conv2 w, b; conv3 w, b."""
+        return self._side_params(getattr(self, f"{s}_local_atten"), getattr(self, f"{s}_global_atten"))
+
     @staticmethod
     def _side_params(local: LocalAttention, glob: GlobalAttention):
         return [local.attn[0].weight, local.attn[0].bias, local.conv[0].weight, local.conv[0].bias,
@@ -73,13 +78,12 @@ class DualAtt(HotPathModule):
     def encode(self, docs, sides, arena=None):
         """Fused encoder: docs = list of [bz, doc_len] id tensors, sides = matching list of "u" / "i" → list of
         [bz, l_out + 3*g_out] features (dual_att.py:45-50, 53-56 without the FC)."""
-        mods = {"u": (self.u_local_atten, self.u_global_atten), "i": (self.i_local_atten, self.i_global_atten)}
         params, args = [], []
         for ids, s in zip(docs, sides):
             if ids.shape[-1] != self.doc_len:
                 raise ValueError(f"DualAtt was built for doc_len={self.doc_len}, got {ids.shape[-1]} "
                                  "(the global attention kernel spans the whole document)")
-            prm = self._side_params(*mods[s])
+            prm = self.side_params(s)
             params.append(prm)
             args += [ids, *prm]
         table = self.word_embeddings.embedding.weight

@@ -23,6 +23,7 @@ D-ATT's score is already a dot product of the two FC outputs.
 """
 from __future__ import annotations
 
+import functools
 from dataclasses import dataclass
 from typing import Optional, Tuple
 
@@ -31,7 +32,7 @@ import torch
 from . import ops
 from .deepconn import DeepCoNNpp
 from .dual_att import DualAtt
-from .layers import FM, fused_head
+from .layers import FM, fused_head, head_params
 from .narre import NARRE
 from .simple_siamese import SimpleSiamese
 
@@ -45,18 +46,6 @@ def fm_factors(u_lat: torch.Tensor, i_lat: torch.Tensor, h: torch.Tensor, user_b
     A = torch.cat([hv * torch.relu(u_lat), hv * torch.relu(-u_lat)], dim=1)
     B = torch.cat([torch.relu(i_lat), torch.relu(-i_lat)], dim=1)
     return A, user_bias.reshape(-1) + g_bias.reshape(()), B, item_bias.reshape(-1)
-
-
-def _is_narre(model) -> bool:
-    return isinstance(model, NARRE)
-
-
-def _is_datt(model) -> bool:
-    return isinstance(model, DualAtt)
-
-
-def _is_siamese(model) -> bool:
-    return isinstance(model, SimpleSiamese)
 
 
 class PairScorer:
@@ -89,6 +78,7 @@ class PairScorer:
         SimpleSiamese: user_docs [U, R_u, T], item_docs [I, R_i, T] (the entity's reviews; R_u and R_i may differ), optional
           word masks of the same shapes (default ids != 0) and user_rev_masks [U, R_u] / item_rev_masks [I, R_i] (default:
           the review has a masked-in word, models/simple_siamese/utils.py get_rev_mask).
+        Each side is encoded in chunks of `chunk` documents (review models: chunk // R entities of R reviews).
         explain=True also keeps what `explain` needs per entity (references to the documents and masks; for DeepCoNN and
         NARRE the conv arg-max and the tap contributions of every pooled window (K12a), for NARRE the per-review features
         and attention weights; for D-ATT the two K5 gates, the conv arg-max, the FC hidden ReLU mask and the per-entity
@@ -96,194 +86,133 @@ class PairScorer:
         logit gradients a (K13), and the LastFeat outputs where the head is not fused).  The cached features are the same
         either way."""
         m = self.model
-        self.model.eval()
+        m.eval()
         self._factors = None
         self._explain = None
-        if _is_siamese(m):
-            self._build_siamese_cache(user_docs, item_docs, user_masks, item_masks, user_rev_masks, item_rev_masks, chunk,
-                                      explain)
-            return
-        if explain and not _is_datt(m) and m.ngram.arch != "CNN":
-            raise NotImplementedError("PairScorer.explain covers the CNN encoder; arch='HierPooling' pools averages, "
-                                      "which have no per-window tap contributions")
-        if _is_datt(m):
+        # per side: (documents, masks, the model's per-review input: NARRE's review ids, SimpleSiamese's review masks)
+        sides = {"user": (user_docs, user_masks, None), "item": (item_docs, item_masks, None)}
+        if isinstance(m, SimpleSiamese):
+            sides = {"user": (user_docs, user_masks, user_rev_masks), "item": (item_docs, item_masks, item_rev_masks)}
+            for name, (docs, wm, rm) in sides.items():
+                if (docs.dim() != 3 or (wm is not None and tuple(wm.shape) != tuple(docs.shape))
+                        or (rm is not None and tuple(rm.shape) != tuple(docs.shape[:2]))):
+                    raise ValueError(f"SimpleSiamese takes {name}_docs [n, R, T] with word masks [n, R, T] and review masks "
+                                     f"[n, R], got {tuple(docs.shape)} / {None if wm is None else tuple(wm.shape)} / "
+                                     f"{None if rm is None else tuple(rm.shape)}")
+            encode = functools.partial(self._encode_siamese, att64=self._siamese_att64() if explain else None)
+        elif isinstance(m, DualAtt):
             if user_masks is not None or item_masks is not None:
                 raise ValueError("DualAtt takes no masks")
-
-            if explain:
-                self._build_datt_explain_cache(user_docs, item_docs, chunk)
-                return
-
-            def side(docs, s):
-                return torch.cat([m.fc(m.encode([docs[lo:lo + chunk]], [s])[0]) for lo in range(0, docs.shape[0], chunk)], 0)
-            self.user_feat, self.item_feat = side(user_docs, "u"), side(item_docs, "i")
-            return
-        if explain:
-            self._build_explain_cache(user_docs, item_docs, user_masks, item_masks, chunk, user_rev_ids, item_rev_ids)
-            return
-        if _is_narre(m):
+            for docs in (user_docs, item_docs):
+                if docs.shape[-1] != m.doc_len:
+                    raise ValueError(f"DualAtt was built for doc_len={m.doc_len}, got {docs.shape[-1]} "
+                                     "(the global attention kernel spans the whole document)")
+            encode = self._encode_datt
+        elif explain and m.ngram.arch != "CNN":
+            raise NotImplementedError("PairScorer.explain covers the CNN encoder; arch='HierPooling' pools averages, "
+                                      "which have no per-window tap contributions")
+        elif isinstance(m, NARRE):
             if user_rev_ids is None or item_rev_ids is None:
                 raise ValueError("NARRE's build_cache needs user_rev_ids [U, R] and item_rev_ids [I, R]")
-            R, T = m.doc_num, m.doc_len
-            ent_chunk = max(1, chunk // R)
+            sides = {"user": (user_docs, user_masks, user_rev_ids), "item": (item_docs, item_masks, item_rev_ids)}
+            for docs, _, rev_ids in sides.values():
+                if docs.shape[1:] != (m.doc_num, m.doc_len) or rev_ids.shape != docs.shape[:2]:
+                    raise ValueError(f"NARRE was built for [*, {m.doc_num}, {m.doc_len}] reviews with [*, {m.doc_num}] review "
+                                     f"ids, got {tuple(docs.shape)} / {tuple(rev_ids.shape)}")
+            encode = self._encode_narre
+        else:
+            encode = self._encode_deepconn
+        feats, kept = {}, {}
+        for name, (docs, masks, rev) in sides.items():
+            step = max(1, chunk // docs.shape[1]) if docs.dim() == 3 else chunk
+            parts = [encode(name, explain, *(None if t is None else t[lo:lo + step] for t in (docs, masks, rev)))
+                     for lo in range(0, docs.shape[0], step)]
+            feats[name] = torch.cat([f for f, _ in parts])
+            if explain:
+                kept[name] = {"docs": docs, "masks": masks, **{k: torch.cat([x[k] for _, x in parts]) for k in parts[0][1]}}
+        self.user_feat, self.item_feat = feats["user"], feats["item"]
+        if explain:
+            if isinstance(m, SimpleSiamese) and not self._siamese_fused_g():
+                kept["user"]["lat"], kept["item"]["lat"] = (t.float() for t in self._latents64())
+            self._explain = kept
 
-            def side(docs, masks, rev_ids, att):
-                if docs.shape[1:] != (R, T) or rev_ids.shape != docs.shape[:2]:
-                    raise ValueError(f"NARRE was built for [*, {R}, {T}] reviews with [*, {R}] review ids, got "
-                                     f"{tuple(docs.shape)} / {tuple(rev_ids.shape)}")
-                outs = []
-                for lo in range(0, docs.shape[0], ent_chunk):
-                    d = docs[lo:lo + ent_chunk]
-                    mk = None if masks is None else masks[lo:lo + ent_chunk].reshape(-1, T)
-                    (f,) = m.ngram.encode(m.word_embeddings, [d.reshape(-1, T)], [mk])
-                    outs.append(att(f.view(d.shape[0], R, -1), rev_ids[lo:lo + ent_chunk])[0])
-                return torch.cat(outs, 0)
-            self.user_feat = side(user_docs, user_masks, user_rev_ids, m.user_att)
-            self.item_feat = side(item_docs, item_masks, item_rev_ids, m.item_att)
-            return
+    # build_cache's chunk encoders, one per model: (side, explain, documents, masks, per-review input) of a chunk of entities
+    # → (the entities' cached features, None or with explain a dict of their per-entity explain tensors)
 
-        def encode(docs, masks):
-            outs = []
-            for lo in range(0, docs.shape[0], chunk):
-                mk = None if masks is None else masks[lo:lo + chunk]
-                (f,) = m.ngram.encode(m.word_embeddings, [docs[lo:lo + chunk]], [mk])
-                outs.append(f)
-            return torch.cat(outs, dim=0)
-        self.user_feat = encode(user_docs, user_masks)
-        self.item_feat = encode(item_docs, item_masks)
-
-    def _datt_side_prm(self, s: str):
+    def _encode_deepconn(self, side, explain, docs, masks, _):
         m = self.model
-        return [p.detach() for p in m._side_params(getattr(m, f"{s}_local_atten"), getattr(m, f"{s}_global_atten"))]
+        out = m.ngram.encode(m.word_embeddings, [docs], [masks], return_argmax=explain)      # (HierPooling: no arg-max)
+        if not explain:
+            return out[0], None
+        feat, amax = out
+        return feat, {"feat": feat, "argmax": amax, "contrib": self._window_contrib(docs, masks, amax)}
 
-    def _build_datt_explain_cache(self, user_docs, item_docs, chunk):
-        """D-ATT with explain=True: the encoder once per chunk (ops.datt_encode_side, the kernels DualAtt.encode runs), the FC
-        stack layer by layer (the same modules in the same order as m.fc, so the cached features are bit-identical to
-        build_cache(explain=False)) to keep its hidden ReLU mask, then K12's per-entity terms (ops.datt_explain_contrib)."""
+    def _encode_narre(self, side, explain, docs, masks, rev_ids):
+        m = self.model
+        n, R, T = docs.shape
+        docs = docs.reshape(-1, T)
+        masks = None if masks is None else masks.reshape(-1, T)
+        out = m.ngram.encode(m.word_embeddings, [docs], [masks], return_argmax=explain)
+        feat, att = (m.user_att if side == "user" else m.item_att)(out[0].view(n, R, -1), rev_ids)
+        if not explain:
+            return feat, None
+        return feat, {"rev_ids": rev_ids, "feat": out[0], "argmax": out[1], "att": att.view(-1, R),
+                      "contrib": self._window_contrib(docs, masks, out[1])}
+
+    def _encode_datt(self, side, explain, docs, masks, _):
+        """The encoder (ops.datt_encode_side, the kernels DualAtt.encode runs), then the FC stack layer by layer (the modules
+        of m.fc in its order) to keep its hidden ReLU mask; with explain K12's per-entity terms (ops.datt_explain_contrib)."""
         m = self.model
         table = m.word_embeddings.embedding.weight.detach()
         shadow = m.word_embeddings.bf16_shadow() if m.precision == "bf16" else None
+        prm = m.side_params("u" if side == "user" else "i")
+        packed = ops.datt_side_packs(prm)
+        feat, amax, _, gl, gg = ops.datt_encode_side(table, docs, prm, m.precision, shadow, packed, conv_flags=m.conv_flags)
         lin0, relu, drop, lin1 = m.fc
-        sides, outs = {}, {}
-        for name, s, docs in (("user", "u", user_docs), ("item", "i", item_docs)):
-            if docs.shape[-1] != m.doc_len:
-                raise ValueError(f"DualAtt was built for doc_len={m.doc_len}, got {docs.shape[-1]}")
-            prm = self._datt_side_prm(s)
-            packed = ops.datt_side_packs(prm)
-            keep = {k: [] for k in ("gate_l", "gate_g", "argmax", "contrib", "gate_coef", "gate_vec", "hid_mask")}
-            out = []
-            for lo in range(0, docs.shape[0], chunk):
-                d = docs[lo:lo + chunk]
-                feat, amax, _, gl, gg = ops.datt_encode_side(table, d, prm, m.precision, shadow, packed)
-                z = lin0(feat)
-                out.append(lin1(drop(relu(z))))
-                contrib, coef, vec = ops.datt_explain_contrib(table, d, prm, gl, gg, feat, amax, packed)
-                for k, v in (("gate_l", gl), ("gate_g", gg), ("argmax", amax), ("contrib", contrib), ("gate_coef", coef),
-                             ("gate_vec", vec), ("hid_mask", z > 0)):
-                    keep[k].append(v)
-            sides[name] = {"docs": docs, **{k: torch.cat(v) for k, v in keep.items()}}
-            outs[name] = torch.cat(out, 0)
-        self.user_feat, self.item_feat = outs["user"], outs["item"]
-        self._explain = sides
+        hid = lin0(feat)
+        out = lin1(drop(relu(hid)))
+        if not explain:
+            return out, None
+        contrib, coef, vec = ops.datt_explain_contrib(table, docs, prm, gl, gg, feat, amax, packed)
+        return out, {"gate_l": gl, "gate_g": gg, "argmax": amax, "contrib": contrib, "gate_coef": coef, "gate_vec": vec,
+                     "hid_mask": hid > 0}
+
+    def _encode_siamese(self, side, explain, docs, masks, rev_masks, att64):
+        """SimpleSiamese.encode_side; explain also keeps per entity the attention's inputs v [R, F] and weights s [R], and
+        a = P^T (w * (1 - tanh^2(P v + c))) [R, F] (zero for a masked review; in float64, then fp32)."""
+        rm = ((docs != 0) if masks is None else masks).any(-1) if rev_masks is None else rev_masks
+        feat, s, v = self.model.encode_side(docs, masks, rm)
+        if not explain:
+            return feat, None
+        P, c, w = att64
+        th = torch.tanh(v.double() @ P.t() + c)
+        return feat, {"v": v.contiguous(), "att": s.reshape(-1, docs.shape[1]),
+                      "a": (((w * (1 - th * th)) @ P) * rm.unsqueeze(-1)).float()}
+
+    def _siamese_att64(self):
+        """(P, c, w) of SimpleSiamese's review attention in float64."""
+        att = self.model.review_att_layer
+        proj = att.proj_layer[0]
+        return proj.weight.detach().double(), proj.bias.detach().double(), att.inner_product.weight.detach().double().view(-1)
 
     def _conv_specs(self):
         conv = self.model.ngram.conv
         return [(c.weight.shape[0], k, (k - 1) // 2) for c, k in zip(conv.list_of_conv1d, conv.kernel_sizes)]
 
-    def _encode_explain(self, docs: torch.Tensor, masks: Optional[torch.Tensor], chunk: int):
-        """docs [N, L] (masks None: ids != 0) → (feat [N, H], argmax int32 [N, H], contrib [N, sum_c H_c * k_c]): the encoder's
-        own features and first arg-max (EncodeDocsFn), then the tap contributions of every pooled window (K12a)."""
+    def _window_contrib(self, docs: torch.Tensor, masks: Optional[torch.Tensor], argmax: torch.Tensor) -> torch.Tensor:
+        """K12a: the tap contributions [N, sum_c H_c * k_c] of every pooled window of docs [N, L] at the arg-max."""
         m = self.model
         conv = m.ngram.conv
         table = m.word_embeddings.embedding.weight.detach()
         specs = self._conv_specs()
-        taps = sum(h * k for h, k, _ in specs)
-        feats, amaxes = [], []
-        contrib = torch.empty(docs.shape[0], taps, dtype=torch.float32, device=table.device)
-        for lo in range(0, docs.shape[0], chunk):
-            d = docs[lo:lo + chunk]
-            mk = None if masks is None else masks[lo:lo + chunk]
-            f, a = m.ngram.encode(m.word_embeddings, [d], [mk], return_argmax=True)
-            col = tcol = 0
-            for i, (h, k, pad) in enumerate(specs):
-                ops.conv_window_contrib(table, d, mk, conv.list_of_conv1d[i].weight.detach(), pad, a[:, col:col + h],
-                                        packed=conv.packed(i), mask_from_ids=True, out=contrib[lo:lo + chunk, tcol:tcol + h * k])
-                col += h
-                tcol += h * k
-            feats.append(f)
-            amaxes.append(a)
-        return torch.cat(feats), torch.cat(amaxes), contrib
-
-    def _build_explain_cache(self, user_docs, item_docs, user_masks, item_masks, chunk, user_rev_ids, item_rev_ids):
-        m = self.model
-        if not _is_narre(m):
-            sides = {}
-            for name, docs, masks in (("user", user_docs, user_masks), ("item", item_docs, item_masks)):
-                feat, amax, contrib = self._encode_explain(docs, masks, chunk)
-                sides[name] = {"docs": docs, "masks": masks, "feat": feat, "argmax": amax, "contrib": contrib}
-            self.user_feat, self.item_feat = sides["user"]["feat"], sides["item"]["feat"]
-            self._explain = sides
-            return
-        if user_rev_ids is None or item_rev_ids is None:
-            raise ValueError("NARRE's build_cache needs user_rev_ids [U, R] and item_rev_ids [I, R]")
-        R, T = m.doc_num, m.doc_len
-        ent_chunk = max(1, chunk // R)
-        sides = {}
-        for name, docs, masks, rev_ids, att in (("user", user_docs, user_masks, user_rev_ids, m.user_att),
-                                                ("item", item_docs, item_masks, item_rev_ids, m.item_att)):
-            if docs.shape[1:] != (R, T) or rev_ids.shape != docs.shape[:2]:
-                raise ValueError(f"NARRE was built for [*, {R}, {T}] reviews with [*, {R}] review ids, got "
-                                 f"{tuple(docs.shape)} / {tuple(rev_ids.shape)}")
-            n = docs.shape[0]
-            feat, amax, contrib = self._encode_explain(docs.reshape(n * R, T), None if masks is None else masks.reshape(n * R, T),
-                                                       ent_chunk * R)
-            outs, scores = [], []
-            for lo in range(0, n, ent_chunk):
-                o, s = att(feat[lo * R:(lo + ent_chunk) * R].view(-1, R, feat.shape[1]), rev_ids[lo:lo + ent_chunk])
-                outs.append(o)
-                scores.append(s.view(-1, R))
-            sides[name] = {"docs": docs, "masks": masks, "rev_ids": rev_ids, "feat": feat, "argmax": amax, "contrib": contrib,
-                           "att": torch.cat(scores), "out": torch.cat(outs)}
-        self.user_feat, self.item_feat = sides["user"].pop("out"), sides["item"].pop("out")
-        self._explain = sides
-
-    def _build_siamese_cache(self, user_docs, item_docs, user_masks, item_masks, user_rev_masks, item_rev_masks, chunk, explain):
-        """SimpleSiamese: SimpleSiamese.encode_side over chunks of chunk // R entities.  explain=True also keeps per entity the
-        attention's inputs v [R, F] and weights s [R], a = P^T (w * (1 - tanh^2(P v + c))) [R, F] (zero for a masked review;
-        in float64, then fp32) and, where the head is not fused (K13 then forms g itself), the LastFeat outputs [K]."""
-        m = self.model
-        proj = m.review_att_layer.proj_layer[0]
-        P, c = proj.weight.detach().double(), proj.bias.detach().double()
-        w = m.review_att_layer.inner_product.weight.detach().double().view(-1)
-        feats, sides = {}, {}
-        for name, docs, wm, rm in (("user", user_docs, user_masks, user_rev_masks), ("item", item_docs, item_masks, item_rev_masks)):
-            if (docs.dim() != 3 or (wm is not None and tuple(wm.shape) != tuple(docs.shape))
-                    or (rm is not None and tuple(rm.shape) != tuple(docs.shape[:2]))):
-                raise ValueError(f"SimpleSiamese takes {name}_docs [n, R, T] with word masks [n, R, T] and review masks [n, R], "
-                                 f"got {tuple(docs.shape)} / {None if wm is None else tuple(wm.shape)} / "
-                                 f"{None if rm is None else tuple(rm.shape)}")
-            R = docs.shape[1]
-            step = max(1, chunk // R)
-            keep = {k: [] for k in ("feat", "v", "att", "a")}
-            for lo in range(0, docs.shape[0], step):
-                d = docs[lo:lo + step]
-                wmk = None if wm is None else wm[lo:lo + step]
-                rmk = ((d != 0) if wmk is None else wmk).any(-1) if rm is None else rm[lo:lo + step]
-                f, s, v = m.encode_side(d, wmk, rmk)
-                keep["feat"].append(f)
-                if explain:
-                    th = torch.tanh(v.double() @ P.t() + c)
-                    keep["a"].append((((w * (1 - th * th)) @ P) * rmk.unsqueeze(-1)).float())
-                    keep["v"].append(v.contiguous())
-                    keep["att"].append(s.reshape(-1, R))
-            feats[name] = torch.cat(keep.pop("feat"))
-            if explain:
-                sides[name] = {"docs": docs, "masks": wm, **{k: torch.cat(t) for k, t in keep.items()}}
-        self.user_feat, self.item_feat = feats["user"], feats["item"]
-        if explain:
-            if not self._siamese_fused_g():
-                sides["user"]["lat"], sides["item"]["lat"] = (t.float() for t in self._latents64())
-            self._explain = sides
+        contrib = torch.empty(docs.shape[0], sum(h * k for h, k, _ in specs), dtype=torch.float32, device=table.device)
+        col = tcol = 0
+        for i, (h, k, pad) in enumerate(specs):
+            ops.conv_window_contrib(table, docs, masks, conv.list_of_conv1d[i].weight.detach(), pad, argmax[:, col:col + h],
+                                    packed=conv.packed(i), mask_from_ids=True, out=contrib[:, tcol:tcol + h * k])
+            col += h
+            tcol += h * k
+        return contrib
 
     def _siamese_fused_g(self) -> bool:
         """Whether g = d pred / d feat comes from K4's backward (ops.head_text_grads) rather than from K13 itself."""
@@ -298,30 +227,29 @@ class PairScorer:
         m = self.model
         u_text = ops.gather_rows(self.user_feat, u_ids)
         i_text = ops.gather_rows(self.item_feat, i_ids)
-        if _is_datt(m):
+        if not u_text.shape[0]:                 # no pairs (K4 takes batches of at least one)
+            return u_text.new_empty(0)
+        if isinstance(m, DualAtt):
             return torch.sum(torch.mul(u_text, i_text), 1).view(-1)
-        if _is_siamese(m):
+        if isinstance(m, SimpleSiamese):
             return m.head(u_text, i_text, u_ids, i_ids).view(-1)
         return fused_head(m.user_feat, m.item_feat, m.fm, u_text, i_text, u_ids, i_ids, False, None).view(-1)
 
     def _last_feats(self):
         m = self.model
-        return (m.user_last_feat_layer, m.item_last_feat_layer) if _is_siamese(m) else (m.user_feat, m.item_feat)
+        return (m.user_last_feat_layer, m.item_last_feat_layer) if isinstance(m, SimpleSiamese) else (m.user_feat, m.item_feat)
 
     def _head_params(self):
+        """K4's parameters for the model's head in layers.head_params' order (D-ATT: none)."""
         m = self.model
-        if _is_datt(m):
-            return []
-        uf, itf = self._last_feats()
-        bias = [m.fm.user_bias.weight, m.fm.item_bias.weight] if isinstance(m.fm, FM) else []     # not FMWithoutUIBias
-        return [uf.W, uf.b, uf.ebd.weight, itf.W, itf.b, itf.ebd.weight, m.fm.h, *bias, m.fm.g_bias]
+        return [] if isinstance(m, DualAtt) else head_params(*self._last_feats(), m.fm)[0]
 
     def _latents64(self) -> Tuple[torch.Tensor, torch.Tensor]:
         """LastFeat (models/deepconn/layers.py:163) of every cached entity in float64, [U, K] / [I, K]: exact fp32 latents
         whatever the TF32 setting."""
-        (Wu, bu, eu, Wi, bi, ei) = [p.detach().double() for p in self._head_params()[:6]]
-        return (self.user_feat.double() @ Wu + bu + eu[:self.user_feat.shape[0]],
-                self.item_feat.double() @ Wi + bi + ei[:self.item_feat.shape[0]])
+        return tuple(feat.double() @ lf.W.detach().double() + lf.b.detach().double()
+                     + lf.ebd.weight.detach().double()[:feat.shape[0]]
+                     for feat, lf in zip((self.user_feat, self.item_feat), self._last_feats()))
 
     def factors(self) -> Tuple[torch.Tensor, Optional[torch.Tensor], torch.Tensor, Optional[torch.Tensor]]:
         """(A [U, D], row_bias [U] or None, B [I, D], col_bias [I] or None) with score(u, i) = A[u] . B[i] + biases for the
@@ -329,22 +257,24 @@ class PairScorer:
         its version counter) or the cache was rebuilt."""
         if self.user_feat is None:
             raise RuntimeError("PairScorer.build_cache(...) first")
+        m = self.model
         params = self._head_params()
-        key = tuple((p._version, p.data_ptr()) for p in params) + ((self.user_feat.data_ptr(), self.item_feat.data_ptr()),)
+        key = (tuple((p._version, p.data_ptr()) for p in params if p is not None)
+               + ((self.user_feat.data_ptr(), self.item_feat.data_ptr()),))
         if self._factors is None or self._factors[0] != key:
-            if _is_datt(self.model):
+            if isinstance(m, DualAtt):
                 f = (self.user_feat, None, self.item_feat, None)
             else:
                 with torch.no_grad():
                     u_lat, i_lat = self._latents64()
                     n_u, n_i = u_lat.shape[0], i_lat.shape[0]
-                    h, g = params[6].detach().double(), params[-1].detach().double()
-                    if len(params) == 10:
-                        ub, ib = params[7].detach().double()[:n_u], params[8].detach().double()[:n_i]
-                    else:                                # FMWithoutUIBias: row_bias = g_bias, no column bias
-                        ub, ib = u_lat.new_zeros(n_u, 1), i_lat.new_zeros(n_i, 1)
-                    f = tuple(t.float().contiguous() for t in fm_factors(u_lat, i_lat, h, ub, ib, g))
-                    if len(params) != 10:
+                    fm = m.fm
+                    bias = isinstance(fm, FM)            # FMWithoutUIBias: row_bias = g_bias, no column bias
+                    ub = fm.user_bias.weight.detach().double()[:n_u] if bias else u_lat.new_zeros(n_u, 1)
+                    ib = fm.item_bias.weight.detach().double()[:n_i] if bias else i_lat.new_zeros(n_i, 1)
+                    f = tuple(t.float().contiguous()
+                              for t in fm_factors(u_lat, i_lat, fm.h.detach().double(), ub, ib, fm.g_bias.detach().double()))
+                    if not bias:
                         f = f[:3] + (None,)
             self._factors = (key, f)
         return self._factors[1]
@@ -373,7 +303,7 @@ class PairScorer:
         rb_rows = None if rb is None else rb.index_select(0, u_ids)
         pad = None
         if exclude_padding:
-            pad = 0 if _is_datt(self.model) or _is_siamese(self.model) else self.model.fm.item_padding_idx
+            pad = 0 if isinstance(self.model, (DualAtt, SimpleSiamese)) else self.model.fm.item_padding_idx
             if pad is not None and 0 <= pad < B.shape[0]:
                 # a -inf column bias: the padding item's score never beats a threshold, so it is never returned
                 cb = torch.zeros(B.shape[0], dtype=torch.float32, device=B.device) if cb is None else cb.clone()
@@ -456,157 +386,119 @@ class PairScorer:
                 raise ValueError(f"user ids must lie in [0, {n_u}) and item ids in [0, {n_i})")
         m = int(m)
         pred = self.score_cached(u_ids, i_ids)
-        if _is_siamese(mdl):
-            return self._explain_siamese(u_ids, i_ids, pred, m, width, return_maps, chunk)
-        if _is_datt(mdl) and attribution:
-            return self._explain_datt(u_ids, i_ids, pred, m, width, return_maps, chunk)
-        if _is_datt(mdl):
-            L = self._explain["user"]["gate_l"].shape[1]
+        cache = self._explain
+        if isinstance(mdl, DualAtt) and not attribution:
+            L = mdl.doc_len
             if not 1 <= m <= L:
                 raise ValueError(f"m must lie in [1, {L}]")
             sides = []
             for name, ids in (("user", u_ids), ("item", i_ids)):
-                c = self._explain[name]
-                gl = c["gate_l"].index_select(0, ids)
+                gl = cache[name]["gate_l"].index_select(0, ids)
                 # stable sort: equal gates keep the lower position first
                 order = torch.sort(gl, dim=1, descending=True, stable=True).indices[:, :m]
-                sides.append(SideExplanation(local_att=gl, global_att=c["gate_g"].index_select(0, ids), top_pos=order,
+                sides.append(SideExplanation(local_att=gl, global_att=cache[name]["gate_g"].index_select(0, ids), top_pos=order,
                                              top_attr=gl.gather(1, order)))
             return Explanation(pred, *sides)
-        specs = self._conv_specs()
-        R, T = (mdl.doc_num, mdl.doc_len) if _is_narre(mdl) else (1, self._explain["user"]["docs"].shape[1])
-        width = max(k for _, k, _ in specs) if width is None else int(width)
-        if not ops.explain_supported(R * T, m, width, len(specs)):
+
+        # per model: the default width, whether the kernels take (m, width), g_u, g_i = grads(u, i) for a chunk of pairs, g0 =
+        # an empty g, and attrib(side, ids, other side's ids, g) → explain_attrib's dict
+        if isinstance(mdl, SimpleSiamese):
+            table = mdl.word_embedding.embedding.weight.detach()
+            lt_w = mdl.latent_transform_layer[0].weight.detach() if mdl.latent_transform else None
+            last = dict(zip(("user", "item"), self._last_feats()))
+            feats = {"user": self.user_feat, "item": self.item_feat}
+            width = 1 if width is None else int(width)
+            ok = all(ops.explain_avgpool_supported(R * T, R, table.shape[1], self.user_feat.shape[1], m, width)
+                     for R, T in (c["docs"].shape[1:] for c in cache.values()))
+            fused = self._siamese_fused_g()
+            grads = self._head_grads() if fused else lambda u, i: (None, None)      # None: K13 forms g from the latents
+            g0 = torch.empty(0, self.user_feat.shape[1], device=dev) if fused else None
+
+            def attrib(name, ids, other, g):
+                c, o = cache[name], cache["item" if name == "user" else "user"]
+                return ops.explain_avgpool_attrib(table, c["docs"], c["masks"], ids, c["v"], c["a"], c["att"], feats[name], m,
+                                                  width, g=g, other=other, lat=c.get("lat"), lat_other=o.get("lat"),
+                                                  w_side=last[name].W, fm_h=mdl.fm.h, lt_w=lt_w, return_map=return_maps)
+        else:
+            docs = cache["user"]["docs"]
+            R, T = docs.shape[1:] if docs.dim() == 3 else (1, docs.shape[1])
+            if isinstance(mdl, DualAtt):
+                specs = ops.datt_explain_convs(mdl.side_params("u"))
+                width = specs[0][1] if width is None else int(width)              # the local window
+                w0, w3 = mdl.fc[0].weight, mdl.fc[3].weight
+
+                def grads(u, i):
+                    return ops.datt_fc_grads(u, i, self.user_feat, self.item_feat, cache["user"]["hid_mask"],
+                                             cache["item"]["hid_mask"], w0, w3)
+            else:
+                specs = self._conv_specs()
+                width = max(k for _, k, _ in specs) if width is None else int(width)
+                grads = self._head_grads()
+                if isinstance(mdl, NARRE):
+                    grads = self._narre_grads(grads)
+            h_tot = sum(h for h, _, _ in specs)
+            ok = ops.explain_supported(R * T, m, width, len(specs))
+            g0 = torch.empty(0, R, h_tot, device=dev)
+
+            def attrib(name, ids, other, g):
+                c = cache[name]
+                return ops.explain_attrib(ids * R, g.view(ids.numel(), R, h_tot), c.get("feat"), c["argmax"], c["contrib"],
+                                          specs, R, T, m, width, return_map=return_maps, return_review_attr="att" in c,
+                                          dense_coef=c.get("gate_coef"), dense_vec=c.get("gate_vec"))
+        if not ok:
             raise ValueError(f"explain takes 1 <= m <= {ops.EXPLAIN_MAX_M}, 1 <= width <= {ops.EXPLAIN_MAX_WIDTH} and at most "
-                             f"{ops.EXPLAIN_MAX_POSITIONS} positions per entity (got m={m}, width={width}, {R} x {T})")
-        head = self._head_params()
-        pads = (mdl.user_feat.padding_idx, mdl.item_feat.padding_idx, mdl.fm.padding_idx, mdl.fm.item_padding_idx)
-        head_scratch = [torch.empty_like(p) for p in head]
-        if _is_narre(mdl):
-            att_prm = [[a.W_rv, a.W_id, a.h, a.b_1, a.b_2, a.ebd_vals.weight] for a in (mdl.user_att, mdl.item_att)]
-            att_scratch = [[torch.empty_like(p) for p in sp] for sp in att_prm]
-            att_pads = (mdl.user_att.padding_idx, mdl.item_att.padding_idx)
+                             f"{ops.EXPLAIN_MAX_POSITIONS} positions per entity within the kernel's shared memory (got m={m}, "
+                             f"width={width}, documents {tuple(c['docs'].shape[1:] for c in cache.values())})")
         parts = {"user": [], "item": []}
         for lo in range(0, u_ids.numel(), chunk):
             u, i = u_ids[lo:lo + chunk], i_ids[lo:lo + chunk]
-            g_u, g_i = ops.head_text_grads(ops.gather_rows(self.user_feat, u), ops.gather_rows(self.item_feat, i), u, i, head,
-                                           pads, head_scratch)
-            if _is_narre(mdl):
-                cu, ci = self._explain["user"], self._explain["item"]
-                H = cu["feat"].shape[1]
-                g_u, g_i = ops.narre_feat_grads(
-                    [cu["feat"].view(-1, R, H).index_select(0, u), ci["feat"].view(-1, R, H).index_select(0, i)],
-                    [cu["rev_ids"].index_select(0, u), ci["rev_ids"].index_select(0, i)],
-                    [cu["att"].index_select(0, u), ci["att"].index_select(0, i)], [g_u, g_i], att_prm, att_pads, att_scratch)
-            for name, ids, g in (("user", u, g_u), ("item", i, g_i)):
-                c = self._explain[name]
-                parts[name].append(ops.explain_attrib(ids * R, g.view(ids.numel(), R, -1), c["feat"], c["argmax"], c["contrib"],
-                                                      specs, R, T, m, width, return_map=return_maps,
-                                                      return_review_attr=_is_narre(mdl)))
-        sides = []
-        for name, ids in (("user", u_ids), ("item", i_ids)):
-            p = parts[name]
-            cat = {k: torch.cat([x[k] for x in p]) if p else None for k in (p[0] if p else {})}
-            if not p:                                   # no pairs: empty results of the right shapes
-                cat = ops.explain_attrib(ids, torch.empty(0, R, sum(h for h, _, _ in specs), device=dev),
-                                         self._explain[name]["feat"], self._explain[name]["argmax"],
-                                         self._explain[name]["contrib"], specs, R, T, m, width, return_maps, _is_narre(mdl))
-            mp = cat.get("map")
-            sides.append(SideExplanation(
-                text_total=cat["text_total"], top_pos=cat["top_pos"], top_attr=cat["top_attr"], bottom_pos=cat["bottom_pos"],
-                bottom_attr=cat["bottom_attr"], map=None if mp is None else (mp.view(-1, R, T) if _is_narre(mdl) else mp),
-                review_weight=self._explain[name]["att"].index_select(0, ids) if _is_narre(mdl) else None,
-                review_attr=cat.get("review_attr")))
-        return Explanation(pred, *sides)
-
-    def _explain_datt(self, u_ids, i_ids, pred, m, width, return_maps, chunk) -> "Explanation":
-        mdl = self.model
-        L = mdl.doc_len
-        specs = ops.datt_explain_convs(self._datt_side_prm("u"))
-        width = specs[0][1] if width is None else int(width)
-        if not ops.explain_supported(L, m, width, len(specs)):
-            raise ValueError(f"explain takes 1 <= m <= {ops.EXPLAIN_MAX_M}, 1 <= width <= {ops.EXPLAIN_MAX_WIDTH} and at most "
-                             f"{ops.EXPLAIN_MAX_POSITIONS} positions per entity (got m={m}, width={width}, L={L})")
-        cu, ci = self._explain["user"], self._explain["item"]
-        w0, w3 = mdl.fc[0].weight.detach(), mdl.fc[3].weight.detach()
-        parts = {"user": [], "item": []}
-        for lo in range(0, u_ids.numel(), chunk):
-            u, i = u_ids[lo:lo + chunk], i_ids[lo:lo + chunk]
-            g_u, g_i = ops.datt_fc_grads(u, i, self.user_feat, self.item_feat, cu["hid_mask"], ci["hid_mask"], w0, w3)
-            for name, ids, g in (("user", u, g_u), ("item", i, g_i)):
-                c = self._explain[name]
-                parts[name].append(ops.explain_attrib(ids, g.view(ids.numel(), 1, -1), None, c["argmax"], c["contrib"], specs, 1,
-                                                      L, m, width, return_map=return_maps, dense_coef=c["gate_coef"],
-                                                      dense_vec=c["gate_vec"]))
-        sides = []
-        for name, ids in (("user", u_ids), ("item", i_ids)):
-            c = self._explain[name]
-            p = parts[name]
-            if p:
-                cat = {k: torch.cat([x[k] for x in p]) for k in p[0]}
-            else:                                       # no pairs: empty results of the right shapes
-                cat = ops.explain_attrib(ids, torch.empty(0, 1, c["argmax"].shape[1], device=ids.device), None, c["argmax"],
-                                         c["contrib"], specs, 1, L, m, width, return_maps, dense_coef=c["gate_coef"],
-                                         dense_vec=c["gate_vec"])
-            sides.append(SideExplanation(
-                text_total=cat["text_total"], top_pos=cat["top_pos"], top_attr=cat["top_attr"], bottom_pos=cat["bottom_pos"],
-                bottom_attr=cat["bottom_attr"], map=cat.get("map"), local_att=c["gate_l"].index_select(0, ids),
-                global_att=c["gate_g"].index_select(0, ids)))
-        return Explanation(pred, *sides)
-
-    def _explain_siamese(self, u_ids, i_ids, pred, m, width, return_maps, chunk) -> "Explanation":
-        """SimpleSiamese: K13 per side, with g from K4's backward where the head is fused (zero bias tables for
-        FMWithoutUIBias: the biases do not enter g), else formed in K13 from the cached LastFeat outputs."""
-        mdl = self.model
-        table = mdl.word_embedding.embedding.weight.detach()
-        feat_w, emb = self.user_feat.shape[1], table.shape[1]
-        width = 1 if width is None else int(width)
-        for name in ("user", "item"):
-            _, R, T = self._explain[name]["docs"].shape
-            if not ops.explain_avgpool_supported(R * T, R, emb, feat_w, m, width):
-                raise ValueError(f"explain takes 1 <= m <= {ops.EXPLAIN_MAX_M}, 1 <= width <= {ops.EXPLAIN_MAX_WIDTH} and at most "
-                                 f"{ops.EXPLAIN_MAX_POSITIONS} positions per entity within 227 KB of shared memory (got m={m}, "
-                                 f"width={width}, {R} x {T}, emb={emb}, feat={feat_w})")
-        uf, itf = self._last_feats()
-        fm = mdl.fm
-        lt_w = mdl.latent_transform_layer[0].weight.detach() if mdl.latent_transform else None
-        fused = self._siamese_fused_g()
-        if fused:
-            head = self._head_params()
-            if not isinstance(fm, FM):
-                head = head[:7] + [torch.zeros(e.shape[0], 1, device=e.device) for e in (head[2], head[5])] + head[7:]
-            pads = (uf.padding_idx, itf.padding_idx, getattr(fm, "padding_idx", 0), getattr(fm, "item_padding_idx", 0))
-            head_scratch = [torch.empty_like(p) for p in head]
-        sides = {"user": (uf, "item"), "item": (itf, "user")}
-
-        def attrib(name, ids, other, g):
-            c, (lf, oname) = self._explain[name], sides[name]
-            return ops.explain_avgpool_attrib(table, c["docs"], c["masks"], ids, c["v"], c["a"], c["att"],
-                                              self.user_feat if name == "user" else self.item_feat, m, width, g=g, other=other,
-                                              lat=c.get("lat"), lat_other=self._explain[oname].get("lat"), w_side=lf.W,
-                                              fm_h=fm.h, lt_w=lt_w, return_map=return_maps)
-        parts = {"user": [], "item": []}
-        for lo in range(0, u_ids.numel(), chunk):
-            u, i = u_ids[lo:lo + chunk], i_ids[lo:lo + chunk]
-            g_u = g_i = None
-            if fused:
-                g_u, g_i = ops.head_text_grads(ops.gather_rows(self.user_feat, u), ops.gather_rows(self.item_feat, i), u, i, head,
-                                               pads, head_scratch)
+            g_u, g_i = grads(u, i)
             parts["user"].append(attrib("user", u, i, g_u))
             parts["item"].append(attrib("item", i, u, g_i))
-        out = []
+        sides = []
         for name, ids in (("user", u_ids), ("item", i_ids)):
-            c, p = self._explain[name], parts[name]
-            if p:
-                cat = {k: torch.cat([x[k] for x in p]) for k in p[0]}
-            else:                                       # no pairs: empty results of the right shapes
-                cat = attrib(name, ids, ids, torch.empty(0, feat_w, device=ids.device) if fused else None)
+            c = cache[name]
+            # no pairs: K4 takes at least one, so only the attribution runs, on an empty g (empty results of the right shapes)
+            p = parts[name] or [attrib(name, ids, ids, g0)]
+            cat = {k: torch.cat([x[k] for x in p]) for k in p[0]}
             mp = cat.get("map")
-            out.append(SideExplanation(
+            sides.append(SideExplanation(
                 text_total=cat["text_total"], top_pos=cat["top_pos"], top_attr=cat["top_attr"], bottom_pos=cat["bottom_pos"],
                 bottom_attr=cat["bottom_attr"], map=None if mp is None else mp.view(-1, *c["docs"].shape[1:]),
-                review_weight=c["att"].index_select(0, ids), review_attr=cat["review_attr"]))
-        return Explanation(pred, *out)
+                review_weight=c["att"].index_select(0, ids) if "att" in c else None, review_attr=cat.get("review_attr"),
+                local_att=c["gate_l"].index_select(0, ids) if "gate_l" in c else None,
+                global_att=c["gate_g"].index_select(0, ids) if "gate_g" in c else None))
+        return Explanation(pred, *sides)
+
+    def _head_grads(self):
+        """grads(u, i) → (g_u, g_i) = d pred / d feat of both sides for pairs (u, i) from K4's backward on the cached
+        features."""
+        mdl = self.model
+        head, pads = head_params(*self._last_feats(), mdl.fm, zero_bias=True)
+        scratch = [torch.empty_like(p) for p in head]
+
+        def grads(u, i):
+            u_text, i_text = ops.gather_rows(self.user_feat, u), ops.gather_rows(self.item_feat, i)
+            return ops.head_text_grads(u_text, i_text, u, i, head, pads, scratch)
+        return grads
+
+    def _narre_grads(self, head_grads):
+        """grads(u, i) → (g_u, g_i) = d pred / d feat [P, R, H] of each review's features: head_grads(u, i) through K3's
+        backward, with the cached attention weights."""
+        mdl = self.model
+        cu, ci = self._explain["user"], self._explain["item"]
+        R, H = mdl.doc_num, cu["feat"].shape[1]
+        atts = (mdl.user_att, mdl.item_att)
+        att_prm = [a.kernel_params() for a in atts]
+        att_scratch = [[torch.empty_like(p) for p in sp] for sp in att_prm]
+
+        def grads(u, i):
+            return ops.narre_feat_grads(
+                [cu["feat"].view(-1, R, H).index_select(0, u), ci["feat"].view(-1, R, H).index_select(0, i)],
+                [cu["rev_ids"].index_select(0, u), ci["rev_ids"].index_select(0, i)],
+                [cu["att"].index_select(0, u), ci["att"].index_select(0, i)], head_grads(u, i), att_prm,
+                [a.padding_idx for a in atts], att_scratch)
+        return grads
 
     def tokens_at(self, side: str, ent_ids: torch.Tensor, pos: torch.Tensor) -> torch.Tensor:
         """Token ids at flat positions pos [B, m] (explain's top_pos / bottom_pos) of the kept documents of entities

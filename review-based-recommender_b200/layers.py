@@ -304,6 +304,22 @@ class FM(nn.Module):
         return fm @ self.h + ub + ib + self.g_bias
 
 
+def head_params(user_feat: LastFeat, item_feat: LastFeat, fm: nn.Module, zero_bias: bool = False):
+    """K4's parameters (Wu, bu, ebd_u, Wi, bi, ebd_i, fm_h, user_bias, item_bias, g_bias) and padding indices (user, item,
+    FM user, FM item) for LastFeat(user) + LastFeat(item) + `fm`.  An FM without user / item bias tables (SimpleSiamese's
+    FMWithoutUIBias) has None in their two slots and padding index 0 for them, or with zero_bias zero tables of the LastFeat
+    embeddings' heights, which K4 can read (the biases do not enter d pred / d text)."""
+    if isinstance(fm, FM):
+        bias, fm_pads = [fm.user_bias.weight, fm.item_bias.weight], (fm.padding_idx, fm.item_padding_idx)
+    else:
+        bias, fm_pads = [None, None], (0, 0)
+        if zero_bias:
+            bias = [torch.zeros(f.ebd.weight.shape[0], 1, device=f.ebd.weight.device) for f in (user_feat, item_feat)]
+    params = [user_feat.W, user_feat.b, user_feat.ebd.weight, item_feat.W, item_feat.b, item_feat.ebd.weight, fm.h, *bias,
+              fm.g_bias]
+    return params, (user_feat.padding_idx, item_feat.padding_idx, *fm_pads)
+
+
 def fused_head(user_feat: LastFeat, item_feat: LastFeat, fm: FM, u_text, i_text, u_id, i_id, training: bool, arena,
                ratings: Optional[torch.Tensor] = None):
     """K4: LastFeat(user) + LastFeat(item) + FM in one kernel (reference deepconn.py:48-51).  With `ratings` the same launch
@@ -313,9 +329,7 @@ def fused_head(user_feat: LastFeat, item_feat: LastFeat, fm: FM, u_text, i_text,
     # base plus a step counter that lives on the device and is bumped at the start of every replay
     seed_dev = fm.__dict__.get("_rbr_seed_dev") if p > 0 else None
     seed = 0 if p <= 0 else (0x5EED if seed_dev is not None else int(torch.randint(0, 2 ** 62, (1,)).item()))
-    params = [user_feat.W, user_feat.b, user_feat.ebd.weight, item_feat.W, item_feat.b, item_feat.ebd.weight, fm.h,
-              fm.user_bias.weight, fm.item_bias.weight, fm.g_bias]
-    pads = (user_feat.padding_idx, item_feat.padding_idx, fm.padding_idx, fm.item_padding_idx)
+    params, pads = head_params(user_feat, item_feat, fm)
     fm.__dict__["_rbr_last_drop"] = (p, seed, seed_dev)          # for tests: ops.head_dropout_mask(B, K, *this)
     if ratings is not None:
         return ops.HeadLossFn.apply(u_text, i_text, u_id, i_id, ratings, *params, p, seed, pads, arena, params, seed_dev)
@@ -335,8 +349,12 @@ class LinearAttention(nn.Module):
         self.dropout = nn.Dropout(p=dropout)
         self._arena = None
 
+    def kernel_params(self) -> List[torch.Tensor]:
+        """The six parameters in K3's order: (W_rv, W_id, h, b_1, b_2, ebd_vals)."""
+        return [self.W_rv, self.W_id, self.h, self.b_1, self.b_2, self.ebd_vals.weight]
+
     def forward(self, feat, other_id):
         """feat [bz, dnum, H], other_id [bz, dnum] → (out [bz, H], att_scores [bz, dnum, 1])  (narre.py:40-64)."""
-        params = [self.W_rv, self.W_id, self.h, self.b_1, self.b_2, self.ebd_vals.weight]
+        params = self.kernel_params()
         out, scores = ops.NarreAttnFn.apply(feat, other_id, *params, self.padding_idx, self._arena, params)
         return self.dropout(out), scores

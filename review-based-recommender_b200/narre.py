@@ -62,8 +62,7 @@ class NARRE(HotPathModule):
         ua, ia = self.user_att, self.item_att
         if self.fused_attention and ops.narre_attn_pair_supported(self.doc_num, self.hiddem_dim, ua.W_rv.shape[1]):
             # both sides in one launch per direction on the tensor cores (csrc/attn_tc.cu); dropout as in LinearAttention.forward
-            pu = [ua.W_rv, ua.W_id, ua.h, ua.b_1, ua.b_2, ua.ebd_vals.weight]
-            pi = [ia.W_rv, ia.W_id, ia.h, ia.b_1, ia.b_2, ia.ebd_vals.weight]
+            pu, pi = ua.kernel_params(), ia.kernel_params()
             u_out, u_att_scores, i_out, i_att_scores = ops.NarreAttnPairFn.apply(
                 u_feat, reuid, i_feat, reiid, *pu, *pi, (ua.padding_idx, ia.padding_idx), self.last_arena, pu + pi)
             return ua.dropout(u_out), ia.dropout(i_out), u_att_scores, i_att_scores

@@ -392,3 +392,29 @@ def test_feature_cache_scores_are_bit_identical_to_per_pair_scoring():
     assert torch.equal(cached, direct)
     rp = orc.deepconn_forward(_f64(params, round_bf16=True), ud, idd, ud != 0, idd != 0, u_ids, i_ids)
     assert rel_err(cached.cpu(), rp.cpu()) < 2e-3
+
+
+@pytest.mark.parametrize("H", [100, 300], ids=["proj", "noproj"])
+def test_feature_cache_scores_hier_pooling(H):
+    """arch="HierPooling" (K8, then the Linear projection when E != H): the feature cache's scores against per-pair scoring."""
+    from rbr_b200.inference import PairScorer
+    U, I, V, E, K, L = 300, 200, 5000, 300, 32, 500
+    model = rbr_b200.DeepCoNNpp(U, I, V, [3], E, H, K, L, None, 0.5, arch="HierPooling")
+    model.load_state_dict(synth.deepconn_hier_params(U, I, V, E, H, K, seed=4))
+    scorer = PairScorer(model.cuda())
+    user_docs, _ = synth.doc_batch(U, L, V, seed=1)
+    item_docs, _ = synth.doc_batch(I, L, V, seed=2)
+    user_docs[0] = 0
+    item_docs[0] = 0
+    user_docs, item_docs = user_docs.cuda(), item_docs.cuda()
+    scorer.build_cache(user_docs, item_docs, chunk=128)
+    gen = torch.Generator().manual_seed(3)
+    u_ids = torch.randint(0, U, (4096,), generator=gen).cuda()
+    i_ids = torch.randint(0, I, (4096,), generator=gen).cuda()
+    cached = scorer.score_cached(u_ids, i_ids)
+    ud, idd = user_docs[u_ids], item_docs[i_ids]
+    direct = scorer.score_pairs(ud, idd, ud != 0, idd != 0, u_ids, i_ids)
+    if H == E:
+        assert torch.equal(cached, direct)
+    else:                       # the projection is a library GEMM, whose bits may depend on the batch (128 entities vs 4096 pairs)
+        assert rel_err(cached, direct) < FP32_TOL

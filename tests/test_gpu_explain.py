@@ -109,12 +109,12 @@ def _narre(prec, R=10, T=60, explain=True):
     return sc, (ud, idd, urev, irev)
 
 
-def _datt(prec, L=120):
+def _datt(prec, L=120, explain=True):
     m = rbr_b200.DualAtt(V, L, 5, 200, 100, 100, 500, 50, 0.0, None, precision=prec)
     m.load_state_dict(synth.dual_att_params(V, L, 5, 200, 100, 100, 500, 50, seed=0))
     sc = PairScorer(m.cuda())
     ud, idd = _docs(U, L, 6), _docs(I, L, 7)
-    sc.build_cache(ud, idd, explain=True)
+    sc.build_cache(ud, idd, explain=explain)
     return sc, (ud, idd)
 
 
@@ -346,6 +346,13 @@ def test_consistency(name):
             assert torch.equal(a, getattr(getattr(e3, side), f)), f
             assert torch.equal(a[perm], getattr(getattr(ep, side), f)), f
     assert torch.equal(e1.pred[perm], ep.pred)
+    empty = sc.explain(u[:0], i[:0], m=5, return_maps=True)
+    assert empty.pred.shape == (0,) and empty.user.top_pos.shape == (0, 5) and empty.item.bottom_attr.shape == (0, 5)
+    if name == "narre":
+        assert empty.user.map.shape == (0, 10, 60) and empty.item.review_weight.shape == (0, 10)
+        assert empty.item.review_attr.shape == (0, 10)
+    else:
+        assert empty.user.map.shape == (0, 60) and empty.item.review_weight is None
 
 
 def test_explain_needs_the_explain_cache():
@@ -383,3 +390,17 @@ def test_kernels_in_profiler_trace():
     names = " ".join(evt.key for evt in prof.key_averages())
     assert "conv_window_contrib_kernel" in names
     assert "explain_attrib_kernel" in names
+
+
+def test_plain_cache_launches_no_explain_kernels():
+    """build_cache(explain=False) does the encoder's work only: no K12a contributions, no D-ATT per-entity terms"""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for make in (_deepconn, _narre, _datt):
+            sc, _ = make("bf16", explain=False)
+            assert sc._explain is None
+        torch.cuda.synchronize()
+    names = " ".join(evt.key for evt in prof.key_averages())
+    assert "gate" in names                                              # the trace holds the encoders' kernels
+    assert "conv_window_contrib_kernel" not in names
+    assert "datt_explain_contrib_kernel" not in names

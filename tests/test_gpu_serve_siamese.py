@@ -268,10 +268,9 @@ def test_determinism(ub, lt):
         assert _nan_equal(getattr(e1.user, f), getattr(e4.user, f)), f
     tok = sc.tokens_at("user", u, e1.user.top_pos)
     assert bool((tok[e1.user.top_pos >= 0] >= 0).all())
-    # no pairs (the library-op head; K4 itself takes batches of at least one pair)
-    if not sc._siamese_fused_g():
-        e0 = sc.explain(u[:0], i[:0], return_maps=True)
-        assert e0.user.top_pos.shape == (0, 5) and e0.item.map.shape[0] == 0
+    # no pairs, with g from K4's backward or from K13
+    e0 = sc.explain(u[:0], i[:0], return_maps=True)
+    assert e0.user.top_pos.shape == (0, 5) and e0.item.map.shape[0] == 0
 
 
 def test_ids_outside_the_table_read_as_zero_rows():
