@@ -500,6 +500,26 @@ int rbr_explain_avgpool_attrib(const float* table, int64_t vocab, int64_t emb, c
                                float* text_total, int64_t* top_pos, float* top_attr, int64_t* bottom_pos, float* bottom_attr,
                                float* map, float* review_attr, int flags, void* stream);
 
+/* ---- K14: diversified top-k — maximal marginal relevance over a relevance pool -------------------------------------------
+ * Row r's pool is pool_scores / pool_items [n_rows, pool] (row-major), e.g. rbr_factor_topk's output for k = pool: score
+ * descending then item id ascending.  Position c is eligible when 0 <= pool_items[r, c] < n_items and its score is finite
+ * (K10's (-inf, -1) slots are not).  item_vecs [n_items, dim] fp32 row-major are the items' unit-normalised vectors
+ * (a zero row is allowed: its similarity to anything is 0);  sim(a, b) = v_a . v_b, an fp32 dot product with one fmaf per
+ * element in ascending element order from 0, so every sim has the same bits in every call.
+ *   rel(c) = (s_c - lo) / (hi - lo)  with lo / hi the min / max of the row's eligible scores (rel = 1 when hi == lo);
+ *   step 0 picks the largest rel; step t picks, over the eligible positions not yet picked, the largest
+ *   obj(c) = lam * rel(c) - (1 - lam) * maxsim(c),  maxsim(c) = max over the picked j of sim(c, j),
+ * each operation rounded to fp32 (no contraction; 1 - lam is rounded to fp32 once, -0 counts as +0).  Ties go to the lower
+ * pool position (64-bit key: order-preserving objective bits << 32 | ~position).  out_scores / out_items [n_rows, k] get
+ * the picked positions' pool scores and items in selection order; a row with fewer than k eligible positions ends in
+ * (-inf, -1).  Results are bit-identical across calls, batches, row orders and chunkings.  lam = 1 returns the pool's
+ * first k eligible entries in pool order.  One CTA per row; k * pool * dim FMAs per row.
+ * Limits (rbr_mmr_supported, host-only): 1 <= k <= pool <= 256 (K10's largest k), 1 <= dim <= 512 (K10's largest dim);
+ * otherwise rbr_mmr_select returns RBR_EUNSUPPORTED before any launch; lam outside [0, 1] is RBR_EINVAL.                  */
+int rbr_mmr_supported(int64_t pool, int64_t dim, int64_t k);
+int rbr_mmr_select(const float* pool_scores, const int64_t* pool_items, int64_t n_rows, int64_t pool, const float* item_vecs,
+                   int64_t n_items, int64_t dim, int64_t k, float lam, float* out_scores, int64_t* out_items, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

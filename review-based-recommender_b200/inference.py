@@ -16,7 +16,10 @@ encoder work.  In eval mode every model puts an entity's side through that entit
 
 `PairScorer.recommend` answers "the k best items for these users out of the whole catalogue" with K10 (ops.factor_topk),
 which never materialises the users x items score matrix; `rank_items` / `evaluate` give the exact full-catalogue rank of
-held-out items and HR@k / Recall@k / NDCG@k / MRR / AUC from it with K11 (ops.factor_rank), on the same scores.  The FM head factorises exactly:
+held-out items and HR@k / Recall@k / NDCG@k / MRR / AUC from it with K11 (ops.factor_rank), on the same scores;
+`recommend_diverse` re-ranks recommend's top-P by maximal marginal relevance over item-vector similarity with K14
+(ops.mmr_select), and `list_metrics` gives the lists' intra-list diversity and catalogue coverage.  The FM head factorises
+exactly:
   relu(u*i) = relu(u)*relu(i) + relu(-u)*relu(-i)   ⇒   score(u,i) = A[u] . B[i] + row_bias[u] + col_bias[i]
 with A = [h*relu(u_lat), h*relu(-u_lat)], B = [relu(i_lat), relu(-i_lat)], row_bias = ub + g, col_bias = ib (fm_factors);
 D-ATT's score is already a dot product of the two FC outputs.
@@ -56,6 +59,7 @@ class PairScorer:
         self.user_feat: Optional[torch.Tensor] = None
         self.item_feat: Optional[torch.Tensor] = None
         self._factors = None         # (key, (A, row_bias, B, col_bias)) derived from the current head parameters
+        self._unit_items = None      # (key, source, unit-normalised item vectors) of recommend_diverse
         self._explain = None         # per-side tensors kept by build_cache(explain=True)
 
     @torch.no_grad()
@@ -88,6 +92,7 @@ class PairScorer:
         m = self.model
         m.eval()
         self._factors = None
+        self._unit_items = None
         self._explain = None
         # per side: (documents, masks, the model's per-review input: NARRE's review ids, SimpleSiamese's review masks)
         sides = {"user": (user_docs, user_masks, None), "item": (item_docs, item_masks, None)}
@@ -290,6 +295,47 @@ class PairScorer:
         (-inf, -1).  Scores agree with score_cached on the same pairs to fp32 rounding."""
         A_rows, rb_rows, B, cb, _ = self._user_rows(u_ids, exclude_padding)
         return ops.factor_topk(A_rows, rb_rows, B, cb, k, exclude=exclude)
+
+    @torch.no_grad()
+    def recommend_diverse(self, u_ids: torch.Tensor, k: int, lam: float = 0.5, pool: Optional[int] = None,
+                          exclude: Optional[Tuple[torch.Tensor, torch.Tensor]] = None, exclude_padding: bool = True,
+                          item_vecs: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """k items per user u_ids[r], relevant and not redundant: maximal marginal relevance (K14, ops.mmr_select) over the
+        pool recommend(u_ids, pool, exclude, exclude_padding) (K10; default pool = min(256, 4 k)).  Step 0 takes the pool's
+        best item; each later step the eligible unpicked item with the largest lam * rel - (1 - lam) * max sim to the items
+        picked so far, rel = the score min-max scaled over the row's pool, sim = the cosine of the items' vectors: item_vecs
+        [I, D] (default: the cached item features; e.g. factors()[2]), rows unit-normalised once (a zero row has sim 0 to
+        everything).  Returns (scores [len(u_ids), k] fp32, items [len(u_ids), k] int64) in selection order; the scores are
+        recommend's, bit for bit, and rows with fewer than k eligible items end in (-inf, -1).  lam = 1 is recommend(u_ids,
+        k); pool = k gives a permutation of it.  Results do not depend on the other rows of the call."""
+        k = int(k)
+        pool = min(ops.MMR_MAX_POOL, 4 * k) if pool is None else int(pool)
+        lam = float(lam)
+        vecs = self._unit_item_vecs(item_vecs)
+        if not 0.0 <= lam <= 1.0:
+            raise ValueError(f"lam must lie in [0, 1], got {lam}")
+        if not ops.mmr_supported(pool, vecs.shape[1], k):
+            raise ValueError(f"recommend_diverse takes 1 <= k <= pool <= {ops.MMR_MAX_POOL} and item vectors of at most "
+                             f"{ops.MMR_MAX_DIM} columns (got k={k}, pool={pool}, dim={vecs.shape[1]})")
+        A_rows, rb_rows, B, cb, _ = self._user_rows(u_ids, exclude_padding)
+        pool_scores, pool_items = ops.factor_topk(A_rows, rb_rows, B, cb, pool, exclude=exclude)
+        return ops.mmr_select(pool_scores, pool_items, vecs, k, lam)
+
+    def _unit_item_vecs(self, item_vecs: Optional[torch.Tensor]) -> torch.Tensor:
+        """ops.unit_rows of item_vecs (default: the cached item features), kept until the source changes: keyed by its data
+        pointer, layout and version counter, and holding a reference to it so that the pointer cannot be reused."""
+        if self.item_feat is None:
+            raise RuntimeError("PairScorer.build_cache(...) first")
+        src = self.item_feat if item_vecs is None else item_vecs
+        if not isinstance(src, torch.Tensor) or src.dim() != 2 or src.shape[0] != self.item_feat.shape[0]:
+            raise ValueError(f"item_vecs must be [{self.item_feat.shape[0]}, D] (one row per cached item), got "
+                             f"{tuple(src.shape) if isinstance(src, torch.Tensor) else type(src).__name__}")
+        if src.device != self.item_feat.device:
+            raise ValueError(f"item_vecs is on {src.device}, the cache on {self.item_feat.device}")
+        key = (src.data_ptr(), tuple(src.shape), src.stride(), src.dtype, src._version)
+        if self._unit_items is None or self._unit_items[0] != key:
+            self._unit_items = (key, src, ops.unit_rows(src).contiguous())
+        return self._unit_items[2]
 
     def _user_rows(self, u_ids: torch.Tensor, exclude_padding: bool):
         """(A rows, row_bias rows, B, col_bias, padding item or None) for users u_ids under the current head parameters;
@@ -592,3 +638,35 @@ def ranking_metrics(ranks: torch.Tensor, indptr: torch.Tensor, n_candidates: tor
     out["auc"] = mean(row_sum(term) / m.clamp_min(1), has & (n_cand > m))
     out["n_rows"] = n_rows
     return out
+
+
+def list_metrics(items: torch.Tensor, item_vecs: torch.Tensor, n_items: int, chunk: int = 1024) -> dict:
+    """List-level metrics of recommendation lists (any device, no GPU needed), e.g. to compare recommend with
+    recommend_diverse.
+
+    items [n, k] int64: each row's list, -1 for an empty slot (recommend's tail); item_vecs [I, D]: the item vectors the
+    similarity is taken on, unit-normalised as recommend_diverse does (ops.unit_rows: float64, then fp32; a zero row has
+    sim 0 to everything); n_items: the number of items a list could hold (e.g. I - 1 without the padding item).
+      ild       intra-list diversity: per row, the mean over pairs of its valid items of 1 - sim(a, b) (in float64), then
+                the mean over the rows with at least two valid items (n_rows of them); 0.0 when there is none
+      coverage  the number of distinct valid items over all lists / n_items"""
+    items = items.to(torch.int64)
+    if items.dim() != 2:
+        raise ValueError(f"items must be [n, k], got {tuple(items.shape)}")
+    vecs = ops.unit_rows(item_vecs).to(items.device).double()
+    valid = items >= 0
+    if bool((items >= vecs.shape[0]).any()):
+        raise ValueError(f"item ids must lie in [-1, {vecs.shape[0]})")
+    total, n_rows = 0.0, 0
+    for lo in range(0, items.shape[0], chunk):
+        it, ok = items[lo:lo + chunk], valid[lo:lo + chunk]
+        v = vecs[it.clamp_min(0)] * ok.unsqueeze(-1)
+        dist = 1.0 - v @ v.transpose(1, 2)
+        pair = ok.unsqueeze(2) & ok.unsqueeze(1)
+        pair &= torch.triu(torch.ones_like(pair[0]), diagonal=1)
+        n_pairs = pair.sum((1, 2))
+        has = n_pairs > 0
+        total += float(((dist * pair).sum((1, 2))[has] / n_pairs[has]).sum())
+        n_rows += int(has.sum())
+    coverage = torch.unique(items[valid]).numel() / max(int(n_items), 1)
+    return {"ild": total / n_rows if n_rows else 0.0, "coverage": coverage, "n_rows": n_rows}

@@ -1288,6 +1288,62 @@ def factor_rank(A: torch.Tensor, row_bias: Optional[torch.Tensor], B: torch.Tens
 
 
 # ---------------------------------------------------------------------------------------------------
+# K14: diversified top-k — maximal marginal relevance over a relevance pool
+# ---------------------------------------------------------------------------------------------------
+MMR_MAX_POOL, MMR_MAX_DIM = 256, 512
+
+
+def mmr_supported(pool: int, dim: int, k: int) -> bool:
+    """Whether rbr_mmr_select takes pools of `pool` entries, `dim`-wide item vectors and k picks (host-only query)."""
+    return bool(lib.rbr_mmr_supported(int(pool), int(dim), int(k)))
+
+
+def unit_rows(x: torch.Tensor) -> torch.Tensor:
+    """x [n, dim] with every row scaled to unit length, in float64 and then rounded to fp32; a zero row stays zero."""
+    x64 = x.detach().double()
+    norm = x64.norm(dim=1, keepdim=True)
+    return torch.where(norm > 0, x64 / norm.clamp_min(torch.finfo(torch.float64).tiny), torch.zeros_like(x64)).float()
+
+
+def mmr_select(pool_scores: torch.Tensor, pool_items: torch.Tensor, item_vecs: torch.Tensor, k: int, lam: float
+               ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """K14: per row, k picks from the row's pool by maximal marginal relevance (include/rbr_b200.h, K14).
+
+    pool_scores [n, P] fp32 / pool_items [n, P] int64 CUDA: the row's candidates (e.g. factor_topk's output for k = P); a
+    position is eligible when its item lies in [0, n_items) and its score is finite.  item_vecs [n_items, dim] fp32 CUDA:
+    unit-normalised item vectors (unit_rows), sim = fp32 dot product.  Step 0 picks the largest relevance (the score min-max
+    scaled over the row's eligible positions), step t the largest lam * rel - (1 - lam) * max sim to the items picked so
+    far; ties to the lower position.  Returns (scores [n, k] fp32, items [n, k] int64) in selection order, the pool's own
+    scores; rows with fewer than k eligible positions end in (-inf, -1)."""
+    pool_scores = _req(pool_scores, torch.float32, "pool_scores")
+    pool_items = _req(pool_items, torch.int64, "pool_items")
+    item_vecs = _req(item_vecs, torch.float32, "item_vecs")
+    for t, name in ((pool_items, "pool_items"), (item_vecs, "item_vecs")):
+        if t.device != pool_scores.device:
+            raise ValueError(f"rbr_b200: `{name}` is on {t.device}, pool_scores on {pool_scores.device}")
+    if pool_scores.dim() != 2 or pool_items.shape != pool_scores.shape or item_vecs.dim() != 2:
+        raise ValueError(f"rbr_b200: mmr_select takes pool_scores / pool_items [n, P] and item_vecs [n_items, dim], got "
+                         f"{tuple(pool_scores.shape)} / {tuple(pool_items.shape)} / {tuple(item_vecs.shape)}")
+    n, P = pool_scores.shape
+    n_items, dim = item_vecs.shape
+    k, lam = int(k), float(lam)
+    if not 0.0 <= lam <= 1.0:
+        raise ValueError(f"rbr_b200: lam must lie in [0, 1], got {lam}")
+    if not mmr_supported(P, dim, k):
+        raise ValueError(f"rbr_b200: mmr_select does not take k={k}, pool={P}, dim={dim} "
+                         f"(1 <= k <= pool <= {MMR_MAX_POOL}, 1 <= dim <= {MMR_MAX_DIM})")
+    dev = pool_scores.device
+    scores = torch.empty(n, k, dtype=torch.float32, device=dev)
+    items = torch.empty(n, k, dtype=torch.int64, device=dev)
+    if n == 0:
+        return scores, items
+    with torch.cuda.device(dev):
+        lib.check(lib.rbr_mmr_select(_p(pool_scores), _p(pool_items), n, P, _p(item_vecs), n_items, dim, k, lam, _p(scores),
+                                     _p(items), _stream(True)), "rbr_mmr_select")
+    return scores, items
+
+
+# ---------------------------------------------------------------------------------------------------
 # K12: token attributions of a predicted rating from the per-entity feature cache
 # ---------------------------------------------------------------------------------------------------
 EXPLAIN_MAX_POSITIONS, EXPLAIN_MAX_M, EXPLAIN_MAX_WIDTH, EXPLAIN_MAX_CONVS = 16384, 32, 16, 8
