@@ -18,7 +18,9 @@ encoder work.  In eval mode every model puts an entity's side through that entit
 which never materialises the users x items score matrix; `rank_items` / `evaluate` give the exact full-catalogue rank of
 held-out items and HR@k / Recall@k / NDCG@k / MRR / AUC from it with K11 (ops.factor_rank), on the same scores;
 `recommend_diverse` re-ranks recommend's top-P by maximal marginal relevance over item-vector similarity with K14
-(ops.mmr_select), and `list_metrics` gives the lists' intra-list diversity and catalogue coverage.  The FM head factorises
+(ops.mmr_select), and `list_metrics` gives the lists' intra-list diversity and catalogue coverage.  `add` / `update` grow
+the cache by new entities (served under the side's padding id through a row -> model-id map) and re-encode changed ones in
+place, encoding and re-deriving only those rows (DESIGN.md §5).  The FM head factorises
 exactly:
   relu(u*i) = relu(u)*relu(i) + relu(-u)*relu(-i)   ⇒   score(u,i) = A[u] . B[i] + row_bias[u] + col_bias[i]
 with A = [h*relu(u_lat), h*relu(-u_lat)], B = [relu(i_lat), relu(-i_lat)], row_bias = ub + g, col_bias = ib (fm_factors);
@@ -51,16 +53,97 @@ def fm_factors(u_lat: torch.Tensor, i_lat: torch.Tensor, h: torch.Tensor, user_b
     return A, user_bias.reshape(-1) + g_bias.reshape(()), B, item_bias.reshape(-1)
 
 
+SIDES = ("user", "item")
+_CHUNK = 4096                   # entities per encoder launch in add / update (build_cache's default chunk)
+
+
+def _reserve(buf: torch.Tensor, used: int, need: int) -> torch.Tensor:
+    """buf if it has `need` rows, else a new buffer of max(need, 2 x its rows) rows holding its first `used` rows: a run of
+    appends copies O(total) rows."""
+    if buf.shape[0] >= need:
+        return buf
+    out = buf.new_empty((max(need, 2 * buf.shape[0]),) + tuple(buf.shape[1:]))
+    out[:used] = buf[:used]
+    return out
+
+
+class _Side:
+    """One side of the feature cache.  Every per-entity tensor lives in a buffer with spare rows (`bufs`; "cached" = the
+    cached features, "model_ids" = the row -> model-id map, the rest build_cache(explain=True)'s tensors, `per[key]` rows of
+    it per entity); the first n entities are in use.  `log` holds (generation, rows) of every add / update since the
+    derived caches (factors, unit item vectors) last took them in.  `shape` is the documents' shape past the entity axis
+    (None when the features were assigned, not built from documents)."""
+
+    def __init__(self, feat: torch.Tensor, kept: Optional[dict] = None, shape: Optional[tuple] = None):
+        n = feat.shape[0]
+        self.n = self.n_built = n
+        self.shape = None if shape is None else tuple(shape)
+        self.bufs = {"cached": feat, "model_ids": torch.arange(n, device=feat.device), **(kept or {})}
+        self.kept = None if kept is None else list(kept)
+        self.per = {k: 1 if t is None or not n else t.shape[0] // n for k, t in self.bufs.items()}
+        self.caller_owned = {"docs", "masks"}      # build_cache keeps references to the caller's documents and masks
+        self.gen, self.log = 0, []
+
+    def view(self, key: str) -> Optional[torch.Tensor]:
+        t = self.bufs[key]
+        return None if t is None else t[:self.n * self.per[key]]
+
+    def write(self, rows: Optional[torch.Tensor], new: dict) -> None:
+        """Entity rows `rows` (None: append) <- new {key: rows of that buffer}; a caller's tensor is copied on the first
+        write, never written."""
+        need = self.n + (new["cached"].shape[0] if rows is None else 0)
+        for k, v in new.items():
+            buf, p = self.bufs[k], self.per[k]
+            if k in self.caller_owned:
+                buf = buf[:self.n * p].clone(memory_format=torch.contiguous_format)
+                self.caller_owned.discard(k)
+            buf = _reserve(buf, self.n * p, need * p)
+            if rows is None:
+                buf[self.n * p:need * p] = v
+            else:
+                at = rows if p == 1 else (rows.view(-1, 1) * p + torch.arange(p, device=rows.device)).view(-1)
+                buf.index_copy_(0, at, v.to(buf.dtype))
+            self.bufs[k] = buf
+        if rows is None:
+            rows = torch.arange(self.n, need, device=new["cached"].device)
+        self.n = need
+        self.gen += 1
+        self.log.append((self.gen, rows))
+
+    def changed(self, since: int) -> Optional[torch.Tensor]:
+        """The rows added or updated after generation `since`, ascending; None if there are none."""
+        rows = [r for g, r in self.log if g > since]
+        return torch.unique(torch.cat(rows)) if rows else None
+
+
 class PairScorer:
     def __init__(self, model):
         if not isinstance(model, (DeepCoNNpp, NARRE, DualAtt, SimpleSiamese)):
             raise TypeError("PairScorer serves DeepCoNNpp, NARRE, DualAtt and SimpleSiamese")
         self.model = model.eval()
-        self.user_feat: Optional[torch.Tensor] = None
-        self.item_feat: Optional[torch.Tensor] = None
-        self._factors = None         # (key, (A, row_bias, B, col_bias)) derived from the current head parameters
-        self._unit_items = None      # (key, source, unit-normalised item vectors) of recommend_diverse
-        self._explain = None         # per-side tensors kept by build_cache(explain=True)
+        self._sides = dict.fromkeys(SIDES)   # name -> _Side
+        self._factors = None         # dict: head-parameter key, per side the generation and rows taken in, factor buffers
+        self._unit_items = None      # dict: source key (None: the cached item features), unit-normalised item vectors
+
+    def _get_feat(self, name):
+        s = self._sides[name]
+        return None if s is None else s.view("cached")
+
+    def _set_feat(self, name, feat):
+        self._sides[name] = None if feat is None else _Side(feat)
+        self._factors = self._unit_items = None
+
+    user_feat = property(lambda self: self._get_feat("user"), lambda self, t: self._set_feat("user", t),
+                         doc="The cached user features [U, D] (row e = cache row e)")
+    item_feat = property(lambda self: self._get_feat("item"), lambda self, t: self._set_feat("item", t),
+                         doc="The cached item features [I, D]")
+
+    @property
+    def _explain(self) -> Optional[dict]:
+        """Per side, the per-entity tensors build_cache(explain=True) keeps (views of the rows in use), or None."""
+        if any(s is None or s.kept is None for s in self._sides.values()):
+            return None
+        return {name: {k: s.view(k) for k in s.kept} for name, s in self._sides.items()}
 
     @torch.no_grad()
     def score_pairs(self, *inputs) -> torch.Tensor:
@@ -91,9 +174,6 @@ class PairScorer:
         either way."""
         m = self.model
         m.eval()
-        self._factors = None
-        self._unit_items = None
-        self._explain = None
         # per side: (documents, masks, the model's per-review input: NARRE's review ids, SimpleSiamese's review masks)
         sides = {"user": (user_docs, user_masks, None), "item": (item_docs, item_masks, None)}
         if isinstance(m, SimpleSiamese):
@@ -104,7 +184,6 @@ class PairScorer:
                     raise ValueError(f"SimpleSiamese takes {name}_docs [n, R, T] with word masks [n, R, T] and review masks "
                                      f"[n, R], got {tuple(docs.shape)} / {None if wm is None else tuple(wm.shape)} / "
                                      f"{None if rm is None else tuple(rm.shape)}")
-            encode = functools.partial(self._encode_siamese, att64=self._siamese_att64() if explain else None)
         elif isinstance(m, DualAtt):
             if user_masks is not None or item_masks is not None:
                 raise ValueError("DualAtt takes no masks")
@@ -112,7 +191,6 @@ class PairScorer:
                 if docs.shape[-1] != m.doc_len:
                     raise ValueError(f"DualAtt was built for doc_len={m.doc_len}, got {docs.shape[-1]} "
                                      "(the global attention kernel spans the whole document)")
-            encode = self._encode_datt
         elif explain and m.ngram.arch != "CNN":
             raise NotImplementedError("PairScorer.explain covers the CNN encoder; arch='HierPooling' pools averages, "
                                       "which have no per-window tap contributions")
@@ -124,22 +202,154 @@ class PairScorer:
                 if docs.shape[1:] != (m.doc_num, m.doc_len) or rev_ids.shape != docs.shape[:2]:
                     raise ValueError(f"NARRE was built for [*, {m.doc_num}, {m.doc_len}] reviews with [*, {m.doc_num}] review "
                                      f"ids, got {tuple(docs.shape)} / {tuple(rev_ids.shape)}")
-            encode = self._encode_narre
-        else:
-            encode = self._encode_deepconn
+        encode = self._encoder(explain)
         feats, kept = {}, {}
         for name, (docs, masks, rev) in sides.items():
-            step = max(1, chunk // docs.shape[1]) if docs.dim() == 3 else chunk
-            parts = [encode(name, explain, *(None if t is None else t[lo:lo + step] for t in (docs, masks, rev)))
-                     for lo in range(0, docs.shape[0], step)]
-            feats[name] = torch.cat([f for f, _ in parts])
-            if explain:
-                kept[name] = {"docs": docs, "masks": masks, **{k: torch.cat([x[k] for _, x in parts]) for k in parts[0][1]}}
-        self.user_feat, self.item_feat = feats["user"], feats["item"]
+            feats[name], kept[name] = self._encode_rows(encode, name, explain, docs, masks, rev, chunk)
+        if explain and isinstance(m, SimpleSiamese) and not ops.head_supported(feats["user"].shape[1], m.fm.h.shape[0]):
+            for name in SIDES:
+                kept[name]["lat"] = self._latent64(name, feats[name]).float()
+        for name in SIDES:
+            self._sides[name] = _Side(feats[name], kept[name], sides[name][0].shape[1:])
+        self._factors = self._unit_items = None
+
+    def _encoder(self, explain: bool):
+        """The model's chunk encoder (below)."""
+        m = self.model
+        if isinstance(m, SimpleSiamese):
+            return functools.partial(self._encode_siamese, att64=self._siamese_att64() if explain else None)
+        if isinstance(m, DualAtt):
+            return self._encode_datt
+        return self._encode_narre if isinstance(m, NARRE) else self._encode_deepconn
+
+    @staticmethod
+    def _encode_rows(encode, name, explain, docs, masks, rev, chunk):
+        """One side's entities through `encode` in chunks of `chunk` documents (review models: chunk // R entities) →
+        (cached features, None or with explain the per-entity explain tensors with the documents and masks)."""
+        step = max(1, chunk // docs.shape[1]) if docs.dim() == 3 else chunk
+        parts = [encode(name, explain, *(None if t is None else t[lo:lo + step] for t in (docs, masks, rev)))
+                 for lo in range(0, docs.shape[0], step)]
+        feat = torch.cat([f for f, _ in parts])
+        if not explain:
+            return feat, None
+        return feat, {"docs": docs, "masks": masks, **{k: torch.cat([x[k] for _, x in parts]) for k in parts[0][1]}}
+
+    @torch.no_grad()
+    def add(self, side: str, docs: torch.Tensor, masks: Optional[torch.Tensor] = None, *,
+            rev_ids: Optional[torch.Tensor] = None, rev_masks: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Encode new entities on `side` ("user" / "item") from their documents and append them to the cache; returns their
+        cache rows (int64, from the current row count up), which every serving method takes as ids from then on.
+        docs, masks, rev_ids / rev_masks: what build_cache takes for that side and model, for the new entities only.  A new
+        entity has no row in the model's ID tables: it is served under the side's padding id (DeepCoNN / NARRE:
+        fm.padding_idx / fm.item_padding_idx, SimpleSiamese 0; D-ATT has no ids), i.e. exactly as the model's eval forward
+        scores the same documents under that id.  NARRE's rev_ids are MODEL ids of the counterparts, as K3 gathers them from
+        ebd_vals: a review by a counterpart the model has no id for is given as the padding id.  With an explain cache the
+        new rows' explain tensors are appended too.  Nothing is written when a check fails."""
+        s = self._check_rows(side, None, docs, masks, rev_ids, rev_masks)
+        n = docs.shape[0]
+        if not n:
+            return torch.empty(0, dtype=torch.int64, device=s.bufs["cached"].device)
+        pad = 0 if isinstance(self.model, (DualAtt, SimpleSiamese)) else (
+            self.model.fm.padding_idx if side == "user" else self.model.fm.item_padding_idx)
+        mids = torch.full((n,), pad, dtype=torch.int64, device=s.bufs["cached"].device)
+        new = self._encode_new(side, s, docs, masks, rev_ids, rev_masks, mids)
+        new["model_ids"] = mids
+        first = s.n
+        s.write(None, new)
+        self._trim(side)
+        return torch.arange(first, s.n, device=mids.device)
+
+    @torch.no_grad()
+    def update(self, side: str, ids: torch.Tensor, docs: torch.Tensor, masks: Optional[torch.Tensor] = None, *,
+               rev_ids: Optional[torch.Tensor] = None, rev_masks: Optional[torch.Tensor] = None) -> None:
+        """Re-encode the cached entities `ids` (distinct cache rows) on `side` from new documents, in place: e.g. after a
+        user posted a review, or to refresh an entity cached with stale text.  Their model ids are kept.  Inputs as for
+        `add`, one entity per id.  Only these rows are encoded, and factors() / recommend_diverse's item vectors then
+        re-derive only these rows.  The caller's tensors that build_cache(explain=True) kept are copied, never written."""
+        s = self._check_rows(side, ids, docs, masks, rev_ids, rev_masks)
+        ids = ids.to(device=s.bufs["cached"].device, dtype=torch.int64).reshape(-1)
+        if not ids.numel():
+            return
+        s.write(ids, self._encode_new(side, s, docs, masks, rev_ids, rev_masks, s.view("model_ids").index_select(0, ids)))
+        self._trim(side)
+
+    def _check_rows(self, side, ids, docs, masks, rev_ids, rev_masks) -> _Side:
+        """add / update's checks of the caller's input (ValueError before anything is launched) → the side."""
+        m = self.model
+        if side not in SIDES:
+            raise ValueError(f"side must be 'user' or 'item', got {side!r}")
+        s = self._sides[side]
+        if s is None or s.shape is None:
+            raise ValueError("PairScorer.build_cache(...) first: add / update extend a cache built from documents")
+        dev = s.bufs["cached"].device
+        if (not isinstance(docs, torch.Tensor) or docs.device != dev or docs.dim() != len(s.shape) + 1
+                or tuple(docs.shape[1:]) != s.shape or docs.is_floating_point()):
+            raise ValueError(f"{side} documents must be a [n, {', '.join(map(str, s.shape))}] tensor on {dev} (the cached "
+                             f"side's shape), got {tuple(docs.shape) if isinstance(docs, torch.Tensor) else type(docs).__name__}")
+        n = docs.shape[0]
+        if masks is not None and (isinstance(m, DualAtt) or not isinstance(masks, torch.Tensor)
+                                  or masks.device != dev or masks.shape != docs.shape):
+            raise ValueError(f"masks must be None or of the documents' shape {tuple(docs.shape)} on {dev}"
+                             + (" (DualAtt takes no masks)" if isinstance(m, DualAtt) else ""))
+        for name, t, ok in (("rev_ids", rev_ids, isinstance(m, NARRE)), ("rev_masks", rev_masks, isinstance(m, SimpleSiamese))):
+            if t is None and not (ok and name == "rev_ids"):
+                continue
+            if not ok:
+                raise ValueError(f"{type(m).__name__} takes no {name}")
+            if not isinstance(t, torch.Tensor) or t.device != dev or tuple(t.shape) != tuple(docs.shape[:2]):
+                raise ValueError(f"{name} must be a [{n}, {s.shape[0]}] tensor on {dev}, got "
+                                 f"{tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__}")
+        if isinstance(m, NARRE) and rev_ids.numel():
+            n_other = (m.user_att if side == "user" else m.item_att).ebd_vals.weight.shape[0]
+            lo, hi = torch.stack([rev_ids.min(), rev_ids.max()]).tolist()
+            if lo < 0 or hi >= n_other:
+                raise ValueError(f"rev_ids are model ids of the counterparts and must lie in [0, {n_other}) (a counterpart "
+                                 f"the model has no id for is given as the padding id), got [{lo}, {hi}]")
+        if not isinstance(m, DualAtt):
+            n_ids = self._last_feats()[side == "item"].ebd.weight.shape[0]
+            if s.n_built > n_ids:
+                raise ValueError(f"the {side} cache was built with {s.n_built} rows, more than the model's {n_ids} ids")
+        if ids is not None:
+            if not isinstance(ids, torch.Tensor) or ids.dim() != 1 or ids.numel() != n or ids.is_floating_point():
+                raise ValueError(f"ids must be a 1-D integer tensor with one id per document ({n}), got "
+                                 f"{tuple(ids.shape) if isinstance(ids, torch.Tensor) else type(ids).__name__}")
+            if n:
+                lo, hi = torch.stack([ids.min(), ids.max()]).tolist()
+                if lo < 0 or hi >= s.n:
+                    raise ValueError(f"ids must lie in [0, {s.n}) (the cached {side} rows), got [{lo}, {hi}]")
+                if torch.unique(ids).numel() != n:
+                    raise ValueError("ids must be distinct")
+        return s
+
+    def _encode_new(self, side, s, docs, masks, rev_ids, rev_masks, mids) -> dict:
+        """The chunk encoder on new documents of entities with model ids `mids` → {buffer key: new rows} for _Side.write."""
+        m = self.model
+        m.eval()
+        explain = s.kept is not None
+        rev = rev_ids if isinstance(m, NARRE) else rev_masks
+        feat, kept = self._encode_rows(self._encoder(explain), side, explain, docs, masks, rev, _CHUNK)
+        new = {"cached": feat}
         if explain:
-            if isinstance(m, SimpleSiamese) and not self._siamese_fused_g():
-                kept["user"]["lat"], kept["item"]["lat"] = (t.float() for t in self._latents64())
-            self._explain = kept
+            if kept["masks"] is None and s.bufs["masks"] is not None:
+                kept["masks"] = docs != 0                               # the default mask, as the encoder took it
+            elif kept["masks"] is not None and s.bufs["masks"] is None:
+                s.bufs["masks"] = s.view("docs") != 0                   # the cached rows' default masks, materialised
+                s.per["masks"], s.caller_owned = s.per["docs"], s.caller_owned - {"masks"}
+            if kept["masks"] is None:
+                del kept["masks"]
+            if "lat" in s.kept:
+                kept["lat"] = self._latent64(side, feat, mids).float()
+            new.update(kept)
+        return new
+
+    def _trim(self, name):
+        """Drop the change-log entries that every derived cache has taken in."""
+        s = self._sides[name]
+        gens = [] if self._factors is None else [self._factors["gen"][name]]
+        if name == "item" and self._unit_items is not None and self._unit_items["key"] is None:
+            gens.append(self._unit_items["gen"])
+        lo = min(gens, default=s.gen)
+        s.log = [(g, r) for g, r in s.log if g > lo]
 
     # build_cache's chunk encoders, one per model: (side, explain, documents, masks, per-review input) of a chunk of entities
     # → (the entities' cached features, None or with explain a dict of their per-entity explain tensors)
@@ -236,9 +446,19 @@ class PairScorer:
             return u_text.new_empty(0)
         if isinstance(m, DualAtt):
             return torch.sum(torch.mul(u_text, i_text), 1).view(-1)
+        u_ids, i_ids = self._model_ids("user", u_ids), self._model_ids("item", i_ids)
         if isinstance(m, SimpleSiamese):
             return m.head(u_text, i_text, u_ids, i_ids).view(-1)
         return fused_head(m.user_feat, m.item_feat, m.fm, u_text, i_text, u_ids, i_ids, False, None).view(-1)
+
+    def _model_ids(self, name: str, rows: torch.Tensor) -> torch.Tensor:
+        """The model ids of cache rows `rows` (the row -> model-id map); a row outside the cache passes unchanged (K1 reads
+        it as a zero row, K4 as an id outside its tables, as without the map)."""
+        s = self._sides[name]
+        if s.n == s.n_built:                     # rows build_cache wrote map to themselves
+            return rows
+        inside = (rows >= 0) & (rows < s.n)
+        return torch.where(inside, s.view("model_ids").index_select(0, rows.clamp(0, s.n - 1)), rows)
 
     def _last_feats(self):
         m = self.model
@@ -249,40 +469,68 @@ class PairScorer:
         m = self.model
         return [] if isinstance(m, DualAtt) else head_params(*self._last_feats(), m.fm)[0]
 
-    def _latents64(self) -> Tuple[torch.Tensor, torch.Tensor]:
-        """LastFeat (models/deepconn/layers.py:163) of every cached entity in float64, [U, K] / [I, K]: exact fp32 latents
-        whatever the TF32 setting."""
-        return tuple(feat.double() @ lf.W.detach().double() + lf.b.detach().double()
-                     + lf.ebd.weight.detach().double()[:feat.shape[0]]
-                     for feat, lf in zip((self.user_feat, self.item_feat), self._last_feats()))
+    def _latent64(self, name: str, feat: torch.Tensor, mids: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """LastFeat (models/deepconn/layers.py:163) in float64 of `name`-side features feat [n, H] of entities with model ids
+        `mids` (None: rows 0..n-1) → [n, K]: exact fp32 latents whatever the TF32 setting."""
+        lf = self._last_feats()[name == "item"]
+        ebd = lf.ebd.weight.detach().double()
+        return (feat.double() @ lf.W.detach().double() + lf.b.detach().double()
+                + (ebd[:feat.shape[0]] if mids is None else ebd.index_select(0, mids)))
 
     def factors(self) -> Tuple[torch.Tensor, Optional[torch.Tensor], torch.Tensor, Optional[torch.Tensor]]:
         """(A [U, D], row_bias [U] or None, B [I, D], col_bias [I] or None) with score(u, i) = A[u] . B[i] + biases for the
-        cached entities under the CURRENT head parameters.  Re-derived when a parameter changed (optimizer steps bump
-        its version counter) or the cache was rebuilt."""
+        cached entities under the CURRENT head parameters, each row from its entity's model id (the row -> model-id map).
+        Re-derived when a parameter changed (optimizer steps bump its version counter) or the cache was rebuilt; after
+        add / update only the added and updated rows are derived (the same float64 expression, row by row)."""
         if self.user_feat is None:
             raise RuntimeError("PairScorer.build_cache(...) first")
         m = self.model
-        params = self._head_params()
-        key = (tuple((p._version, p.data_ptr()) for p in params if p is not None)
-               + ((self.user_feat.data_ptr(), self.item_feat.data_ptr()),))
-        if self._factors is None or self._factors[0] != key:
-            if isinstance(m, DualAtt):
-                f = (self.user_feat, None, self.item_feat, None)
+        if isinstance(m, DualAtt):
+            return self.user_feat, None, self.item_feat, None
+        key = tuple((p._version, p.data_ptr()) for p in self._head_params() if p is not None)
+        f = self._factors
+        full = f is None or f["key"] != key
+        rows = dict.fromkeys(SIDES) if full else {name: self._sides[name].changed(f["gen"][name]) for name in SIDES}
+        if full or any(r is not None for r in rows.values()):
+            with torch.no_grad():
+                lat, bias = {}, {}
+                fm = m.fm
+                for name, tab in zip(SIDES, (getattr(fm, "user_bias", None), getattr(fm, "item_bias", None))):
+                    s, r = self._sides[name], rows[name]
+                    mids = None if s.n == s.n_built else s.view("model_ids")
+                    feat = s.view("cached")
+                    if not full:
+                        r = r if r is not None else torch.empty(0, dtype=torch.int64, device=feat.device)
+                        feat, mids = feat.index_select(0, r), (r if mids is None else mids.index_select(0, r))
+                    lat[name] = self._latent64(name, feat, mids)
+                    if isinstance(fm, FM):                   # FMWithoutUIBias: row_bias = g_bias, no column bias
+                        w = tab.weight.detach().double()
+                        bias[name] = w[:feat.shape[0]] if mids is None else w.index_select(0, mids)
+                    else:
+                        bias[name] = lat[name].new_zeros(feat.shape[0], 1)
+                new = [t.float().contiguous() for t in fm_factors(lat["user"], lat["item"], fm.h.detach().double(), bias["user"],
+                                                                  bias["item"], fm.g_bias.detach().double())]
+                if not isinstance(fm, FM):
+                    new[3] = None
+            if full:
+                f = {"key": key, "user": new[:2], "item": new[2:]}
             else:
-                with torch.no_grad():
-                    u_lat, i_lat = self._latents64()
-                    n_u, n_i = u_lat.shape[0], i_lat.shape[0]
-                    fm = m.fm
-                    bias = isinstance(fm, FM)            # FMWithoutUIBias: row_bias = g_bias, no column bias
-                    ub = fm.user_bias.weight.detach().double()[:n_u] if bias else u_lat.new_zeros(n_u, 1)
-                    ib = fm.item_bias.weight.detach().double()[:n_i] if bias else i_lat.new_zeros(n_i, 1)
-                    f = tuple(t.float().contiguous()
-                              for t in fm_factors(u_lat, i_lat, fm.h.detach().double(), ub, ib, fm.g_bias.detach().double()))
-                    if not bias:
-                        f = f[:3] + (None,)
-            self._factors = (key, f)
-        return self._factors[1]
+                for name, vals in (("user", new[:2]), ("item", new[2:])):
+                    if rows[name] is None:
+                        continue
+                    n = self._sides[name].n
+                    for j, v in enumerate(vals):
+                        if v is not None:
+                            f[name][j] = _reserve(f[name][j], f["n"][name], n)
+                            f[name][j].index_copy_(0, rows[name], v)
+            f["n"] = {name: self._sides[name].n for name in SIDES}
+            f["gen"] = {name: self._sides[name].gen for name in SIDES}
+            self._factors = f
+            for name in SIDES:
+                self._trim(name)
+        f = self._factors
+        n_u, n_i = f["n"]["user"], f["n"]["item"]
+        return tuple(None if t is None else t[:n] for t, n in zip(f["user"] + f["item"], (n_u, n_u, n_i, n_i)))
 
     @torch.no_grad()
     def recommend(self, u_ids: torch.Tensor, k: int, exclude: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
@@ -322,20 +570,34 @@ class PairScorer:
         return ops.mmr_select(pool_scores, pool_items, vecs, k, lam)
 
     def _unit_item_vecs(self, item_vecs: Optional[torch.Tensor]) -> torch.Tensor:
-        """ops.unit_rows of item_vecs (default: the cached item features), kept until the source changes: keyed by its data
-        pointer, layout and version counter, and holding a reference to it so that the pointer cannot be reused."""
+        """ops.unit_rows of item_vecs (default: the cached item features), kept until the source changes.  The default
+        source follows the item side's change log, so add / update normalise only their rows; a caller's tensor is keyed
+        by its data pointer, layout and version counter, and referenced so that the pointer cannot be reused."""
         if self.item_feat is None:
             raise RuntimeError("PairScorer.build_cache(...) first")
-        src = self.item_feat if item_vecs is None else item_vecs
+        if item_vecs is None:
+            s, u = self._sides["item"], self._unit_items
+            if u is None or u["key"] is not None:
+                u = {"key": None, "vecs": ops.unit_rows(self.item_feat).contiguous()}
+            else:
+                rows = s.changed(u["gen"])
+                if rows is not None:
+                    u["vecs"] = _reserve(u["vecs"], u["n"], s.n)
+                    u["vecs"].index_copy_(0, rows, ops.unit_rows(self.item_feat.index_select(0, rows)))
+            u["n"], u["gen"] = s.n, s.gen
+            self._unit_items = u
+            self._trim("item")
+            return u["vecs"][:u["n"]]
+        src = item_vecs
         if not isinstance(src, torch.Tensor) or src.dim() != 2 or src.shape[0] != self.item_feat.shape[0]:
             raise ValueError(f"item_vecs must be [{self.item_feat.shape[0]}, D] (one row per cached item), got "
                              f"{tuple(src.shape) if isinstance(src, torch.Tensor) else type(src).__name__}")
         if src.device != self.item_feat.device:
             raise ValueError(f"item_vecs is on {src.device}, the cache on {self.item_feat.device}")
         key = (src.data_ptr(), tuple(src.shape), src.stride(), src.dtype, src._version)
-        if self._unit_items is None or self._unit_items[0] != key:
-            self._unit_items = (key, src, ops.unit_rows(src).contiguous())
-        return self._unit_items[2]
+        if self._unit_items is None or self._unit_items["key"] != key:
+            self._unit_items = {"key": key, "src": src, "vecs": ops.unit_rows(src).contiguous()}
+        return self._unit_items["vecs"]
 
     def _user_rows(self, u_ids: torch.Tensor, exclude_padding: bool):
         """(A rows, row_bias rows, B, col_bias, padding item or None) for users u_ids under the current head parameters;
@@ -525,7 +787,8 @@ class PairScorer:
 
         def grads(u, i):
             u_text, i_text = ops.gather_rows(self.user_feat, u), ops.gather_rows(self.item_feat, i)
-            return ops.head_text_grads(u_text, i_text, u, i, head, pads, scratch)
+            return ops.head_text_grads(u_text, i_text, self._model_ids("user", u), self._model_ids("item", i), head, pads,
+                                       scratch)
         return grads
 
     def _narre_grads(self, head_grads):
