@@ -125,11 +125,6 @@ int rbr_conv_act_maxpool_fwd(int precision, int activation, const void* table, c
                              const void* packed, const float* bias, int64_t filters, int64_t ksize,
                              int64_t pad, float* feat, int32_t* argmax, float* pool_raw, int64_t feat_ld,
                              void* ws, int64_t ws_bytes, int flags, void* stream);
-/* Timing experiments only.  With RBR_TC2_DEBUG=4 in the environment the CTA-pair conv kernel accumulates per-CTA cycle
- * counters; this copies out[cta][12] = {MMA warp total, its wait for operands, its wait for a free accumulator, producer warp 0
- * total, its wait for a free ring slot, epilogue warp 0 total, its wait for a finished accumulator, tiles, epilogue warp 0's
- * TMEM loads + column max, its per-document finalisation, producer warp 0's per-tile prologue, 0} of the last launch (synchronises the device). */
-int rbr_debug_conv_tc2_prof(int64_t* out, int n_ctas);
 
 /* ---- K2b: arg-max-sparse backward of K2 ------------------------------------------------------------
  * Replaces aten::convolution_backward + max_pool1d backward + relu backward + masked_fill backward +
@@ -167,8 +162,6 @@ int rbr_conv_act_maxpool_bwd(int precision, int activation, const void* table, c
  *   rbr_conv_bwd_cmat_scatter(side, c)    once per document side — the sides may run on different streams
  *   rbr_conv_bwd_cmat_finish(1, c)        splits the block into the bf16 hi|lo operand while it is still in L2
  * then rbr_conv_bwd_cmat_finish(2 / 4, -1) for the two gradients.  chunk = -1 means "every block" in all three calls.
- * Bit 2 computes table rows [row_lo, row_hi) (cut on multiples of 128; 0, 0 = all): data-parallel training produces the
- * gradient in row slices and starts the all-reduce of each slice while the next one is still being computed.
  * `ws`: rbr_conv_bwd_cmat_workspace_bytes() bytes that the CALLER ZERO-FILLS ONCE (the weight scratch is left zeroed again
  * by bit 4).
  * `what`: 1 = close the accumulation of block `chunk` (split C; required once per block after its scatters, before 2 / 4),
@@ -187,7 +180,7 @@ int rbr_conv_bwd_cmat_scatter(const void* ids, const uint8_t* mask, int64_t n_do
                               int64_t filters, int64_t ksize, int64_t pad, int activation, const float* feat,
                               const int32_t* argmax, const float* feat_grad, int64_t feat_ld, float* bias_grad, int chunk,
                               void* ws, int64_t ws_bytes, int flags, void* stream);
-int rbr_conv_bwd_cmat_finish(int what, int chunk, int64_t row_lo, int64_t row_hi, const void* shadow_bf16, const void* packed,
+int rbr_conv_bwd_cmat_finish(int what, int chunk, const void* shadow_bf16, const void* packed,
                              int64_t vocab, int64_t emb, int64_t filters, int64_t ksize, int64_t padding_idx, float* table_grad,
                              float* weight_grad, void* ws, int64_t ws_bytes, void* stream);
 

@@ -617,10 +617,6 @@ static bool attn_tc_plan(int64_t B, int R, int H, int A, bool bwd, AttnArgs* a, 
     a->Hp8 = (H + 7) & ~7;
     // samples per tile: as many as keep the tile within 80..128 review rows and 8 warps
     int ts = 80 / R;
-    static const char* ts_env = getenv("RBR_ATTN_TS");                // timing experiments: samples per tile
-    static const char* tsb_env = getenv("RBR_ATTN_TS_BWD");
-    if (!bwd && ts_env && atoi(ts_env) > 0) ts = atoi(ts_env);
-    if (bwd && tsb_env && atoi(tsb_env) > 0) ts = atoi(tsb_env);
     if (ts < 1) ts = 1;
     while ((ts * R + 15) / 16 > AT_MAXW) --ts;
     if (ts < 1) return false;
@@ -637,7 +633,7 @@ static bool attn_tc_plan(int64_t B, int R, int H, int A, bool bwd, AttnArgs* a, 
     *smem_bytes = (size_t)attn_tc_smem(*a, bwd).total * 4;
     // forward: a smaller tile that lets TWO CTAs share an SM hides one CTA's tile load behind the other's math
     // (R = 10, H = 150: 6 samples / 107 KB instead of 8 / 122 KB — 89.9 -> 74.4 us; the backward does not fit twice either way)
-    if (!bwd && !(ts_env && atoi(ts_env) > 0) && *smem_bytes > 112 * 1024) {
+    if (!bwd && *smem_bytes > 112 * 1024) {
         for (int t2 = ts - 1; t2 >= 1 && t2 * R >= 48; --t2) {
             AttnArgs b = *a;
             b.TS = t2; b.rows = t2 * R; b.NW = (b.rows + 15) / 16;

@@ -62,8 +62,7 @@ static CmatLayout cmat_layout(int64_t vocab, int64_t emb, int64_t filters, int64
     l.off_chl = off; off += round_up(vocab * 2 * l.HJp * 2, 1024);
     l.off_dw = off; off += round_up(l.HJ * l.epad4 * 4, 1024);
     l.total = off;
-    static const char* ch_env = getenv("RBR_CMAT_CHUNKS");                      // timing experiments: force the block count
-    int64_t want = ch_env ? atoi(ch_env) : (vocab * l.HJp * 4 + (80ll << 20) - 1) / (80ll << 20);
+    int64_t want = (vocab * l.HJp * 4 + (80ll << 20) - 1) / (80ll << 20);
     want = std::max<int64_t>(1, std::min<int64_t>(want, 16));
     l.hc = round_up((filters + want - 1) / want, 4);                            // block widths stay float4-aligned
     l.n_chunks = (filters + l.hc - 1) / l.hc;
@@ -267,7 +266,6 @@ struct TableGemmArgs {
     int64_t padding_idx;
     float* table_grad;         // [vocab][E]
     int overwrite;             // 1: table_grad = tile (every row and column of the gradient is written, padding row = 0); 0: +=
-    int tile0;                 // first 128-token tile of this launch (the gradient can be produced in row slices)
 };
 
 __global__ void __launch_bounds__(CM_THREADS, 2)
@@ -281,7 +279,7 @@ cmat_table_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_con
     const int stage_bytes = 16384 + b_bytes;
     const uint32_t bars = sbase + CM_STAGES_T * stage_bytes;            // full[S], empty[S], acc_full
     volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem + CM_STAGES_T * stage_bytes + 8 * (2 * CM_STAGES_T + 1));
-    const int m0 = ((int)blockIdx.x + a.tile0) * 128, n0 = blockIdx.y * a.NT;
+    const int m0 = (int)blockIdx.x * 128, n0 = blockIdx.y * a.NT;
 
     if (threadIdx.x == 0) {
         for (int i = 0; i < CM_STAGES_T; ++i) { mbar_init(bars + 8 * i, 1); mbar_init(bars + 8 * (CM_STAGES_T + i), 1); }
@@ -570,11 +568,9 @@ static int cmat_scatter_block(const CmatLayout& l, const CmatChunk& k, const voi
         int64_t g = filters, r = 256;
         while (r) { const int64_t t = g % r; g = r; r = t; }            // g = gcd(filters, 256)
         const int64_t m = filters / g;                                  // grid must be a multiple of m
-        static const char* fast_env = getenv("RBR_SCATTER_FAST");
-        const bool fast_on = !(fast_env && atoi(fast_env) == 0);
         const bool small = n_docs * std::max(feat_ld, doc_len) < (1ll << 31) - 1 && vocab < (1ll << 31) - 1 && vocab * k.width < (1ll << 32) &&
                            filters * ksize < (1 << 20);
-        if (fast_on && small && m <= 148 * 8 && (ksize == 1 || ksize == 3 || ksize == 5)) {
+        if (small && m <= 148 * 8 && (ksize == 1 || ksize == 3 || ksize == 5)) {
             constexpr int IT = 2;
             int64_t blocks = (total + 256 * IT - 1) / (256 * IT);
             if (blocks > 148 * 8) blocks = 148 * 8;
@@ -635,7 +631,7 @@ extern "C" int rbr_conv_bwd_cmat_scatter(const void* ids_raw, const uint8_t* mas
     return RBR_OK;
 }
 
-extern "C" int rbr_conv_bwd_cmat_finish(int what, int chunk, int64_t row_lo, int64_t row_hi, const void* shadow_bf16, const void* packed,
+extern "C" int rbr_conv_bwd_cmat_finish(int what, int chunk, const void* shadow_bf16, const void* packed,
                                         int64_t vocab, int64_t emb, int64_t filters, int64_t ksize, int64_t padding_idx, float* table_grad,
                                         float* weight_grad, void* ws, int64_t ws_bytes, void* stream) {
     RBR_REQUIRE(ws && packed, RBR_EINVAL, "conv_bwd_cmat_finish: null pointer");
@@ -674,10 +670,6 @@ extern "C" int rbr_conv_bwd_cmat_finish(int what, int chunk, int64_t row_lo, int
         a.vocab = vocab; a.E = (int)emb; a.NT = (int)pl.NT; a.nkb = (int)(2 * l.HJp / 64); a.padding_idx = padding_idx;
         a.table_grad = table_grad;
         a.overwrite = (what & 8) ? 1 : 0;
-        if (row_lo == 0 && row_hi == 0) row_hi = vocab;
-        RBR_REQUIRE(row_lo >= 0 && row_lo < row_hi && row_hi <= vocab && row_lo % 128 == 0 && (row_hi % 128 == 0 || row_hi == vocab), RBR_EINVAL,
-                    "conv_bwd_cmat_finish: the table row range must be cut on multiples of 128 rows");
-        a.tile0 = (int)(row_lo / 128);
         const int smem = cmat_smem(emb).table;
         static bool attr = false;
         if (!attr) {
@@ -685,7 +677,7 @@ extern "C" int rbr_conv_bwd_cmat_finish(int what, int chunk, int64_t row_lo, int
             attr = true;
         }
         RBR_REQUIRE(smem <= CM_SMEM_T_MAX, RBR_EUNSUPPORTED, "conv_bwd_cmat_finish: shared memory");
-        dim3 grid((unsigned)((row_hi - row_lo + 127) / 128), (unsigned)pl.n_tiles);
+        dim3 grid((unsigned)((vocab + 127) / 128), (unsigned)pl.n_tiles);
         cmat_table_gemm_kernel<<<grid, CM_THREADS, smem, s>>>(tmA, tmB, a);
         RBR_LAUNCH_CHECK("cmat_table_gemm_kernel");
     }

@@ -17,7 +17,6 @@
 // Pipeline: per CTA four TMA producer warps, 16 epilogue warps; the LEADER CTA's MMA warp issues every tcgen05.mma for the
 // pair.  full[s] lives in the leader (both CTAs' TMA bytes complete on it), empty[s] / acc_full[b] are multicast by
 // tcgen05.commit to both CTAs, acc_empty[b] collects one arrive per epilogue warp of both CTAs.
-#include <stdlib.h>
 #include <cuda.h>   // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint, no -lcuda)
 
 #include "rbr_common.cuh"
@@ -30,12 +29,13 @@ constexpr int T2_M = 128;                  // positions per CTA tile (UMMA M = 2
 // the 16-column chunks.  The max-reduction is a chain of fixed-latency warp ops: 16 warps hide it when there is a lot of it
 // per tile relative to the MMA/gather work (many filter chunks, short documents = per-tile finalisation, or a narrow
 // embedding = few K blocks per tile), 8 leave more issue slots to the MMA warp.
-// Warp roles: [0, EW) epilogue, [EW, EW+PW) TMA producers (TMA issue is serialised per warp), EW+PW = TMEM owner + MMA issuer,
-// EW+PW+1 = index warp (resolves the table row of every staged tile row ahead of the producers).
-// Producer warps PW (template parameter): issuing one gather4 costs a warp ~100 cycles (the TMA unit accepts the instruction's
-// uniform-register operands serially per warp), so the 32 + halo gather4s of a K block are spread over PW warps; each
-// stages 128 / PW tile rows.
-constexpr int t2_threads(int ew, int pw) { return (ew + pw + 2) * 32; }
+// Warp roles: [0, EW) epilogue, [EW, EW+4) TMA producers (TMA issue is serialised per warp), EW+4 = TMEM owner + MMA issuer,
+// EW+5 = index warp (resolves the table row of every staged tile row ahead of the producers).
+// Producer warps: issuing one gather4 costs a warp ~100 cycles (the TMA unit accepts the instruction's uniform-register
+// operands serially per warp), so the 32 + halo gather4s of a K block are spread over 4 warps; each stages 32 tile rows.
+// 8 measured = 4: the floor is the TMA unit's row rate, not per-warp issue.
+constexpr int T2_PROD_WARPS = 4;
+constexpr int t2_threads(int ew) { return (ew + T2_PROD_WARPS + 2) * 32; }
 constexpr int T2_IDX_BUFS = 3;               // index buffers at most (plan: nib = as many as fit without costing a ring stage, >= 1; the
                                              // producers copy a tile's indices to registers at the top of the tile, so one buffer already
                                              // lets the index warp finish tile g+1 while tile g streams — more only absorb jitter)
@@ -70,7 +70,6 @@ struct Tc2Plan {
     int off_ring, off_w, off_bias, off_keys, off_idx, off_bars, off_slot, smem_bytes;   // offsets from the 1024-aligned base
     int act;
     uint32_t boff[4 * 8];   // B-descriptor offset (16-byte units) of (K-step ks, tap j) inside a K block: [ks * 8 + j]
-    int dbg;          // RBR_TC2_DEBUG bits (timing experiments only; results are wrong): 1 = skip the MMAs, 2 = skip the max-reduction
 };
 
 static inline int t2_stage_bytes(int K) {
@@ -126,20 +125,14 @@ struct Tc2Args {
     Tc2Plan p;
 };
 
-// RBR_TC2_DEBUG bit 4: per-CTA cycle counters (timing experiments): [0] MMA warp total, [1] its wait on the ring (full), [2] its wait on
-// the accumulators (acc_empty), [3] producer warp 0 total, [4] its wait on the ring (empty), [5] epilogue warp 0 total, [6] its wait
-// on the accumulators (acc_full), [7] tiles, [8] epilogue warp 0: TMEM loads + column max, [9] its document finalisation (named barrier
-// + stores), [10] producer warp 0: per-tile prologue (row indices of the tile: ids, range checks, shuffles) before its first gather4
-__device__ long long g_tc2_prof[1024][12];
-
 // list slot li (unit * D + slot) → document index
 __device__ __forceinline__ int64_t t2_doc_of(const int32_t* live, int64_t li) { return live ? (int64_t)__ldg(live + 1 + li) : li; }
 
-template <int KT, int EW, int PW>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(t2_threads(EW, PW), 1)
+template <int KT, int EW>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(t2_threads(EW), 1)
 conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
-    constexpr int T2_PROD_WARPS = PW, ROWS_PW = T2_M / PW, G4_PW = ROWS_PW / 4;
-    constexpr int T2_EPI_WARPS = EW, T2_EPI_SHARES = EW / 4, T2_EPI_THREADS = EW * 32;
+    constexpr int ROWS_PW = T2_M / T2_PROD_WARPS, G4_PW = ROWS_PW / 4;
+    constexpr int T2_EPI_WARPS = EW, T2_EPI_SHARES = EW / 4;
     constexpr int MAXC = 1;   // TMEM chunks held in registers at once (2 or 4 with an earlier accumulator release measured slower: 0.34 / 0.38 vs 0.31 ms)
     constexpr int T2_PROD_WARP0 = EW, T2_MMA_WARP = EW + T2_PROD_WARPS, T2_IDX_WARP = T2_MMA_WARP + 1;
     extern __shared__ uint8_t smem_raw[];
@@ -225,26 +218,20 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
                 uint32_t ph = 0;
                 uint32_t full_bar = bar_full, empty_bar = bar_empty;
                 uint64_t ad = a_desc0;
-                const bool prof = (p.dbg & 4) != 0;
-                long long pt0 = prof ? clock64() : 0, pw_full = 0, pw_acce = 0, pt;
                 for (int64_t g = 0; g < pair_tiles; ++g) {
                     const int buf = (int)(g & ((1 << p.nacc_log2) - 1));
-                    if (prof) pt = clock64();
                     mbar_wait(bar_acce + 8 * buf, (uint32_t)(((g >> p.nacc_log2) & 1) ^ 1));        // both CTAs' epilogues drained this buffer
-                    if (prof) pw_acce += clock64() - pt;
                     tc_fence_after();
                     const uint32_t d_tmem = tmem_base + (uint32_t)(buf * p.acc_stride);
                     uint64_t bd = b_desc0;
                     int ks_left = p.ksteps;
                     for (int kb = 0; kb < p.nkb; ++kb) {
-                        if (prof) pt = clock64();
                         mbar_wait(full_bar, ph);                                           // both CTAs' TMA bytes have landed
-                        if (prof) pw_full += clock64() - pt;
                         tc_fence_after();
                         if (leader_lane) {
 #pragma unroll
                             for (int ks = 0; ks < 4; ++ks) {
-                                if (ks < ks_left && !(p.dbg & 1)) {
+                                if (ks < ks_left) {
 #pragma unroll
                                     for (int j = 0; j < KT; ++j)
                                         umma_bf16_2(d_tmem, ad + (uint64_t)(ks * 2 + j * 8), bd + (uint64_t)p.boff[ks * 8 + j], idesc,
@@ -262,10 +249,6 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
                         empty_bar += 8;
                         if (++stage == p.nst) { stage = 0; ph ^= 1; ad = a_desc0; full_bar = bar_full; empty_bar = bar_empty; }
                     }
-                }
-                if (prof && lane == 0 && blockIdx.x < 1024) {
-                    g_tc2_prof[blockIdx.x][0] = clock64() - pt0; g_tc2_prof[blockIdx.x][1] = pw_full; g_tc2_prof[blockIdx.x][2] = pw_acce;
-                    g_tc2_prof[blockIdx.x][7] = pair_tiles;
                 }
             }
         }
@@ -285,11 +268,7 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
         bool w_checked = false;
         const uint32_t dst0 = ring_s + (uint32_t)(pw * G4_PW) * 512u;
         const uint32_t dst_halo = ring_s + 32u * 512u;
-        const bool prof = (p.dbg & 4) != 0 && pw == 0;
-        long long pt0 = prof ? clock64() : 0, pw_empty = 0, pt;
-        long long pw_pro = 0, pt_pro = 0;
         for (int64_t g = 0; g < pair_tiles; ++g) {
-            if (prof) pt_pro = clock64();
             mbar_wait(bar_idxf + 8 * ib, iph);
             int idx[ROWS_PW], hidx[8];
             {
@@ -307,11 +286,8 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_idxe + 8 * ib);          // the buffer may be rewritten (tile g + nib)
             if (++ib == p.nib) { ib = 0; iph ^= 1; }
-            if (prof) pw_pro += clock64() - pt_pro;
             for (int kb = 0; kb < p.nkb; ++kb) {
-                if (prof) pt = clock64();
                 mbar_wait(bar_empty + 8 * stage, ph ^ 1);
-                if (prof) pw_empty += clock64() - pt;
                 const uint32_t fb = bar_full + 8 * stage;
                 if (pw == 0 && lane == 0) {
                     if (rank == 0) {
@@ -335,9 +311,6 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
                 __syncwarp();
                 if (++stage == p.nst) { stage = 0; ph ^= 1; }
             }
-        }
-        if (prof && lane == 0 && blockIdx.x < 1024) {
-            g_tc2_prof[blockIdx.x][3] = clock64() - pt0; g_tc2_prof[blockIdx.x][4] = pw_empty; g_tc2_prof[blockIdx.x][10] = pw_pro;
         }
     } else if (warp == T2_IDX_WARP) {
         // =========================== index warp: table row (or -1) of every staged row, a few tiles ahead of the producers ===========
@@ -498,8 +471,6 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
         stage_a();                          // tile 1
         int ib = 0;
         uint32_t iph = 0;
-        const bool prof = (p.dbg & 4) != 0;
-        long long pt0 = prof ? clock64() : 0, pw_wait = 0, pt;
         for (int64_t g = 0; g < pair_tiles; ++g) {
             int mine[NS];
 #pragma unroll
@@ -518,9 +489,7 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
             stage_b();                      // tile g + 1
             advance();
             stage_a();                      // tile g + 2
-            if (prof) pt = clock64();
             mbar_wait(bar_idxe + 8 * ib, iph ^ 1);                  // every producer warp has read this buffer's previous tile
-            if (prof) pw_wait += clock64() - pt;
             int* dst = idx_s + ib * T2_IDX_ROWS;
 #pragma unroll
             for (int i = 0; i < 4; ++i) dst[row[i]] = mine[i];
@@ -528,7 +497,6 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
             mbar_arrive(bar_idxf + 8 * ib);                         // 32 arrivals (release): the tile's indices are visible
             if (++ib == p.nib) { ib = 0; iph ^= 1; }
         }
-        if (prof && lane == 0 && blockIdx.x < 1024) g_tc2_prof[blockIdx.x][11] = clock64() - pt0 - pw_wait;
         }
     } else {
         // =========================== epilogue (16 warps; warp w reads TMEM lanes 32(w&3)..+31 and reduces 1/4 of the column chunks:
@@ -550,10 +518,7 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
         const int qps = p.mode_b ? p.S / 32 : 4;              // quadrants (warps of a share) per document slot
         const int grp_bar = 1 + share * (4 / qps) + quad / qps, grp_threads = qps * 32, grp_tid = (quad % qps) * 32 + lane;
         int32_t fin_doc = -1;
-        const bool prof = (p.dbg & 4) != 0 && warp == 0;
-        long long pt0 = prof ? clock64() : 0, pw_accf = 0, pw_red = 0, pw_fin = 0, pt;
         for (int64_t g = 0; g < pair_tiles; ++g) {
-            if (prof && g > 0) pw_fin += clock64() - pt;
             if (++tt >= unt) { ++uj; tt = 0; unt = step_tiles(uj); }
             const int64_t unit = ci + uj * ctas_per_pass;
             const int buf = (int)(g & ((1 << p.nacc_log2) - 1));
@@ -573,15 +538,12 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
             float row_gate = 1.f;
             if (a.gate_mode == 1 && valid) row_gate = a.gate[t2_doc_of(a.live, my_li) * p.L + t];
 
-            if (prof) pt = clock64();
             mbar_wait(bar_accf + 8 * buf, (uint32_t)((g >> p.nacc_log2) & 1));
-            if (prof) pw_accf += clock64() - pt;
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(buf * p.acc_stride);
             // Chunks are pulled out of TMEM MAXC at a time; the accumulator is handed back to the MMA warp as soon as the warp's
             // LAST chunk is in registers, i.e. before any reduction when all its chunks fit one group (8-warp mode, <= 4 chunks
             // per warp): the max-reduction then overlaps the MMAs of tile g+2 instead of delaying them.
-            if (prof) pt = clock64();
             for (int chg = chunk_lo; chg < chunk_hi; chg += MAXC) {
                 uint32_t v[MAXC][16];
 #pragma unroll
@@ -601,18 +563,16 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
 #pragma unroll
                         for (int i = 0; i < 16; ++i) v[u][i] = __float_as_uint(__uint_as_float(v[u][i]) * row_gate);
                     }
-                    if (!(p.dbg & 2)) {
-                        uint32_t keep_v = 0, keep_b = 0;
-                        if (__all_sync(0xffffffffu, valid)) tc_colmax<true>(v[u], true, lane, keep_v, keep_b);
-                        else tc_colmax<false>(v[u], valid, lane, keep_v, keep_b);
-                        if (lane < 16 && keep_b) {
-                            const int first = __ffs(keep_b) - 1;          // first (smallest-position) row attaining the max
-                            const int tf = p.mode_b ? (quad * 32 + first - slot * p.S) : (tt * T2_M + quad * 32 + first);
-                            const unsigned long long key =
-                                ((unsigned long long)f2ord(keep_v) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)tf);
-                            unsigned long long* kp = keys_u + quad * p.Nb + c0 + lane;
-                            if (key > *kp) *kp = key;
-                        }
+                    uint32_t keep_v = 0, keep_b = 0;
+                    if (__all_sync(0xffffffffu, valid)) tc_colmax<true>(v[u], true, lane, keep_v, keep_b);
+                    else tc_colmax<false>(v[u], valid, lane, keep_v, keep_b);
+                    if (lane < 16 && keep_b) {
+                        const int first = __ffs(keep_b) - 1;          // first (smallest-position) row attaining the max
+                        const int tf = p.mode_b ? (quad * 32 + first - slot * p.S) : (tt * T2_M + quad * 32 + first);
+                        const unsigned long long key =
+                            ((unsigned long long)f2ord(keep_v) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)tf);
+                        unsigned long long* kp = keys_u + quad * p.Nb + c0 + lane;
+                        if (key > *kp) *kp = key;
                     }
                 }
             }
@@ -621,7 +581,6 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
                 __syncwarp();
                 if (lane == 0) mbar_arrive_cluster(bar_acce + 8 * buf, 0);
             }
-            if (prof) { pw_red += clock64() - pt; pt = clock64(); }
             if (tt == unt - 1) {
                 // (A/B on one box, DeepCoNN shape: the group barrier 4258 clk per tile, a CTA-wide one 4338)
                 if (qps > 1) asm volatile("bar.sync %0, %1;" ::"r"(grp_bar), "r"(grp_threads) : "memory");
@@ -645,10 +604,6 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const Tc2Args a) {
                     }
                 }
             }
-        }
-        if (prof && lane == 0 && blockIdx.x < 1024) {
-            g_tc2_prof[blockIdx.x][5] = clock64() - pt0; g_tc2_prof[blockIdx.x][6] = pw_accf;
-            g_tc2_prof[blockIdx.x][8] = pw_red; g_tc2_prof[blockIdx.x][9] = pw_fin;
         }
     }
     // teardown: neither CTA may free TMEM / exit while the pair's MMAs can still touch its shared or tensor memory
@@ -934,11 +889,11 @@ static EncodeTiledFn tc2_encoder() {
     return fn;
 }
 
-template <int KT, int EW, int PW>
+template <int KT, int EW>
 static int tc2_launch(const CUtensorMap& tm, const Tc2Args& a, cudaStream_t s) {
     static int max_clusters = -1;
-    constexpr int T2_THREADS = t2_threads(EW, PW);
-    auto kern = conv_tc2_kernel<KT, EW, PW>;
+    constexpr int T2_THREADS = t2_threads(EW);
+    auto kern = conv_tc2_kernel<KT, EW>;
     if (max_clusters < 0) {
         RBR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_MAX));
         cudaLaunchConfig_t cfg{};
@@ -974,12 +929,6 @@ int conv_tc2_dispatch(const __nv_bfloat16* shadow, int64_t vocab, int E, IdView 
                       int64_t ws_bytes, cudaStream_t s) {
     Tc2Args a{};
     if (vocab >= (1ll << 31) || n_docs >= (1ll << 31) || !tc2_make_plan(E, H, K, L, pad, act, n_docs, &a.p)) return RBR_EUNSUPPORTED;
-    {
-        static const char* dbg = getenv("RBR_TC2_DEBUG");
-        a.p.dbg = dbg ? atoi(dbg) : 0;
-        static const char* nacc = getenv("RBR_TC2_ACC_BUFS");                    // timing experiments: 2 = two accumulator buffers always
-        if (nacc && atoi(nacc) == 2) a.p.nacc_log2 = 1;
-    }
     if (K != 1 && K != 2 && K != 3 && K != 4 && K != 5 && K != 7) return RBR_EUNSUPPORTED;
     EncodeTiledFn enc = tc2_encoder();
     if (!enc) return RBR_EUNSUPPORTED;
@@ -989,12 +938,9 @@ int conv_tc2_dispatch(const __nv_bfloat16* shadow, int64_t vocab, int E, IdView 
     cuuint64_t gstr[1] = {(cuuint64_t)emb_pad * 2};
     cuuint32_t box[2] = {64, 1};
     cuuint32_t estr[2] = {1, 1};
-    static const char* promo_env = getenv("RBR_TMA_PROMO");           // tuning knob: 0 none, 1 64B, 2 128B, 3 256B (default)
-    const int promo = promo_env ? atoi(promo_env) : 3;
-    const CUtensorMapL2promotion l2p = promo == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : promo == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-                                       : promo == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
     const CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<__nv_bfloat16*>(shadow), gdim, gstr, box, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, l2p, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     RBR_REQUIRE(r == CUDA_SUCCESS, RBR_ECUDA, "conv_fwd[bf16]: cuTensorMapEncodeTiled failed (%d)", (int)r);
     // all-padding documents are cheap to find and need no tensor-core work (short documents only: NARRE's padded review slots)
     a.live = nullptr;
@@ -1002,14 +948,10 @@ int conv_tc2_dispatch(const __nv_bfloat16* shadow, int64_t vocab, int E, IdView 
     a.rowidx = nullptr;
     // Row-index table (written by the pre-pass that reads the ids / masks anyway: the tile-count pass for long documents, the
     // document selection for short ones; a pass of its own otherwise).
-    static const char* ri_env = getenv("RBR_TC2_ROWIDX");      // timing experiments: 0 = never (the index warp resolves ids itself)
-    const int ri_mode = ri_env ? atoi(ri_env) : 1;
-    const bool want_ri = ri_mode != 0 && ws && ws_bytes >= conv_tc2_workspace_bytes(n_docs, L, K, pad) &&
+    const bool want_ri = ws && ws_bytes >= conv_tc2_workspace_bytes(n_docs, L, K, pad) &&
                          ws_bytes > conv_tc2_select_bytes(n_docs) && (reinterpret_cast<uintptr_t>(ws) & 15) == 0;
     int32_t* ri = want_ri ? reinterpret_cast<int32_t*>(reinterpret_cast<char*>(ws) + conv_tc2_select_bytes(n_docs)) : nullptr;
-    static const char* sel_env = getenv("RBR_TC2_SELECT");                      // timing experiments: 0 disables both selections
-    const bool sel_on = !(sel_env && atoi(sel_env) == 0);
-    if (sel_on && ws && ws_bytes >= conv_tc2_select_bytes(n_docs) && (mask || ids.mask_ids) && gate_mode == 0 && n_docs >= 64 &&
+    if (ws && ws_bytes >= conv_tc2_select_bytes(n_docs) && (mask || ids.mask_ids) && gate_mode == 0 && n_docs >= 64 &&
         n_docs < (1ll << 30)) {
         int32_t* w32 = reinterpret_cast<int32_t*>(ws);
         if (a.p.mode_b) {
@@ -1056,18 +998,13 @@ int conv_tc2_dispatch(const __nv_bfloat16* shadow, int64_t vocab, int E, IdView 
     }
     a.vocab = vocab; a.ids = ids; a.mask = mask; a.n_docs = n_docs; a.wpack = umma_w2; a.bias = bias;
     a.feat = feat; a.argmax = argmax; a.preact = preact; a.gate = gate; a.gate_mode = gate_mode; a.feat_ld = feat_ld;
-    static const char* ew_env = getenv("RBR_TC2_EPI_WARPS");                    // timing experiments: force 8 or 16
-    const bool wide = ew_env ? atoi(ew_env) == 16 : (a.p.mode_b || a.p.Nb / 16 >= 9 || a.p.nkb <= 2);
-    static const char* pw_env = getenv("RBR_TC2_PROD_WARPS");                   // timing experiments: 4 or 8
-    const bool pw8 = pw_env ? atoi(pw_env) == 8 : false;      // measured: 8 producer warps = 4 (the floor is the TMA unit's row rate, not per-warp issue)
+    const bool wide = a.p.mode_b || a.p.Nb / 16 >= 9 || a.p.nkb <= 2;
     // (Tried and rejected: the column max as a transposed shuffle butterfly (24 shfl.bfly per 16 columns, value + first row carried
     // along) instead of redux.sync + ballot: DeepCoNN conv 299 -> 361 us, NARRE 313 -> 380 us — the redux form is the cheap one.)
     // (Tried and rejected: 20 epilogue warps = five column shares, so that Nb = 160 = 10 chunks splits 2,2,2,2,2 instead of 3,2,3,2 and
     // the per-document finalisation waits less for the slowest warp.  NARRE conv 305 -> 340 us: the extra warps take issue slots
     // from the producer warps, and gather issue is what bounds the kernel.)
-#define RBR_T2(KT_)                                                                                                   \
-    return wide ? (pw8 ? tc2_launch<KT_, 16, 8>(tm, a, s) : tc2_launch<KT_, 16, 4>(tm, a, s))                          \
-                : (pw8 ? tc2_launch<KT_, 8, 8>(tm, a, s) : tc2_launch<KT_, 8, 4>(tm, a, s))
+#define RBR_T2(KT_) return wide ? tc2_launch<KT_, 16>(tm, a, s) : tc2_launch<KT_, 8>(tm, a, s)
     switch (K) {
         case 1: RBR_T2(1);
         case 2: RBR_T2(2);
@@ -1096,11 +1033,3 @@ extern "C" int rbr_conv_tc2_plan(int64_t emb, int64_t filters, int64_t ksize, in
 }
 
 RBR_DEFINE_OOB_ACCESSOR(conv_tc2)
-
-// timing experiments (RBR_TC2_DEBUG=4): copies the per-CTA cycle counters of the last conv_tc2 launch to the host
-extern "C" int rbr_debug_conv_tc2_prof(int64_t* out, int n_ctas) {
-    if (!out || n_ctas < 1 || n_ctas > 1024) return RBR_EINVAL;
-    RBR_CUDA(cudaDeviceSynchronize());
-    RBR_CUDA(cudaMemcpyFromSymbol(out, rbr::g_tc2_prof, sizeof(long long) * 12 * (size_t)n_ctas));
-    return RBR_OK;
-}

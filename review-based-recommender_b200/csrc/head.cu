@@ -508,15 +508,13 @@ extern "C" int rbr_head_fwd(const float* u_text, const float* i_text, const int6
     RBR_REQUIRE(drop_p >= 0.f && drop_p < 1.f, RBR_EINVAL, "rbr_head_fwd: dropout p must be in [0,1)");
     if (batch == 0) return RBR_OK;
     const int H = (int)hidden, K = (int)latent;
-    static const char* v2_env = getenv("RBR_HEAD_V2");                 // timing experiments: 0 = the scalar kernels
-    const bool v2_on = !(v2_env && atoi(v2_env) == 0);
     {   // register-tiled kernel (latent % 4 == 0: float4 views of the latent gradients; everything else is padded in shared memory)
         const int Hp = (H + 3) & ~3;
         const bool small = batch <= 32 * 148 * 2;                      // few tiles: 16-sample CTAs fill the SMs twice over
         const int ts = small ? 16 : 32;
         const size_t smem2 = ((size_t)2 * Hp * K + (size_t)2 * ts * Hp) * 4;
         const bool aligned = (((uintptr_t)u_text | (uintptr_t)i_text | (uintptr_t)Wu | (uintptr_t)Wi) & 15) == 0;
-        if (v2_on && K % 4 == 0 && smem2 <= 200 * 1024) {
+        if (K % 4 == 0 && smem2 <= 200 * 1024) {
             static bool attr2 = false;
             if (!attr2) {
                 RBR_CUDA(cudaFuncSetAttribute(head_fwd2_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
@@ -560,15 +558,13 @@ extern "C" int rbr_head_bwd(const float* u_text, const float* i_text, const int6
                 "rbr_head_bwd: latent_dim must be in [1,%d]", 32 * HD_KQ);
     if (batch == 0) return RBR_OK;
     const int H = (int)hidden, K = (int)latent;
-    static const char* v2_env = getenv("RBR_HEAD_V2");
-    const bool v2_on = !(v2_env && atoi(v2_env) == 0);
     {
         const int Hp = (H + 3) & ~3;
         const bool small = false;                                      // 32-sample tiles: half the weight-gradient atomics of 16 (22.6 vs 26.8 us)
         const int ts = small ? 16 : 32;
         const size_t smem2 = ((size_t)2 * H * (K + 1) + 4 + (size_t)2 * ts * Hp + (size_t)2 * ts * K) * 4;
         const bool aligned = (((uintptr_t)u_text | (uintptr_t)i_text) & 15) == 0;
-        if (v2_on && K % 4 == 0 && smem2 <= 200 * 1024) {
+        if (K % 4 == 0 && smem2 <= 200 * 1024) {
             static bool attr2 = false;
             if (!attr2) {
                 RBR_CUDA(cudaFuncSetAttribute(head_bwd2_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));

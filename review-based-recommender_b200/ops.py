@@ -6,8 +6,6 @@ int64 / bool — anything else raises (there is no CPU path).
 """
 from __future__ import annotations
 
-import os
-
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
@@ -425,7 +423,7 @@ class EncodeDocsFn(torch.autograd.Function):
                 for c in range(lib.rbr_conv_bwd_cmat_chunks(vocab, emb, h, k)):
                     lib.check(lib.rbr_conv_bwd_cmat_begin(c, vocab, emb, h, k, _p(ws), ws.numel(), _stream()), "rbr_conv_bwd_cmat_begin")
                     per_side(dense_scatter_chunk(i, c))
-                    lib.check(lib.rbr_conv_bwd_cmat_finish(1, c, 0, 0, None, _p(ctx.packed[i]), vocab, emb, h, k, cfg["padding_idx"], None, None,
+                    lib.check(lib.rbr_conv_bwd_cmat_finish(1, c, None, _p(ctx.packed[i]), vocab, emb, h, k, cfg["padding_idx"], None, None,
                                                            _p(ws), ws.numel(), _stream()), "rbr_conv_bwd_cmat_finish")
 
         # the arena left the table slot un-zeroed because this backward writes every element of it (NgramFeat.encode decided)
@@ -434,12 +432,12 @@ class EncodeDocsFn(torch.autograd.Function):
             g_table.zero_()                 # nothing will overwrite it after all
             overwrite = False
 
-        def dense_finish(what, rows=(0, 0)):
+        def dense_finish(what):
             if overwrite and (what & 2):
                 what |= 8
             for i, ws in cm_ws.items():
                 h, _, k = shapes[i]
-                lib.check(lib.rbr_conv_bwd_cmat_finish(what, -1, rows[0], rows[1], _p(ctx.shadow), _p(ctx.packed[i]), vocab, emb, h, k,
+                lib.check(lib.rbr_conv_bwd_cmat_finish(what, -1, _p(ctx.shadow), _p(ctx.packed[i]), vocab, emb, h, k,
                                                        cfg["padding_idx"], _p(g_table), _p(g_w[i]), _p(ws), ws.numel(), _stream()),
                           "rbr_conv_bwd_cmat_finish")
 
@@ -450,25 +448,9 @@ class EncodeDocsFn(torch.autograd.Function):
                 per_side(sparse_part(True, not two_pass) if need_table else sparse_part(False, True))
             if cm_ws:
                 dense_accumulate()
-            # Data-parallel: the word-table gradient (~90 % of the exchanged bytes) CAN be produced in row slices, the hook starting
-            # the all-reduce of each slice on its own stream while the next slice's GEMM runs (only when the dense path is the one
-            # and only writer of the gradient).  Measured on 2 x B200 (bench.py, DeepCoNN): exposed exchange 0.164 ms with one
-            # slice, 0.177 with 4, 0.230 with 8 — the table GEMM is only ~48 us long and every slice pays two cross-GPU barriers,
-            # so the default stays ONE slice; RBR_TABLE_GRAD_SLICES is kept for experiments with larger vocabularies.
-            n_slices = 1
-            if getattr(hook, "accepts_slices", False) and cm_ws and need_table and not any_sparse and len(cm_ws) == 1:
-                n_slices = max(1, min(int(os.environ.get("RBR_TABLE_GRAD_SLICES", "1")), vocab // 1024))
             if cm_ws and need_table:
-                if n_slices == 1:
-                    dense_finish(2)
-                else:
-                    step = (vocab + n_slices - 1) // n_slices
-                    step = (step + 127) // 128 * 128
-                    for lo in range(0, vocab, step):
-                        hi = min(vocab, lo + step)
-                        dense_finish(2, (lo, hi))
-                        hook(g_table[lo:hi])
-            if hook is not None and n_slices == 1:
+                dense_finish(2)
+            if hook is not None:
                 hook(g_table)
             if any_sparse and two_pass:
                 per_side(sparse_part(False, True))

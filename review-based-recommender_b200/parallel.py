@@ -165,7 +165,7 @@ def enable_nvls_allreduce(model: torch.nn.Module, group=None, overlap: bool = Tr
     overlap = bool(overlap and ngram is not None and hasattr(ngram, "table_grad_hook"))
     world = dist.get_world_size(group)
     if kind == "auto":
-        kind = os.environ.get("RBR_ALLREDUCE_KIND", "p2p" if world == 2 else "multimem")
+        kind = "p2p" if world == 2 else "multimem"
     if kind == "p2p" and world not in (2, 4, 8):
         kind = "multimem"
     st = _NvlsState(hdl, mc, n, dist.get_rank(group), world, dev, overlap, kind)
@@ -187,10 +187,8 @@ def enable_nvls_allreduce(model: torch.nn.Module, group=None, overlap: bool = Tr
                 st.reduce(lo, cnt, 1.0 / st.world, st.side.cuda_stream)
                 hdl.barrier(channel=3)
                 st.ev_done.record(st.side)
-            # called once per row slice of the table gradient (consecutive slices): the reduced range grows
-            st.early = (lo, lo + cnt) if st.early is None or st.early[1] != lo else (st.early[0], lo + cnt)
+            st.early = (lo, lo + cnt)
 
-        hook.accepts_slices = True           # may be called once per consecutive row slice of the table gradient
         ngram.table_grad_hook = hook
     return True
 

@@ -28,6 +28,21 @@ def test_cabi_loads_and_exports_every_declared_symbol():
     assert lib.rbr_embgrad_workspace_bytes(1000, 50000) > 0
 
 
+def test_library_reads_no_environment_variable():
+    """Kernel variants are chosen per call (`flags`) and by shape.  No process-wide switch in the environment changes what the
+    CUDA library or the autograd operators compute: a variable left set in a shell cannot silently alter a later run."""
+    import glob
+    csrc = os.path.join(ROOT, "review-based-recommender_b200", "csrc")
+    sources = sorted(glob.glob(os.path.join(csrc, "*.cu")) + glob.glob(os.path.join(csrc, "*.cuh")))
+    assert len(sources) > 10
+    for path in sources:
+        with open(path) as f:
+            assert "getenv(" not in f.read(), path
+    with open(os.path.join(ROOT, "review-based-recommender_b200", "ops.py")) as f:
+        src = f.read()
+    assert "environ" not in src and "getenv" not in src
+
+
 def test_no_cpu_fallback():
     m = rbr_b200.DeepCoNNpp(9, 7, 60, [3], 12, 8, 6, 20, None, 0.0)
     ids = torch.zeros(2, 20, dtype=torch.long)

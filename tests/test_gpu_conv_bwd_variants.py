@@ -367,20 +367,18 @@ def test_wide_embedding_bf16_model_trains():
 
 
 # ----------------------------------------------------------------------------------------------------------------------
-# the gradient arena: overwrite mode (the table slot is not zero-filled), row slices, a repeated step
+# the gradient arena: overwrite mode (the table slot is not zero-filled), a repeated step
 # ----------------------------------------------------------------------------------------------------------------------
-ARENA_CASES = {"overwrite": ((3,), 1), "overwrite_3_row_slices": ((3,), 3), "two_convs_zero_filled": ((3, 5), 1)}
+ARENA_CASES = {"overwrite": (3,), "two_convs_zero_filled": (3, 5)}
 
 
 @pytest.mark.parametrize("name", list(ARENA_CASES))
-def test_arena_table_gradient(name, monkeypatch, tmp_path):
+def test_arena_table_gradient(name, tmp_path):
     """DeepCoNN bf16 with a persistent arena buffer filled with NaN before each step.  With one conv the table slot is not
-    zero-filled (K2c overwrites every element), with two it is.  Row slices: RBR_TABLE_GRAD_SLICES=3 and a hook that accepts
-    slices, V = 5000 → [0, 1792), [1792, 3584), [3584, 5000); each slice must be final when the hook sees it.  A second step on
-    the same model (the coefficient blocks re-zeroed before their atomics) gives the same gradients."""
-    ks, n_slices = ARENA_CASES[name]
+    zero-filled (K2c overwrites every element), with two it is.  The table-gradient hook sees the whole gradient once per step.
+    A second step on the same model (the coefficient blocks re-zeroed before their atomics) gives the same gradients."""
+    ks = ARENA_CASES[name]
     V, E, H, L, n = 5000, 100, 40, 80, 16
-    monkeypatch.setenv("RBR_TABLE_GRAD_SLICES", str(n_slices))
     params = synth.deepconn_params(7, 6, V, E, H, 8, ks, seed=3)
     batch, ratings = synth.deepconn_batch(n, L, V, 7, 6, seed=4)
     model = rbr_b200.DeepCoNNpp(7, 6, V, list(ks), E, H, 8, L, None, 0.0, precision="bf16")
@@ -411,17 +409,16 @@ def test_arena_table_gradient(name, monkeypatch, tmp_path):
         return list(outs) if return_argmax else list(feats)
 
     model.ngram.encode = encode_capturing
-    slices = []
+    hooked = []
 
     def hook(g):
-        slices.append(g.detach().clone())
+        hooked.append(g.detach().clone())
 
-    hook.accepts_slices = True
     model.ngram.table_grad_hook = hook
     results = []
     for rep in range(2):
         buf.fill_(float("nan"))
-        slices.clear()
+        hooked.clear()
         model.zero_grad(set_to_none=True)
 
         def step():
@@ -431,20 +428,13 @@ def test_arena_table_gradient(name, monkeypatch, tmp_path):
         g = table.grad
         assert bool(torch.isfinite(g).all()) and float(g[0].abs().max()) == 0.0
         gemm = [gx for nm, gx in launched if "cmat_table_gemm_kernel" in nm]
-        bounds = [(0, V)] if n_slices == 1 else [(0, 1792), (1792, 3584), (3584, V)]
-        assert gemm == [(hi - lo + 127) // 128 for lo, hi in bounds] * len(ks), gemm
+        assert gemm == [(V + 127) // 128] * len(ks), gemm
         gt, gw, gb = _reference_grads(c, table.detach().cpu(), ws, bs, ref_sides, cap["ams"], cap["point"], cap["G"])
         assert _note("bf16", "table", rel_err(g, gt)) < GRAD_TOL
         for i, cv in enumerate(convs):
             assert _note("bf16", "weight", rel_err(cv.weight.grad, gw[i])) < GRAD_TOL, i
             assert _note("bf16", "bias", rel_err(cv.bias.grad, gb[i])) < GRAD_TOL, i
-        if n_slices > 1:
-            assert len(slices) == 3
-            for got, (lo, hi) in zip(slices, bounds):
-                assert got.shape[0] == hi - lo and bool(torch.isfinite(got).all())
-                assert rel_err(got, gt[lo:hi]) < GRAD_TOL, (lo, hi)
-        else:
-            assert len(slices) == 1
+        assert len(hooked) == 1
         results.append({k: p.grad.detach().clone() for k, p in model.named_parameters()})
     for k in results[0]:
         assert rel_err(results[1][k], results[0][k], 1e-9) < 1e-6, k

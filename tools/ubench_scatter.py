@@ -1,5 +1,5 @@
 """Timing harness for the K2c coefficient scatter on synthetic NARRE / DeepCoNN shaped inputs (L2 flushed between launches).
-    [RBR_CMAT_CHUNKS=n] [UB_I64=1] [UB_FLUSH=write|read|none] python tools/ubench_scatter.py narre|deepconn
+    [UB_I64=1] [UB_FLUSH=write|read|none] python tools/ubench_scatter.py narre|deepconn
 (The numbers in profiles/r02_ub_scatter.txt with "dbg=1" were taken with a since-removed switch that disabled the atomics.)"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
